@@ -298,6 +298,13 @@ def run_reference(args):
     print(json.dumps(line))
 
 
+def dump_outputs(out_dir, arrays):
+    """Write every tensor of ``arrays`` as ``out_dir/<name>.npy`` in float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------
 def run_native(args):
     import torch.distributed as dist
@@ -341,6 +348,8 @@ def run_native(args):
     gen = torch.Generator(device=dev).manual_seed(1234 + rank)
     batch = SPEAKERS * UTTS
 
+    last = {}
+
     def step(mel):
         opt.zero_grad(set_to_none=True)
         d = model(mel)
@@ -348,6 +357,7 @@ def run_native(args):
         loss.backward()
         opt.step()
         sched.step()
+        last["dvectors"] = d
         return loss
 
     def barrier():
@@ -377,6 +387,12 @@ def run_native(args):
     ms_total = float(t.item())
     value = world * K / (ms_total * 1e-3)
     last_loss = float(loss.item())
+    if args.dump_outputs and rank == 0:
+        arrays = {"loss": loss.reshape(1), "dvectors": last["dvectors"]}
+        for n, p in model.named_parameters():
+            arrays["param." + n] = p
+            arrays["grad." + n] = p.grad
+        dump_outputs(args.dump_outputs, arrays)
     del dev_mels
 
     # ---- end to end through the public API: pinned host batch -> H2D -> step -> loss D2H
@@ -789,10 +805,18 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="train workload: after the timed steps, write what the last one computed (loss, d-vectors, "
+                         "updated parameters and their gradients, ~21 MB) as DIR/<name>.npy in float32; the inputs "
+                         "depend only on the arguments, so two builds can be compared output for output.  Weight "
+                         "gradients are summed with fp32 atomics, so two runs of one build already differ by rounding "
+                         "(and the few ReLU gates it flips): ~1e-6 in the loss, up to a few 1e-3 relative per gradient")
     ap.add_argument("--workload", default="train", choices=["train", "infer", "ge2e"],
                     help="train: GE2E training step (headline, BASELINE config 2/4, the line also carries config 3); "
                          "infer: multi-slice extraction alone (config 3); ge2e: fused-loss sweep (config 5)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "native" or args.workload != "train"):
+        ap.error("--dump-outputs writes the outputs of the native train workload only")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "infer":

@@ -31,6 +31,18 @@ def fingerprint_indices(numel, k=64):
     return rng.integers(0, numel, size=min(k, numel))
 
 
+def sample_rows(rows, k):
+    """Sorted seeded sample of ``k`` distinct row indices out of ``rows``: the rows of an output too large to store
+    whole (a golden file stays under 1 MB) that the file keeps, next to the values under ``<name>_rows``."""
+    rng = np.random.default_rng(FP_IDX_SEED + rows)
+    return np.sort(rng.choice(rows, size=min(k, rows), replace=False))
+
+
+def stored_rows(golden, key):
+    """Index of the rows a golden file holds of an output: ``golden[key]`` when it keeps a sample, else every row."""
+    return golden[key] if key in golden.files else slice(None)
+
+
 def load_reference():
     sys.path.insert(0, REF)
     warnings.filterwarnings("ignore")
@@ -86,13 +98,17 @@ def main():
     ]
     for i, (sd, N, M, un, w, b) in enumerate(lcases):
         E = synth.make_embeddings(sd, N, M, unit_norm=bool(un))
+        rows = slice(None)
+        if N * M > 240:                       # the 960 x 256 dE of case 3 is kept as a quarter of its rows
+            rows = los["case%d_rows" % i] = sample_rows(N * M, 240)
         for tag, dt in (("f32", torch.float32), ("f64", torch.float64)):
             crit = GE2E_Loss(init_weight=w, init_bias=b).to(dt)
             e = torch.as_tensor(E).to(dt).requires_grad_(True)
             loss = crit(e, M)
             loss.backward()
             los["case%d_%s_loss" % (i, tag)] = loss.detach().numpy()
-            los["case%d_%s_dE" % (i, tag)] = e.grad.numpy()
+            if tag == "f64":                  # the fp32 run is checked through its loss only
+                los["case%d_%s_dE" % (i, tag)] = e.grad.numpy()[rows]
             los["case%d_%s_dw" % (i, tag)] = crit.weight.grad.numpy()
             los["case%d_%s_db" % (i, tag)] = (crit.bias.grad if crit.bias.grad is not None
                                                else torch.zeros(())).numpy()

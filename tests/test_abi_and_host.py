@@ -164,7 +164,7 @@ def test_dropin_harness_is_what_the_reference_expects(tmp_path):
     import sys
     ref = os.path.join(ROOT, "baseline", "_ref")
     if not os.path.exists(os.path.join(ref, "Train.py")):
-        pytest.skip("baseline/_ref is staged by __graft_entry__.build() where /root/reference exists")
+        pytest.skip("needs a reference checkout, staged to baseline/_ref by build() from SPK_REFERENCE")
     env = dict(os.environ, SPK_DROPIN_REFERENCE_MODULES="1", CUDA_VISIBLE_DEVICES="")
     proc = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "dropin_train_worker.py"), ref, str(tmp_path)],
                           capture_output=True, text=True, timeout=600, cwd=str(tmp_path), env=env)

@@ -14,7 +14,7 @@ REF = os.path.join(ROOT, "baseline", "_ref")
 
 
 @pytest.mark.skipif(not os.path.exists(os.path.join(REF, "Train.py")),
-                    reason="baseline/_ref is staged by __graft_entry__.build() where /root/reference exists")
+                    reason="needs a reference checkout, staged to baseline/_ref by build() from SPK_REFERENCE")
 @pytest.mark.parametrize("device_collater", ["0", "1"])
 def test_reference_train_py_runs_unmodified_on_the_drop_in_modules(tmp_path, device_collater):
     """device_collater = 1 additionally shadows Datasets.Collater with the on-device collater (RaggedMel batches)."""

@@ -21,7 +21,7 @@ def _free_port():
     return port
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_two_rank_nccl_gradient_mean_and_identical_weights():
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr",
            "127.0.0.1", "--master-port", str(_free_port()), os.path.join(ROOT, "tests", "nccl_worker.py")]
