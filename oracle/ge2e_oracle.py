@@ -56,7 +56,7 @@ def _dropout(x, p, gen, scale=None):
 
 
 def encoder_forward(state, mel, samples=1, heads=4, layers=3, dropout_p=0.0, gen=None,
-                    return_intermediates=False, drop_scales=None):
+                    return_intermediates=False, drop_scales=None, relu_masks=None):
     """d-vectors [B/samples, D] from mel [B, mel_dim, T]  (Modules.py:46-59).
 
     ``state`` is a dict of torch tensors with the reference's state_dict names.
@@ -66,12 +66,20 @@ def encoder_forward(state, mel, samples=1, heads=4, layers=3, dropout_p=0.0, gen
     replaces the random masks by given ones (sites numbered as in include/spkemb.h: 0 positional encoding,
     1 + 4l attention probabilities [B, H, T, T], 2 + 4l dropout1, 3 + 4l FFN inner [B, T, 4D], 4 + 4l dropout2),
     which is how the tests check that the CUDA forward and backward apply one and the same mask per site.
+    ``relu_masks`` = {site: bool tensor} likewise replaces ``relu(u)`` by ``u * mask`` (sites ``"prenet"`` [B, T, D]
+    and ``"ffn<l>"`` [B, T, 4D]): fed the gates a kernel chose, the fp64 gradients are those of the kernel's own
+    piecewise-linear function, free of the gates that flip when a pre-activation lies within rounding of zero.
     """
     ds = drop_scales or {}
+    rm = relu_masks or {}
+
+    def relu(u, site):
+        return u * rm[site].to(u.dtype) if site in rm else torch.relu(u)
+
     x = mel.transpose(1, 2)                                   # [B, T, mel]
     B, T, _ = x.shape
     w_pre = state["prenet.weight"][:, :, 0]                   # [D, mel]
-    h = torch.relu(x @ w_pre.t() + state["prenet.bias"])      # Modules.py:50-51
+    h = relu(x @ w_pre.t() + state["prenet.bias"], "prenet")  # Modules.py:50-51
     D = h.shape[-1]
     pe = state["positional_encoding.pe"][0, :, :T].t()        # [T, D]  (Modules.py:107-109)
     h = h + state["positional_encoding.alpha"] * pe           # Modules.py:102
@@ -93,7 +101,7 @@ def encoder_forward(state, mel, samples=1, heads=4, layers=3, dropout_p=0.0, gen
         a = a @ state[p + "self_attn.out_proj.weight"].t() + state[p + "self_attn.out_proj.bias"]
         h = _layer_norm(h + _dropout(a, dropout_p, gen, ds.get(2 + 4 * l)), state[p + "norm1.weight"],
                         state[p + "norm1.bias"])
-        f = torch.relu(h @ state[p + "linear1.weight"].t() + state[p + "linear1.bias"])
+        f = relu(h @ state[p + "linear1.weight"].t() + state[p + "linear1.bias"], "ffn%d" % l)
         f = _dropout(f, dropout_p, gen, ds.get(3 + 4 * l))
         f = f @ state[p + "linear2.weight"].t() + state[p + "linear2.bias"]
         h = _layer_norm(h + _dropout(f, dropout_p, gen, ds.get(4 + 4 * l)), state[p + "norm2.weight"],
@@ -205,12 +213,13 @@ def ge2e_closed_form_chunked(emb, per_speaker, weight=10.0, bias=-5.0, rows_per_
 
 
 def train_step_grads(state_np, mel_np, per_speaker, weight=10.0, bias=-5.0, dtype=torch.float64,
-                     samples=1, drop_scales=None):
+                     samples=1, drop_scales=None, relu_masks=None):
     """Loss, d-vectors and every parameter gradient via autograd through the restatement."""
     st = to_torch_state(state_np, dtype=dtype, requires_grad=True)
     w = torch.tensor(weight, dtype=dtype, requires_grad=True)
     b = torch.tensor(bias, dtype=dtype, requires_grad=True)
-    d = encoder_forward(st, torch.as_tensor(mel_np).to(dtype), samples=samples, drop_scales=drop_scales)
+    d = encoder_forward(st, torch.as_tensor(mel_np).to(dtype), samples=samples, drop_scales=drop_scales,
+                        relu_masks=relu_masks)
     loss = ge2e_loss(d, per_speaker, w, b)
     loss.backward()
     grads = {k: v.grad.detach().numpy() for k, v in st.items() if v.requires_grad}

@@ -282,6 +282,26 @@ def read_split(ws, layout, name, rows, cols, planes):
     return out
 
 
+def _ws_bytes(ws, layout, name, nbytes):
+    off, _ = layout[name]
+    base = (ws.data_ptr() + 255) // 256 * 256 - ws.data_ptr() + off
+    return ws[base:base + nbytes]
+
+
+def read_f32(ws, layout, name, n):
+    """Read ``n`` fp32 values of a workspace buffer (statistics, head vectors, gradient scale) as a 1-D tensor."""
+    return _ws_bytes(ws, layout, name, n * 4).view(torch.float32).clone()
+
+
+def read_bits(ws, layout, name, rows, cols):
+    """Read a 1-bit mask of a [rows, cols] tensor as bool [rows, cols].  The words are chunk-major ``[cols/32][rows]``:
+    bit i of word (c, r) is element (r, 32c + i)."""
+    words = _ws_bytes(ws, layout, name, (cols // 32) * rows * 4).view(torch.int32).view(cols // 32, rows)
+    shifts = torch.arange(32, dtype=torch.int32, device=ws.device)
+    bits = (words.unsqueeze(-1) >> shifts) & 1                       # [cols/32, rows, 32]
+    return bits.permute(1, 0, 2).reshape(rows, cols).bool()
+
+
 def prof_enable(on=True):
     lib().spk_prof_enable(int(on))
 

@@ -223,15 +223,29 @@ int encoder_debug_layout(const spk_encoder_config& c, int B, int T, int S, int P
   };
   put("", -1, "x0", pl.x0.off, pl.x0.ps); put("", -1, "h0", pl.h0.off, pl.h0.ps);
   put("", -1, "scr", pl.scr.off, pl.scr.ps); put("", -1, "pe_t", pl.pe_t, 0);
+  if (keep) put("", -1, "h0bits", pl.h0bits, 0);
   for (int l = 0; l < (pl.prune ? pl.L - 1 : pl.L); ++l) {
     const LayerBufs& b = pl.Lb[l];
     put("", l, "qkv", b.qkv.off, b.qkv.ps); put("", l, "p", b.p.off, b.p.ps); put("", l, "att", b.att.off, b.att.ps);
+    put("", l, "pd", b.pd.off, b.pd.ps);
     put("", l, "z1", b.z1.off, b.z1.ps); put("", l, "h1", b.h1.off, b.h1.ps); put("", l, "f", b.f.off, b.f.ps);
     put("", l, "z2", b.z2.off, b.z2.ps); put("", l, "hout", b.hout.off, b.hout.ps);
-    put("", l, "st1", b.st1, 0); put("", l, "st2", b.st2, 0);
+    put("", l, "st1", b.st1, 0); put("", l, "st2", b.st2, 0); put("", l, "fbits", b.fbits, 0);
+    if (pl.attn_tr) { put("", l, "astat", b.astat, 0); put("", l, "abits", b.abits, 0); }
   }
-  put("", -1, "hn", pl.hn, 0); put("", -1, "emean", pl.emean, 0); put("", -1, "epre", pl.epre, 0); put("", -1, "de", pl.de, 0);
+  if (pl.prune) {
+    const LastBufs& lb = pl.last;
+    put("", -1, "last.kv", lb.kv.off, lb.kv.ps); put("", -1, "last.q0", lb.q0.off, lb.q0.ps);
+    put("", -1, "last.att0", lb.att0.off, lb.att0.ps); put("", -1, "last.z1", lb.z1.off, lb.z1.ps);
+    put("", -1, "last.h1", lb.h1.off, lb.h1.ps); put("", -1, "last.f", lb.f.off, lb.f.ps);
+    put("", -1, "last.z2", lb.z2.off, lb.z2.ps); put("", -1, "last.hout", lb.hout.off, lb.hout.ps);
+    put("", -1, "last.st1", lb.st1, 0); put("", -1, "last.st2", lb.st2, 0);
+    put("", -1, "last.p0", lb.p0, 0); put("", -1, "last.pd0", lb.pd0, 0);
+  }
+  put("", -1, "hn", pl.hn, 0); put("", -1, "hst", pl.hst, 0); put("", -1, "emean", pl.emean, 0);
+  put("", -1, "epre", pl.epre, 0); put("", -1, "de", pl.de, 0);
   if (keep) {
+    put("", -1, "gscale", pl.gscale, 0);
     put("", -1, "dh_a", pl.dh_a.off, pl.dh_a.ps); put("", -1, "dh_b", pl.dh_b.off, pl.dh_b.ps);
     put("", -1, "dz", pl.dz.off, pl.dz.ps); put("", -1, "dzd", pl.dzd.off, pl.dzd.ps);
     put("", -1, "df", pl.df.off, pl.df.ps); put("", -1, "datt", pl.datt.off, pl.datt.ps);

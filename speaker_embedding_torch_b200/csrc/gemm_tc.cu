@@ -407,7 +407,10 @@ __device__ __forceinline__ void ln_epilogue_tile(const GemmEpilogue& e, uint32_t
   const CoopIO io_res = has_res ? make_coop(lane, res_boff, row0, e.res_ld, M, 8) : io_out;
   const bool use_drop = (e.flags & EPI_DROPOUT) && e.drop.thresh != 0;
   const int64_t row = row0 + lane;
-  float s1 = 0.f, s2 = 0.f;
+  // Shifted sums: each warp sums d = z - piv, piv being the first z of the row it sees.  A one-pass E[z^2] - mean^2
+  // loses the variance when |mean| >> std (relative error ~ (mean / std)^2 * 2^-24); about a pivot taken from the row
+  // itself the sums stay of the order of the row's spread, whatever its offset.
+  float s1 = 0.f, s2 = 0.f, piv = 0.f;
 #pragma unroll 1
   for (int c = cgroup; c < BLOCK_N / 32; c += EPI_CG) {
     const int col0 = c * 32;
@@ -442,27 +445,36 @@ __device__ __forceinline__ void ln_epilogue_tile(const GemmEpilogue& e, uint32_t
 #pragma unroll
       for (int i = 0; i < 32; ++i) v[i] += rr[i];
     }
+    if (c == cgroup) piv = v[0];
 #pragma unroll
-    for (int i = 0; i < 32; ++i) { s1 += v[i]; s2 = fmaf(v[i], v[i], s2); }
+    for (int i = 0; i < 32; ++i) { const float d = v[i] - piv; s1 += d; s2 = fmaf(d, d, s2); }
     tmem_st_32x32_acc(t_row + c * 32, v);
     if (e.ln_z != nullptr)      // training: the backward pass needs the pre-normalisation rows (v is consumed by the split)
       store_split_tile(stage_buf, lane, e.ln_z, e.ln_z_plane_stride, e.out_planes, io_out, col0, N, v);
   }
   asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
   // the quarter's EPI_CG warps meet: partial sums through the (currently idle) staging tiles
-  asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(stage_buf + lane * 8), "f"(s1), "f"(s2) : "memory");
+  asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(stage_buf + lane * 16), "f"(s1), "f"(s2), "f"(piv),
+               "f"(0.f) : "memory");
   asm volatile("bar.sync %0, %1;" ::"r"(quarter + 1), "r"(32 * EPI_CG) : "memory");
-  float t1 = 0.f, t2 = 0.f;
+  // merge about the pivot p0 of warp 0: sum (z - p0) = s1 + n dp, sum (z - p0)^2 = s2 + dp (2 s1 + n dp), dp = piv - p0
+  // (two values of the same row: their difference is exact or of the order of the spread)
+  float t1 = 0.f, t2 = 0.f, p0 = 0.f;
 #pragma unroll
   for (int g = 0; g < EPI_CG; ++g) {
-    float a, b;
-    asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(a), "=f"(b)
-                 : "r"(stage_buf + (g - cgroup) * 4 * (EPI_STAGE_BYTES + EPI_BIAS_BYTES) + lane * 8) : "memory");
-    t1 += a; t2 += b;
+    float a, b, p, unused;
+    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(a), "=f"(b), "=f"(p), "=f"(unused)
+                 : "r"(stage_buf + (g - cgroup) * 4 * (EPI_STAGE_BYTES + EPI_BIAS_BYTES) + lane * 16) : "memory");
+    if (g == 0) p0 = p;
+    const float n = static_cast<float>((BLOCK_N / 32 - g + EPI_CG - 1) / EPI_CG * 32);   // columns warp g summed
+    const float dp = p - p0;
+    t1 += fmaf(n, dp, a);
+    t2 += fmaf(dp, fmaf(n, dp, 2.f * a), b);
   }
   asm volatile("bar.sync %0, %1;" ::"r"(quarter + 1), "r"(32 * EPI_CG) : "memory");   // read before the tiles are reused
-  const float mean = t1 * (1.f / BLOCK_N);
-  const float var = fmaxf(t2 * (1.f / BLOCK_N) - mean * mean, 0.f);
+  const float mc = t1 * (1.f / BLOCK_N);                  // mean - p0
+  const float mean = p0 + mc;
+  const float var = fmaxf(t2 * (1.f / BLOCK_N) - mc * mc, 0.f);
   const float rstd = rsqrtf(var + e.ln_eps);
   if (e.ln_stats != nullptr && cgroup == 0 && row < M) reinterpret_cast<float2*>(e.ln_stats)[row] = make_float2(mean, rstd);
 #pragma unroll 1

@@ -170,3 +170,33 @@ def test_dropin_harness_is_what_the_reference_expects(tmp_path):
                           capture_output=True, text=True, timeout=600, cwd=str(tmp_path), env=env)
     assert proc.returncode == 0, proc.stdout[-2000:] + proc.stderr[-2000:]
     assert "DROPIN_TRAIN_OK" in proc.stdout
+
+
+def test_debug_layout_lists_the_stage_buffers_and_the_readers_decode_them(native):
+    """The workspace map names every stage buffer the stage-parity tests read (fused attention statistics and keep
+    bits, ReLU bits, the pruned last layer's compact rows, the head statistics, the gradient scale), and read_bits /
+    read_f32 decode the chunk-major bit layout ([cols/32][rows] words, bit i of word (c, r) = element (r, 32c + i))."""
+    cfg = native.EncoderConfig(80, 256, 4, 1024, 3, 1024, 0.1, 0.1)
+    flags = native.plan_flags()
+    lay = native.debug_layout(cfg, 6, 129, 1, 2 | flags, True)
+    for name in ("h0bits", "L0.fbits", "L1.astat", "L1.abits", "L1.pd", "last.kv", "last.q0", "last.att0",
+                 "last.z1", "last.st1", "last.h1", "last.f", "last.z2", "last.st2", "last.hout", "last.p0",
+                 "last.pd0", "hst", "gscale"):
+        assert name in lay, name
+    infer = native.debug_layout(cfg, 6, 129, 1, 1 | flags, False)
+    assert "h0bits" not in infer and "gscale" not in infer and "L0.astat" not in infer
+    rows, cols = 5, 64
+    mask = torch.rand(rows, cols, generator=torch.Generator().manual_seed(3)) > 0.5
+    words = torch.zeros(cols // 32, rows, dtype=torch.int64)
+    for c in range(cols // 32):
+        for i in range(32):
+            words[c] |= mask[:, 32 * c + i].long() << i
+    ws = torch.zeros(4096, dtype=torch.uint8)
+    base = (ws.data_ptr() + 255) // 256 * 256 - ws.data_ptr()
+    payload = words.numpy().astype(np.uint32)
+    ws[base + 256:base + 256 + payload.nbytes] = torch.from_numpy(payload.view(np.uint8).reshape(-1).copy())
+    vals = torch.arange(7, dtype=torch.float32)
+    ws[base + 1024:base + 1024 + 28] = vals.view(torch.uint8)
+    fake = {"bits": (256, 0), "vals": (1024, 0)}
+    assert torch.equal(native.read_bits(ws, fake, "bits", rows, cols), mask)
+    assert torch.equal(native.read_f32(ws, fake, "vals", 7), vals)
