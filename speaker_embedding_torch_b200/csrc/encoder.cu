@@ -35,18 +35,25 @@ struct Split {
   int64_t ps = 0;      // plane stride, elements
 };
 
-struct LayerBufs {
-  Split qkv, p, pd, att, z1, h1, f, z2, hout;
+// The sublayer after the attention: out-proj + residual -> LayerNorm1 -> FFN -> residual -> LayerNorm2.
+struct SublayerBufs {
+  Split att, z1, h1, f, z2, hout;
   size_t st1 = 0, st2 = 0;
-  size_t fbits = 0;   // ReLU mask of the FFN hidden activation, one bit per element ([F/32, Mt] words), for the backward
+  size_t fbits = 0;   // dense layers: ReLU mask of the FFN hidden activation, one bit per element ([F/32, Mt] words)
+};
+
+struct LayerBufs {
+  Split qkv, p, pd;
   size_t astat = 0;   // fused training attention: (row max, row sum) per (slice, head, query)
   size_t abits = 0;   // fused training attention: dropout keep bits [B*H][ceil(Tp/32)][T]
+  SublayerBufs sub;
 };
 
 // Last layer, t = 0 rows only (see attn_row0.cu): compact [B, .] buffers + K|V for every frame.
 struct LastBufs {
-  Split kv, q0, att0, z1, h1, f, z2, hout;
-  size_t st1 = 0, st2 = 0, p0 = 0, pd0 = 0;
+  Split kv, q0;
+  SublayerBufs sub;
+  size_t p0 = 0, pd0 = 0;
 };
 
 struct Plan {
@@ -79,6 +86,22 @@ static size_t take_f32(size_t& cur, int64_t elems) {
   size_t o = cur;
   cur = align_up(cur + static_cast<size_t>(elems) * 4, 1024);
   return o;
+}
+// `rows` rows of the sublayer.  fbits: allocate the FFN ReLU mask; hout: the buffer the output aliases, or nullptr for
+// one of its own.
+static SublayerBufs take_sublayer(size_t& cur, int64_t rows, int64_t D, int64_t F, int P, bool fbits,
+                                  const Split* hout) {
+  SublayerBufs s;
+  s.att = take_split(cur, rows * D, P);
+  s.z1 = take_split(cur, rows * D, P);
+  s.st1 = take_f32(cur, rows * 2);
+  s.h1 = take_split(cur, rows * D, P);
+  s.f = take_split(cur, rows * F, P);
+  if (fbits) s.fbits = take_f32(cur, rows * (F / 32));
+  s.z2 = take_split(cur, rows * D, P);
+  s.st2 = take_f32(cur, rows * 2);
+  s.hout = hout ? *hout : take_split(cur, rows * D, P);
+  return s;
 }
 
 static bool g_prune_last = true;   // spk_set_option("prune_last_layer", 0/1)
@@ -152,28 +175,13 @@ static int make_plan(const spk_encoder_config& c, int B, int T, int S, int Pflag
       b.astat = take_f32(cur, pl.BH * T * 2);
       b.abits = take_f32(cur, pl.BH * ((pl.Tp + 31) / 32) * T);
     }
-    b.att = take_split(cur, Mt * D, P);
-    b.z1 = take_split(cur, Mt * D, P);
-    b.st1 = take_f32(cur, Mt * 2);
-    b.h1 = take_split(cur, Mt * D, P);
-    b.f = take_split(cur, Mt * F, P);
-    b.fbits = take_f32(cur, Mt * (F / 32));
-    b.z2 = take_split(cur, Mt * D, P);
-    b.st2 = take_f32(cur, Mt * 2);
-    b.hout = keep ? take_split(cur, Mt * D, P) : pl.h0;
+    b.sub = take_sublayer(cur, Mt, D, F, P, true, keep ? nullptr : &pl.h0);
   }
   if (pl.prune) {
     LastBufs& lb = pl.last;
     lb.kv = take_split(cur, Mt * 2 * D, P);
     lb.q0 = take_split(cur, B * D, P);
-    lb.att0 = take_split(cur, B * D, P);
-    lb.z1 = take_split(cur, B * D, P);
-    lb.st1 = take_f32(cur, static_cast<int64_t>(B) * 2);
-    lb.h1 = take_split(cur, B * D, P);
-    lb.f = take_split(cur, B * F, P);
-    lb.z2 = take_split(cur, B * D, P);
-    lb.st2 = take_f32(cur, static_cast<int64_t>(B) * 2);
-    lb.hout = take_split(cur, B * D, P);
+    lb.sub = take_sublayer(cur, B, D, F, P, false, nullptr);
     lb.p0 = take_f32(cur, pl.BH * pl.Tp);
     lb.pd0 = take_f32(cur, pl.BH * pl.Tp);
   }
@@ -215,41 +223,42 @@ int encoder_debug_layout(const spk_encoder_config& c, int B, int T, int S, int P
   Plan pl;
   SPK_TRY(make_plan(c, B, T, S, P, keep != 0, pl));
   size_t off = 0;
-  auto put = [&](const char* pre, int l, const char* name, size_t o, int64_t ps) {
-    int n = l >= 0 ? snprintf(buf + off, off < cap ? cap - off : 0, "L%d.%s %zu %lld\n", l, name, o, (long long)ps)
-                   : snprintf(buf + off, off < cap ? cap - off : 0, "%s %zu %lld\n", name, o, (long long)ps);
-    (void)pre;
+  auto put = [&](const char* pre, const char* name, size_t o, int64_t ps) {
+    int n = snprintf(buf + off, off < cap ? cap - off : 0, "%s%s %zu %lld\n", pre, name, o, (long long)ps);
     if (n > 0 && off + n < cap) off += n;
   };
-  put("", -1, "x0", pl.x0.off, pl.x0.ps); put("", -1, "h0", pl.h0.off, pl.h0.ps);
-  put("", -1, "scr", pl.scr.off, pl.scr.ps); put("", -1, "pe_t", pl.pe_t, 0);
-  if (keep) put("", -1, "h0bits", pl.h0bits, 0);
+  auto put_sub = [&](const char* pre, const SublayerBufs& s, const char* att) {
+    put(pre, att, s.att.off, s.att.ps);
+    put(pre, "z1", s.z1.off, s.z1.ps); put(pre, "h1", s.h1.off, s.h1.ps); put(pre, "f", s.f.off, s.f.ps);
+    put(pre, "z2", s.z2.off, s.z2.ps); put(pre, "hout", s.hout.off, s.hout.ps);
+    put(pre, "st1", s.st1, 0); put(pre, "st2", s.st2, 0);
+  };
+  put("", "x0", pl.x0.off, pl.x0.ps); put("", "h0", pl.h0.off, pl.h0.ps);
+  put("", "scr", pl.scr.off, pl.scr.ps); put("", "pe_t", pl.pe_t, 0);
+  if (keep) put("", "h0bits", pl.h0bits, 0);
   for (int l = 0; l < (pl.prune ? pl.L - 1 : pl.L); ++l) {
     const LayerBufs& b = pl.Lb[l];
-    put("", l, "qkv", b.qkv.off, b.qkv.ps); put("", l, "p", b.p.off, b.p.ps); put("", l, "att", b.att.off, b.att.ps);
-    put("", l, "pd", b.pd.off, b.pd.ps);
-    put("", l, "z1", b.z1.off, b.z1.ps); put("", l, "h1", b.h1.off, b.h1.ps); put("", l, "f", b.f.off, b.f.ps);
-    put("", l, "z2", b.z2.off, b.z2.ps); put("", l, "hout", b.hout.off, b.hout.ps);
-    put("", l, "st1", b.st1, 0); put("", l, "st2", b.st2, 0); put("", l, "fbits", b.fbits, 0);
-    if (pl.attn_tr) { put("", l, "astat", b.astat, 0); put("", l, "abits", b.abits, 0); }
+    char pre[16];
+    snprintf(pre, sizeof(pre), "L%d.", l);
+    put(pre, "qkv", b.qkv.off, b.qkv.ps); put(pre, "p", b.p.off, b.p.ps); put(pre, "pd", b.pd.off, b.pd.ps);
+    put_sub(pre, b.sub, "att");
+    put(pre, "fbits", b.sub.fbits, 0);
+    if (pl.attn_tr) { put(pre, "astat", b.astat, 0); put(pre, "abits", b.abits, 0); }
   }
   if (pl.prune) {
     const LastBufs& lb = pl.last;
-    put("", -1, "last.kv", lb.kv.off, lb.kv.ps); put("", -1, "last.q0", lb.q0.off, lb.q0.ps);
-    put("", -1, "last.att0", lb.att0.off, lb.att0.ps); put("", -1, "last.z1", lb.z1.off, lb.z1.ps);
-    put("", -1, "last.h1", lb.h1.off, lb.h1.ps); put("", -1, "last.f", lb.f.off, lb.f.ps);
-    put("", -1, "last.z2", lb.z2.off, lb.z2.ps); put("", -1, "last.hout", lb.hout.off, lb.hout.ps);
-    put("", -1, "last.st1", lb.st1, 0); put("", -1, "last.st2", lb.st2, 0);
-    put("", -1, "last.p0", lb.p0, 0); put("", -1, "last.pd0", lb.pd0, 0);
+    put("last.", "kv", lb.kv.off, lb.kv.ps); put("last.", "q0", lb.q0.off, lb.q0.ps);
+    put_sub("last.", lb.sub, "att0");
+    put("last.", "p0", lb.p0, 0); put("last.", "pd0", lb.pd0, 0);
   }
-  put("", -1, "hn", pl.hn, 0); put("", -1, "hst", pl.hst, 0); put("", -1, "emean", pl.emean, 0);
-  put("", -1, "epre", pl.epre, 0); put("", -1, "de", pl.de, 0);
+  put("", "hn", pl.hn, 0); put("", "hst", pl.hst, 0); put("", "emean", pl.emean, 0);
+  put("", "epre", pl.epre, 0); put("", "de", pl.de, 0);
   if (keep) {
-    put("", -1, "gscale", pl.gscale, 0);
-    put("", -1, "dh_a", pl.dh_a.off, pl.dh_a.ps); put("", -1, "dh_b", pl.dh_b.off, pl.dh_b.ps);
-    put("", -1, "dz", pl.dz.off, pl.dz.ps); put("", -1, "dzd", pl.dzd.off, pl.dzd.ps);
-    put("", -1, "df", pl.df.off, pl.df.ps); put("", -1, "datt", pl.datt.off, pl.datt.ps);
-    put("", -1, "dqkv", pl.dqkv.off, pl.dqkv.ps); put("", -1, "ds", pl.ds.off, pl.ds.ps);
+    put("", "gscale", pl.gscale, 0);
+    put("", "dh_a", pl.dh_a.off, pl.dh_a.ps); put("", "dh_b", pl.dh_b.off, pl.dh_b.ps);
+    put("", "dz", pl.dz.off, pl.dz.ps); put("", "dzd", pl.dzd.off, pl.dzd.ps);
+    put("", "df", pl.df.off, pl.df.ps); put("", "datt", pl.datt.off, pl.datt.ps);
+    put("", "dqkv", pl.dqkv.off, pl.dqkv.ps); put("", "ds", pl.ds.off, pl.ds.ps);
   }
   return static_cast<int>(off);
 }
@@ -552,6 +561,14 @@ struct Ctx {
   char* ws;
   cudaStream_t st;
   int P;
+  const float* gs = nullptr;   // backward: the device scalars (S, 1 / S) of grad_scale_kernel
+  // backward: gemm_run, handing 1 / S to every epilogue that produces parameter gradients (fp32 atomics of the weight
+  // gradients, fused bias column sums)
+  int run(GemmProblem& g) const {
+    if (g.epi.flags & EPI_OUT_ATOMIC) g.epi.alpha_ptr = gs + 1;
+    if (g.epi.flags & EPI_COLSUM) g.epi.colsum_scale_ptr = gs + 1;
+    return gemm_run(g, st);
+  }
   elem_t* ptr(const Split& s, int64_t elem_off = 0) const {
     return reinterpret_cast<elem_t*>(ws + s.off) + elem_off;
   }
@@ -584,20 +601,145 @@ int wgrad_ksplit(int64_t K, int M, int N) {
   return ks < 1 ? 1 : ks;
 }
 
-// dW[M_out, N_in] += dY^T[M_out, tokens] * X[tokens, N_in]   (both operands read MN-major, split-K, fp32 atomics)
-int wgrad(const Ctx& c, const Split& dy, int64_t dy_cols, const Split& x, int64_t x_cols, float* dw,
-          const char* tag, const float* inv_scale) {
+// Y[rows, N] = X[rows, K] W^T, W = the packed weight [N, K] at w_off   (both operands K-major)
+GemmProblem linear(const Ctx& c, const char* tag, const Split& x, int64_t rows, int64_t K, int64_t x_ld, int64_t w_off,
+                   int64_t N) {
   GemmProblem g;
   g.tag = tag;
-  g.A = c.mat(dy, 0, c.pl.Mt, dy_cols, dy_cols);
-  g.B = c.mat(x, 0, c.pl.Mt, x_cols, x_cols);
+  g.A = c.mat(x, 0, rows, K, x_ld);
+  g.B = c.mat(c.pl.wpack, w_off, N, K, K);
+  g.planes = c.P;
+  g.M = static_cast<int>(rows); g.N = static_cast<int>(N); g.K = static_cast<int>(K);
+  return g;
+}
+
+// dX[rows, K] = dY[rows, N] W, W = the packed weight [N, K] at w_off   (W read MN-major)
+GemmProblem dgrad(const Ctx& c, const char* tag, const Split& dy, int64_t rows, int64_t N, int64_t w_off, int64_t K) {
+  GemmProblem g;
+  g.tag = tag;
+  g.A = c.mat(dy, 0, rows, N, N);
+  g.B = c.mat(c.pl.wpack, w_off, N, K, K);
+  g.b_mn = true;
+  g.planes = c.P;
+  g.M = static_cast<int>(rows); g.N = static_cast<int>(K); g.K = static_cast<int>(N);
+  return g;
+}
+
+// dW[M_out, N_in] += dY^T[M_out, rows] * X[rows, N_in]   (both operands read MN-major, split-K, fp32 atomics; dY arrives
+// scaled by S, c.run multiplies by 1 / S)
+int wgrad(const Ctx& c, const char* tag, int64_t rows, const Split& dy, int64_t dy_cols, const Split& x, int64_t x_cols,
+          int64_t x_ld, float* dw) {
+  GemmProblem g;
+  g.tag = tag;
+  g.A = c.mat(dy, 0, rows, dy_cols, dy_cols);
+  g.B = c.mat(x, 0, rows, x_cols, x_ld);
   g.a_mn = true; g.b_mn = true; g.planes = c.P;
-  g.M = static_cast<int>(dy_cols); g.N = static_cast<int>(x_cols); g.K = static_cast<int>(c.pl.Mt);
-  g.ksplit = wgrad_ksplit(c.pl.Mt, g.M, g.N);
+  g.M = static_cast<int>(dy_cols); g.N = static_cast<int>(x_cols); g.K = static_cast<int>(rows);
+  g.ksplit = wgrad_ksplit(rows, g.M, g.N);
   g.epi.flags = EPI_OUT_ATOMIC;
-  g.epi.alpha_ptr = inv_scale;       // dY arrives scaled by S (grad_scale_kernel)
   g.epi.out = dw; g.epi.out_ld = x_cols;
-  return gemm_run(g, c.st);
+  return c.run(g);
+}
+
+// The sublayer of layer l after its attention, over `rows` rows of s.att: out-proj + dropout1 + residual ->
+// LayerNorm1 -> FFN1 + ReLU + dropout -> FFN2 + dropout2 + residual -> LayerNorm2.  The residual rows are read from
+// hin every hin_ld elements (D; the pruned last layer gathers the t = 0 rows of every slice with T*D).
+//   fuse_ln    both LayerNorms run inside the out-proj / FFN2 epilogues (EPI_LN); a plan that keeps the stash also
+//              stores the pre-normalisation rows and the row statistics the backward needs
+//   emit_bits  FFN1 writes its ReLU mask to s.fbits for the backward's gate
+//   last       the pruned last layer (its profiler tags)
+int sublayer_fwd(const Ctx& c, const spk_layer_params& lw, int l, const SublayerBufs& s, int64_t rows, const Split& hin,
+                 int64_t hin_ld, bool fuse_ln, bool emit_bits, DropCfg drop, bool last) {
+  const Plan& pl = c.pl;
+  const int64_t D = pl.D, F = pl.F;
+  const uint32_t drop_flag = drop.thresh ? EPI_DROPOUT : 0;
+  // Runs a GEMM whose output rows z are LayerNorm-ed into y: inside its epilogue (the tile owns whole rows; inference:
+  // z never leaves the SM) or by ln_fwd after it.
+  auto gemm_ln = [&](GemmProblem& g, const float* gamma, const float* beta, const Split& z, size_t stats,
+                     const Split& y) -> int {
+    if (!fuse_ln) {
+      c.out(g.epi, z, 0, D);
+      SPK_TRY(gemm_run(g, c.st));
+      return ln_fwd(c.ptr(z), z.ps, c.P, 1, gamma, beta, c.ptr(y), y.ps, c.P, c.f32(stats), rows, c.st);
+    }
+    g.epi.flags |= EPI_LN; g.epi.ln_gamma = gamma; g.epi.ln_beta = beta;
+    c.out(g.epi, y, 0, D);
+    if (pl.keep) { g.epi.ln_z = c.ptr(z); g.epi.ln_z_plane_stride = z.ps; g.epi.ln_stats = c.f32(stats); }
+    return gemm_run(g, c.st);
+  };
+  {  // out-proj + dropout1 + residual -> LayerNorm1
+    GemmProblem g = linear(c, last ? "gemm.last.out_proj" : "gemm.out_proj", s.att, rows, D, D, pl.w_out[l], D);
+    g.epi.flags = EPI_BIAS | EPI_RES | drop_flag;
+    g.epi.bias = lw.out_proj_b; g.epi.drop = drop; g.epi.drop_site = 2 + 4 * l;
+    c.res(g.epi, hin, hin_ld);
+    SPK_TRY(gemm_ln(g, lw.norm1_w, lw.norm1_b, s.z1, s.st1, s.h1));
+  }
+  {  // linear1 + ReLU + dropout
+    GemmProblem g = linear(c, last ? "gemm.last.ffn1" : "gemm.ffn1", s.h1, rows, D, D, pl.w_l1[l], F);
+    g.epi.flags = EPI_BIAS | EPI_RELU | drop_flag;
+    g.epi.bias = lw.linear1_b; g.epi.drop = drop; g.epi.drop_site = 3 + 4 * l;
+    if (emit_bits) {   // the backward's ReLU gate reads one bit per element instead of a whole plane of f
+      g.epi.flags |= EPI_EMIT_BITS;
+      g.epi.gate_bits = reinterpret_cast<uint32_t*>(c.f32(s.fbits));
+    }
+    c.out(g.epi, s.f, 0, F);
+    SPK_TRY(gemm_run(g, c.st));
+  }
+  // linear2 + dropout2 + residual -> LayerNorm2
+  GemmProblem g = linear(c, last ? "gemm.last.ffn2" : "gemm.ffn2", s.f, rows, F, F, pl.w_l2[l], D);
+  g.epi.flags = EPI_BIAS | EPI_RES | drop_flag;
+  g.epi.bias = lw.linear2_b; g.epi.drop = drop; g.epi.drop_site = 4 + 4 * l;
+  c.res(g.epi, s.h1, D);
+  return gemm_ln(g, lw.norm2_w, lw.norm2_b, s.z2, s.st2, s.hout);
+}
+
+// Backward of sublayer_fwd from the gradient dh of its output: LayerNorm2 -> FFN2 -> FFN1 (dH1 into dh_b) ->
+// LayerNorm1 -> out-proj (dATT into datt), the parameter gradients on the way.  The FFN2 dgrad's ReLU gate reads the
+// forward's mask bits s.fbits (gate_bits) or the sign of plane 0 of s.f.
+int sublayer_bwd(const Ctx& c, const spk_layer_params& lw, const spk_layer_params& lg, int l, const SublayerBufs& s,
+                 int64_t rows, const Split& dh, bool gate_bits, DropCfg drop, bool last) {
+  const Plan& pl = c.pl;
+  const int64_t D = pl.D, F = pl.F;
+  const int P = c.P;
+  const Split& dy = drop.thresh ? pl.dzd : pl.dz;
+  // ---- LayerNorm2 backward: dH(out) -> dZ2 (residual path) and dZ2 * mask (FFN path)
+  SPK_TRY(ln_bwd(c.ptr(dh), dh.ps, P, c.ptr(s.z2), s.z2.ps, P, c.f32(s.st2), lw.norm2_w, c.ptr(pl.dz), pl.dz.ps, P,
+                 c.ptr(pl.dzd), drop, 4 + 4 * l, lg.norm2_w, lg.norm2_b, lg.linear2_b, rows, c.gs, c.st));
+  SPK_TRY(wgrad(c, last ? "gemm.last.bwd.ffn2_wgrad" : "gemm.bwd.ffn2_wgrad", rows, dy, D, s.f, F, F, lg.linear2_w));
+  {  // dU = (dY2 W2) * 1[f > 0] / (1 - p)
+    GemmProblem g = dgrad(c, last ? "gemm.last.bwd.ffn2_dgrad" : "gemm.bwd.ffn2_dgrad", dy, rows, D, pl.w_l2[l], F);
+    g.epi.flags = EPI_COLSUM;
+    g.epi.colsum = lg.linear1_b;
+    if (gate_bits) {
+      g.epi.flags |= EPI_GATE_BITS;
+      g.epi.gate_bits = reinterpret_cast<uint32_t*>(c.f32(s.fbits));   // written by the forward FFN1 epilogue
+    } else {
+      g.epi.flags |= EPI_GATE_POS;
+      g.epi.gate = c.ptr(s.f); g.epi.gate_plane_stride = s.f.ps; g.epi.gate_ld = F; g.epi.gate_planes = 1;
+    }
+    g.epi.gate_scale = drop.inv_keep;
+    c.out(g.epi, pl.df, 0, F);
+    SPK_TRY(c.run(g));
+  }
+  SPK_TRY(wgrad(c, last ? "gemm.last.bwd.ffn1_wgrad" : "gemm.bwd.ffn1_wgrad", rows, pl.df, F, s.h1, D, D,
+                lg.linear1_w));
+  {  // dH1 = dU W1 + dZ2
+    GemmProblem g = dgrad(c, last ? "gemm.last.bwd.ffn1_dgrad" : "gemm.bwd.ffn1_dgrad", pl.df, rows, F, pl.w_l1[l], D);
+    g.epi.flags = EPI_RES;
+    c.res(g.epi, pl.dz, D);
+    c.out(g.epi, pl.dh_b, 0, D);
+    SPK_TRY(c.run(g));
+  }
+  // ---- LayerNorm1 backward
+  SPK_TRY(ln_bwd(c.ptr(pl.dh_b), pl.dh_b.ps, P, c.ptr(s.z1), s.z1.ps, P, c.f32(s.st1), lw.norm1_w, c.ptr(pl.dz),
+                 pl.dz.ps, P, c.ptr(pl.dzd), drop, 2 + 4 * l, lg.norm1_w, lg.norm1_b, lg.out_proj_b, rows, c.gs, c.st));
+  SPK_TRY(wgrad(c, last ? "gemm.last.bwd.out_wgrad" : "gemm.bwd.out_wgrad", rows, dy, D, s.att, D, D, lg.out_proj_w));
+  {  // dATT = dY1 Wo
+    GemmProblem g = dgrad(c, last ? "gemm.last.bwd.out_dgrad" : "gemm.bwd.out_dgrad", dy, rows, D, pl.w_out[l], D);
+    c.out(g.epi, pl.datt, 0, D);
+    SPK_TRY(c.run(g));
+  }
+  return 0;
 }
 
 }  // namespace
@@ -627,7 +769,7 @@ int encoder_forward(const spk_encoder_config& cfg, const spk_encoder_params& w, 
   SPK_CHECK(!training || keep, "encoder: training forward needs keep_stash (dropout P buffers live in the stash)");
   Ctx c{pl, reinterpret_cast<char*>(ws_v), st, P};
   GemmDependentLaunchScope dependent_launch(!keep && !training);   // inference: GEMM prologues under the previous kernel's tail
-  const int64_t Mt = pl.Mt, D = pl.D, F = pl.F;
+  const int64_t Mt = pl.Mt, D = pl.D;
   const int Tp = pl.Tp, H = pl.H;
   const DropCfg drop_pe = make_drop(seed, cfg.pe_dropout, training != 0);
   const DropCfg drop = make_drop(seed, cfg.dropout, training != 0);
@@ -640,11 +782,7 @@ int encoder_forward(const spk_encoder_config& cfg, const spk_encoder_params& w, 
   SPK_TRY(pe_transpose(w.pe, c.f32(pl.pe_t), pl.D, cfg.max_pos, T, st));
 
   {  // prenet k=1 conv + ReLU + alpha * PE (+ dropout)        Modules.py:50-52,98-105
-    GemmProblem g;
-    g.tag = "gemm.prenet";
-    g.A = c.mat(pl.x0, 0, Mt, pl.C, pl.C);
-    g.B = c.mat(pl.wpack, pl.w_pre, D, pl.C, pl.C);
-    g.planes = P; g.M = (int)Mt; g.N = (int)D; g.K = pl.C;
+    GemmProblem g = linear(c, "gemm.prenet", pl.x0, Mt, pl.C, pl.C, pl.w_pre, D);
     g.epi.flags = EPI_BIAS | EPI_RELU | EPI_PE | (drop_pe.thresh ? EPI_DROPOUT : 0);
     if (pl.keep && P >= 2) {   // the backward gates dH0 with the forward's own ReLU decisions
       g.epi.flags |= EPI_EMIT_BITS;
@@ -656,19 +794,14 @@ int encoder_forward(const spk_encoder_config& cfg, const spk_encoder_params& w, 
     SPK_TRY(gemm_run(g, st));
   }
   const int dense_layers = pl.prune ? pl.L - 1 : pl.L;
-  // both LayerNorms of the dense layers run inside the out-proj / FFN2 epilogues (EPI_LN); a training forward also
-  // stores the pre-normalisation rows and the row statistics the backward needs
+  // both LayerNorms of the dense layers run inside the GEMM epilogues (the pruned last layer keeps ln_fwd)
   const bool fuse_ln = g_fuse_ln && P <= 2 && (!keep || (g_fuse_ln_train && P == 2));   // EPI_LN kernels exist for 1 and 2 planes
   for (int l = 0; l < dense_layers; ++l) {
     const LayerBufs& b = pl.Lb[l];
-    const Split& hin = (l == 0) ? pl.h0 : pl.Lb[l - 1].hout;
+    const Split& hin = (l == 0) ? pl.h0 : pl.Lb[l - 1].sub.hout;
     const spk_layer_params& lw = w.layer[l];
     {  // in-proj
-      GemmProblem g;
-      g.tag = "gemm.qkv";
-      g.A = c.mat(hin, 0, Mt, D, D);
-      g.B = c.mat(pl.wpack, pl.w_in[l], 3 * D, D, D);
-      g.planes = P; g.M = (int)Mt; g.N = (int)(3 * D); g.K = (int)D;
+      GemmProblem g = linear(c, "gemm.qkv", hin, Mt, D, D, pl.w_in[l], 3 * D);
       g.epi.flags = EPI_BIAS; g.epi.bias = lw.in_proj_b;
       c.out(g.epi, b.qkv, 0, 3 * D);
       SPK_TRY(gemm_run(g, st));
@@ -676,11 +809,11 @@ int encoder_forward(const spk_encoder_config& cfg, const spk_encoder_params& w, 
     // inference (one plane, nothing kept for a backward pass): scores, softmax and PV in one tcgen05 kernel
     const bool fused_attn = (P == 1) && !keep && !training && T <= 256 && pl.fused_infer;
     if (fused_attn && T <= 192 && g_infer_attn_two) {      // two CTAs per SM (attn_train.cu, inference variant)
-      SPK_TRY(attn_infer_fwd(c.ptr(b.qkv), c.ptr(b.att), D, B, H, T, st));
+      SPK_TRY(attn_infer_fwd(c.ptr(b.qkv), c.ptr(b.sub.att), D, B, H, T, st));
     } else if (fused_attn) {
-      SPK_TRY(attn_fused_fwd(c.ptr(b.qkv), c.ptr(b.att), D, B, H, T, st));
+      SPK_TRY(attn_fused_fwd(c.ptr(b.qkv), c.ptr(b.sub.att), D, B, H, T, st));
     } else if (pl.attn_tr) {
-      SPK_TRY(attn_train_fwd(c.ptr(b.qkv), b.qkv.ps, P, c.ptr(b.att), b.att.ps, D, c.f32(b.astat),
+      SPK_TRY(attn_train_fwd(c.ptr(b.qkv), b.qkv.ps, P, c.ptr(b.sub.att), b.sub.att.ps, D, c.f32(b.astat),
                              reinterpret_cast<uint32_t*>(c.f32(b.abits)), drop, 1 + 4 * l, B, H, T, Tp, st));
     } else {
     {  // S = Q K^T / sqrt(dh), per (slice, head)
@@ -704,133 +837,35 @@ int encoder_forward(const spk_encoder_config& cfg, const spk_encoder_params& w, 
       g.B = c.mat(b.qkv, 2 * D, T, 64, 3 * D, 64, (int64_t)T * 3 * D);
       g.b_mn = true;
       g.planes = P; g.M = T; g.N = 64; g.K = T; g.nb0 = H; g.nb1 = B;
-      c.out(g.epi, b.att, 0, D, 64, (int64_t)T * D);
+      c.out(g.epi, b.sub.att, 0, D, 64, (int64_t)T * D);
       SPK_TRY(gemm_run(g, st));
     }
     }
-    {  // out-proj + dropout1 + residual
-      GemmProblem g;
-      g.tag = "gemm.out_proj";
-      g.A = c.mat(b.att, 0, Mt, D, D);
-      g.B = c.mat(pl.wpack, pl.w_out[l], D, D, D);
-      g.planes = P; g.M = (int)Mt; g.N = (int)D; g.K = (int)D;
-      g.epi.flags = EPI_BIAS | EPI_RES | (drop.thresh ? EPI_DROPOUT : 0);
-      g.epi.bias = lw.out_proj_b; g.epi.drop = drop; g.epi.drop_site = 2 + 4 * l;
-      c.res(g.epi, hin, D);
-      if (fuse_ln) {   // inference: LayerNorm1 inside the epilogue (the tile owns whole rows), z1 never leaves the SM
-        g.epi.flags |= EPI_LN; g.epi.ln_gamma = lw.norm1_w; g.epi.ln_beta = lw.norm1_b;
-        c.out(g.epi, b.h1, 0, D);
-        if (keep) { g.epi.ln_z = c.ptr(b.z1); g.epi.ln_z_plane_stride = b.z1.ps; g.epi.ln_stats = c.f32(b.st1); }
-      } else {
-        c.out(g.epi, b.z1, 0, D);
-      }
-      SPK_TRY(gemm_run(g, st));
-    }
-    if (!fuse_ln)
-      SPK_TRY(ln_fwd(c.ptr(b.z1), b.z1.ps, P, 1, lw.norm1_w, lw.norm1_b, c.ptr(b.h1), b.h1.ps, P, c.f32(b.st1), Mt, st));
-    {  // linear1 + ReLU + dropout
-      GemmProblem g;
-      g.tag = "gemm.ffn1";
-      g.A = c.mat(b.h1, 0, Mt, D, D);
-      g.B = c.mat(pl.wpack, pl.w_l1[l], F, D, D);
-      g.planes = P; g.M = (int)Mt; g.N = (int)F; g.K = (int)D;
-      g.epi.flags = EPI_BIAS | EPI_RELU | (drop.thresh ? EPI_DROPOUT : 0);
-      g.epi.bias = lw.linear1_b; g.epi.drop = drop; g.epi.drop_site = 3 + 4 * l;
-      if (keep) {   // the backward's ReLU gate reads one bit per element instead of a whole plane of f
-        g.epi.flags |= EPI_EMIT_BITS;
-        g.epi.gate_bits = reinterpret_cast<uint32_t*>(c.f32(b.fbits));
-      }
-      c.out(g.epi, b.f, 0, F);
-      SPK_TRY(gemm_run(g, st));
-    }
-    {  // linear2 + dropout2 + residual
-      GemmProblem g;
-      g.tag = "gemm.ffn2";
-      g.A = c.mat(b.f, 0, Mt, F, F);
-      g.B = c.mat(pl.wpack, pl.w_l2[l], D, F, F);
-      g.planes = P; g.M = (int)Mt; g.N = (int)D; g.K = (int)F;
-      g.epi.flags = EPI_BIAS | EPI_RES | (drop.thresh ? EPI_DROPOUT : 0);
-      g.epi.bias = lw.linear2_b; g.epi.drop = drop; g.epi.drop_site = 4 + 4 * l;
-      c.res(g.epi, b.h1, D);
-      if (fuse_ln) {
-        g.epi.flags |= EPI_LN; g.epi.ln_gamma = lw.norm2_w; g.epi.ln_beta = lw.norm2_b;
-        c.out(g.epi, b.hout, 0, D);
-        if (keep) { g.epi.ln_z = c.ptr(b.z2); g.epi.ln_z_plane_stride = b.z2.ps; g.epi.ln_stats = c.f32(b.st2); }
-      } else {
-        c.out(g.epi, b.z2, 0, D);
-      }
-      SPK_TRY(gemm_run(g, st));
-    }
-    if (!fuse_ln)
-      SPK_TRY(ln_fwd(c.ptr(b.z2), b.z2.ps, P, 1, lw.norm2_w, lw.norm2_b, c.ptr(b.hout), b.hout.ps, P, c.f32(b.st2), Mt, st));
+    SPK_TRY(sublayer_fwd(c, lw, l, b.sub, Mt, hin, D, fuse_ln, pl.keep, drop, false));
   }
   if (pl.prune) {
     // ---- last layer: only the t = 0 query row of every slice is consumed (Modules.py:54)
     const int l = pl.L - 1;
     const LastBufs& lb = pl.last;
-    const Split& hin = (l == 0) ? pl.h0 : pl.Lb[l - 1].hout;
+    const Split& hin = (l == 0) ? pl.h0 : pl.Lb[l - 1].sub.hout;
     const spk_layer_params& lw = w.layer[l];
     {  // K | V for every frame
-      GemmProblem g;
-      g.tag = "gemm.last.kv";
-      g.A = c.mat(hin, 0, Mt, D, D);
-      g.B = c.mat(pl.wpack, pl.w_in[l] + D * D, 2 * D, D, D);
-      g.planes = P; g.M = (int)Mt; g.N = (int)(2 * D); g.K = (int)D;
+      GemmProblem g = linear(c, "gemm.last.kv", hin, Mt, D, D, pl.w_in[l] + D * D, 2 * D);
       g.epi.flags = EPI_BIAS; g.epi.bias = lw.in_proj_b + D;
       c.out(g.epi, lb.kv, 0, 2 * D);
       SPK_TRY(gemm_run(g, st));
     }
     {  // Q for the first frame of every slice (rows gathered by the row stride T*D)
-      GemmProblem g;
-      g.tag = "gemm.last.q0";
-      g.A = c.mat(hin, 0, B, D, (int64_t)T * D);
-      g.B = c.mat(pl.wpack, pl.w_in[l], D, D, D);
-      g.planes = P; g.M = B; g.N = (int)D; g.K = (int)D;
+      GemmProblem g = linear(c, "gemm.last.q0", hin, B, D, (int64_t)T * D, pl.w_in[l], D);
       g.epi.flags = EPI_BIAS; g.epi.bias = lw.in_proj_b;
       c.out(g.epi, lb.q0, 0, D);
       SPK_TRY(gemm_run(g, st));
     }
-    SPK_TRY(attn_row0_fwd(c.ptr(lb.q0), lb.q0.ps, c.ptr(lb.kv), lb.kv.ps, P, c.ptr(lb.att0), lb.att0.ps,
+    SPK_TRY(attn_row0_fwd(c.ptr(lb.q0), lb.q0.ps, c.ptr(lb.kv), lb.kv.ps, P, c.ptr(lb.sub.att), lb.sub.att.ps,
                           keep ? c.f32(lb.p0) : nullptr, keep ? c.f32(lb.pd0) : nullptr, drop, 1 + 4 * l, B, H, T, Tp, st));
-    {  // out-proj + dropout1 + residual (t = 0 rows of the layer input)
-      GemmProblem g;
-      g.tag = "gemm.last.out_proj";
-      g.A = c.mat(lb.att0, 0, B, D, D);
-      g.B = c.mat(pl.wpack, pl.w_out[l], D, D, D);
-      g.planes = P; g.M = B; g.N = (int)D; g.K = (int)D;
-      g.epi.flags = EPI_BIAS | EPI_RES | (drop.thresh ? EPI_DROPOUT : 0);
-      g.epi.bias = lw.out_proj_b; g.epi.drop = drop; g.epi.drop_site = 2 + 4 * l;
-      c.res(g.epi, hin, (int64_t)T * D);
-      c.out(g.epi, lb.z1, 0, D);
-      SPK_TRY(gemm_run(g, st));
-    }
-    SPK_TRY(ln_fwd(c.ptr(lb.z1), lb.z1.ps, P, 1, lw.norm1_w, lw.norm1_b, c.ptr(lb.h1), lb.h1.ps, P, c.f32(lb.st1), B, st));
-    {
-      GemmProblem g;
-      g.tag = "gemm.last.ffn1";
-      g.A = c.mat(lb.h1, 0, B, D, D);
-      g.B = c.mat(pl.wpack, pl.w_l1[l], F, D, D);
-      g.planes = P; g.M = B; g.N = (int)F; g.K = (int)D;
-      g.epi.flags = EPI_BIAS | EPI_RELU | (drop.thresh ? EPI_DROPOUT : 0);
-      g.epi.bias = lw.linear1_b; g.epi.drop = drop; g.epi.drop_site = 3 + 4 * l;
-      c.out(g.epi, lb.f, 0, F);
-      SPK_TRY(gemm_run(g, st));
-    }
-    {
-      GemmProblem g;
-      g.tag = "gemm.last.ffn2";
-      g.A = c.mat(lb.f, 0, B, F, F);
-      g.B = c.mat(pl.wpack, pl.w_l2[l], D, F, F);
-      g.planes = P; g.M = B; g.N = (int)D; g.K = (int)F;
-      g.epi.flags = EPI_BIAS | EPI_RES | (drop.thresh ? EPI_DROPOUT : 0);
-      g.epi.bias = lw.linear2_b; g.epi.drop = drop; g.epi.drop_site = 4 + 4 * l;
-      c.res(g.epi, lb.h1, D);
-      c.out(g.epi, lb.z2, 0, D);
-      SPK_TRY(gemm_run(g, st));
-    }
-    SPK_TRY(ln_fwd(c.ptr(lb.z2), lb.z2.ps, P, 1, lw.norm2_w, lw.norm2_b, c.ptr(lb.hout), lb.hout.ps, P, c.f32(lb.st2), B, st));
+    SPK_TRY(sublayer_fwd(c, lw, l, lb.sub, B, hin, (int64_t)T * D, false, false, drop, true));
   }
-  const Split& hl = pl.prune ? pl.last.hout : pl.Lb[pl.L - 1].hout;
+  const Split& hl = pl.prune ? pl.last.sub.hout : pl.Lb[pl.L - 1].sub.hout;
   const int head_T = pl.prune ? 1 : T;     // the compact buffer holds one row per slice
   ProfScope prof_head("head_fwd", 2.0 * (B / S) * 256 * 256, 4.0 * B * 256 * 2, st);
   head_fwd_kernel<<<(B / S + HEAD_UPB - 1) / HEAD_UPB, 256, 0, st>>>(
@@ -849,23 +884,17 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
   if (ws_bytes < pl.total) { set_error("encoder: workspace too small (%zu < %zu)", ws_bytes, pl.total); return SPK_ENOMEM; }
   const int P = P_fwd < 2 ? P_fwd : 2;   // the stash may hold 3 planes; the backward pass reads / writes 2
   Ctx c{pl, reinterpret_cast<char*>(ws_v), st, P};
-  const int64_t Mt = pl.Mt, D = pl.D, F = pl.F;
+  const int64_t Mt = pl.Mt, D = pl.D;
   const int Tp = pl.Tp, H = pl.H;
   const DropCfg drop_pe = make_drop(seed, cfg.pe_dropout, training != 0);
   const DropCfg drop = make_drop(seed, cfg.dropout, training != 0);
-  // gradient scale of this pass (device scalars S, 1 / S) and a gemm_run that hands 1 / S to every epilogue that
-  // produces parameter gradients (fp32 atomics of the weight gradients, fused bias column sums)
-  float* gs = c.f32(pl.gscale);
-  auto run = [&](GemmProblem& g) {
-    if (g.epi.flags & EPI_OUT_ATOMIC) g.epi.alpha_ptr = gs + 1;
-    if (g.epi.flags & EPI_COLSUM) g.epi.colsum_scale_ptr = gs + 1;
-    return gemm_run(g, st);
-  };
+  float* gs = c.f32(pl.gscale);   // gradient scale of this pass (device scalars S, 1 / S)
+  c.gs = gs;
   grad_scale_kernel<<<1, 1024, 0, st>>>(d_dvec, static_cast<int64_t>(B / S) * 256, gs, g_grad_scale_log2);
   SPK_CUDA(cudaGetLastError());
 
   // ---- head
-  const Split& hl = pl.prune ? pl.last.hout : pl.Lb[pl.L - 1].hout;
+  const Split& hl = pl.prune ? pl.last.sub.hout : pl.Lb[pl.L - 1].sub.hout;
   const int head_T = pl.prune ? 1 : T;
   // dense: the gradient of the last layer's output is zero except the t = 0 rows; pruned: compact [B, 256] in dh_b
   const Split& dhead = pl.prune ? pl.dh_b : pl.dh_a;
@@ -885,165 +914,42 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
     // ---- last layer on the compact t = 0 rows (buffers dh_b / dz / dzd / df / datt hold B rows here)
     const int l = pl.L - 1;
     const LastBufs& lb = pl.last;
-    const Split& hin = (l == 0) ? pl.h0 : pl.Lb[l - 1].hout;
-    const spk_layer_params& lw = w.layer[l];
+    const Split& hin = (l == 0) ? pl.h0 : pl.Lb[l - 1].sub.hout;
     const spk_layer_params& lg = gr.layer[l];
-    const Split& dy = drop.thresh ? pl.dzd : pl.dz;
-    auto small_wgrad = [&](const Split& dyt, int64_t dy_cols, const Split& x, int64_t x_cols, int64_t x_ld, float* dw,
-                           const char* tag) {
-      GemmProblem g;
-      g.tag = tag;
-      g.A = c.mat(dyt, 0, B, dy_cols, dy_cols);
-      g.B = c.mat(x, 0, B, x_cols, x_ld);
-      g.a_mn = true; g.b_mn = true; g.planes = P;
-      g.M = (int)dy_cols; g.N = (int)x_cols; g.K = B;
-      g.ksplit = wgrad_ksplit(B, g.M, g.N);
-      g.epi.flags = EPI_OUT_ATOMIC;
-      g.epi.out = dw; g.epi.out_ld = x_cols;
-      return run(g);
-    };
-    SPK_TRY(ln_bwd(c.ptr(pl.dh_b), pl.dh_b.ps, P, c.ptr(lb.z2), lb.z2.ps, P, c.f32(lb.st2), lw.norm2_w, c.ptr(pl.dz),
-                   pl.dz.ps, P, c.ptr(pl.dzd), drop, 4 + 4 * l, lg.norm2_w, lg.norm2_b, lg.linear2_b, B, gs, st));
-    SPK_TRY(small_wgrad(dy, D, lb.f, F, F, lg.linear2_w, "gemm.last.bwd.ffn2_wgrad"));
-    {
-      GemmProblem g;
-      g.tag = "gemm.last.bwd.ffn2_dgrad";
-      g.A = c.mat(dy, 0, B, D, D);
-      g.B = c.mat(pl.wpack, pl.w_l2[l], D, F, F);
-      g.b_mn = true;
-      g.planes = P; g.M = B; g.N = (int)F; g.K = (int)D;
-      g.epi.flags = EPI_GATE_POS | EPI_COLSUM;
-      g.epi.colsum = lg.linear1_b;
-      g.epi.gate = c.ptr(lb.f); g.epi.gate_plane_stride = lb.f.ps; g.epi.gate_ld = F; g.epi.gate_planes = 1;
-      g.epi.gate_scale = drop.inv_keep;
-      c.out(g.epi, pl.df, 0, F);
-      SPK_TRY(run(g));
-    }
-    SPK_TRY(small_wgrad(pl.df, F, lb.h1, D, D, lg.linear1_w, "gemm.last.bwd.ffn1_wgrad"));
-    {
-      GemmProblem g;
-      g.tag = "gemm.last.bwd.ffn1_dgrad";
-      g.A = c.mat(pl.df, 0, B, F, F);
-      g.B = c.mat(pl.wpack, pl.w_l1[l], F, D, D);
-      g.b_mn = true;
-      g.planes = P; g.M = B; g.N = (int)D; g.K = (int)F;
-      g.epi.flags = EPI_RES;
-      c.res(g.epi, pl.dz, D);
-      c.out(g.epi, pl.dh_b, 0, D);
-      SPK_TRY(run(g));
-    }
-    SPK_TRY(ln_bwd(c.ptr(pl.dh_b), pl.dh_b.ps, P, c.ptr(lb.z1), lb.z1.ps, P, c.f32(lb.st1), lw.norm1_w, c.ptr(pl.dz),
-                   pl.dz.ps, P, c.ptr(pl.dzd), drop, 2 + 4 * l, lg.norm1_w, lg.norm1_b, lg.out_proj_b, B, gs, st));
-    SPK_TRY(small_wgrad(dy, D, lb.att0, D, D, lg.out_proj_w, "gemm.last.bwd.out_wgrad"));
-    {
-      GemmProblem g;
-      g.tag = "gemm.last.bwd.out_dgrad";
-      g.A = c.mat(dy, 0, B, D, D);
-      g.B = c.mat(pl.wpack, pl.w_out[l], D, D, D);
-      g.b_mn = true;
-      g.planes = P; g.M = B; g.N = (int)D; g.K = (int)D;
-      c.out(g.epi, pl.datt, 0, D);
-      SPK_TRY(run(g));
-    }
+    // the FFN2 dgrad gates on the sign of f: the last layer keeps no ReLU mask bits
+    SPK_TRY(sublayer_bwd(c, w.layer[l], lg, l, lb.sub, B, pl.dh_b, false, drop, true));
     // single-query attention backward: dq0 (compact [B, 256]), dK | dV -> dqkv viewed as [Mt, 512]
     SPK_TRY(attn_row0_bwd(c.ptr(pl.datt), pl.datt.ps, P, c.ptr(lb.q0), lb.q0.ps, c.ptr(lb.kv), lb.kv.ps, P_fwd,
                           c.f32(lb.p0), c.f32(lb.pd0), c.ptr(pl.dq0), pl.dq0.ps, c.ptr(pl.dqkv), pl.dqkv.ps,
                           lg.in_proj_b, gs, B, H, T, Tp, st));
-    SPK_TRY(small_wgrad(pl.dq0, D, hin, D, (int64_t)T * D, lg.in_proj_w, "gemm.last.bwd.q_wgrad"));
-    {  // dW[K|V rows] = dKV^T hin
-      GemmProblem g;
-      g.tag = "gemm.last.bwd.kv_wgrad";
-      g.A = c.mat(pl.dqkv, 0, Mt, 2 * D, 2 * D);
-      g.B = c.mat(hin, 0, Mt, D, D);
-      g.a_mn = true; g.b_mn = true; g.planes = P;
-      g.M = (int)(2 * D); g.N = (int)D; g.K = (int)Mt;
-      g.ksplit = wgrad_ksplit(Mt, g.M, g.N);
-      g.epi.flags = EPI_OUT_ATOMIC;
-      g.epi.out = lg.in_proj_w + D * D; g.epi.out_ld = D;
-      SPK_TRY(run(g));
-    }
+    SPK_TRY(wgrad(c, "gemm.last.bwd.q_wgrad", B, pl.dq0, D, hin, D, (int64_t)T * D, lg.in_proj_w));
+    // dW[K|V rows] = dKV^T hin
+    SPK_TRY(wgrad(c, "gemm.last.bwd.kv_wgrad", Mt, pl.dqkv, 2 * D, hin, D, D, lg.in_proj_w + D * D));
     {  // dH(in) = dKV W[K|V rows]  for every frame
-      GemmProblem g;
-      g.tag = "gemm.last.bwd.kv_dgrad";
-      g.A = c.mat(pl.dqkv, 0, Mt, 2 * D, 2 * D);
-      g.B = c.mat(pl.wpack, pl.w_in[l] + D * D, 2 * D, D, D);
-      g.b_mn = true;
-      g.planes = P; g.M = (int)Mt; g.N = (int)D; g.K = (int)(2 * D);
+      GemmProblem g = dgrad(c, "gemm.last.bwd.kv_dgrad", pl.dqkv, Mt, 2 * D, pl.w_in[l] + D * D, D);
       c.out(g.epi, pl.dh_a, 0, D);
-      SPK_TRY(run(g));
+      SPK_TRY(c.run(g));
     }
     {  // t = 0 rows additionally receive dq0 Wq and the residual path dZ1
-      GemmProblem g;
-      g.tag = "gemm.last.bwd.q_dgrad";
-      g.A = c.mat(pl.dq0, 0, B, D, D);
-      g.B = c.mat(pl.wpack, pl.w_in[l], D, D, D);
-      g.b_mn = true;
-      g.planes = P; g.M = B; g.N = (int)D; g.K = (int)D;
+      GemmProblem g = dgrad(c, "gemm.last.bwd.q_dgrad", pl.dq0, B, D, pl.w_in[l], D);
       g.epi.flags = EPI_RES;
       c.res(g.epi, pl.dz, D);
       c.out(g.epi, pl.dh_b, 0, D);
-      SPK_TRY(run(g));
+      SPK_TRY(c.run(g));
     }
     SPK_TRY(rows_add(c.ptr(pl.dh_a), pl.dh_a.ps, T, c.ptr(pl.dh_b), pl.dh_b.ps, P, B, st));
   }
 
   for (int l = (pl.prune ? pl.L - 2 : pl.L - 1); l >= 0; --l) {
     const LayerBufs& b = pl.Lb[l];
-    const Split& hin = (l == 0) ? pl.h0 : pl.Lb[l - 1].hout;
-    const spk_layer_params& lw = w.layer[l];
+    const Split& hin = (l == 0) ? pl.h0 : pl.Lb[l - 1].sub.hout;
     const spk_layer_params& lg = gr.layer[l];
-    const Split& dy_ffn = drop.thresh ? pl.dzd : pl.dz;
-    // ---- LayerNorm2 backward: dH(out) -> dZ2 (residual path) and dZ2 * mask (FFN path)
-    SPK_TRY(ln_bwd(c.ptr(pl.dh_a), pl.dh_a.ps, P, c.ptr(b.z2), b.z2.ps, P, c.f32(b.st2), lw.norm2_w, c.ptr(pl.dz),
-                   pl.dz.ps, P, c.ptr(pl.dzd), drop, 4 + 4 * l, lg.norm2_w, lg.norm2_b, lg.linear2_b, Mt, gs, st));
-    SPK_TRY(wgrad(c, dy_ffn, D, b.f, F, lg.linear2_w, "gemm.bwd.ffn2_wgrad", gs + 1));
-    {  // dU = (dY2 W2) * 1[f > 0] / (1 - p)
-      GemmProblem g;
-      g.tag = "gemm.bwd.ffn2_dgrad";
-      g.A = c.mat(dy_ffn, 0, Mt, D, D);
-      g.B = c.mat(pl.wpack, pl.w_l2[l], D, F, F);
-      g.b_mn = true;
-      g.planes = P; g.M = (int)Mt; g.N = (int)F; g.K = (int)D;
-      g.epi.flags = EPI_GATE_BITS | EPI_COLSUM;
-      g.epi.colsum = lg.linear1_b;
-      g.epi.gate_bits = reinterpret_cast<uint32_t*>(c.f32(b.fbits));   // written by the forward FFN1 epilogue
-      g.epi.gate_scale = drop.inv_keep;
-      c.out(g.epi, pl.df, 0, F);
-      SPK_TRY(run(g));
-    }
-    SPK_TRY(wgrad(c, pl.df, F, b.h1, D, lg.linear1_w, "gemm.bwd.ffn1_wgrad", gs + 1));
-    {  // dH1 = dU W1 + dZ2
-      GemmProblem g;
-      g.tag = "gemm.bwd.ffn1_dgrad";
-      g.A = c.mat(pl.df, 0, Mt, F, F);
-      g.B = c.mat(pl.wpack, pl.w_l1[l], F, D, D);
-      g.b_mn = true;
-      g.planes = P; g.M = (int)Mt; g.N = (int)D; g.K = (int)F;
-      g.epi.flags = EPI_RES;
-      c.res(g.epi, pl.dz, D);
-      c.out(g.epi, pl.dh_b, 0, D);
-      SPK_TRY(run(g));
-    }
-    // ---- LayerNorm1 backward
-    const Split& dy_att = drop.thresh ? pl.dzd : pl.dz;
-    SPK_TRY(ln_bwd(c.ptr(pl.dh_b), pl.dh_b.ps, P, c.ptr(b.z1), b.z1.ps, P, c.f32(b.st1), lw.norm1_w, c.ptr(pl.dz),
-                   pl.dz.ps, P, c.ptr(pl.dzd), drop, 2 + 4 * l, lg.norm1_w, lg.norm1_b, lg.out_proj_b, Mt, gs, st));
-    SPK_TRY(wgrad(c, dy_att, D, b.att, D, lg.out_proj_w, "gemm.bwd.out_wgrad", gs + 1));
-    {  // dATT = dY1 Wo
-      GemmProblem g;
-      g.tag = "gemm.bwd.out_dgrad";
-      g.A = c.mat(dy_att, 0, Mt, D, D);
-      g.B = c.mat(pl.wpack, pl.w_out[l], D, D, D);
-      g.b_mn = true;
-      g.planes = P; g.M = (int)Mt; g.N = (int)D; g.K = (int)D;
-      c.out(g.epi, pl.datt, 0, D);
-      SPK_TRY(run(g));
-    }
+    SPK_TRY(sublayer_bwd(c, w.layer[l], lg, l, b.sub, Mt, pl.dh_a, true, drop, false));
     // ---- attention backward, per (slice, head)
     if (pl.attn_tr) {
-      SPK_TRY(attn_train_bwd(c.ptr(b.qkv), b.qkv.ps, c.ptr(b.att), b.att.ps, c.ptr(pl.datt), pl.datt.ps, c.f32(b.astat),
-                             reinterpret_cast<const uint32_t*>(c.f32(b.abits)), c.f32(pl.adelta), c.ptr(pl.dqkv),
-                             pl.dqkv.ps, lg.in_proj_b, gs, drop, B, H, T, Tp, st));
+      SPK_TRY(attn_train_bwd(c.ptr(b.qkv), b.qkv.ps, c.ptr(b.sub.att), b.sub.att.ps, c.ptr(pl.datt), pl.datt.ps,
+                             c.f32(b.astat), reinterpret_cast<const uint32_t*>(c.f32(b.abits)), c.f32(pl.adelta),
+                             c.ptr(pl.dqkv), pl.dqkv.ps, lg.in_proj_b, gs, drop, B, H, T, Tp, st));
     } else {
     const Split& pdrop = drop.thresh ? b.pd : b.p;
     const int64_t sP0 = (int64_t)T * Tp, sP1 = (int64_t)H * T * Tp;
@@ -1057,7 +963,7 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
       g.planes = P; g.M = T; g.N = 64; g.K = T; g.nb0 = H; g.nb1 = B;
       g.epi.flags = EPI_COLSUM; g.epi.colsum = lg.in_proj_b + 2 * D; g.epi.colsum_sb0 = 64;
       c.out(g.epi, pl.dqkv, 2 * D, 3 * D, sQ0, sQ1);
-      SPK_TRY(run(g));
+      SPK_TRY(c.run(g));
     }
     {  // dP_drop = dO V^T
       GemmProblem g;
@@ -1068,7 +974,7 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
       c.out(g.epi, pl.scr, 0, Tp, sP0, sP1);
       if (P >= 2) g.epi.flags |= EPI_OUT_F32;
       if (P >= 2) g.block_n = 64;   // as for QK^T
-      SPK_TRY(run(g));
+      SPK_TRY(c.run(g));
     }
     SPK_TRY(softmax_bwd(c.ptr(b.p), c.ptr(pl.scr), P >= 2 ? reinterpret_cast<const float*>(c.ptr(pl.scr)) : nullptr,
                         b.p.ps, P, c.ptr(pl.ds), drop, 1 + 4 * l, 0.125f, pl.BH * T, T, Tp, st));
@@ -1081,7 +987,7 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
       g.planes = P; g.M = T; g.N = 64; g.K = T; g.nb0 = H; g.nb1 = B;
       g.epi.flags = EPI_COLSUM; g.epi.colsum = lg.in_proj_b; g.epi.colsum_sb0 = 64;
       c.out(g.epi, pl.dqkv, 0, 3 * D, sQ0, sQ1);
-      SPK_TRY(run(g));
+      SPK_TRY(c.run(g));
     }
     {  // dK = dS^T Q
       GemmProblem g;
@@ -1092,22 +998,17 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
       g.planes = P; g.M = T; g.N = 64; g.K = T; g.nb0 = H; g.nb1 = B;
       g.epi.flags = EPI_COLSUM; g.epi.colsum = lg.in_proj_b + D; g.epi.colsum_sb0 = 64;
       c.out(g.epi, pl.dqkv, D, 3 * D, sQ0, sQ1);
-      SPK_TRY(run(g));
+      SPK_TRY(c.run(g));
     }
     }
     // ---- in-proj
-    SPK_TRY(wgrad(c, pl.dqkv, 3 * D, hin, D, lg.in_proj_w, "gemm.bwd.qkv_wgrad", gs + 1));
+    SPK_TRY(wgrad(c, "gemm.bwd.qkv_wgrad", Mt, pl.dqkv, 3 * D, hin, D, D, lg.in_proj_w));
     {  // dH(in) = dQKV Win + dZ1
-      GemmProblem g;
-      g.tag = "gemm.bwd.qkv_dgrad";
-      g.A = c.mat(pl.dqkv, 0, Mt, 3 * D, 3 * D);
-      g.B = c.mat(pl.wpack, pl.w_in[l], 3 * D, D, D);
-      g.b_mn = true;
-      g.planes = P; g.M = (int)Mt; g.N = (int)D; g.K = (int)(3 * D);
+      GemmProblem g = dgrad(c, "gemm.bwd.qkv_dgrad", pl.dqkv, Mt, 3 * D, pl.w_in[l], D);
       g.epi.flags = EPI_RES;
       c.res(g.epi, pl.dz, D);
       c.out(g.epi, pl.dh_a, 0, D);
-      SPK_TRY(run(g));
+      SPK_TRY(c.run(g));
     }
   }
   // ---- embedding: positional alpha, prenet weight / bias
@@ -1117,21 +1018,17 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
   } else {        // one-plane plans keep no mask: the gate is recomputed from x0 W^T + b
     SPK_TRY(pe_alpha_grad(c.ptr(pl.dh_a), pl.dh_a.ps, P, c.f32(pl.pe_t), drop_pe, 0, gr.pe_alpha, Mt, T, gs, st));
     {
-      GemmProblem g;
-      g.tag = "gemm.bwd.prenet_gate";
-      g.A = c.mat(pl.x0, 0, Mt, pl.C, pl.C);
-      g.B = c.mat(pl.wpack, pl.w_pre, D, pl.C, pl.C);
-      // same operand planes as the forward prenet GEMM, so the recomputed ReLU gate is the forward's gate
-      g.planes = P_fwd; g.M = (int)Mt; g.N = (int)D; g.K = pl.C;
+      GemmProblem g = linear(c, "gemm.bwd.prenet_gate", pl.x0, Mt, pl.C, pl.C, pl.w_pre, D);
+      g.planes = P_fwd;   // same operand planes as the forward prenet GEMM, so the recomputed ReLU gate is the forward's gate
       g.epi.flags = EPI_BIAS | EPI_ACC_GATES_AUX | EPI_COLSUM;
       g.epi.colsum = gr.prenet_b;
       g.epi.bias = w.prenet_b; g.epi.drop = drop_pe; g.epi.drop_site = 0;
       c.res(g.epi, pl.dh_a, D);
       c.out(g.epi, pl.dh_b, 0, D);
-      SPK_TRY(run(g));
+      SPK_TRY(c.run(g));
     }
   }
-  SPK_TRY(wgrad(c, pl.dh_b, D, pl.x0, pl.C, gr.prenet_w, "gemm.bwd.prenet_wgrad", gs + 1));
+  SPK_TRY(wgrad(c, "gemm.bwd.prenet_wgrad", Mt, pl.dh_b, D, pl.x0, pl.C, pl.C, gr.prenet_w));
   return 0;
 }
 

@@ -1087,19 +1087,23 @@ int encode_map_4d(CUtensorMap* map, const void* base, const int64_t dims[4], con
   return 0;
 }
 
-// Opt in to the dynamic shared memory size and make the kernel resident (CUDA loads kernels lazily: a first launch of
-// a new instantiation inside a timed region -- a new frame length picks another BLOCK_N -- would pay for the load).
-template <bool A_MN, bool B_MN, int PLANES, int BLOCK_N>
-static int configure() {
-  using Cfg = TileCfg<PLANES, BLOCK_N>;
-  auto kern = gemm_tc_kernel<A_MN, B_MN, PLANES, BLOCK_N>;
-  SPK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+// Opt in to the kernel's dynamic shared memory size and check its register count (per device: callers run it under a
+// PerDeviceOnce).
+template <class Kern>
+static int configure_kernel(Kern kern, int smem) {
+  SPK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   cudaFuncAttributes fa;
   SPK_CUDA(cudaFuncGetAttributes(&fa, kern));
   // setmaxnreg re-partitions the launch allocation; another launch register count would dead-lock the epilogue warps
   SPK_CHECK(fa.numRegs == LAUNCH_REGS, "gemm kernel was built with %d registers/thread, expected %d", fa.numRegs,
             LAUNCH_REGS);
   return 0;
+}
+// The single-CTA kernels are configured up front (CUDA loads kernels lazily: a first launch of a new instantiation
+// inside a timed region -- a new frame length picks another BLOCK_N -- would pay for the load).
+template <bool A_MN, bool B_MN, int PLANES, int BLOCK_N>
+static int configure() {
+  return configure_kernel(gemm_tc_kernel<A_MN, B_MN, PLANES, BLOCK_N>, TileCfg<PLANES, BLOCK_N>::SMEM_BYTES);
 }
 template <bool A_MN, bool B_MN, int PLANES>
 static int configure_bn() {
@@ -1161,13 +1165,7 @@ static int launch_ln(const GemmKernelArgs& args, int grid, cudaStream_t stream) 
   using Cfg = TileCfg<PLANES, 256>;
   auto kern = gemm_tc_kernel<false, false, PLANES, 256, true>;
   static PerDeviceOnce once;
-  SPK_TRY(once.run([&]() -> int {
-    SPK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-    cudaFuncAttributes fa;
-    SPK_CUDA(cudaFuncGetAttributes(&fa, kern));
-    SPK_CHECK(fa.numRegs == LAUNCH_REGS, "gemm LN kernel was built with %d registers/thread, expected %d", fa.numRegs, LAUNCH_REGS);
-    return 0;
-  }));
+  SPK_TRY(once.run([&]() -> int { return configure_kernel(kern, Cfg::SMEM_BYTES); }));
   return launch_gemm_kernel(kern, grid, Cfg::SMEM_BYTES, stream, args);
 }
 
@@ -1186,14 +1184,7 @@ static int launch_pair(const GemmKernelArgs& args, int pairs, cudaStream_t strea
   using Cfg = PairCfg<PLANES, BLOCK_N>;
   auto kern = gemm_pair_kernel<B_MN, PLANES, BLOCK_N, LN>;
   static PerDeviceOnce once;
-  SPK_TRY(once.run([&]() -> int {
-    SPK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-    cudaFuncAttributes fa;
-    SPK_CUDA(cudaFuncGetAttributes(&fa, kern));
-    SPK_CHECK(fa.numRegs == LAUNCH_REGS, "gemm pair kernel was built with %d registers/thread, expected %d", fa.numRegs,
-              LAUNCH_REGS);
-    return 0;
-  }));
+  SPK_TRY(once.run([&]() -> int { return configure_kernel(kern, Cfg::SMEM_BYTES); }));
   return launch_gemm_kernel(kern, 2 * pairs, Cfg::SMEM_BYTES, stream, args);   // __cluster_dims__(2,1,1)
 }
 
@@ -1255,55 +1246,23 @@ int gemm_run(const GemmProblem& p, cudaStream_t stream) {
   const bool ln_pair = (p.epi.flags & EPI_LN) && p.planes == 2 && p.M > 2048 && g_cta_pairs;
   if ((p.epi.flags & EPI_LN) && !ln_pair) req_bn = 256;      // the fused LayerNorm runs in its own instantiations
 
-  // CTA-pair path: K-major A, two or three planes, no split-K, 256-wide N tiles
-  if (g_cta_pairs && !p.a_mn && p.planes >= 2 && p.ksplit <= 1 && req_bn == 0 && p.N % 128 == 0 && p.M >= 256) {
-    constexpr int BN = 256;
-    GemmKernelArgs a;
-    memset(&a, 0, sizeof(a));
-    for (int pl = 0; pl < p.planes; ++pl) {
-      SPK_TRY(make_map(&a.a_map[pl], p.A, pl, p.nb0, p.nb1, BLOCK_M));
-      SPK_TRY(make_map(&a.b_map[pl], p.B, pl, p.nb0, p.nb1, p.b_mn ? BLOCK_K : BN / 2));
-    }
-    a.M = p.M; a.N = p.N; a.K = p.K;
-    a.tiles_m = (p.M + 2 * BLOCK_M - 1) / (2 * BLOCK_M);
-    a.tiles_n = (p.N + BN - 1) / BN;
-    a.nb0 = p.nb0; a.nb1 = p.nb1;
-    a.kb_total = (p.K + BLOCK_K - 1) / BLOCK_K;
-    a.kb_per_split = a.kb_total; a.ksplit = 1;
-    a.a_batched = (p.A.sb0 != 0 || p.A.sb1 != 0);
-    a.b_batched = (p.B.sb0 != 0 || p.B.sb1 != 0);
-    a.epi = p.epi;
-    const long long total = 1LL * a.nb0 * a.nb1 * a.tiles_m * a.tiles_n;
-    SPK_CHECK(total < (1LL << 30), "gemm: too many tiles");
-    const int max_pairs = device_sm_count() / 2;
-    const int pairs = static_cast<int>(total < max_pairs ? total : max_pairs);
-    const double nb = 1.0 * p.nb0 * p.nb1, esz = 2.0 * p.planes;
-    const double out_b = (p.epi.flags & (EPI_OUT_F32 | EPI_OUT_ATOMIC)) ? 4.0 : esz;
-    double bytes = nb * (1.0 * p.M * p.K * esz + 1.0 * p.M * p.N * out_b) + (a.b_batched ? nb : 1.0) * p.N * p.K * esz;
-    if (p.epi.flags & (EPI_RES | EPI_ACC_GATES_AUX)) bytes += nb * p.M * p.N * 2.0 * p.epi.res_planes;
-    if (p.epi.flags & EPI_GATE_POS) bytes += nb * p.M * p.N * 2.0 * p.epi.gate_planes;
-    ProfScope prof(p.tag, 2.0 * nb * p.M * p.N * p.K, bytes, stream);
-    if (p.epi.flags & EPI_LN) return launch_pair<false, 2, BN, true>(a, pairs, stream);
-    if (p.planes == 3) {
-      if (p.b_mn) return launch_pair<true, 3, BN>(a, pairs, stream);
-      return launch_pair<false, 3, BN>(a, pairs, stream);
-    }
-    if (p.b_mn) return launch_pair<true, 2, BN>(a, pairs, stream);
-    return launch_pair<false, 2, BN>(a, pairs, stream);
-  }
-
-  int bn = req_bn;
+  // CTA-pair path: K-major A, two or three planes, no split-K, 256-wide N tiles (128 columns of B per CTA)
+  constexpr int PAIR_BN = 256;
+  const bool pair =
+      g_cta_pairs && !p.a_mn && p.planes >= 2 && p.ksplit <= 1 && req_bn == 0 && p.N % 128 == 0 && p.M >= 256;
+  int bn = pair ? PAIR_BN : req_bn;
   if (bn == 0) bn = p.N <= 64 ? 64 : (p.N <= 128 ? 128 : (p.N <= 192 ? 192 : 256));
-  if (p.planes == 3 && bn > 128) bn = 128;
+  if (!pair && p.planes == 3 && bn > 128) bn = 128;
+  const int tile_m = pair ? 2 * BLOCK_M : BLOCK_M;
 
   GemmKernelArgs a;
   memset(&a, 0, sizeof(a));
   for (int pl = 0; pl < p.planes; ++pl) {
     SPK_TRY(make_map(&a.a_map[pl], p.A, pl, p.nb0, p.nb1, p.a_mn ? BLOCK_K : BLOCK_M));
-    SPK_TRY(make_map(&a.b_map[pl], p.B, pl, p.nb0, p.nb1, p.b_mn ? BLOCK_K : bn));
+    SPK_TRY(make_map(&a.b_map[pl], p.B, pl, p.nb0, p.nb1, p.b_mn ? BLOCK_K : (pair ? bn / 2 : bn)));
   }
   a.M = p.M; a.N = p.N; a.K = p.K;
-  a.tiles_m = (p.M + BLOCK_M - 1) / BLOCK_M;
+  a.tiles_m = (p.M + tile_m - 1) / tile_m;
   a.tiles_n = (p.N + bn - 1) / bn;
   a.nb0 = p.nb0; a.nb1 = p.nb1;
   a.kb_total = (p.K + BLOCK_K - 1) / BLOCK_K;
@@ -1316,8 +1275,6 @@ int gemm_run(const GemmProblem& p, cudaStream_t stream) {
   a.epi = p.epi;
   const long long total = 1LL * a.nb0 * a.nb1 * a.ksplit * a.tiles_m * a.tiles_n;
   SPK_CHECK(total < (1LL << 30), "gemm: too many tiles");
-  const int sms = device_sm_count();
-  const int grid = static_cast<int>(total < sms ? total : sms);
   const double nb = 1.0 * p.nb0 * p.nb1;
   const double esz = 2.0 * p.planes;
   const double out_b = (p.epi.flags & (EPI_OUT_F32 | EPI_OUT_ATOMIC)) ? 4.0 : esz;
@@ -1325,7 +1282,21 @@ int gemm_run(const GemmProblem& p, cudaStream_t stream) {
                  (a.b_batched ? nb : 1.0) * p.N * p.K * esz;
   if (p.epi.flags & (EPI_RES | EPI_ACC_GATES_AUX)) bytes += nb * p.M * p.N * 2.0 * p.epi.res_planes;
   if (p.epi.flags & EPI_GATE_POS) bytes += nb * p.M * p.N * 2.0 * p.epi.gate_planes;
+  const int sms = device_sm_count();
   ProfScope prof(p.tag, 2.0 * nb * p.M * p.N * p.K, bytes, stream);
+
+  if (pair) {
+    const int max_pairs = sms / 2;
+    const int pairs = static_cast<int>(total < max_pairs ? total : max_pairs);
+    if (p.epi.flags & EPI_LN) return launch_pair<false, 2, PAIR_BN, true>(a, pairs, stream);
+    if (p.planes == 3) {
+      if (p.b_mn) return launch_pair<true, 3, PAIR_BN>(a, pairs, stream);
+      return launch_pair<false, 3, PAIR_BN>(a, pairs, stream);
+    }
+    if (p.b_mn) return launch_pair<true, 2, PAIR_BN>(a, pairs, stream);
+    return launch_pair<false, 2, PAIR_BN>(a, pairs, stream);
+  }
+  const int grid = static_cast<int>(total < sms ? total : sms);
   if (p.epi.flags & EPI_LN) return p.planes == 1 ? launch_ln<1>(a, grid, stream) : launch_ln<2>(a, grid, stream);
   if (p.planes == 1) return launch_major<1>(p.a_mn, p.b_mn, bn, a, grid, stream);
   if (p.planes == 2) return launch_major<2>(p.a_mn, p.b_mn, bn, a, grid, stream);
