@@ -8,16 +8,16 @@
 // * one elected thread issues tcgen05.mma (UMMA 128 x BLOCK_N x 16, fp16 in, fp32 accumulate in
 //   TMEM); with two planes it issues Ah*Bh + Ah*Bl + Al*Bh into the same accumulator, with three
 //   planes the six products down to 2^-16 (fp32-equivalent operands);
-// * the accumulator is double-buffered in TMEM so the 8 epilogue warps (tcgen05.ld -> registers
+// * the accumulator is double-buffered in TMEM so the 12 epilogue warps (tcgen05.ld -> registers
 //   -> fused bias / ReLU / positional term / dropout / residual / gate -> global) drain tile i
 //   while the MMA warp works on tile i+1;
 // * grid = min(#tiles, #SMs); tiles are assigned round-robin (persistent CTAs);
 // * multi-plane problems with a K-major A and M >= 256 run on CTA pairs instead (gemm_pair_kernel below:
 //   tcgen05.mma.cta_group::2, 256 x 256 tiles, each CTA stages half of B).
 //
-// Warp roles (384 threads): 0 = TMA producer, 1 = MMA issuer, 2 = TMEM allocator, 3 = idle,
-// 4..11 = epilogue (warp w owns TMEM lanes 32*(w%4) .. +31 == accumulator rows; warps 4-7 take the even
-// 32-column chunks of a tile, warps 8-11 the odd ones).
+// Warp roles (512 threads): 0 = TMA producer, 1 = MMA issuer, 2 = TMEM allocator, 3 = idle,
+// 4..15 = epilogue (warp w owns TMEM lanes 32*(w%4) .. +31 == accumulator rows; the three warps of a lane quarter
+// take its 32-column chunks round-robin: warp w the chunks c with c % 3 == (w-4) / 4).
 #include "gemm.h"
 #include "ptx.cuh"
 
@@ -53,7 +53,8 @@ struct GemmKernelArgs {
 template <int PLANES, int BLOCK_N>
 struct TileCfg {
   static constexpr int A_BYTES = BLOCK_M * BLOCK_K * 2;
-  static constexpr int B_BYTES = BLOCK_N * BLOCK_K * 2;
+  static constexpr int B_ROWS = BLOCK_N;
+  static constexpr int B_BYTES = B_ROWS * BLOCK_K * 2;
   static constexpr int STAGE_BYTES = PLANES * (A_BYTES + B_BYTES);
   static constexpr int RAW_STAGES = (SMEM_LIMIT - 1024 - BAR_BYTES - EPI_SMEM) / STAGE_BYTES;
   static constexpr int STAGES = RAW_STAGES > 8 ? 8 : RAW_STAGES;
@@ -532,6 +533,161 @@ __device__ __forceinline__ void epilogue_tile(const GemmEpilogue& e, uint32_t st
 }
 
 // ------------------------------------------------------------------------------------------------
+// Pieces shared by the single-CTA and the CTA-pair kernel.
+
+// Tiles are numbered N tile fastest, then M tile, K split, batch index i0, batch index i1.
+struct TileIdx {
+  int tn, tm;
+  int batch, i0, i1;          // batch = i0 + nb0 * i1
+  int kb_begin, kb_end;       // the tile's k-blocks (its K split)
+};
+__device__ __forceinline__ int num_tiles(const GemmKernelArgs& a) {
+  return a.nb0 * a.nb1 * a.ksplit * a.tiles_m * a.tiles_n;
+}
+__device__ __forceinline__ TileIdx decode_tile(const GemmKernelArgs& a, int tile) {
+  TileIdx t;
+  const int mn_tiles = a.tiles_m * a.tiles_n;
+  const int outer = tile / mn_tiles;                  // the k-block range needs only this division and the next
+  const int ks = outer % a.ksplit;
+  const int mn = tile - outer * mn_tiles;
+  t.tn = mn % a.tiles_n; t.tm = mn / a.tiles_n;
+  t.batch = outer / a.ksplit;
+  t.i0 = t.batch % a.nb0; t.i1 = t.batch / a.nb0;
+  t.kb_begin = ks * a.kb_per_split;
+  t.kb_end = min(t.kb_begin + a.kb_per_split, a.kb_total);
+  return t;
+}
+
+// An operand ring stage (Cfg = TileCfg or PairCfg) holds the PLANES planes of A (BLOCK_M rows each, Cfg::A_BYTES apart
+// from sa on), then those of B (Cfg::B_ROWS rows each, Cfg::B_BYTES apart from sb on).
+
+// TMA load of k-block kb of one operand plane, ROWS rows from `row` on.  K-major: one box of BLOCK_K x ROWS.  MN-major:
+// BLOCK_K rows of the stored [K, rows] tensor, in 64-element-wide chunks (one 128-byte swizzle row each).
+template <bool MN, int ROWS>
+__device__ __forceinline__ void tma_load_operand(uint32_t dst, const CUtensorMap* map, uint32_t bar, int kb, int row,
+                                                 int i0, int i1) {
+  if (!MN) {
+    tma_load_4d(dst, map, bar, kb * BLOCK_K, row, i0, i1);
+  } else {
+#pragma unroll
+    for (int c = 0; c < ROWS / 64; ++c) tma_load_4d(dst + c * (BLOCK_K * 128), map, bar, row + c * 64, kb * BLOCK_K, i0, i1);
+  }
+}
+
+// Every plane of k-block kb into one stage: A rows from a_row, B rows from b_row, batch (i0, i1) of a batched operand.
+template <class Cfg, int PLANES, bool A_MN, bool B_MN>
+__device__ __forceinline__ void load_stage(const GemmKernelArgs& args, uint32_t sa, uint32_t sb, uint32_t bar, int kb,
+                                           int a_row, int b_row, int i0, int i1) {
+  const int a0 = args.a_batched ? i0 : 0, a1 = args.a_batched ? i1 : 0;
+  const int b0 = args.b_batched ? i0 : 0, b1 = args.b_batched ? i1 : 0;
+#pragma unroll
+  for (int p = 0; p < PLANES; ++p) {
+    tma_load_operand<A_MN, BLOCK_M>(sa + p * Cfg::A_BYTES, &args.a_map[p], bar, kb, a_row, a0, a1);
+    tma_load_operand<B_MN, Cfg::B_ROWS>(sb + p * Cfg::B_BYTES, &args.b_map[p], bar, kb, b_row, b0, b1);
+  }
+}
+
+// Plane products of one k-step, smallest terms first (plane 0 = hi, 1 = mid/lo, 2 = lo):
+//   2 planes: a1*b0, a0*b1, a0*b0           3 planes: a1*b1, a0*b2, a2*b0, a0*b1, a1*b0, a0*b0
+// Both kernels add them in this order, so a CTA-pair tile and a single-CTA tile agree bit for bit.
+__host__ __device__ constexpr int plane_products(int planes) { return planes == 1 ? 1 : (planes == 2 ? 3 : 6); }
+__device__ __forceinline__ int2 plane_product(int planes, int i) {   // (plane of A, plane of B) of product i
+  constexpr int PA2[3] = {1, 0, 0}, PB2[3] = {0, 1, 0};
+  constexpr int PA3[6] = {1, 0, 2, 0, 1, 0}, PB3[6] = {1, 2, 0, 1, 0, 0};
+  if (planes == 1) return make_int2(0, 0);
+  return planes == 2 ? make_int2(PA2[i], PB2[i]) : make_int2(PA3[i], PB3[i]);
+}
+
+// The MMAs of one stage into the accumulator at d_tmem; the first MMA of a tile (accumulate == 0) overwrites it.
+// PAIR: tcgen05.mma.cta_group::2, issued by the leader of a CTA pair for both CTAs.
+template <class Cfg, int PLANES, bool A_MN, bool B_MN, bool PAIR>
+__device__ __forceinline__ void mma_stage(uint32_t sa, uint32_t sb, uint32_t d_tmem, uint32_t idesc, uint32_t& accumulate) {
+#pragma unroll
+  for (int i = 0; i < plane_products(PLANES); ++i) {
+    const int2 pp = plane_product(PLANES, i);
+    const uint32_t a_base = sa + pp.x * Cfg::A_BYTES, b_base = sb + pp.y * Cfg::B_BYTES;
+#pragma unroll
+    for (int k = 0; k < BLOCK_K / UMMA_K; ++k) {
+      const uint64_t da = A_MN ? umma_smem_desc(a_base + k * (UMMA_K * 128), BLOCK_K * 128, 1024)
+                               : umma_smem_desc(a_base + k * (UMMA_K * 2), 16, 1024);
+      const uint64_t db = B_MN ? umma_smem_desc(b_base + k * (UMMA_K * 128), BLOCK_K * 128, 1024)
+                               : umma_smem_desc(b_base + k * (UMMA_K * 2), 16, 1024);
+      if constexpr (PAIR) umma_f16_pair(d_tmem, da, db, idesc, accumulate);
+      else umma_f16(d_tmem, da, db, idesc, accumulate);
+      accumulate = 1;
+    }
+  }
+}
+
+// The epilogue warps (4 .. 15) of either kernel: tiles first_tile, first_tile + tile_stride, ...  A tile has tile_rows
+// accumulator rows; this CTA holds BLOCK_M of them from row_off on.  full_bar / drained_bar: the CTA's barriers
+// "accumulator a complete" and "accumulator a drained" (32 * NUM_EPI_WARPS arrivals), a = 0 at the address given,
+// a = 1 eight bytes on.  The wait for accumulator a reports wait_code + a to the watchdog.
+template <int PLANES, int BLOCK_N, bool LN>
+__device__ __forceinline__ void epilogue_role(const GemmKernelArgs& args, int warp, int lane, uint32_t epi_stage_base,
+                                              uint32_t tmem_base, int first_tile, int tile_stride, int tile_rows,
+                                              int row_off, uint32_t full_bar, uint32_t drained_bar, uint32_t wait_code) {
+  setmaxnreg_inc<EPI_REGS>();
+  const int w = (warp - 4) & 3;          // TMEM lane quarter (warp % 4) -> accumulator rows 32w .. 32w+31
+  const int cgroup = (warp - 4) >> 2;    // this warp handles the 32-column chunks with c % EPI_CG == cgroup
+  const GemmEpilogue& e = args.epi;
+  const float pe_alpha = (e.flags & EPI_PE) ? __ldg(e.pe_alpha) : 0.f;
+  const float alpha = e.alpha * (e.alpha_ptr != nullptr ? __ldg(e.alpha_ptr) : 1.f);
+  const float cs_scale = e.colsum_scale_ptr != nullptr ? __ldg(e.colsum_scale_ptr) : 1.f;
+  const uint32_t stage_buf = epi_stage_base + (warp - 4) * (EPI_STAGE_BYTES + EPI_BIAS_BYTES);
+  const uint32_t bias_buf = stage_buf + EPI_STAGE_BYTES;
+  const int total_tiles = num_tiles(args);
+  int it = 0;
+  for (int tile = first_tile; tile < total_tiles; tile += tile_stride, ++it) {
+    const TileIdx t = decode_tile(args, tile);
+    const int acc = it & 1;
+    const uint32_t acc_phase = (it >> 1) & 1;
+    if (e.flags & EPI_BIAS) {   // bias of this warp's chunks (cgroup + EPI_CG j) -> shared memory, before the accumulator is due
+      const int j = lane >> 3;
+      const int cloc = (cgroup + j * EPI_CG) * 32;
+      const int col = t.tn * BLOCK_N + cloc + (lane & 7) * 4;
+      float4 b = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (cloc < BLOCK_N && col < args.N) b = __ldg(reinterpret_cast<const float4*>(e.bias + col));
+      asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(bias_buf + lane * 16), "f"(b.x), "f"(b.y), "f"(b.z), "f"(b.w) : "memory");
+      __syncwarp();
+    }
+    mbar_wait(full_bar + 8u * acc, acc_phase, wait_code + acc);
+    tc_fence_after();
+    const int64_t row0 = static_cast<int64_t>(t.tm) * tile_rows + row_off + w * 32;
+    const int64_t out_boff = t.i0 * e.out_sb0 + t.i1 * e.out_sb1;
+    const int64_t res_boff = t.i0 * e.res_sb0 + t.i1 * e.res_sb1;
+    const uint32_t t_row = tmem_base + (static_cast<uint32_t>(w * 32) << 16) + acc * BLOCK_N;
+    const int64_t cs_boff = t.i0 * e.colsum_sb0;
+    if constexpr (LN) {
+      if (row0 < args.M)
+        ln_epilogue_tile<BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, w, t_row, args.M, args.N, row0, t.batch, out_boff,
+                                  res_boff, alpha);
+    } else
+    if (row0 < args.M) {   // warp-uniform
+      constexpr uint32_t CT_LEAN = EPI_BIAS | EPI_RELU | EPI_OUT_F32;
+      // the bit-mask classes only exist in the multi-plane kernels: the one-plane (inference) kernels stay small
+      constexpr uint32_t CT_FWD = CT_LEAN | EPI_PE | EPI_DROPOUT | EPI_RES | (PLANES >= 2 ? EPI_EMIT_BITS : 0u);
+      constexpr uint32_t CT_BWD = EPI_GATE_BITS | EPI_COLSUM | EPI_RES | EPI_OUT_F32;   // data gradients
+      if ((e.flags & ~CT_LEAN) == 0)
+        epilogue_tile<CT_LEAN, BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, t_row, args.M, args.N, row0, t.batch, out_boff,
+                                        res_boff, cs_boff, t.tn, pe_alpha, alpha, cs_scale);
+      else if ((e.flags & ~CT_FWD) == 0)
+        epilogue_tile<CT_FWD, BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, t_row, args.M, args.N, row0, t.batch, out_boff,
+                                       res_boff, cs_boff, t.tn, pe_alpha, alpha, cs_scale);
+      else if (PLANES >= 2 && (e.flags & ~CT_BWD) == 0)
+        epilogue_tile<(PLANES >= 2 ? CT_BWD : 0xFFFFFFFFu), BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, t_row, args.M, args.N,
+                                                                     row0, t.batch, out_boff, res_boff, cs_boff, t.tn, pe_alpha,
+                                                                     alpha, cs_scale);
+      else
+        epilogue_tile<0xFFFFFFFFu, BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, t_row, args.M, args.N, row0, t.batch, out_boff,
+                                            res_boff, cs_boff, t.tn, pe_alpha, alpha, cs_scale);
+    }
+    tc_fence_before();
+    mbar_arrive(drained_bar + 8u * acc);
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
 // LN = true: the instantiation whose ONLY epilogue is the fused LayerNorm (EPI_LN); it is a kernel of its own so that the
 // extra code and registers do not touch the other epilogues (built into the common kernel it cost them 2 %).
 template <bool A_MN, bool B_MN, int PLANES, int BLOCK_N, bool LN = false>
@@ -551,8 +707,8 @@ __global__ void __launch_bounds__(128 + 32 * NUM_EPI_WARPS, 1) gemm_tc_kernel(co
   auto tempty_bar = [&](int a) { return bar_base + 8u * (2 * STAGES + 2 + a); };
   const uint32_t tmem_slot = bar_base + 8u * (2 * STAGES + 4);
   const uint32_t epi_stage_base = bar_base + BAR_BYTES;
-  auto sA = [&](int s, int p) { return smem_base + s * Cfg::STAGE_BYTES + p * Cfg::A_BYTES; };
-  auto sB = [&](int s, int p) { return smem_base + s * Cfg::STAGE_BYTES + PLANES * Cfg::A_BYTES + p * Cfg::B_BYTES; };
+  auto sA = [&](int s) { return smem_base + s * Cfg::STAGE_BYTES; };   // stage s: planes of A, then planes of B
+  auto sB = [&](int s) { return sA(s) + PLANES * Cfg::A_BYTES; };
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -586,8 +742,7 @@ __global__ void __launch_bounds__(128 + 32 * NUM_EPI_WARPS, 1) gemm_tc_kernel(co
   uint32_t tmem_base;
   asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
 
-  const int tiles_per_batch = args.ksplit * args.tiles_m * args.tiles_n;
-  const int total_tiles = args.nb0 * args.nb1 * tiles_per_batch;
+  const int total_tiles = num_tiles(args);
 
   if (warp < 4) {
     setmaxnreg_dec<CTRL_REGS>();
@@ -597,37 +752,12 @@ __global__ void __launch_bounds__(128 + 32 * NUM_EPI_WARPS, 1) gemm_tc_kernel(co
         int stage = 0;
         uint32_t phase = 0;
         for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-          int t = tile;
-          const int tn = t % args.tiles_n; t /= args.tiles_n;
-          const int tm = t % args.tiles_m; t /= args.tiles_m;
-          const int ks = t % args.ksplit;  t /= args.ksplit;
-          const int i0 = t % args.nb0, i1 = t / args.nb0;
-          const int a0 = args.a_batched ? i0 : 0, a1 = args.a_batched ? i1 : 0;
-          const int b0 = args.b_batched ? i0 : 0, b1 = args.b_batched ? i1 : 0;
-          const int kb_begin = ks * args.kb_per_split;
-          const int kb_end = min(kb_begin + args.kb_per_split, args.kb_total);
-          for (int kb = kb_begin; kb < kb_end; ++kb) {
+          const TileIdx t = decode_tile(args, tile);
+          for (int kb = t.kb_begin; kb < t.kb_end; ++kb) {
             mbar_wait(empty_bar(stage), phase ^ 1u, 0x100u + stage);
             mbar_arrive_expect_tx(full_bar(stage), Cfg::STAGE_BYTES);
-#pragma unroll
-            for (int p = 0; p < PLANES; ++p) {
-              if (!A_MN) {
-                tma_load_4d(sA(stage, p), &args.a_map[p], full_bar(stage), kb * BLOCK_K, tm * BLOCK_M, a0, a1);
-              } else {
-#pragma unroll
-                for (int c = 0; c < BLOCK_M / 64; ++c)
-                  tma_load_4d(sA(stage, p) + c * (BLOCK_K * 128), &args.a_map[p], full_bar(stage),
-                              tm * BLOCK_M + c * 64, kb * BLOCK_K, a0, a1);
-              }
-              if (!B_MN) {
-                tma_load_4d(sB(stage, p), &args.b_map[p], full_bar(stage), kb * BLOCK_K, tn * BLOCK_N, b0, b1);
-              } else {
-#pragma unroll
-                for (int c = 0; c < BLOCK_N / 64; ++c)
-                  tma_load_4d(sB(stage, p) + c * (BLOCK_K * 128), &args.b_map[p], full_bar(stage),
-                              tn * BLOCK_N + c * 64, kb * BLOCK_K, b0, b1);
-              }
-            }
+            load_stage<Cfg, PLANES, A_MN, B_MN>(args, sA(stage), sB(stage), full_bar(stage), kb, t.tm * BLOCK_M,
+                                                t.tn * BLOCK_N, t.i0, t.i1);
             if (++stage == STAGES) { stage = 0; phase ^= 1u; }
           }
         }
@@ -639,38 +769,17 @@ __global__ void __launch_bounds__(128 + 32 * NUM_EPI_WARPS, 1) gemm_tc_kernel(co
         uint32_t phase = 0;
         int it = 0;
         for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++it) {
-          int t = tile / (args.tiles_n * args.tiles_m);
-          const int ks = t % args.ksplit;
-          const int kb_begin = ks * args.kb_per_split;
-          const int kb_end = min(kb_begin + args.kb_per_split, args.kb_total);
+          const TileIdx t = decode_tile(args, tile);
           const int acc = it & 1;
           const uint32_t acc_phase = (it >> 1) & 1;
           mbar_wait(tempty_bar(acc), acc_phase ^ 1u, 0x200u + acc);
           tc_fence_after();
           const uint32_t d_tmem = tmem_base + acc * BLOCK_N;
           uint32_t accumulate = 0;
-          for (int kb = kb_begin; kb < kb_end; ++kb) {
+          for (int kb = t.kb_begin; kb < t.kb_end; ++kb) {
             mbar_wait(full_bar(stage), phase, 0x300u + stage);
             tc_fence_after();
-#pragma unroll
-            for (int combo = 0; combo < (PLANES == 1 ? 1 : (PLANES == 2 ? 3 : 6)); ++combo) {
-              // plane products, smallest terms first (plane 0 = hi, 1 = mid/lo, 2 = lo):
-              //   2 planes: a1*b0, a0*b1, a0*b0           3 planes: a1*b1, a0*b2, a2*b0, a0*b1, a1*b0, a0*b0
-              constexpr int PA2[3] = {1, 0, 0}, PB2[3] = {0, 1, 0};
-              constexpr int PA3[6] = {1, 0, 2, 0, 1, 0}, PB3[6] = {1, 2, 0, 1, 0, 0};
-              const int pa = (PLANES == 1) ? 0 : (PLANES == 2 ? PA2[combo % 3] : PA3[combo]);
-              const int pb = (PLANES == 1) ? 0 : (PLANES == 2 ? PB2[combo % 3] : PB3[combo]);
-              const uint32_t a_base = sA(stage, pa), b_base = sB(stage, pb);
-#pragma unroll
-              for (int k = 0; k < BLOCK_K / UMMA_K; ++k) {
-                const uint64_t da = A_MN ? umma_smem_desc(a_base + k * (UMMA_K * 128), BLOCK_K * 128, 1024)
-                                         : umma_smem_desc(a_base + k * (UMMA_K * 2), 16, 1024);
-                const uint64_t db = B_MN ? umma_smem_desc(b_base + k * (UMMA_K * 128), BLOCK_K * 128, 1024)
-                                         : umma_smem_desc(b_base + k * (UMMA_K * 2), 16, 1024);
-                umma_f16(d_tmem, da, db, IDESC, accumulate);
-                accumulate = 1;
-              }
-            }
+            mma_stage<Cfg, PLANES, A_MN, B_MN, false>(sA(stage), sB(stage), d_tmem, IDESC, accumulate);
             umma_commit(empty_bar(stage));        // frees the smem slot when these MMAs retire
             if (++stage == STAGES) { stage = 0; phase ^= 1u; }
           }
@@ -680,66 +789,8 @@ __global__ void __launch_bounds__(128 + 32 * NUM_EPI_WARPS, 1) gemm_tc_kernel(co
     }
   } else {
     // ===================================================================== epilogue
-    setmaxnreg_inc<EPI_REGS>();
-    const int w = (warp - 4) & 3;          // TMEM lane quarter (warp % 4) -> accumulator rows 32w .. 32w+31
-    const int cgroup = (warp - 4) >> 2;    // this warp handles the 32-column chunks with c % EPI_CG == cgroup
-    const GemmEpilogue& e = args.epi;
-    const float pe_alpha = (e.flags & EPI_PE) ? __ldg(e.pe_alpha) : 0.f;
-    const float alpha = e.alpha * (e.alpha_ptr != nullptr ? __ldg(e.alpha_ptr) : 1.f);
-    const float cs_scale = e.colsum_scale_ptr != nullptr ? __ldg(e.colsum_scale_ptr) : 1.f;
-    const uint32_t stage_buf = epi_stage_base + (warp - 4) * (EPI_STAGE_BYTES + EPI_BIAS_BYTES);
-    const uint32_t bias_buf = stage_buf + EPI_STAGE_BYTES;
-    int it = 0;
-    for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++it) {
-      int t = tile;
-      const int tn = t % args.tiles_n; t /= args.tiles_n;
-      const int tm = t % args.tiles_m; t /= args.tiles_m;
-      t /= args.ksplit;
-      const int i0 = t % args.nb0, i1 = t / args.nb0;
-      const int acc = it & 1;
-      const uint32_t acc_phase = (it >> 1) & 1;
-      if (e.flags & EPI_BIAS) {   // bias of this warp's chunks (cgroup + EPI_CG j) -> shared memory, before the accumulator is due
-        const int j = lane >> 3;
-        const int cloc = (cgroup + j * EPI_CG) * 32;
-        const int col = tn * BLOCK_N + cloc + (lane & 7) * 4;
-        float4 b = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (cloc < BLOCK_N && col < args.N) b = __ldg(reinterpret_cast<const float4*>(e.bias + col));
-        asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(bias_buf + lane * 16), "f"(b.x), "f"(b.y), "f"(b.z), "f"(b.w) : "memory");
-        __syncwarp();
-      }
-      mbar_wait(tfull_bar(acc), acc_phase, 0x400u + acc);
-      tc_fence_after();
-      const int64_t row0 = static_cast<int64_t>(tm) * BLOCK_M + w * 32;
-      const int64_t out_boff = i0 * e.out_sb0 + i1 * e.out_sb1;
-      const int64_t res_boff = i0 * e.res_sb0 + i1 * e.res_sb1;
-      const uint32_t t_row = tmem_base + (static_cast<uint32_t>(w * 32) << 16) + acc * BLOCK_N;
-      const int64_t cs_boff = i0 * e.colsum_sb0;
-      if constexpr (LN) {
-        if (row0 < args.M)
-          ln_epilogue_tile<BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, w, t_row, args.M, args.N, row0, t, out_boff, res_boff,
-                                    alpha);
-      } else
-      if (row0 < args.M) {   // warp-uniform
-        constexpr uint32_t CT_LEAN = EPI_BIAS | EPI_RELU | EPI_OUT_F32;
-        // the bit-mask classes only exist in the multi-plane kernels: the one-plane (inference) kernels stay small
-        constexpr uint32_t CT_FWD = CT_LEAN | EPI_PE | EPI_DROPOUT | EPI_RES | (PLANES >= 2 ? EPI_EMIT_BITS : 0u);
-        constexpr uint32_t CT_BWD = EPI_GATE_BITS | EPI_COLSUM | EPI_RES | EPI_OUT_F32;   // data gradients
-        if ((e.flags & ~CT_LEAN) == 0)
-          epilogue_tile<CT_LEAN, BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, t_row, args.M, args.N, row0, t, out_boff, res_boff,
-                                          cs_boff, tn, pe_alpha, alpha, cs_scale);
-        else if ((e.flags & ~CT_FWD) == 0)
-          epilogue_tile<CT_FWD, BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, t_row, args.M, args.N, row0, t, out_boff, res_boff,
-                                         cs_boff, tn, pe_alpha, alpha, cs_scale);
-        else if (PLANES >= 2 && (e.flags & ~CT_BWD) == 0)
-          epilogue_tile<(PLANES >= 2 ? CT_BWD : 0xFFFFFFFFu), BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, t_row, args.M, args.N, row0,
-                                                                       t, out_boff, res_boff, cs_boff, tn, pe_alpha, alpha, cs_scale);
-        else
-          epilogue_tile<0xFFFFFFFFu, BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, t_row, args.M, args.N, row0, t, out_boff,
-                                              res_boff, cs_boff, tn, pe_alpha, alpha, cs_scale);
-      }
-      tc_fence_before();
-      mbar_arrive(tempty_bar(acc));
-    }
+    epilogue_role<PLANES, BLOCK_N, LN>(args, warp, lane, epi_stage_base, tmem_base, blockIdx.x, gridDim.x, BLOCK_M, 0,
+                                       tfull_bar(0), tempty_bar(0), 0x400u);
   }
 
   tc_fence_before();
@@ -761,13 +812,14 @@ __global__ void __launch_bounds__(128 + 32 * NUM_EPI_WARPS, 1) gemm_tc_kernel(co
 //   peer_full[s] leader only: the peer's stage s is loaded           (remote arrive by the peer's relay lane)
 //   empty[s]     both CTAs, signalled by the leader's commit (multicast)
 //   tfull[a]     both CTAs, leader's commit (multicast): accumulator a complete
-//   tlocal[a]    each CTA: its 256 epilogue threads have drained accumulator a (CTA-scope arrives: a cluster-scope
+//   tlocal[a]    each CTA: its 384 epilogue threads have drained accumulator a (CTA-scope arrives: a cluster-scope
 //                release from every epilogue thread would wait for its outstanding global stores)
 //   tempty[a]    leader only: one remote arrive per CTA, forwarded by the idle warp 3 once tlocal[a] completes
 template <int PLANES, int BLOCK_N>
 struct PairCfg {
   static constexpr int A_BYTES = BLOCK_M * BLOCK_K * 2;
-  static constexpr int B_BYTES = (BLOCK_N / 2) * BLOCK_K * 2;
+  static constexpr int B_ROWS = BLOCK_N / 2;
+  static constexpr int B_BYTES = B_ROWS * BLOCK_K * 2;
   static constexpr int STAGE_BYTES = PLANES * (A_BYTES + B_BYTES);
   static constexpr int RAW_STAGES = (SMEM_LIMIT - 1024 - BAR_BYTES - EPI_SMEM) / STAGE_BYTES;
   static constexpr int STAGES = RAW_STAGES > 6 ? 6 : RAW_STAGES;
@@ -783,7 +835,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * NUM_EPI_W
   pdl_trigger();   // the next kernel of the stream may start its prologue (ptx.cuh)
   using Cfg = PairCfg<PLANES, BLOCK_N>;
   constexpr int STAGES = Cfg::STAGES;
-  constexpr int HALF_N = BLOCK_N / 2;
   constexpr uint32_t IDESC = umma_idesc_f16(2 * BLOCK_M, BLOCK_N, false, B_MN);
 
   extern __shared__ uint8_t smem_raw[];
@@ -797,14 +848,16 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * NUM_EPI_W
   auto tlocal_bar = [&](int a) { return bar_base + 8u * (3 * STAGES + 4 + a); };
   const uint32_t tmem_slot = bar_base + 8u * (3 * STAGES + 6);
   const uint32_t epi_stage_base = bar_base + BAR_BYTES;
-  auto sA = [&](int s, int p) { return smem_base + s * Cfg::STAGE_BYTES + p * Cfg::A_BYTES; };
-  auto sB = [&](int s, int p) { return smem_base + s * Cfg::STAGE_BYTES + PLANES * Cfg::A_BYTES + p * Cfg::B_BYTES; };
+  auto sA = [&](int s) { return smem_base + s * Cfg::STAGE_BYTES; };   // stage s: planes of A, then planes of B
+  auto sB = [&](int s) { return sA(s) + PLANES * Cfg::A_BYTES; };
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();
-  const int pair = static_cast<int>(cluster_id_x());
-  const int npairs = static_cast<int>(cluster_count_x());
+  // This pair's tiles: pair_id(), + num_pairs(), ...  The two are read where used: kept in registers across all warp
+  // roles they cost spill slots (ptxas: 92 / 88 spill bytes instead of 120 / 132 at two planes).
+  auto pair_id = [] { return static_cast<int>(cluster_id_x()); };
+  auto num_pairs = [] { return static_cast<int>(cluster_count_x()); };
 
   if (warp == 0 && lane == 0) {
 #pragma unroll
@@ -838,8 +891,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * NUM_EPI_W
   uint32_t tmem_base;
   asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
 
-  const int tiles_per_batch = args.tiles_m * args.tiles_n;       // tiles_m counts 256-row tiles here
-  const int total_tiles = args.nb0 * args.nb1 * tiles_per_batch;
+  const int total_tiles = num_tiles(args);       // tiles_m counts 256-row tiles here
 
   if (warp < 4) {
     setmaxnreg_dec<CTRL_REGS>();
@@ -848,30 +900,14 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * NUM_EPI_W
       if (lane == 0) {
         int stage = 0;
         uint32_t phase = 0;
-        for (int tile = pair; tile < total_tiles; tile += npairs) {
-          int t = tile;
-          const int tn = t % args.tiles_n; t /= args.tiles_n;
-          const int tm = t % args.tiles_m; t /= args.tiles_m;
-          const int i0 = t % args.nb0, i1 = t / args.nb0;
-          const int a0 = args.a_batched ? i0 : 0, a1 = args.a_batched ? i1 : 0;
-          const int b0 = args.b_batched ? i0 : 0, b1 = args.b_batched ? i1 : 0;
-          const int arow = tm * 2 * BLOCK_M + static_cast<int>(rank) * BLOCK_M;
-          const int brow = tn * BLOCK_N + static_cast<int>(rank) * HALF_N;
-          for (int kb = 0; kb < args.kb_total; ++kb) {
+        for (int tile = pair_id(); tile < total_tiles; tile += num_pairs()) {
+          const TileIdx t = decode_tile(args, tile);
+          const int arow = t.tm * 2 * BLOCK_M + static_cast<int>(rank) * BLOCK_M;
+          const int brow = t.tn * BLOCK_N + static_cast<int>(rank) * Cfg::B_ROWS;
+          for (int kb = t.kb_begin; kb < t.kb_end; ++kb) {
             mbar_wait(empty_bar(stage), phase ^ 1u, 0x900u + stage);
             mbar_arrive_expect_tx(full_bar(stage), Cfg::STAGE_BYTES);
-#pragma unroll
-            for (int p = 0; p < PLANES; ++p) {
-              tma_load_4d(sA(stage, p), &args.a_map[p], full_bar(stage), kb * BLOCK_K, arow, a0, a1);
-              if (!B_MN) {
-                tma_load_4d(sB(stage, p), &args.b_map[p], full_bar(stage), kb * BLOCK_K, brow, b0, b1);
-              } else {
-#pragma unroll
-                for (int c = 0; c < HALF_N / 64; ++c)
-                  tma_load_4d(sB(stage, p) + c * (BLOCK_K * 128), &args.b_map[p], full_bar(stage), brow + c * 64,
-                              kb * BLOCK_K, b0, b1);
-              }
-            }
+            load_stage<Cfg, PLANES, false, B_MN>(args, sA(stage), sB(stage), full_bar(stage), kb, arow, brow, t.i0, t.i1);
             if (++stage == STAGES) { stage = 0; phase ^= 1u; }
           }
         }
@@ -882,8 +918,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * NUM_EPI_W
         uint32_t phase = 0;
         if (rank != 0) {
           // =================================================================== peer: relay "my stage is loaded"
-          for (int tile = pair; tile < total_tiles; tile += npairs) {
-            for (int kb = 0; kb < args.kb_total; ++kb) {
+          for (int tile = pair_id(); tile < total_tiles; tile += num_pairs()) {
+            const TileIdx t = decode_tile(args, tile);
+            for (int kb = t.kb_begin; kb < t.kb_end; ++kb) {
               mbar_wait(full_bar(stage), phase, 0xA00u + stage);
               mbar_arrive_cluster(mapa_shared(pfull_bar(stage), 0));
               if (++stage == STAGES) { stage = 0; phase ^= 1u; }
@@ -892,33 +929,19 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * NUM_EPI_W
         } else {
           // =================================================================== leader: MMA issuer for the pair
           int it = 0;
-          for (int tile = pair; tile < total_tiles; tile += npairs, ++it) {
+          for (int tile = pair_id(); tile < total_tiles; tile += num_pairs(), ++it) {
+            const TileIdx t = decode_tile(args, tile);
             const int acc = it & 1;
             const uint32_t acc_phase = (it >> 1) & 1;
             mbar_wait_cluster(tempty_bar(acc), acc_phase ^ 1u, 0xB00u + acc);
             tc_fence_after();
             const uint32_t d_tmem = tmem_base + acc * BLOCK_N;
             uint32_t accumulate = 0;
-            for (int kb = 0; kb < args.kb_total; ++kb) {
+            for (int kb = t.kb_begin; kb < t.kb_end; ++kb) {
               mbar_wait(full_bar(stage), phase, 0xC00u + stage);
               mbar_wait_cluster(pfull_bar(stage), phase, 0xD00u + stage);
               tc_fence_after();
-#pragma unroll
-              for (int combo = 0; combo < (PLANES == 1 ? 1 : (PLANES == 2 ? 3 : 6)); ++combo) {
-                constexpr int PA2[3] = {1, 0, 0}, PB2[3] = {0, 1, 0};
-                constexpr int PA3[6] = {1, 0, 2, 0, 1, 0}, PB3[6] = {1, 2, 0, 1, 0, 0};
-                const int pa = (PLANES == 1) ? 0 : (PLANES == 2 ? PA2[combo % 3] : PA3[combo]);
-                const int pb = (PLANES == 1) ? 0 : (PLANES == 2 ? PB2[combo % 3] : PB3[combo]);
-                const uint32_t a_base = sA(stage, pa), b_base = sB(stage, pb);
-#pragma unroll
-                for (int k = 0; k < BLOCK_K / UMMA_K; ++k) {
-                  const uint64_t da = umma_smem_desc(a_base + k * (UMMA_K * 2), 16, 1024);
-                  const uint64_t db = B_MN ? umma_smem_desc(b_base + k * (UMMA_K * 128), BLOCK_K * 128, 1024)
-                                           : umma_smem_desc(b_base + k * (UMMA_K * 2), 16, 1024);
-                  umma_f16_pair(d_tmem, da, db, IDESC, accumulate);
-                  accumulate = 1;
-                }
-              }
+              mma_stage<Cfg, PLANES, false, B_MN, true>(sA(stage), sB(stage), d_tmem, IDESC, accumulate);
               umma_commit_pair(empty_bar(stage));       // frees the slot in both CTAs when these MMAs retire
               if (++stage == STAGES) { stage = 0; phase ^= 1u; }
             }
@@ -931,7 +954,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * NUM_EPI_W
       if (lane == 0) {
         const uint32_t te0 = mapa_shared(tempty_bar(0), 0), te1 = mapa_shared(tempty_bar(1), 0);
         int it = 0;
-        for (int tile = pair; tile < total_tiles; tile += npairs, ++it) {
+        for (int tile = pair_id(); tile < total_tiles; tile += num_pairs(), ++it) {
           const int acc = it & 1;
           mbar_wait(tlocal_bar(acc), (it >> 1) & 1, 0xF00u + acc);
           mbar_arrive_cluster(acc ? te1 : te0);
@@ -940,65 +963,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * NUM_EPI_W
     }
   } else {
     // ===================================================================== epilogue (both CTAs, own rows)
-    setmaxnreg_inc<EPI_REGS>();
-    const int w = (warp - 4) & 3;
-    const int cgroup = (warp - 4) >> 2;
-    const GemmEpilogue& e = args.epi;
-    const float pe_alpha = (e.flags & EPI_PE) ? __ldg(e.pe_alpha) : 0.f;
-    const float alpha = e.alpha * (e.alpha_ptr != nullptr ? __ldg(e.alpha_ptr) : 1.f);
-    const float cs_scale = e.colsum_scale_ptr != nullptr ? __ldg(e.colsum_scale_ptr) : 1.f;
-    const uint32_t stage_buf = epi_stage_base + (warp - 4) * (EPI_STAGE_BYTES + EPI_BIAS_BYTES);
-    const uint32_t bias_buf = stage_buf + EPI_STAGE_BYTES;
-    int it = 0;
-    for (int tile = pair; tile < total_tiles; tile += npairs, ++it) {
-      int t = tile;
-      const int tn = t % args.tiles_n; t /= args.tiles_n;
-      const int tm = t % args.tiles_m; t /= args.tiles_m;
-      const int i0 = t % args.nb0, i1 = t / args.nb0;
-      const int acc = it & 1;
-      const uint32_t acc_phase = (it >> 1) & 1;
-      if (e.flags & EPI_BIAS) {
-        const int j = lane >> 3;
-        const int cloc = (cgroup + j * EPI_CG) * 32;
-        const int col = tn * BLOCK_N + cloc + (lane & 7) * 4;
-        float4 b = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (cloc < BLOCK_N && col < args.N) b = __ldg(reinterpret_cast<const float4*>(e.bias + col));
-        asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(bias_buf + lane * 16), "f"(b.x), "f"(b.y), "f"(b.z), "f"(b.w) : "memory");
-        __syncwarp();
-      }
-      mbar_wait(tfull_bar(acc), acc_phase, 0xE00u + acc);
-      tc_fence_after();
-      const int64_t row0 = static_cast<int64_t>(tm) * 2 * BLOCK_M + static_cast<int64_t>(rank) * BLOCK_M + w * 32;
-      const int64_t out_boff = i0 * e.out_sb0 + i1 * e.out_sb1;
-      const int64_t res_boff = i0 * e.res_sb0 + i1 * e.res_sb1;
-      const uint32_t t_row = tmem_base + (static_cast<uint32_t>(w * 32) << 16) + acc * BLOCK_N;
-      const int64_t cs_boff = i0 * e.colsum_sb0;
-      if constexpr (LN) {
-        if (row0 < args.M)
-          ln_epilogue_tile<BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, w, t_row, args.M, args.N, row0, t, out_boff, res_boff,
-                                    alpha);
-      } else
-      if (row0 < args.M) {   // warp-uniform
-        constexpr uint32_t CT_LEAN = EPI_BIAS | EPI_RELU | EPI_OUT_F32;
-        // the bit-mask classes only exist in the multi-plane kernels: the one-plane (inference) kernels stay small
-        constexpr uint32_t CT_FWD = CT_LEAN | EPI_PE | EPI_DROPOUT | EPI_RES | (PLANES >= 2 ? EPI_EMIT_BITS : 0u);
-        constexpr uint32_t CT_BWD = EPI_GATE_BITS | EPI_COLSUM | EPI_RES | EPI_OUT_F32;   // data gradients
-        if ((e.flags & ~CT_LEAN) == 0)
-          epilogue_tile<CT_LEAN, BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, t_row, args.M, args.N, row0, t, out_boff, res_boff,
-                                          cs_boff, tn, pe_alpha, alpha, cs_scale);
-        else if ((e.flags & ~CT_FWD) == 0)
-          epilogue_tile<CT_FWD, BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, t_row, args.M, args.N, row0, t, out_boff, res_boff,
-                                         cs_boff, tn, pe_alpha, alpha, cs_scale);
-        else if (PLANES >= 2 && (e.flags & ~CT_BWD) == 0)
-          epilogue_tile<(PLANES >= 2 ? CT_BWD : 0xFFFFFFFFu), BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, t_row, args.M, args.N, row0,
-                                                                       t, out_boff, res_boff, cs_boff, tn, pe_alpha, alpha, cs_scale);
-        else
-          epilogue_tile<0xFFFFFFFFu, BLOCK_N>(e, stage_buf, bias_buf, lane, cgroup, t_row, args.M, args.N, row0, t, out_boff,
-                                              res_boff, cs_boff, tn, pe_alpha, alpha, cs_scale);
-      }
-      tc_fence_before();
-      mbar_arrive(tlocal_bar(acc));
-    }
+    epilogue_role<PLANES, BLOCK_N, LN>(args, warp, lane, epi_stage_base, tmem_base, pair_id(), num_pairs(), 2 * BLOCK_M,
+                                       static_cast<int>(rank) * BLOCK_M, tfull_bar(0), tlocal_bar(0), 0xE00u);
   }
 
   tc_fence_before();
@@ -1087,51 +1053,99 @@ int encode_map_4d(CUtensorMap* map, const void* base, const int64_t dims[4], con
   return 0;
 }
 
-// Opt in to the kernel's dynamic shared memory size and check its register count (per device: callers run it under a
-// PerDeviceOnce).
-template <class Kern>
-static int configure_kernel(Kern kern, int smem) {
-  SPK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  cudaFuncAttributes fa;
-  SPK_CUDA(cudaFuncGetAttributes(&fa, kern));
-  // setmaxnreg re-partitions the launch allocation; another launch register count would dead-lock the epilogue warps
-  SPK_CHECK(fa.numRegs == LAUNCH_REGS, "gemm kernel was built with %d registers/thread, expected %d", fa.numRegs,
-            LAUNCH_REGS);
-  return 0;
-}
-// The single-CTA kernels are configured up front (CUDA loads kernels lazily: a first launch of a new instantiation
-// inside a timed region -- a new frame length picks another BLOCK_N -- would pay for the load).
-template <bool A_MN, bool B_MN, int PLANES, int BLOCK_N>
-static int configure() {
-  return configure_kernel(gemm_tc_kernel<A_MN, B_MN, PLANES, BLOCK_N>, TileCfg<PLANES, BLOCK_N>::SMEM_BYTES);
+// A kernel instantiation, its dynamic shared memory size and its one-time set-up (per device).
+struct GemmKernel {
+  void (*fn)(GemmKernelArgs) = nullptr;
+  int smem = 0;
+  PerDeviceOnce* configured = nullptr;
+};
+
+// Three planes of A and B only fit a double-buffered operand ring up to BLOCK_N = 128.
+constexpr int max_block_n(int planes) { return planes == 3 ? 128 : 256; }
+constexpr int PAIR_BN = 256;
+
+template <bool A_MN, bool B_MN, int PLANES, int BLOCK_N, bool LN = false>
+static GemmKernel tc_entry() {
+  if constexpr (BLOCK_N > max_block_n(PLANES)) {
+    return {};
+  } else {
+    static PerDeviceOnce once;
+    return {gemm_tc_kernel<A_MN, B_MN, PLANES, BLOCK_N, LN>, TileCfg<PLANES, BLOCK_N>::SMEM_BYTES, &once};
+  }
 }
 template <bool A_MN, bool B_MN, int PLANES>
-static int configure_bn() {
-  SPK_TRY((configure<A_MN, B_MN, PLANES, 64>()));
-  SPK_TRY((configure<A_MN, B_MN, PLANES, 128>()));
-  if constexpr (PLANES < 3) {
-    SPK_TRY((configure<A_MN, B_MN, PLANES, 192>()));
-    SPK_TRY((configure<A_MN, B_MN, PLANES, 256>()));
+static GemmKernel tc_entry_bn(int block_n) {
+  switch (block_n) {
+    case 64: return tc_entry<A_MN, B_MN, PLANES, 64>();
+    case 128: return tc_entry<A_MN, B_MN, PLANES, 128>();
+    case 192: return tc_entry<A_MN, B_MN, PLANES, 192>();
+    case 256: return tc_entry<A_MN, B_MN, PLANES, 256>();
   }
-  return 0;
+  return {};
 }
 template <int PLANES>
-static int configure_planes() {
-  SPK_TRY((configure_bn<false, false, PLANES>()));
-  SPK_TRY((configure_bn<false, true, PLANES>()));
-  SPK_TRY((configure_bn<true, true, PLANES>()));
-  return 0;
+static GemmKernel tc_entry_planes(bool a_mn, bool b_mn, int block_n, bool ln) {
+  if (ln) {   // the fused LayerNorm: K-major operands, BLOCK_N = N = 256, one or two planes
+    if constexpr (PLANES <= 2)
+      if (!a_mn && !b_mn && block_n == 256) return tc_entry<false, false, PLANES, 256, true>();
+    return {};
+  }
+  if (!a_mn) return b_mn ? tc_entry_bn<false, true, PLANES>(block_n) : tc_entry_bn<false, false, PLANES>(block_n);
+  return b_mn ? tc_entry_bn<true, true, PLANES>(block_n) : GemmKernel{};   // A MN-major with B K-major is not built
 }
-static int configure_all() {
+// The single-CTA instantiations: (A, B) K/K-, K/MN- or MN/MN-major, BLOCK_N = 64 / 128 / 192 / 256 up to
+// max_block_n(planes), one to three planes, and the fused-LayerNorm kernels; {} for a combination that is not built.
+static GemmKernel tc_kernel(bool a_mn, bool b_mn, int planes, int block_n, bool ln) {
+  switch (planes) {
+    case 1: return tc_entry_planes<1>(a_mn, b_mn, block_n, ln);
+    case 2: return tc_entry_planes<2>(a_mn, b_mn, block_n, ln);
+    case 3: return tc_entry_planes<3>(a_mn, b_mn, block_n, ln);
+  }
+  return {};
+}
+
+template <bool B_MN, int PLANES, bool LN = false>
+static GemmKernel pair_entry() {
   static PerDeviceOnce once;
-  return once.run([]() -> int {
-    SPK_TRY(configure_planes<1>());
-    SPK_TRY(configure_planes<2>());
-    SPK_TRY(configure_planes<3>());
+  return {gemm_pair_kernel<B_MN, PLANES, PAIR_BN, LN>, PairCfg<PLANES, PAIR_BN>::SMEM_BYTES, &once};
+}
+// The CTA-pair instantiations (A K-major, BLOCK_N = PAIR_BN): two or three planes; the fused LayerNorm at two planes
+// with B K-major.
+static GemmKernel pair_kernel(bool b_mn, int planes, bool ln) {
+  if (ln) return (planes == 2 && !b_mn) ? pair_entry<false, 2, true>() : GemmKernel{};
+  if (planes == 2) return b_mn ? pair_entry<true, 2>() : pair_entry<false, 2>();
+  if (planes == 3) return b_mn ? pair_entry<true, 3>() : pair_entry<false, 3>();
+  return {};
+}
+
+// Opt in to the kernel's dynamic shared memory size and check its register count, once per device.
+static int configure(const GemmKernel& k) {
+  return k.configured->run([&]() -> int {
+    SPK_CUDA(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, k.smem));
+    cudaFuncAttributes fa;
+    SPK_CUDA(cudaFuncGetAttributes(&fa, k.fn));
+    // setmaxnreg re-partitions the launch allocation; another launch register count would dead-lock the epilogue warps
+    SPK_CHECK(fa.numRegs == LAUNCH_REGS, "gemm kernel was built with %d registers/thread, expected %d", fa.numRegs,
+              LAUNCH_REGS);
     return 0;
   });
 }
-
+// The single-CTA kernels without the fused LayerNorm are configured up front (CUDA loads kernels lazily: a first launch
+// of a new instantiation inside a timed region -- a new frame length picks another BLOCK_N -- would pay for the load).
+// The fused-LayerNorm and CTA-pair kernels are configured on first use.
+static int configure_all() {
+  static PerDeviceOnce once;
+  return once.run([]() -> int {
+    for (int planes = 1; planes <= 3; ++planes)
+      for (const bool a_mn : {false, true})
+        for (const bool b_mn : {false, true})
+          for (int block_n = 64; block_n <= 256; block_n += 64) {
+            const GemmKernel k = tc_kernel(a_mn, b_mn, planes, block_n, false);
+            if (k.fn != nullptr) SPK_TRY(configure(k));
+          }
+    return 0;
+  });
+}
 
 // spk_set_option("gemm_dependent_launch", 0 | 1 | 2): 0 off, 1 inside the inference forward only, 2 (default) every GEMM.
 // Measured (same process, alternating): inference 960 x 200 frames 1.904 -> 1.842 ms, 7 x 33 frames 0.246 -> 0.237 ms,
@@ -1144,77 +1158,23 @@ GemmDependentLaunchScope::~GemmDependentLaunchScope() { if (on_) --t_gemm_pdl_sc
 
 // A GEMM launched with the programmatic-stream-serialisation attribute runs its prologue under the tail of the kernel
 // before it (which calls pdl_trigger() at its start) and its main part after pdl_wait().
-template <class Kern>
-static int launch_gemm_kernel(Kern kern, int grid, size_t smem, cudaStream_t stream, const GemmKernelArgs& args) {
+static int launch_gemm_kernel(const GemmKernel& k, int grid, cudaStream_t stream, const GemmKernelArgs& args) {
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(static_cast<unsigned>(grid));
   cfg.blockDim = dim3(128 + 32 * NUM_EPI_WARPS);
-  cfg.dynamicSmemBytes = smem;
+  cfg.dynamicSmemBytes = k.smem;
   cfg.stream = stream;
   cfg.attrs = attr;
   cfg.numAttrs = (g_gemm_pdl >= 2 || (g_gemm_pdl == 1 && t_gemm_pdl_scope > 0)) ? 1 : 0;
-  SPK_CUDA(cudaLaunchKernelEx(&cfg, kern, args));
+  SPK_CUDA(cudaLaunchKernelEx(&cfg, k.fn, args));
   return 0;
-}
-
-template <int PLANES>
-static int launch_ln(const GemmKernelArgs& args, int grid, cudaStream_t stream) {
-  using Cfg = TileCfg<PLANES, 256>;
-  auto kern = gemm_tc_kernel<false, false, PLANES, 256, true>;
-  static PerDeviceOnce once;
-  SPK_TRY(once.run([&]() -> int { return configure_kernel(kern, Cfg::SMEM_BYTES); }));
-  return launch_gemm_kernel(kern, grid, Cfg::SMEM_BYTES, stream, args);
-}
-
-template <bool A_MN, bool B_MN, int PLANES, int BLOCK_N>
-static int launch(const GemmKernelArgs& args, int grid, cudaStream_t stream) {
-  using Cfg = TileCfg<PLANES, BLOCK_N>;
-  auto kern = gemm_tc_kernel<A_MN, B_MN, PLANES, BLOCK_N>;
-  return launch_gemm_kernel(kern, grid, Cfg::SMEM_BYTES, stream, args);
 }
 
 static int g_cta_pairs = 1;            // spk_set_option("gemm_cta_pairs", 0/1)
 void gemm_set_cta_pairs(int on) { g_cta_pairs = on; }
-
-template <bool B_MN, int PLANES, int BLOCK_N, bool LN = false>
-static int launch_pair(const GemmKernelArgs& args, int pairs, cudaStream_t stream) {
-  using Cfg = PairCfg<PLANES, BLOCK_N>;
-  auto kern = gemm_pair_kernel<B_MN, PLANES, BLOCK_N, LN>;
-  static PerDeviceOnce once;
-  SPK_TRY(once.run([&]() -> int { return configure_kernel(kern, Cfg::SMEM_BYTES); }));
-  return launch_gemm_kernel(kern, 2 * pairs, Cfg::SMEM_BYTES, stream, args);   // __cluster_dims__(2,1,1)
-}
-
-template <bool A_MN, bool B_MN, int PLANES>
-static int launch_bn(int block_n, const GemmKernelArgs& args, int grid, cudaStream_t stream) {
-  if constexpr (PLANES == 3) {   // three planes of A and B only fit a double-buffered ring up to N = 128
-    switch (block_n) {
-      case 64: return launch<A_MN, B_MN, PLANES, 64>(args, grid, stream);
-      case 128: return launch<A_MN, B_MN, PLANES, 128>(args, grid, stream);
-    }
-  } else {
-    switch (block_n) {
-      case 64: return launch<A_MN, B_MN, PLANES, 64>(args, grid, stream);
-      case 128: return launch<A_MN, B_MN, PLANES, 128>(args, grid, stream);
-      case 192: return launch<A_MN, B_MN, PLANES, 192>(args, grid, stream);
-      case 256: return launch<A_MN, B_MN, PLANES, 256>(args, grid, stream);
-    }
-  }
-  set_error("unsupported block_n %d", block_n);
-  return SPK_EINVAL;
-}
-
-template <int PLANES>
-static int launch_major(bool a_mn, bool b_mn, int block_n, const GemmKernelArgs& args, int grid, cudaStream_t stream) {
-  if (!a_mn && !b_mn) return launch_bn<false, false, PLANES>(block_n, args, grid, stream);
-  if (!a_mn && b_mn) return launch_bn<false, true, PLANES>(block_n, args, grid, stream);
-  if (a_mn && b_mn) return launch_bn<true, true, PLANES>(block_n, args, grid, stream);
-  set_error("A MN-major with B K-major is not instantiated");
-  return SPK_EINVAL;
-}
 
 int gemm_run(const GemmProblem& p, cudaStream_t stream) {
   SPK_CHECK(p.M > 0 && p.N > 0 && p.K > 0, "gemm: empty problem %d x %d x %d", p.M, p.N, p.K);
@@ -1233,7 +1193,8 @@ int gemm_run(const GemmProblem& p, cudaStream_t stream) {
 
   SPK_TRY(configure_all());
 
-  if (p.epi.flags & EPI_LN)
+  const bool ln = (p.epi.flags & EPI_LN) != 0;
+  if (ln)
     SPK_CHECK(p.N == 256 && p.nb0 * p.nb1 == 1 && p.ksplit <= 1 && p.epi.ln_gamma != nullptr && p.epi.ln_beta != nullptr &&
                   !p.a_mn && !p.b_mn && p.planes <= 2 &&
                   !(p.epi.flags & (EPI_OUT_F32 | EPI_OUT_ATOMIC | EPI_RELU | EPI_PE | EPI_COLSUM | EPI_GATE_BITS |
@@ -1243,17 +1204,20 @@ int gemm_run(const GemmProblem& p, cudaStream_t stream) {
   // CTAs that each walk the whole K loop; 64-wide single-CTA tiles spread the same work over 4x as many SMs.
   int req_bn = p.block_n;
   if (req_bn == 0 && !p.a_mn && p.ksplit <= 1 && p.nb0 * p.nb1 == 1 && p.M <= 2048 && p.N >= 128) req_bn = 64;
-  const bool ln_pair = (p.epi.flags & EPI_LN) && p.planes == 2 && p.M > 2048 && g_cta_pairs;
-  if ((p.epi.flags & EPI_LN) && !ln_pair) req_bn = 256;      // the fused LayerNorm runs in its own instantiations
+  const bool ln_pair = ln && p.planes == 2 && p.M > 2048 && g_cta_pairs;
+  if (ln && !ln_pair) req_bn = 256;      // the fused LayerNorm runs in its own instantiations
 
   // CTA-pair path: K-major A, two or three planes, no split-K, 256-wide N tiles (128 columns of B per CTA)
-  constexpr int PAIR_BN = 256;
   const bool pair =
       g_cta_pairs && !p.a_mn && p.planes >= 2 && p.ksplit <= 1 && req_bn == 0 && p.N % 128 == 0 && p.M >= 256;
   int bn = pair ? PAIR_BN : req_bn;
   if (bn == 0) bn = p.N <= 64 ? 64 : (p.N <= 128 ? 128 : (p.N <= 192 ? 192 : 256));
-  if (!pair && p.planes == 3 && bn > 128) bn = 128;
+  if (!pair && bn > max_block_n(p.planes)) bn = max_block_n(p.planes);
   const int tile_m = pair ? 2 * BLOCK_M : BLOCK_M;
+  const GemmKernel kern = pair ? pair_kernel(p.b_mn, p.planes, ln) : tc_kernel(p.a_mn, p.b_mn, p.planes, bn, ln);
+  SPK_CHECK(kern.fn != nullptr, "gemm: no kernel for %d planes, A %s-major, B %s-major, BLOCK_N %d%s", p.planes,
+            p.a_mn ? "MN" : "K", p.b_mn ? "MN" : "K", bn, ln ? ", fused LayerNorm" : "");
+  SPK_TRY(configure(kern));
 
   GemmKernelArgs a;
   memset(&a, 0, sizeof(a));
@@ -1288,19 +1252,9 @@ int gemm_run(const GemmProblem& p, cudaStream_t stream) {
   if (pair) {
     const int max_pairs = sms / 2;
     const int pairs = static_cast<int>(total < max_pairs ? total : max_pairs);
-    if (p.epi.flags & EPI_LN) return launch_pair<false, 2, PAIR_BN, true>(a, pairs, stream);
-    if (p.planes == 3) {
-      if (p.b_mn) return launch_pair<true, 3, PAIR_BN>(a, pairs, stream);
-      return launch_pair<false, 3, PAIR_BN>(a, pairs, stream);
-    }
-    if (p.b_mn) return launch_pair<true, 2, PAIR_BN>(a, pairs, stream);
-    return launch_pair<false, 2, PAIR_BN>(a, pairs, stream);
+    return launch_gemm_kernel(kern, 2 * pairs, stream, a);   // __cluster_dims__(2,1,1)
   }
-  const int grid = static_cast<int>(total < sms ? total : sms);
-  if (p.epi.flags & EPI_LN) return p.planes == 1 ? launch_ln<1>(a, grid, stream) : launch_ln<2>(a, grid, stream);
-  if (p.planes == 1) return launch_major<1>(p.a_mn, p.b_mn, bn, a, grid, stream);
-  if (p.planes == 2) return launch_major<2>(p.a_mn, p.b_mn, bn, a, grid, stream);
-  return launch_major<3>(p.a_mn, p.b_mn, bn, a, grid, stream);
+  return launch_gemm_kernel(kern, static_cast<int>(total < sms ? total : sms), stream, a);
 }
 
 }  // namespace spk
