@@ -134,6 +134,19 @@ int spk_encoder_backward(const spk_encoder_config* cfg, const spk_encoder_params
                          int samples, int precision, int training, uint64_t seed, void* workspace,
                          size_t workspace_bytes, void* stream);
 
+/* Backward of a forward call with optional outputs (same cfg / shape / precision / training / seed / workspace as
+ * spk_encoder_backward).
+ *   grads  NULL: no parameter gradient is computed (no weight-gradient GEMM, no bias column sums, no LayerNorm /
+ *          head / attention bias sums); otherwise accumulated (+=) exactly as spk_encoder_backward does.
+ *   d_mel  NULL: none; otherwise fp32 [batch, mel_dim, frames] receives (=) dL/d(slices): the gradient of the
+ *          [batch, mel_dim, frames] slice tensor the forward consumed, whichever of plain / view / ragged produced it.
+ * At least one of grads / d_mel is non-NULL.  Needs no more workspace than spk_encoder_backward.
+ * spk_encoder_backward is this call with d_mel = NULL. */
+int spk_encoder_backward_input(const spk_encoder_config* cfg, const spk_encoder_params* weights,
+                               const spk_encoder_params* grads, float* d_mel, const float* d_dvec, int batch,
+                               int frames, int samples, int precision, int training, uint64_t seed,
+                               void* workspace, size_t workspace_bytes, void* stream);
+
 /* Test aid: text table "name byte_offset plane_stride" of the workspace buffers (returns bytes written). */
 int spk_encoder_debug_layout(const spk_encoder_config* cfg, int batch, int frames, int samples, int precision,
                              int keep_stash, char* buf, size_t cap);

@@ -189,7 +189,9 @@ def _run_forward(cfg, names, params, pe, features, samples, precision, training,
 
 class _EncoderFunction(torch.autograd.Function):
     """Differentiable encoder call: forward keeps the activation stash, backward runs
-    spk_encoder_backward into one flat fp32 gradient buffer (returned as per-parameter views)."""
+    spk_encoder_backward into one flat fp32 gradient buffer (returned as per-parameter views).  When ``features`` needs
+    a gradient the backward is spk_encoder_backward_input, which also writes dL/d(features); with every parameter
+    frozen it computes no parameter gradient at all and allocates no gradient arena."""
 
     @staticmethod
     def forward(ctx, features, module, samples, precision, training, seed, *params):
@@ -201,6 +203,7 @@ class _EncoderFunction(torch.autograd.Function):
                                                                     keep=True)
         ctx.module, ctx.ws, ctx.nbytes = module, ws, nbytes
         ctx.meta = (batch, frames, samples, precision, training, seed)
+        ctx.features_dtype = features.dtype if isinstance(features, torch.Tensor) else None
         ctx.save_for_backward(*params)
         ctx.pe = pe
         return dvec
@@ -213,26 +216,41 @@ class _EncoderFunction(torch.autograd.Function):
         batch, frames, samples, precision, training, seed = ctx.meta
         device = grad_dvec.device
         grad_dvec = grad_dvec.contiguous().float()
-        sizes = [p.numel() for p in params]
-        offsets, total = [], 0
-        for s in sizes:
-            offsets.append(total)
-            total += (s + 3) // 4 * 4          # keep every view 16-byte aligned
-        arena = module._grad_arena(total, device, params)
-        views = [arena[o:o + s].view_as(p) for o, s, p in zip(offsets, sizes, params)]
+        want_mel = ctx.needs_input_grad[0]
+        # partial freezing keeps the full arena: only a fully frozen encoder skips the parameter gradients
+        want_params = not want_mel or any(ctx.needs_input_grad[6:])
+        views, d_mel = None, None
+        if want_params:
+            sizes = [p.numel() for p in params]
+            offsets, total = [], 0
+            for s in sizes:
+                offsets.append(total)
+                total += (s + 3) // 4 * 4          # keep every view 16-byte aligned
+            arena = module._grad_arena(total, device, params)
+            views = [arena[o:o + s].view_as(p) for o, s, p in zip(offsets, sizes, params)]
         with torch.cuda.device(device):
             weights = _fill_params(N.EncoderParams(), dict(zip(names, [p.detach() for p in params])), ctx.pe,
                                    cfg.layers)
-            grads = _fill_params(N.EncoderParams(), dict(zip(names, views)), None, cfg.layers)
-            N.check(N.lib().spk_encoder_backward(ctypes.byref(cfg), ctypes.byref(weights), ctypes.byref(grads),
-                                                 N.ptr(grad_dvec), batch, frames, samples, precision, int(training),
-                                                 ctypes.c_uint64(seed), _aligned_ptr(ctx.ws), ctx.nbytes,
-                                                 N.stream_ptr(device)),
-                    "spk_encoder_backward")
+            grads = _fill_params(N.EncoderParams(), dict(zip(names, views)), None, cfg.layers) if want_params else None
+            if not want_mel:
+                N.check(N.lib().spk_encoder_backward(ctypes.byref(cfg), ctypes.byref(weights), ctypes.byref(grads),
+                                                     N.ptr(grad_dvec), batch, frames, samples, precision,
+                                                     int(training), ctypes.c_uint64(seed), _aligned_ptr(ctx.ws),
+                                                     ctx.nbytes, N.stream_ptr(device)),
+                        "spk_encoder_backward")
+            else:
+                d_mel = torch.empty((batch, cfg.mel_dim, frames), dtype=torch.float32, device=device)
+                N.check(N.lib().spk_encoder_backward_input(ctypes.byref(cfg), ctypes.byref(weights),
+                                                           ctypes.byref(grads) if want_params else None, N.ptr(d_mel),
+                                                           N.ptr(grad_dvec), batch, frames, samples, precision,
+                                                           int(training), ctypes.c_uint64(seed),
+                                                           _aligned_ptr(ctx.ws), ctx.nbytes, N.stream_ptr(device)),
+                        "spk_encoder_backward_input")
+                d_mel = d_mel.to(ctx.features_dtype)      # fp16 patterns get an fp16 gradient
         if getattr(module, "_debug_keep_ws", False):      # parity tests read the stage buffers back
             module._last_ws, module._last_meta = ctx.ws, ctx.meta
         ctx.ws = None
-        return (None, None, None, None, None, None) + tuple(views)
+        return (d_mel, None, None, None, None, None) + (tuple(views) if want_params else (None,) * len(params))
 
 
 class GE2E(torch.nn.Module):
@@ -297,7 +315,9 @@ class GE2E(torch.nn.Module):
         """features: [Batch * Sample, Mel_dim, Time] -> [Batch, Emb_dim] unit-norm d-vectors."""
         samples = int(samples)
         params = list(self.parameters())
-        need_grad = torch.is_grad_enabled() and any(p.requires_grad for p in params)
+        # a frozen encoder used as a critic still differentiates with respect to its input
+        input_grad = isinstance(features, torch.Tensor) and features.requires_grad
+        need_grad = torch.is_grad_enabled() and (input_grad or any(p.requires_grad for p in params))
         if need_grad:
             seed = int(torch.empty((), dtype=torch.int64).random_().item()) if self.training else 0
             return _EncoderFunction.apply(features, self, samples, self.train_precision, self.training, seed,

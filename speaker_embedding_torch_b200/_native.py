@@ -25,7 +25,7 @@ EXPORTS = (
     "spk_gemm", "spk_split_pack", "spk_device_info", "spk_prof_enable", "spk_prof_report",
     "spk_encoder_debug_layout", "spk_set_option", "spk_encoder_forward_view", "spk_plan_flags",
     "spk_dropout_keep", "spk_encoder_forward_ragged",
-    "spk_mel_frames", "spk_mel_spectrogram", "spk_set_debug_buffer",
+    "spk_mel_frames", "spk_mel_spectrogram", "spk_set_debug_buffer", "spk_encoder_backward_input",
 )
 
 c_f32p = ctypes.c_void_p  # device pointers travel as integers
@@ -137,6 +137,10 @@ def lib():
         L.spk_encoder_backward.argtypes = [ctypes.POINTER(EncoderConfig), ctypes.POINTER(EncoderParams),
                                            ctypes.POINTER(EncoderParams), vp, i32, i32, i32, i32, i32, u64,
                                            vp, sz, vp]
+        L.spk_encoder_backward_input.restype = i32
+        L.spk_encoder_backward_input.argtypes = [ctypes.POINTER(EncoderConfig), ctypes.POINTER(EncoderParams),
+                                                 ctypes.POINTER(EncoderParams), vp, vp, i32, i32, i32, i32, i32, u64,
+                                                 vp, sz, vp]
         L.spk_ge2e_workspace_bytes.restype = sz
         L.spk_ge2e_workspace_bytes.argtypes = [i32, i32]
         L.spk_ge2e_loss.restype = i32

@@ -59,8 +59,18 @@ int spk_encoder_backward(const spk_encoder_config* cfg, const spk_encoder_params
                          int precision, int training, uint64_t seed, void* workspace, size_t workspace_bytes,
                          void* stream) {
   SPK_CHECK(cfg && weights && grads && d_dvec && workspace, "spk_encoder_backward: null argument");
-  return encoder_backward(*cfg, *weights, *grads, d_dvec, batch, frames, samples, precision, training, seed, workspace,
-                          workspace_bytes, as_stream(stream));
+  return encoder_backward(*cfg, *weights, grads, nullptr, d_dvec, batch, frames, samples, precision, training, seed,
+                          workspace, workspace_bytes, as_stream(stream));
+}
+
+int spk_encoder_backward_input(const spk_encoder_config* cfg, const spk_encoder_params* weights,
+                               const spk_encoder_params* grads, float* d_mel, const float* d_dvec, int batch,
+                               int frames, int samples, int precision, int training, uint64_t seed,
+                               void* workspace, size_t workspace_bytes, void* stream) {
+  SPK_CHECK(cfg && weights && d_dvec && workspace, "spk_encoder_backward_input: null argument");
+  SPK_CHECK(grads || d_mel, "spk_encoder_backward_input: grads and d_mel are both NULL (nothing to compute)");
+  return encoder_backward(*cfg, *weights, grads, d_mel, d_dvec, batch, frames, samples, precision, training, seed,
+                          workspace, workspace_bytes, as_stream(stream));
 }
 
 int spk_encoder_debug_layout(const spk_encoder_config* cfg, int batch, int frames, int samples, int precision,

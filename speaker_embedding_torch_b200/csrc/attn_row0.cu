@@ -280,6 +280,7 @@ __global__ void __launch_bounds__(32 * R0_WARPS) attn_row0_bwd_kernel(
   }
   if (g == 0) {
     store8_split(dq0, dq_ps, g_planes, static_cast<int64_t>(b) * 256 + col, dq);
+    if (dbias == nullptr) return;     // no parameter gradients wanted
     const float inv_s = gscale != nullptr ? __ldg(gscale + 1) : 1.f;     // gradients arrive scaled by gscale[0]
 #pragma unroll
     for (int i = 0; i < 8; ++i) {

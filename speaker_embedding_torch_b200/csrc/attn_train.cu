@@ -943,7 +943,7 @@ struct AttnTrainBwdArgs {
   const uint16_t* mbits;    // [B*H][nC][T] or null (no dropout)
   elem_t* dqkv;      // [2][B*T, 768]
   int64_t dqkv_ps;
-  float* dbias;             // [768] += column sums of dQ | dK | dV, times *(gscale + 1)
+  float* dbias;             // [768] += column sums of dQ | dK | dV, times *(gscale + 1); null: not wanted
   const float* gscale;      // device (S, 1 / S): the gradients arrive scaled by S (may be null)
   float inv_keep;
   unsigned long long* timeline;
@@ -1354,7 +1354,7 @@ __global__ void __launch_bounds__(ATB_THREADS, 1) attn_train_bwd_kernel(const __
       mbar_arrive(bar_dqd);
     }
     // ---- in-proj bias gradient: one atomic per warp, tensor and column for the whole kernel
-    if (blockIdx.x < items && lane < 16) {
+    if (a.dbias != nullptr && blockIdx.x < items && lane < 16) {   // null: no parameter gradients wanted
       const int col = h * 64 + part * 16 + lane;
       const float inv_s = a.gscale != nullptr ? __ldg(a.gscale + 1) : 1.f;
       atomicAdd(a.dbias + col, acc_dq * inv_s);

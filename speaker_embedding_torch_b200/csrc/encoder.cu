@@ -402,7 +402,7 @@ __global__ void __launch_bounds__(256) head_fwd_kernel(const elem_t* __restrict_
 }
 
 // Backward of the head, eight utterances per block (one warp each): d_dvec -> de (pre-normalisation), d_emean,
-// final-LN backward into the t = 0 rows of dH (pre-zeroed), dgamma / dbeta of the final LayerNorm.
+// final-LN backward into the t = 0 rows of dH (pre-zeroed), dgamma / dbeta of the final LayerNorm (both null: skipped).
 __global__ void __launch_bounds__(256) head_bwd_kernel(const float* __restrict__ g_dvec, const float* __restrict__ epre,
                                                        const float* __restrict__ wp, const elem_t* __restrict__ h,
                                                        int64_t h_ps, int planes, const float2* __restrict__ hst,
@@ -503,6 +503,7 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(const float* __restrict__
     }
   }
   // ---- dgamma / dbeta: the block's eight utterances meet in shared memory, one atomic per column and block
+  if (dgamma == nullptr) return;   // no parameter gradients wanted (block-uniform)
   __syncthreads();
 #pragma unroll
   for (int j = 0; j < 8; ++j) { wt[warp][lane + 32 * j] = ag[j]; wt[8 + warp][lane + 32 * j] = ab[j]; }
@@ -562,6 +563,8 @@ struct Ctx {
   cudaStream_t st;
   int P;
   const float* gs = nullptr;   // backward: the device scalars (S, 1 / S) of grad_scale_kernel
+  bool pgrad = true;           // backward: parameter gradients are wanted (spk_encoder_backward_input, grads != NULL)
+  uint32_t colsum() const { return pgrad ? EPI_COLSUM : 0u; }   // bias gradients fused into a data-gradient GEMM
   // backward: gemm_run, handing 1 / S to every epilogue that produces parameter gradients (fp32 atomics of the weight
   // gradients, fused bias column sums)
   int run(GemmProblem& g) const {
@@ -590,6 +593,9 @@ struct Ctx {
     e.res_plane_stride = s.ps; e.res_ld = ld; e.res_planes = P;
   }
 };
+
+// p + off, or null when no parameter gradient is wanted
+float* at(float* p, int64_t off) { return p != nullptr ? p + off : nullptr; }
 
 int wgrad_ksplit(int64_t K, int M, int N) {
   const int tiles = ((M + 127) / 128) * ((N + 255) / 256);
@@ -629,6 +635,7 @@ GemmProblem dgrad(const Ctx& c, const char* tag, const Split& dy, int64_t rows, 
 // scaled by S, c.run multiplies by 1 / S)
 int wgrad(const Ctx& c, const char* tag, int64_t rows, const Split& dy, int64_t dy_cols, const Split& x, int64_t x_cols,
           int64_t x_ld, float* dw) {
+  if (dw == nullptr) return 0;   // no parameter gradients wanted
   GemmProblem g;
   g.tag = tag;
   g.A = c.mat(dy, 0, rows, dy_cols, dy_cols);
@@ -708,7 +715,7 @@ int sublayer_bwd(const Ctx& c, const spk_layer_params& lw, const spk_layer_param
   SPK_TRY(wgrad(c, last ? "gemm.last.bwd.ffn2_wgrad" : "gemm.bwd.ffn2_wgrad", rows, dy, D, s.f, F, F, lg.linear2_w));
   {  // dU = (dY2 W2) * 1[f > 0] / (1 - p)
     GemmProblem g = dgrad(c, last ? "gemm.last.bwd.ffn2_dgrad" : "gemm.bwd.ffn2_dgrad", dy, rows, D, pl.w_l2[l], F);
-    g.epi.flags = EPI_COLSUM;
+    g.epi.flags = c.colsum();
     g.epi.colsum = lg.linear1_b;
     if (gate_bits) {
       g.epi.flags |= EPI_GATE_BITS;
@@ -875,15 +882,20 @@ int encoder_forward(const spk_encoder_config& cfg, const spk_encoder_params& w, 
   return 0;
 }
 
-int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w, const spk_encoder_params& gr,
-                     const float* d_dvec, int B, int T, int S, int P_fwd, int training, uint64_t seed, void* ws_v,
-                     size_t ws_bytes, cudaStream_t st) {
+int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w, const spk_encoder_params* grads,
+                     float* d_mel, const float* d_dvec, int B, int T, int S, int P_fwd, int training, uint64_t seed,
+                     void* ws_v, size_t ws_bytes, cudaStream_t st) {
   Plan pl;
   SPK_TRY(make_plan(cfg, B, T, S, P_fwd, true, pl));
   P_fwd = pl.P;
   if (ws_bytes < pl.total) { set_error("encoder: workspace too small (%zu < %zu)", ws_bytes, pl.total); return SPK_ENOMEM; }
   const int P = P_fwd < 2 ? P_fwd : 2;   // the stash may hold 3 planes; the backward pass reads / writes 2
   Ctx c{pl, reinterpret_cast<char*>(ws_v), st, P};
+  // grads == nullptr: every gradient pointer below is null, so no weight-gradient GEMM, column sum or atomic runs;
+  // the data path (dz, dh, dqkv, datt, d_mel) is the same either way
+  static const spk_encoder_params no_grads = {};
+  const spk_encoder_params& gr = grads != nullptr ? *grads : no_grads;
+  c.pgrad = grads != nullptr;
   const int64_t Mt = pl.Mt, D = pl.D;
   const int Tp = pl.Tp, H = pl.H;
   const DropCfg drop_pe = make_drop(seed, cfg.pe_dropout, training != 0);
@@ -905,9 +917,11 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
       d_dvec, c.f32(pl.epre), w.proj_w, c.ptr(hl), hl.ps, P, reinterpret_cast<const float2*>(c.f32(pl.hst)), w.norm_w,
       head_T, S, c.f32(pl.de), c.ptr(dhead), dhead.ps, gr.norm_w, gr.norm_b, gs, static_cast<int64_t>(B / S));
   SPK_CUDA(cudaGetLastError());
-  head_wgrad_kernel<<<dim3(8, (B / S + HEAD_WG_UCH - 1) / HEAD_WG_UCH), 256, 0, st>>>(c.f32(pl.de), c.f32(pl.emean), B / S,
-                                                                                      gr.proj_w, gr.proj_b);
-  SPK_CUDA(cudaGetLastError());
+  if (c.pgrad) {
+    head_wgrad_kernel<<<dim3(8, (B / S + HEAD_WG_UCH - 1) / HEAD_WG_UCH), 256, 0, st>>>(c.f32(pl.de), c.f32(pl.emean),
+                                                                                        B / S, gr.proj_w, gr.proj_b);
+    SPK_CUDA(cudaGetLastError());
+  }
   }
 
   if (pl.prune) {
@@ -924,7 +938,7 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
                           lg.in_proj_b, gs, B, H, T, Tp, st));
     SPK_TRY(wgrad(c, "gemm.last.bwd.q_wgrad", B, pl.dq0, D, hin, D, (int64_t)T * D, lg.in_proj_w));
     // dW[K|V rows] = dKV^T hin
-    SPK_TRY(wgrad(c, "gemm.last.bwd.kv_wgrad", Mt, pl.dqkv, 2 * D, hin, D, D, lg.in_proj_w + D * D));
+    SPK_TRY(wgrad(c, "gemm.last.bwd.kv_wgrad", Mt, pl.dqkv, 2 * D, hin, D, D, at(lg.in_proj_w, D * D)));
     {  // dH(in) = dKV W[K|V rows]  for every frame
       GemmProblem g = dgrad(c, "gemm.last.bwd.kv_dgrad", pl.dqkv, Mt, 2 * D, pl.w_in[l] + D * D, D);
       c.out(g.epi, pl.dh_a, 0, D);
@@ -961,7 +975,7 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
       g.B = c.mat(pl.datt, 0, T, 64, D, 64, sA1);
       g.a_mn = true; g.b_mn = true;
       g.planes = P; g.M = T; g.N = 64; g.K = T; g.nb0 = H; g.nb1 = B;
-      g.epi.flags = EPI_COLSUM; g.epi.colsum = lg.in_proj_b + 2 * D; g.epi.colsum_sb0 = 64;
+      g.epi.flags = c.colsum(); g.epi.colsum = at(lg.in_proj_b, 2 * D); g.epi.colsum_sb0 = 64;
       c.out(g.epi, pl.dqkv, 2 * D, 3 * D, sQ0, sQ1);
       SPK_TRY(c.run(g));
     }
@@ -985,7 +999,7 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
       g.B = c.mat(b.qkv, D, T, 64, 3 * D, sQ0, sQ1);
       g.b_mn = true;
       g.planes = P; g.M = T; g.N = 64; g.K = T; g.nb0 = H; g.nb1 = B;
-      g.epi.flags = EPI_COLSUM; g.epi.colsum = lg.in_proj_b; g.epi.colsum_sb0 = 64;
+      g.epi.flags = c.colsum(); g.epi.colsum = lg.in_proj_b; g.epi.colsum_sb0 = 64;
       c.out(g.epi, pl.dqkv, 0, 3 * D, sQ0, sQ1);
       SPK_TRY(c.run(g));
     }
@@ -996,7 +1010,7 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
       g.B = c.mat(b.qkv, 0, T, 64, 3 * D, sQ0, sQ1);
       g.a_mn = true; g.b_mn = true;
       g.planes = P; g.M = T; g.N = 64; g.K = T; g.nb0 = H; g.nb1 = B;
-      g.epi.flags = EPI_COLSUM; g.epi.colsum = lg.in_proj_b + D; g.epi.colsum_sb0 = 64;
+      g.epi.flags = c.colsum(); g.epi.colsum = at(lg.in_proj_b, D); g.epi.colsum_sb0 = 64;
       c.out(g.epi, pl.dqkv, D, 3 * D, sQ0, sQ1);
       SPK_TRY(c.run(g));
     }
@@ -1020,7 +1034,7 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
     {
       GemmProblem g = linear(c, "gemm.bwd.prenet_gate", pl.x0, Mt, pl.C, pl.C, pl.w_pre, D);
       g.planes = P_fwd;   // same operand planes as the forward prenet GEMM, so the recomputed ReLU gate is the forward's gate
-      g.epi.flags = EPI_BIAS | EPI_ACC_GATES_AUX | EPI_COLSUM;
+      g.epi.flags = EPI_BIAS | EPI_ACC_GATES_AUX | c.colsum();
       g.epi.colsum = gr.prenet_b;
       g.epi.bias = w.prenet_b; g.epi.drop = drop_pe; g.epi.drop_site = 0;
       c.res(g.epi, pl.dh_a, D);
@@ -1029,6 +1043,17 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
     }
   }
   SPK_TRY(wgrad(c, "gemm.bwd.prenet_wgrad", Mt, pl.dh_b, D, pl.x0, pl.C, pl.C, gr.prenet_w));
+  if (d_mel != nullptr) {
+    // ---- input: dX = dU W_pre (fp32, token-major, into dh_a: dead after the prenet backward, Mt * 512 >= Mt * 320
+    // bytes), then transposed to the [B, mel, T] layout of the input.  dU carries the gradient scale S: alpha = 1 / S.
+    float* dx = reinterpret_cast<float*>(c.ptr(pl.dh_a));
+    GemmProblem g = dgrad(c, "gemm.bwd.mel_dgrad", pl.dh_b, Mt, D, pl.w_pre, pl.C);
+    g.epi.flags = EPI_OUT_F32;
+    g.epi.alpha_ptr = gs + 1;
+    g.epi.out = dx; g.epi.out_ld = pl.C; g.epi.out_planes = 1;
+    SPK_TRY(c.run(g));
+    SPK_TRY(mel_grad_unpack(dx, d_mel, B, pl.C, T, st));
+  }
   return 0;
 }
 

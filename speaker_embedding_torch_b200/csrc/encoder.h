@@ -10,9 +10,10 @@ size_t encoder_workspace_bytes(const spk_encoder_config& c, int B, int T, int S,
 int encoder_forward(const spk_encoder_config& cfg, const spk_encoder_params& w, const spk_mel_view* mel,
                     const spk_mel_ragged* ragged, int B, int T, int S, int P, int training, uint64_t seed, float* dvec,
                     void* ws, size_t ws_bytes, int keep, cudaStream_t st);
-int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w, const spk_encoder_params& gr,
-                     const float* d_dvec, int B, int T, int S, int P, int training, uint64_t seed, void* ws,
-                     size_t ws_bytes, cudaStream_t st);
+// grads null: no parameter gradient; d_mel null: no input gradient
+int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w, const spk_encoder_params* grads,
+                     float* d_mel, const float* d_dvec, int B, int T, int S, int P, int training, uint64_t seed,
+                     void* ws, size_t ws_bytes, cudaStream_t st);
 int encoder_debug_layout(const spk_encoder_config& c, int B, int T, int S, int P, int keep, char* buf, size_t cap);
 void encoder_set_prune(bool on);
 void encoder_set_fused_attn(bool on);

@@ -84,6 +84,32 @@ int mel_pack(const spk_mel_view& mel, void* out, int64_t plane_stride, int plane
   return 0;
 }
 
+// The mirror of mel_pack_kernel for the input gradient: token-major fp32 [B*T, C] -> d_mel [B, C, T] fp32.  The block's
+// 32 tokens are C * 32 consecutive floats on the read side and 32-frame runs of every channel on the write side; the
+// shared tile turns one into the other so that both are coalesced.
+template <int C>
+__global__ void mel_grad_unpack_kernel(const float* __restrict__ src, float* __restrict__ d_mel, int T) {
+  __shared__ float tile[C][33];
+  const int b = blockIdx.y;
+  const int t0 = blockIdx.x * 32;
+  const int nt = T - t0 < 32 ? T - t0 : 32;
+  const float* s = src + (static_cast<int64_t>(b) * T + t0) * C;
+  for (int i = threadIdx.x; i < nt * C; i += blockDim.x) tile[i % C][i / C] = __ldg(s + i);
+  __syncthreads();
+  float* dst = d_mel + static_cast<int64_t>(b) * C * T + t0;
+  for (int i = threadIdx.x; i < C * 32; i += blockDim.x) {
+    const int c = i >> 5, tl = i & 31;
+    if (tl < nt) dst[static_cast<int64_t>(c) * T + tl] = tile[c][tl];
+  }
+}
+int mel_grad_unpack(const float* src, float* d_mel, int B, int C, int T, cudaStream_t st) {
+  ProfScope prof("mel_grad_unpack", 0, 8.0 * B * C * T, st);
+  SPK_CHECK(C == 80, "mel_grad_unpack: Mel_Dim %d not supported by this build (80)", C);
+  mel_grad_unpack_kernel<80><<<dim3((T + 31) / 32, B), 256, 0, st>>>(src, d_mel, T);
+  SPK_CUDA(cudaGetLastError());
+  return 0;
+}
+
 // Training collation on the device (Datasets.py:9-19 `Correction`, :72-86 `Collater`): the batch arrives as ONE ragged
 // array [C, total_frames] (the utterances' patterns concatenated along time, fp16 as stored or fp32) plus a table
 // (start, length, offset) per utterance; every utterance is cut (length > T: frames [offset, offset + T)) or
@@ -243,6 +269,7 @@ int ln_fwd(const void* z, int64_t z_ps, int z_planes, int64_t z_row_step, const 
 
 // dz = rstd * (g - mean(g) - xhat * mean(g * xhat)),  g = dy * gamma ; dgamma += dy * xhat ; dbeta += dy
 // Optionally also writes dz_drop = dz * keep(site) (the gradient that enters the sub-layer's GEMMs).
+// dgamma == nullptr: no parameter gradient at all (dbeta and dbias are then null too); dz / dz_drop are unchanged.
 template <int PL>
 __global__ void __launch_bounds__(256, 3) ln_bwd_kernel(const elem_t* __restrict__ dy, int64_t dy_ps, int dy_planes_rt,
                                                         const elem_t* __restrict__ z, int64_t z_ps, int z_planes_rt,
@@ -320,6 +347,7 @@ __global__ void __launch_bounds__(256, 3) ln_bwd_kernel(const elem_t* __restrict
 #pragma unroll
     for (int i = 0; i < 8; ++i) az[i] += o[i];
   }
+  if (dgamma == nullptr) return;     // no parameter gradients wanted (block-uniform)
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
     red[0][wib][lane * 8 + i] = ag[i]; red[1][wib][lane * 8 + i] = ab[i]; red[2][wib][lane * 8 + i] = az[i];
@@ -603,6 +631,7 @@ int colsum(const void* x, int64_t ps, int planes, float* out, int64_t rows, int 
 // Embedding backward in one pass over dH0 (replaces pe_alpha_grad + a recomputing GEMM):
 //   g = dH0 * keep(site 0);   d_alpha += sum g * pe_t[t];   dU = g * 1[u > 0] (mask bits written by the forward prenet
 //   epilogue, layout [256 / 32][rows]);   d_bias[col] += sum_rows dU.        Modules.py:50-52,98-105
+// dbias == nullptr: only dU is written (dalpha is then null too).
 __global__ void __launch_bounds__(256) prenet_bwd_kernel(const elem_t* __restrict__ dh, int64_t ps, int planes,
                                                          const uint32_t* __restrict__ bits, const float* __restrict__ pe_t,
                                                          DropCfg drop, uint32_t site, elem_t* __restrict__ du, int64_t du_ps,
@@ -638,6 +667,7 @@ __global__ void __launch_bounds__(256) prenet_bwd_kernel(const elem_t* __restric
     }
     store8_split(du, du_ps, planes, r * 256 + lane * 8, d);
   }
+  if (dbias == nullptr) return;      // no parameter gradients wanted (block-uniform)
   acc = warp_sum(acc);
   if (lane == 0) red[wib] = acc;
 #pragma unroll
@@ -700,6 +730,7 @@ __global__ void __launch_bounds__(256) pe_alpha_grad_kernel(const elem_t* __rest
 }
 int pe_alpha_grad(const void* dh, int64_t ps, int planes, const float* pe_t, DropCfg drop, uint32_t site, float* dalpha,
                   int64_t rows, int T, const float* gscale, cudaStream_t st) {
+  if (dalpha == nullptr) return 0;   // the kernel computes nothing else
   ProfScope prof("pe_alpha_grad", 0, 512.0 * rows * planes, st);
   const int blocks = static_cast<int>(std::min<int64_t>((rows + 7) / 8, 148 * 4));
   pe_alpha_grad_kernel<<<blocks, 256, 0, st>>>(reinterpret_cast<const elem_t*>(dh), ps, planes, pe_t, drop, site,

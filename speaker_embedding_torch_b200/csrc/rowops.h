@@ -22,6 +22,8 @@ int mel_pack(const spk_mel_view& mel, void* out, int64_t plane_stride, int plane
 // ragged batch (include/spkemb.h spk_mel_ragged) -> token-major split tensor, crop / reflect-pad to T in the load
 int mel_pack_ragged(const spk_mel_ragged& mel, void* out, int64_t plane_stride, int planes, int B, int C, int T,
                     cudaStream_t st);
+// token-major fp32 [B*T, C] (the input gradient) -> fp32 [B, C, T], the layout of the mel input
+int mel_grad_unpack(const float* src, float* d_mel, int B, int C, int T, cudaStream_t st);
 int pe_transpose(const float* pe, float* pe_t, int D, int max_pos, int T, cudaStream_t st);
 
 // y[r] = LN(z[r * z_row_step]) over 256 columns; stats[r] = (mean, rstd) (may be null)
