@@ -161,6 +161,19 @@ int spk_mel_frames(int64_t samples, int n_fft, int hop);
 int spk_mel_spectrogram(const float* audio, int batch, int64_t samples, int n_fft, int hop, int win, const float* basis,
                         const int32_t* ranges, int n_mels, void* out, int out_fp16, void* stream);
 
+/* Backward of spk_mel_spectrogram with respect to the audio (the mel basis and the window are constants): for
+ * d_mel = dL/d(log-mel), fp32 [batch, n_mels, frames], d_audio fp32 [batch, samples] receives (=) dL/d(audio).
+ * The forward is recomputed from `audio`, so it needs to keep nothing.  Same arguments as the forward, plus
+ * bin_ranges: device int32 [n_fft / 2 + 1][2] = [first, last + 1) filter with a non-zero weight at every bin.
+ * Deterministic: no atomics, two identical calls give bit-identical d_audio.  hop > n_fft (negative padding) is
+ * rejected.  workspace: device memory of at least spk_mel_backward_workspace_bytes(batch, samples, n_fft, hop)
+ * bytes (one windowed frame gradient per frame, batch * frames * n_fft fp32), 16-byte aligned; that function
+ * returns 0 for a shape the backward rejects.  Argument errors return SPK_EINVAL before any CUDA call. */
+size_t spk_mel_backward_workspace_bytes(int batch, int64_t samples, int n_fft, int hop);
+int spk_mel_spectrogram_backward(const float* audio, const float* d_mel, int batch, int64_t samples, int n_fft, int hop,
+                                 int win, const float* basis, const int32_t* ranges, const int32_t* bin_ranges,
+                                 int n_mels, float* d_audio, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Test aid: the dropout keep-scale (0 or 1 / (1 - p_q), p_q = round(p * 2^16) / 2^16) of elements
  * [8 * idx8_begin, 8 * (idx8_begin + n8)) of dropout site `site` under `seed` -- the pure function of
  * (seed, site, element) that the forward and backward kernels evaluate.  Sites: 0 = positional encoding

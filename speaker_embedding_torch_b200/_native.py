@@ -26,6 +26,7 @@ EXPORTS = (
     "spk_encoder_debug_layout", "spk_set_option", "spk_encoder_forward_view", "spk_plan_flags",
     "spk_dropout_keep", "spk_encoder_forward_ragged",
     "spk_mel_frames", "spk_mel_spectrogram", "spk_set_debug_buffer", "spk_encoder_backward_input",
+    "spk_mel_backward_workspace_bytes", "spk_mel_spectrogram_backward",
 )
 
 c_f32p = ctypes.c_void_p  # device pointers travel as integers
@@ -162,6 +163,10 @@ def lib():
         L.spk_mel_frames.argtypes = [i64, i32, i32]
         L.spk_mel_spectrogram.restype = i32
         L.spk_mel_spectrogram.argtypes = [vp, i32, i64, i32, i32, i32, vp, vp, i32, vp, i32, vp]
+        L.spk_mel_backward_workspace_bytes.restype = sz
+        L.spk_mel_backward_workspace_bytes.argtypes = [i32, i64, i32, i32]
+        L.spk_mel_spectrogram_backward.restype = i32
+        L.spk_mel_spectrogram_backward.argtypes = [vp, vp, i32, i64, i32, i32, i32, vp, vp, vp, i32, vp, vp, sz, vp]
         L.spk_dropout_keep.restype = i32
         L.spk_dropout_keep.argtypes = [u64, f32, ctypes.c_uint32, u64, i64, vp, vp]
         L.spk_plan_flags.restype = i32

@@ -93,6 +93,17 @@ int spk_mel_spectrogram(const float* audio, int batch, int64_t samples, int n_ff
   return r < 0 ? r : 0;
 }
 
+size_t spk_mel_backward_workspace_bytes(int batch, int64_t samples, int n_fft, int hop) {
+  return mel_backward_workspace_bytes(batch, samples, n_fft, hop);
+}
+
+int spk_mel_spectrogram_backward(const float* audio, const float* d_mel, int batch, int64_t samples, int n_fft, int hop,
+                                 int win, const float* basis, const int32_t* ranges, const int32_t* bin_ranges,
+                                 int n_mels, float* d_audio, void* workspace, size_t workspace_bytes, void* stream) {
+  return mel_spectrogram_backward(audio, d_mel, batch, samples, n_fft, hop, win, basis, ranges, bin_ranges, n_mels,
+                                  d_audio, workspace, workspace_bytes, as_stream(stream));
+}
+
 int spk_dropout_keep(uint64_t seed, float p, uint32_t site, uint64_t idx8_begin, int64_t n8, float* out, void* stream) {
   return dropout_keep(seed, p, site, idx8_begin, n8, out, as_stream(stream));
 }
