@@ -147,6 +147,34 @@ int spk_encoder_backward_input(const spk_encoder_config* cfg, const spk_encoder_
                                int frames, int samples, int precision, int training, uint64_t seed,
                                void* workspace, size_t workspace_bytes, void* stream);
 
+/* Variable-length utterances: mel is a ragged SLICE batch (one table row per slice, see spk_mel_ragged); slices
+ * segments[u] .. segments[u+1]-1 form utterance u and their embeddings are averaged with 1 / count; dvec
+ * [utterances, emb].  segments: device int32 [utterances + 1], segments[0] = 0, non-decreasing, every utterance at
+ * least one slice, segments[utterances] = batch.  The library does not read the device array on the host, so it cannot
+ * check this: entries are clamped to [0, batch] (nothing is read or written past the batch), and a slice that no
+ * segment covers contributes to no d-vector and receives a zero gradient.
+ * segments NULL: batch / utterances slices per utterance, i.e. spk_encoder_forward_ragged at samples = batch /
+ * utterances.  Workspace: spk_encoder_workspace_bytes(cfg, batch, frames, 1, precision, keep_stash) with segments,
+ * samples = batch / utterances without.  Modules.utterance_slices builds the table and the segments from
+ * utterance lengths. */
+int spk_encoder_forward_segments(const spk_encoder_config* cfg, const spk_encoder_params* weights,
+                                 const spk_mel_ragged* mel, const int32_t* segments, int utterances, int batch,
+                                 int frames, int precision, int training, uint64_t seed, float* dvec,
+                                 void* workspace, size_t workspace_bytes, int keep_stash, void* stream);
+/* Backward of spk_encoder_forward_segments, or of spk_encoder_forward_ragged (segments NULL: batch / utterances
+ * slices each), with the same cfg / shape / precision / training / seed / workspace.  grads as in
+ * spk_encoder_backward_input.  d_data NULL or fp32 [mel_dim, total_frames]: receives (=) dL/d(mel->data), the
+ * adjoint of the crop / reflect-pad; columns no slice reads receive 0.  Slices group by utterance; PRECONDITION: the
+ * column spans of different utterances (smallest start .. largest start + length of their slices) do not overlap.
+ * Deterministic: no atomics on d_data, two identical calls give bit-identical results.  Argument errors (utterances
+ * < 1, batch < utterances, segments NULL and batch % utterances != 0, grads and d_data both NULL, missing data /
+ * table, bad dtype) return SPK_EINVAL before any CUDA call. */
+int spk_encoder_backward_segments(const spk_encoder_config* cfg, const spk_encoder_params* weights,
+                                  const spk_encoder_params* grads, const spk_mel_ragged* mel,
+                                  const int32_t* segments, int utterances, float* d_data, const float* d_dvec,
+                                  int batch, int frames, int precision, int training, uint64_t seed,
+                                  void* workspace, size_t workspace_bytes, void* stream);
+
 /* Test aid: text table "name byte_offset plane_stride" of the workspace buffers (returns bytes written). */
 int spk_encoder_debug_layout(const spk_encoder_config* cfg, int batch, int frames, int samples, int precision,
                              int keep_stash, char* buf, size_t cap);

@@ -22,10 +22,17 @@ import torch
 
 class RaggedMel:
     """A batch of variable-length patterns: ``data`` [Mel_Dim, total_frames] (fp16 or fp32), ``table`` int32 [B, 3] =
-    (start column, length, crop offset) per utterance, and the batch's common frame count."""
+    (start column, length, crop offset) per slice, and the batch's common frame count.
 
-    def __init__(self, data, table, frames, _checked=False):
-        self.data, self.table, self.frames = data, table, int(frames)
+    ``segments`` (optional, int32 [U + 1]): slices ``segments[u] .. segments[u+1] - 1`` form utterance ``u``, and
+    ``GE2E.forward`` returns one d-vector per utterance (the mean over its slices; ``Modules.utterance_slices`` builds
+    such a batch).  Without it the slices group in runs of ``samples``.  An input gradient (``data.requires_grad``)
+    needs the column spans of different utterances to be disjoint; the host copy of the table is kept to check that
+    without a device synchronisation."""
+
+    def __init__(self, data, table, frames, segments=None, _checked=False, _host=None):
+        self.data, self.table, self.frames, self.segments = data, table, int(frames), segments
+        self._host = _host              # (table, segments) on the host, when known
         if not _checked and not table.is_cuda:      # host-side construction: validate once, before the copy
             t = table.to(torch.int64)
             if table.dim() != 2 or table.size(1) != 3 or data.dim() != 2 or self.frames < 1:
@@ -34,6 +41,43 @@ class RaggedMel:
                               or int(t[:, 0].min()) < 0 or int(t[:, 2].min()) < 0
                               or bool(((t[:, 1] > self.frames) & (t[:, 2] + self.frames > t[:, 1])).any())):
                 raise RuntimeError("RaggedMel: table entries point outside the pattern array")
+            if segments is not None:
+                if segments.is_cuda:
+                    raise RuntimeError("RaggedMel: table and segments must both be host tensors (or both on the device)")
+                g = segments.to(torch.int64)
+                if (g.dim() != 1 or g.numel() < 2 or int(g[0]) != 0 or int(g[-1]) != table.size(0)
+                        or bool((g[1:] <= g[:-1]).any())):
+                    raise RuntimeError("RaggedMel: segments must be increasing from 0 to the number of slices %d "
+                                       "(every utterance at least one slice)" % table.size(0))
+            self._host = (table, segments)
+
+    @property
+    def utterances(self):
+        """Number of d-vectors with segments; None without (the slices group by ``samples``)."""
+        return None if self.segments is None else self.segments.numel() - 1
+
+    def spans_disjoint(self, samples=1):
+        """True when the column spans of different utterances do not overlap (utterance = segment, or a run of
+        ``samples`` slices without segments).  Uses the host copy of the table; synchronises only when there is none."""
+        key = ("disjoint", samples)
+        cache = getattr(self, "_cache", None)
+        if cache is None:
+            cache = self._cache = {}
+        if key not in cache:
+            table, segments = self._host if self._host is not None else (self.table.cpu(), None)
+            if segments is None and self.segments is not None:
+                segments = self.segments.cpu()
+            t = table.to(torch.int64)
+            B = t.size(0)
+            if segments is None:
+                segments = torch.arange(0, B + 1, samples, dtype=torch.int64)
+            g = segments.to(torch.int64)
+            group = torch.repeat_interleave(torch.arange(g.numel() - 1), g[1:] - g[:-1])
+            lo = torch.full((g.numel() - 1,), 2 ** 62, dtype=torch.int64).scatter_reduce(0, group, t[:, 0], "amin")
+            hi = torch.zeros(g.numel() - 1, dtype=torch.int64).scatter_reduce(0, group, t[:, 0] + t[:, 1], "amax")
+            order = torch.argsort(lo)
+            cache[key] = bool((lo[order][1:] >= hi[order][:-1]).all())
+        return cache[key]
 
     # --- the little of the tensor API that Train.py touches
     @property
@@ -55,11 +99,15 @@ class RaggedMel:
         return self.data.is_cuda
 
     def pin_memory(self):
-        return RaggedMel(self.data.pin_memory(), self.table.pin_memory(), self.frames, _checked=True)
+        return RaggedMel(self.data.pin_memory(), self.table.pin_memory(), self.frames,
+                         None if self.segments is None else self.segments.pin_memory(), _checked=True,
+                         _host=self._host)
 
     def to(self, device, non_blocking=False):
         return RaggedMel(self.data.to(device, non_blocking=non_blocking),
-                         self.table.to(device, non_blocking=non_blocking), self.frames, _checked=True)
+                         self.table.to(device, non_blocking=non_blocking), self.frames,
+                         None if self.segments is None else self.segments.to(device, non_blocking=non_blocking),
+                         _checked=True, _host=self._host)
 
     def cuda(self, non_blocking=False):
         return self.to("cuda", non_blocking=non_blocking)

@@ -27,7 +27,7 @@ import torch
 
 from . import _native as N
 
-__all__ = ["GE2E", "GE2E_Loss", "Conv1d", "Positional_Encoding"]
+__all__ = ["GE2E", "GE2E_Loss", "Conv1d", "Positional_Encoding", "utterance_slices"]
 
 
 # ------------------------------------------------------------------------------------------------
@@ -115,19 +115,26 @@ def _aligned_ptr(ws):
     return ctypes.c_void_p((base + 255) // 256 * 256)
 
 
-def _run_forward(cfg, names, params, pe, features, samples, precision, training, seed, keep, slicing=None):
+def _run_forward(cfg, names, params, pe, features, samples, precision, training, seed, keep, slicing=None,
+                 return_ragged=False):
     """One spk_encoder_forward_view call.  ``features`` is ``[Batch*Samples, Mel_Dim, Time]`` (fp32 or fp16: the
     reference stores its patterns as fp16, the upcast happens in the prenet load), or -- with
     ``slicing = (frame_length, hop, slices_per_window)`` -- un-sliced windows ``[Utterances, Mel_Dim, L]`` whose
-    overlapping slices are cut by the same load."""
+    overlapping slices are cut by the same load.  ``return_ragged``: also return the RaggedMel the call read
+    (contiguous data, int32 table / segments), or None for a dense input."""
     from .Datasets import RaggedMel
     ragged = features if isinstance(features, RaggedMel) else None
     if ragged is not None:            # training batch collated on the device (Datasets.Collater)
         N.require_cuda(ragged.data, "features")
         N.require_cuda(ragged.table, "features.table")
-        if ragged.data.dtype not in (torch.float32, torch.float16):
-            ragged = RaggedMel(ragged.data.float(), ragged.table, ragged.frames, _checked=True)
-        ragged = RaggedMel(ragged.data.contiguous(), ragged.table.to(torch.int32).contiguous(), ragged.frames,
+        data = ragged.data if ragged.data.dtype in (torch.float32, torch.float16) else ragged.data.float()
+        segments = ragged.segments
+        if segments is not None:
+            N.require_cuda(segments, "features.segments")
+            segments = segments.to(torch.int32).contiguous()
+            if samples != 1:
+                raise RuntimeError("a RaggedMel with segments gives one d-vector per segment: samples must be 1")
+        ragged = RaggedMel(data.contiguous(), ragged.table.to(torch.int32).contiguous(), ragged.frames, segments,
                            _checked=True)
         features = ragged.data            # device / dtype bookkeeping below
         if slicing is not None or ragged.data.dim() != 2 or ragged.data.size(0) != cfg.mel_dim:
@@ -145,6 +152,8 @@ def _run_forward(cfg, names, params, pe, features, samples, precision, training,
                            % (cfg.mel_dim, tuple(features.shape)))
     if ragged is not None:
         batch, frames = ragged.table.size(0), ragged.frames
+        if ragged.segments is not None and not 1 <= ragged.utterances <= batch:
+            raise RuntimeError("RaggedMel: %d segments for %d slices" % (ragged.utterances, batch))
     elif slicing is None:
         batch, _, frames = features.shape
         window, hop, spw = frames, 0, 1
@@ -168,10 +177,17 @@ def _run_forward(cfg, names, params, pe, features, samples, precision, training,
     with torch.cuda.device(features.device):
         weights = _fill_params(N.EncoderParams(), tensors, pe, cfg.layers)
         ws, nbytes = _workspace(cfg, batch, frames, samples, precision, int(keep), features.device)
-        dvec = torch.empty((batch // samples, cfg.emb), dtype=torch.float32, device=features.device)
-        if ragged is not None:
-            view = N.MelRagged(ragged.data.data_ptr(), 1 if ragged.data.dtype == torch.float16 else 0,
-                               ragged.data.size(1), ragged.table.data_ptr())
+        dvecs = batch // samples if ragged is None or ragged.segments is None else ragged.utterances
+        dvec = torch.empty((dvecs, cfg.emb), dtype=torch.float32, device=features.device)
+        if ragged is not None and ragged.segments is not None:      # variable slice counts per utterance
+            N.check(N.lib().spk_encoder_forward_segments(ctypes.byref(cfg), ctypes.byref(weights),
+                                                         ctypes.byref(_mel_ragged(ragged)), N.ptr(ragged.segments),
+                                                         ragged.utterances, batch, frames, precision, int(training),
+                                                         ctypes.c_uint64(seed), N.ptr(dvec), _aligned_ptr(ws), nbytes,
+                                                         int(keep), N.stream_ptr(features.device)),
+                    "spk_encoder_forward_segments")
+        elif ragged is not None:
+            view = _mel_ragged(ragged)
             N.check(N.lib().spk_encoder_forward_ragged(ctypes.byref(cfg), ctypes.byref(weights), ctypes.byref(view),
                                                        batch, frames, samples, precision, int(training),
                                                        ctypes.c_uint64(seed), N.ptr(dvec), _aligned_ptr(ws), nbytes,
@@ -184,26 +200,67 @@ def _run_forward(cfg, names, params, pe, features, samples, precision, training,
                                                      ctypes.c_uint64(seed), N.ptr(dvec), _aligned_ptr(ws), nbytes,
                                                      int(keep), N.stream_ptr(features.device)),
                     "spk_encoder_forward_view")
+    if return_ragged:
+        return dvec, ws, nbytes, (batch, frames, precision), ragged
     return dvec, ws, nbytes, (batch, frames, precision)
+
+
+def _mel_ragged(ragged):
+    return N.MelRagged(ragged.data.data_ptr(), 1 if ragged.data.dtype == torch.float16 else 0, ragged.data.size(1),
+                       ragged.table.data_ptr())
+
+
+def utterance_slices(lengths, frame_length, overlap_length, starts=None):
+    """The slicing rule of variable-length utterances, for ``GE2E.embed_utterances`` and ``RaggedMel(segments=...)``.
+
+    An utterance of ``L`` frames gives, with hop ``h = frame_length - overlap_length``:
+      * ``L <= frame_length``: one slice, the utterance reflect-padded to ``frame_length`` (numpy 'reflect', floor of
+        the missing frames on the left, ceil on the right, as ``Datasets.Correction`` does it);
+      * ``L > frame_length``: ``S = ceil((L - frame_length) / h) + 1`` slices at offsets ``min(s * h, L - frame_length)``
+        (the last one end-aligned, so every frame is covered).
+    When ``(L - frame_length) % h == 0`` these are the slices of ``Overlapped_Slices`` / ``GE2E.embed_windows``.
+    ``starts``: the first column of every utterance in the ragged array (default: the utterances back to back).
+    Returns ``(table int32 [slices, 3] = (start, length, offset), segments int32 [utterances + 1])`` on the host."""
+    T, hop = int(frame_length), int(frame_length) - int(overlap_length)
+    if T < 1 or hop <= 0:
+        raise RuntimeError("invalid slicing: frame_length %d, overlap_length %d" % (frame_length, overlap_length))
+    L = torch.as_tensor(lengths, dtype=torch.int64).reshape(-1)
+    if L.numel() == 0 or int(L.min()) < 1:
+        raise RuntimeError("utterance lengths must be >= 1 frame")
+    if starts is None:
+        starts = torch.cumsum(L, 0) - L
+    starts = torch.as_tensor(starts, dtype=torch.int64).reshape(-1)
+    extra = (L - T).clamp(min=0)
+    count = torch.where(L > T, (extra + hop - 1) // hop + 1, torch.ones_like(L))
+    segments = torch.zeros(L.numel() + 1, dtype=torch.int64)
+    segments[1:] = torch.cumsum(count, 0)
+    utt = torch.repeat_interleave(torch.arange(L.numel()), count)
+    s = torch.arange(int(segments[-1])) - segments[:-1][utt]
+    offset = torch.minimum(s * hop, extra[utt])
+    table = torch.stack([starts[utt], L[utt], offset], dim=1)
+    return table.to(torch.int32), segments.to(torch.int32)
 
 
 class _EncoderFunction(torch.autograd.Function):
     """Differentiable encoder call: forward keeps the activation stash, backward runs
     spk_encoder_backward into one flat fp32 gradient buffer (returned as per-parameter views).  When ``features`` needs
     a gradient the backward is spk_encoder_backward_input, which also writes dL/d(features); with every parameter
-    frozen it computes no parameter gradient at all and allocates no gradient arena."""
+    frozen it computes no parameter gradient at all and allocates no gradient arena.  ``ragged``: a RaggedMel whose
+    ``data`` is ``features``; its backward is spk_encoder_backward_segments, which folds the slices' gradient back
+    onto ``data``."""
 
     @staticmethod
-    def forward(ctx, features, module, samples, precision, training, seed, *params):
+    def forward(ctx, features, module, samples, precision, training, seed, ragged, *params):
         names = module._param_names
         cfg = module._cfg
         pe = module.positional_encoding.pe
-        dvec, ws, nbytes, (batch, frames, precision) = _run_forward(cfg, names, [p.detach() for p in params], pe,
-                                                                    features, samples, precision, training, seed,
-                                                                    keep=True)
+        dvec, ws, nbytes, (batch, frames, precision), used = _run_forward(
+            cfg, names, [p.detach() for p in params], pe, ragged if ragged is not None else features, samples,
+            precision, training, seed, keep=True, return_ragged=True)
         ctx.module, ctx.ws, ctx.nbytes = module, ws, nbytes
         ctx.meta = (batch, frames, samples, precision, training, seed)
-        ctx.features_dtype = features.dtype if isinstance(features, torch.Tensor) else None
+        ctx.ragged = used                 # the contiguous int32 table / segments the forward read (kept alive)
+        ctx.features_dtype = features.dtype
         ctx.save_for_backward(*params)
         ctx.pe = pe
         return dvec
@@ -218,7 +275,8 @@ class _EncoderFunction(torch.autograd.Function):
         grad_dvec = grad_dvec.contiguous().float()
         want_mel = ctx.needs_input_grad[0]
         # partial freezing keeps the full arena: only a fully frozen encoder skips the parameter gradients
-        want_params = not want_mel or any(ctx.needs_input_grad[6:])
+        want_params = not want_mel or any(ctx.needs_input_grad[7:])
+        ragged = ctx.ragged
         views, d_mel = None, None
         if want_params:
             sizes = [p.numel() for p in params]
@@ -232,7 +290,21 @@ class _EncoderFunction(torch.autograd.Function):
             weights = _fill_params(N.EncoderParams(), dict(zip(names, [p.detach() for p in params])), ctx.pe,
                                    cfg.layers)
             grads = _fill_params(N.EncoderParams(), dict(zip(names, views)), None, cfg.layers) if want_params else None
-            if not want_mel:
+            if ragged is not None and (want_mel or ragged.segments is not None):
+                utterances = ragged.utterances if ragged.segments is not None else batch // samples
+                if want_mel:
+                    d_mel = torch.empty((cfg.mel_dim, ragged.data.size(1)), dtype=torch.float32, device=device)
+                N.check(N.lib().spk_encoder_backward_segments(ctypes.byref(cfg), ctypes.byref(weights),
+                                                              ctypes.byref(grads) if want_params else None,
+                                                              ctypes.byref(_mel_ragged(ragged)),
+                                                              N.ptr(ragged.segments), utterances, N.ptr(d_mel),
+                                                              N.ptr(grad_dvec), batch, frames, precision,
+                                                              int(training), ctypes.c_uint64(seed),
+                                                              _aligned_ptr(ctx.ws), ctx.nbytes, N.stream_ptr(device)),
+                        "spk_encoder_backward_segments")
+                if want_mel:
+                    d_mel = d_mel.to(ctx.features_dtype)
+            elif not want_mel:
                 N.check(N.lib().spk_encoder_backward(ctypes.byref(cfg), ctypes.byref(weights), ctypes.byref(grads),
                                                      N.ptr(grad_dvec), batch, frames, samples, precision,
                                                      int(training), ctypes.c_uint64(seed), _aligned_ptr(ctx.ws),
@@ -249,8 +321,8 @@ class _EncoderFunction(torch.autograd.Function):
                 d_mel = d_mel.to(ctx.features_dtype)      # fp16 patterns get an fp16 gradient
         if getattr(module, "_debug_keep_ws", False):      # parity tests read the stage buffers back
             module._last_ws, module._last_meta = ctx.ws, ctx.meta
-        ctx.ws = None
-        return (d_mel, None, None, None, None, None) + (tuple(views) if want_params else (None,) * len(params))
+        ctx.ws = ctx.ragged = None
+        return (d_mel, None, None, None, None, None, None) + (tuple(views) if want_params else (None,) * len(params))
 
 
 class GE2E(torch.nn.Module):
@@ -312,20 +384,26 @@ class GE2E(torch.nn.Module):
         return arena
 
     def forward(self, features, samples=1):
-        """features: [Batch * Sample, Mel_dim, Time] -> [Batch, Emb_dim] unit-norm d-vectors."""
+        """features: [Batch * Sample, Mel_dim, Time] -> [Batch, Emb_dim] unit-norm d-vectors.  A ``RaggedMel``
+        (Datasets.py) is cropped / reflect-padded on the device; with ``segments`` it gives one d-vector per segment
+        (``samples`` must be 1).  Its ``data`` gets a gradient like a dense input when it requires one."""
+        from .Datasets import RaggedMel
         samples = int(samples)
         params = list(self.parameters())
+        ragged = features if isinstance(features, RaggedMel) else None
         # a frozen encoder used as a critic still differentiates with respect to its input
-        input_grad = isinstance(features, torch.Tensor) and features.requires_grad
+        input_grad = (ragged.data if ragged is not None else features).requires_grad
         need_grad = torch.is_grad_enabled() and (input_grad or any(p.requires_grad for p in params))
         if need_grad:
+            if ragged is not None and input_grad and not ragged.spans_disjoint(samples):
+                raise RuntimeError("RaggedMel: the column spans of different utterances overlap, so their gradients "
+                                   "cannot be folded back onto `data`; give every utterance its own columns")
             seed = int(torch.empty((), dtype=torch.int64).random_().item()) if self.training else 0
-            return _EncoderFunction.apply(features, self, samples, self.train_precision, self.training, seed,
-                                          *params)
+            return _EncoderFunction.apply(ragged.data if ragged is not None else features, self, samples,
+                                          self.train_precision, self.training, seed, ragged, *params)
         if self.training:
             raise RuntimeError("GE2E.forward in train() mode without gradients is not supported; call eval()")
-        from .Datasets import RaggedMel
-        if isinstance(features, RaggedMel):       # evaluation batches of the device collater (Train.py:198-212)
+        if ragged is not None:       # evaluation batches of the device collater (Train.py:198-212)
             return _run_forward(self._cfg, self._param_names, [p.detach() for p in params],
                                 self.positional_encoding.pe, features, samples, self.eval_precision, False, 0,
                                 keep=False)[0]
@@ -356,6 +434,55 @@ class GE2E(torch.nn.Module):
                 outs.append(_run_forward(self._cfg, self._param_names, params, pe, windows[u:u + per_call], spw,
                                          self.eval_precision, False, 0, keep=False,
                                          slicing=(int(frame_length), hop, spw))[0])
+        return outs[0] if len(outs) == 1 else torch.cat(outs, dim=0)
+
+
+    def embed_utterances(self, mels, frame_length, overlap_length, lengths=None):
+        """Whole-utterance d-vectors of utterances of different lengths in one pass: every utterance is cut into
+        ``frame_length``-frame slices by the rule of ``utterance_slices`` (short ones reflect-padded, long ones
+        covered to their last frame), and its d-vector is the head over its own slices.  Returns ``[U, Emb_dim]``.
+
+        ``mels``: a list of ``[Mel_Dim, L_u]`` tensors, or a padded ``[U, Mel_Dim, L_max]`` tensor with ``lengths``
+        (padding columns are never read and get a zero gradient).  fp32 or fp16.  Runs at ``eval_precision`` in
+        chunks of at most ``max_slices_per_call`` slices that never split an utterance; differentiable (at
+        ``train_precision``, like ``forward``) when gradients are enabled and the mels or any parameter require them."""
+        from .Datasets import RaggedMel
+        if isinstance(mels, (list, tuple)):
+            if lengths is not None:
+                raise RuntimeError("embed_utterances: lengths is only for a padded [U, Mel_Dim, L_max] tensor")
+            if not mels or any(m.dim() != 2 or m.size(0) != self._cfg.mel_dim for m in mels):
+                raise RuntimeError("embed_utterances: every utterance must be [Mel_Dim=%d, L]" % self._cfg.mel_dim)
+            lens = torch.tensor([m.size(1) for m in mels], dtype=torch.int64)
+            starts = torch.cumsum(lens, 0) - lens
+            data = torch.cat(list(mels), dim=1)
+        else:
+            if mels.dim() != 3 or mels.size(1) != self._cfg.mel_dim or lengths is None:
+                raise RuntimeError("embed_utterances: a padded batch is [U, Mel_Dim=%d, L_max] with lengths"
+                                   % self._cfg.mel_dim)
+            lens = torch.as_tensor(lengths, dtype=torch.int64).cpu().reshape(-1)
+            U, _, L_max = mels.shape
+            if lens.numel() != U or int(lens.min()) < 1 or int(lens.max()) > L_max:
+                raise RuntimeError("embed_utterances: lengths must be %d values in [1, %d]" % (U, L_max))
+            starts = torch.arange(U, dtype=torch.int64) * L_max
+            data = mels.permute(1, 0, 2).reshape(mels.size(1), U * L_max)     # one transposing copy
+        table, segments = utterance_slices(lens, frame_length, overlap_length, starts)
+        end = starts + lens
+        device = data.device
+        outs, u0 = [], 0
+        U = lens.numel()
+        seg = segments.to(torch.int64)
+        while u0 < U:
+            # whole utterances, at most max_slices_per_call slices (one utterance always fits a call)
+            u1 = int(torch.searchsorted(seg, seg[u0] + self.max_slices_per_call, right=True)) - 1
+            u1 = min(max(u1, u0 + 1), U)
+            s0, s1 = int(seg[u0]), int(seg[u1])
+            c0, c1 = int(starts[u0:u1].min()), int(end[u0:u1].max())
+            t = table[s0:s1].clone()
+            t[:, 0] -= c0
+            chunk = RaggedMel(data[:, c0:c1], t, frame_length, segments[u0:u1 + 1] - s0, _checked=True,
+                              _host=(t, segments[u0:u1 + 1] - s0))
+            outs.append(self.forward(chunk.to(device)))
+            u0 = u1
         return outs[0] if len(outs) == 1 else torch.cat(outs, dim=0)
 
 

@@ -27,6 +27,7 @@ EXPORTS = (
     "spk_dropout_keep", "spk_encoder_forward_ragged",
     "spk_mel_frames", "spk_mel_spectrogram", "spk_set_debug_buffer", "spk_encoder_backward_input",
     "spk_mel_backward_workspace_bytes", "spk_mel_spectrogram_backward",
+    "spk_encoder_forward_segments", "spk_encoder_backward_segments",
 )
 
 c_f32p = ctypes.c_void_p  # device pointers travel as integers
@@ -134,6 +135,14 @@ def lib():
         L.spk_encoder_forward_ragged.argtypes = [ctypes.POINTER(EncoderConfig), ctypes.POINTER(EncoderParams),
                                                  ctypes.POINTER(MelRagged), i32, i32, i32, i32, i32, u64, vp, vp, sz,
                                                  i32, vp]
+        L.spk_encoder_forward_segments.restype = i32
+        L.spk_encoder_forward_segments.argtypes = [ctypes.POINTER(EncoderConfig), ctypes.POINTER(EncoderParams),
+                                                   ctypes.POINTER(MelRagged), vp, i32, i32, i32, i32, i32, u64, vp,
+                                                   vp, sz, i32, vp]
+        L.spk_encoder_backward_segments.restype = i32
+        L.spk_encoder_backward_segments.argtypes = [ctypes.POINTER(EncoderConfig), ctypes.POINTER(EncoderParams),
+                                                    ctypes.POINTER(EncoderParams), ctypes.POINTER(MelRagged), vp, i32,
+                                                    vp, vp, i32, i32, i32, i32, u64, vp, sz, vp]
         L.spk_encoder_backward.restype = i32
         L.spk_encoder_backward.argtypes = [ctypes.POINTER(EncoderConfig), ctypes.POINTER(EncoderParams),
                                            ctypes.POINTER(EncoderParams), vp, i32, i32, i32, i32, i32, u64,

@@ -54,6 +54,43 @@ int spk_encoder_forward_ragged(const spk_encoder_config* cfg, const spk_encoder_
                          workspace, workspace_bytes, keep_stash, as_stream(stream));
 }
 
+// Shape checks shared by the two segmented entry points; host-only, before any CUDA call.
+static int check_segments(const char* fn, const spk_mel_ragged* mel, const int32_t* segments, int utterances,
+                          int batch) {
+  SPK_CHECK(mel->data && mel->table && (mel->dtype == 0 || mel->dtype == 1) && mel->total_frames > 0,
+            "%s: ragged mel needs data, table, total_frames > 0 and dtype 0 (fp32) / 1 (fp16)", fn);
+  SPK_CHECK(utterances >= 1 && batch >= utterances, "%s: need 1 <= utterances <= batch (got %d, %d)", fn, utterances,
+            batch);
+  SPK_CHECK(segments || batch % utterances == 0, "%s: segments is NULL and batch %d is not a multiple of utterances %d",
+            fn, batch, utterances);
+  return 0;
+}
+
+int spk_encoder_forward_segments(const spk_encoder_config* cfg, const spk_encoder_params* weights,
+                                 const spk_mel_ragged* mel, const int32_t* segments, int utterances, int batch,
+                                 int frames, int precision, int training, uint64_t seed, float* dvec, void* workspace,
+                                 size_t workspace_bytes, int keep_stash, void* stream) {
+  SPK_CHECK(cfg && weights && mel && dvec && workspace, "spk_encoder_forward_segments: null argument");
+  SPK_TRY(check_segments("spk_encoder_forward_segments", mel, segments, utterances, batch));
+  const int samples = segments ? 1 : batch / utterances;
+  return encoder_forward(*cfg, *weights, nullptr, mel, batch, frames, samples, precision, training, seed, dvec,
+                         workspace, workspace_bytes, keep_stash, as_stream(stream), segments, utterances);
+}
+
+int spk_encoder_backward_segments(const spk_encoder_config* cfg, const spk_encoder_params* weights,
+                                  const spk_encoder_params* grads, const spk_mel_ragged* mel, const int32_t* segments,
+                                  int utterances, float* d_data, const float* d_dvec, int batch, int frames,
+                                  int precision, int training, uint64_t seed, void* workspace, size_t workspace_bytes,
+                                  void* stream) {
+  SPK_CHECK(cfg && weights && mel && d_dvec && workspace, "spk_encoder_backward_segments: null argument");
+  SPK_CHECK(grads || d_data, "spk_encoder_backward_segments: grads and d_data are both NULL (nothing to compute)");
+  SPK_TRY(check_segments("spk_encoder_backward_segments", mel, segments, utterances, batch));
+  const int samples = segments ? 1 : batch / utterances;
+  RaggedGrad rg{mel, segments, utterances, d_data};
+  return encoder_backward(*cfg, *weights, grads, nullptr, d_dvec, batch, frames, samples, precision, training, seed,
+                          workspace, workspace_bytes, as_stream(stream), &rg);
+}
+
 int spk_encoder_backward(const spk_encoder_config* cfg, const spk_encoder_params* weights,
                          const spk_encoder_params* grads, const float* d_dvec, int batch, int frames, int samples,
                          int precision, int training, uint64_t seed, void* workspace, size_t workspace_bytes,

@@ -311,13 +311,26 @@ __global__ void __launch_bounds__(1024) grad_scale_kernel(const float* __restric
 // `samples` slices of an utterance, 256x256 projection (fp32), L2 normalisation.
 // Eight utterances per block, one warp each: the 256 KB projection matrix is read once per block (the first version
 // ran one utterance per block and moved 960 x 256 KB through L2 per call: 45 us for 2 MB of real work).
+// SEG (variable-length utterances): utterance u owns slices segments[u] .. segments[u+1] - 1 of the `batch` slices
+// and is averaged with 1 / count; S is unused.  The fixed-S instantiation never reads the two trailing arguments.
 constexpr int HEAD_UPB = 8;
+// First slice and slice count of utterance u: the device table is clamped to [0, batch), whatever it holds.
+__device__ __forceinline__ int seg_bounds(const int32_t* __restrict__ segments, int64_t u, int64_t batch,
+                                          int64_t& first) {
+  int64_t b = __ldg(segments + u), e = __ldg(segments + u + 1);
+  b = b < 0 ? 0 : (b > batch ? batch : b);
+  e = e < b ? b : (e > batch ? batch : e);
+  first = b;
+  return static_cast<int>(e - b);
+}
+template <bool SEG>
 __global__ void __launch_bounds__(256) head_fwd_kernel(const elem_t* __restrict__ h, int64_t ps, int planes,
                                                        int T, int S, const float* __restrict__ gamma,
                                                        const float* __restrict__ beta, const float* __restrict__ wp,
                                                        const float* __restrict__ bp, float* __restrict__ hn,
                                                        float2* __restrict__ hst, float* __restrict__ emean,
-                                                       float* __restrict__ epre, float* __restrict__ dvec, int64_t U) {
+                                                       float* __restrict__ epre, float* __restrict__ dvec, int64_t U,
+                                                       const int32_t* __restrict__ segments, int64_t batch) {
   __shared__ __align__(16) float em[HEAD_UPB][256];
   __shared__ float wt[256][33];                      // projection rows n0 .. n0+31, transposed: wt[k][n - n0]
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -331,29 +344,59 @@ __global__ void __launch_bounds__(256) head_fwd_kernel(const elem_t* __restrict_
     float g[8], b[8];
 #pragma unroll
     for (int i = 0; i < 8; ++i) { g[i] = __ldg(gamma + lane * 8 + i); b[i] = __ldg(beta + lane * 8 + i); }
-    for (int s = 0; s < S; ++s) {
-      const int64_t slice = u * S + s;
-      float v[8];
-      load8_split(h, ps, planes, slice * T * 256 + lane * 8, v);
-      float sum = 0.f;
+    // The fixed-S loop is spelled out apart from the SEG one: sharing the body (a lambda, a common slice range) changed
+    // the register allocation of the fixed-S kernel that the training step and the benchmark run.
+    if constexpr (SEG) {
+      int64_t first;
+      const int count = seg_bounds(segments, u, batch, first);
+      for (int s = 0; s < count; ++s) {
+        const int64_t slice = first + s;
+        float v[8];
+        load8_split(h, ps, planes, slice * T * 256 + lane * 8, v);
+        float sum = 0.f;
 #pragma unroll
-      for (int i = 0; i < 8; ++i) sum += v[i];
-      const float mean = warp_sum(sum) * (1.f / 256.f);
-      float q = 0.f;
+        for (int i = 0; i < 8; ++i) sum += v[i];
+        const float mean = warp_sum(sum) * (1.f / 256.f);
+        float q = 0.f;
 #pragma unroll
-      for (int i = 0; i < 8; ++i) { v[i] -= mean; q += v[i] * v[i]; }
-      const float rstd = rsqrtf(warp_sum(q) * (1.f / 256.f) + 1e-5f);
-      float y[8];
+        for (int i = 0; i < 8; ++i) { v[i] -= mean; q += v[i] * v[i]; }
+        const float rstd = rsqrtf(warp_sum(q) * (1.f / 256.f) + 1e-5f);
+        float y[8];
 #pragma unroll
-      for (int i = 0; i < 8; ++i) { y[i] = v[i] * rstd * g[i] + b[i]; acc[i] += y[i]; }
-      float4* dst = reinterpret_cast<float4*>(hn + slice * 256 + lane * 8);
-      dst[0] = make_float4(y[0], y[1], y[2], y[3]);
-      dst[1] = make_float4(y[4], y[5], y[6], y[7]);
-      if (lane == 0) hst[slice] = make_float2(mean, rstd);
+        for (int i = 0; i < 8; ++i) { y[i] = v[i] * rstd * g[i] + b[i]; acc[i] += y[i]; }
+        float4* dst = reinterpret_cast<float4*>(hn + slice * 256 + lane * 8);
+        dst[0] = make_float4(y[0], y[1], y[2], y[3]);
+        dst[1] = make_float4(y[4], y[5], y[6], y[7]);
+        if (lane == 0) hst[slice] = make_float2(mean, rstd);
+      }
+      const float inv_s = 1.f / static_cast<float>(count > 0 ? count : 1);
+#pragma unroll
+      for (int i = 0; i < 8; ++i) acc[i] *= inv_s;
+    } else {
+      for (int s = 0; s < S; ++s) {
+        const int64_t slice = u * S + s;
+        float v[8];
+        load8_split(h, ps, planes, slice * T * 256 + lane * 8, v);
+        float sum = 0.f;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) sum += v[i];
+        const float mean = warp_sum(sum) * (1.f / 256.f);
+        float q = 0.f;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) { v[i] -= mean; q += v[i] * v[i]; }
+        const float rstd = rsqrtf(warp_sum(q) * (1.f / 256.f) + 1e-5f);
+        float y[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) { y[i] = v[i] * rstd * g[i] + b[i]; acc[i] += y[i]; }
+        float4* dst = reinterpret_cast<float4*>(hn + slice * 256 + lane * 8);
+        dst[0] = make_float4(y[0], y[1], y[2], y[3]);
+        dst[1] = make_float4(y[4], y[5], y[6], y[7]);
+        if (lane == 0) hst[slice] = make_float2(mean, rstd);
+      }
+      const float inv_s = 1.f / static_cast<float>(S);
+#pragma unroll
+      for (int i = 0; i < 8; ++i) acc[i] *= inv_s;
     }
-    const float inv_s = 1.f / static_cast<float>(S);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) acc[i] *= inv_s;
     float4* dst = reinterpret_cast<float4*>(emean + u * 256 + lane * 8);
     dst[0] = make_float4(acc[0], acc[1], acc[2], acc[3]);
     dst[1] = make_float4(acc[4], acc[5], acc[6], acc[7]);
@@ -403,6 +446,8 @@ __global__ void __launch_bounds__(256) head_fwd_kernel(const elem_t* __restrict_
 
 // Backward of the head, eight utterances per block (one warp each): d_dvec -> de (pre-normalisation), d_emean,
 // final-LN backward into the t = 0 rows of dH (pre-zeroed), dgamma / dbeta of the final LayerNorm (both null: skipped).
+// SEG: slices as in head_fwd_kernel<true>; each of an utterance's slices receives d_emean / count.
+template <bool SEG>
 __global__ void __launch_bounds__(256) head_bwd_kernel(const float* __restrict__ g_dvec, const float* __restrict__ epre,
                                                        const float* __restrict__ wp, const elem_t* __restrict__ h,
                                                        int64_t h_ps, int planes, const float2* __restrict__ hst,
@@ -410,7 +455,7 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(const float* __restrict__
                                                        float* __restrict__ de_out, elem_t* __restrict__ dh,
                                                        int64_t dh_ps, float* __restrict__ dgamma,
                                                        float* __restrict__ dbeta, const float* __restrict__ gscale,
-                                                       int64_t U) {
+                                                       int64_t U, const int32_t* __restrict__ segments, int64_t batch) {
   __shared__ float des[HEAD_UPB][256];
   __shared__ float wt[32][256];                      // projection rows n0 .. n0+31 (also the dgamma / dbeta exchange)
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -475,31 +520,66 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(const float* __restrict__
       for (int j = 0; j < 8; ++j) dm[j] = fmaf(wt[nl][lane + 32 * j], dv, dm[j]);
     }
   }
-  const float inv_s = 1.f / static_cast<float>(S);       // gradient of every slice's LayerNorm output
-  float ag[8], ab[8], gam[8];
+  // as in head_fwd_kernel, the fixed-S code is spelled out apart from the SEG code
+  float ag[8], ab[8];
+  if constexpr (SEG) {
+    int64_t first = 0;
+    int count = 0;
+    if (valid) count = seg_bounds(segments, u, batch, first);
+    const float inv_s = 1.f / static_cast<float>(count > 0 ? count : 1);   // gradient of every slice's LN output
+    float gam[8];
 #pragma unroll
-  for (int j = 0; j < 8; ++j) { dm[j] *= inv_s; ag[j] = 0.f; ab[j] = 0.f; gam[j] = __ldg(gamma + lane + 32 * j); }
-  if (valid) {
-    const float gsc = __ldg(gscale);                     // the gradient enters the encoder scaled by S
-    for (int s = 0; s < S; ++s) {
-      const int64_t slice = u * S + s;
-      const int64_t off = slice * T * 256 + lane;
-      const float2 ms = hst[slice];
-      float xh[8], gd[8];
-      float s1 = 0.f, s2 = 0.f;
+    for (int j = 0; j < 8; ++j) { dm[j] *= inv_s; ag[j] = 0.f; ab[j] = 0.f; gam[j] = __ldg(gamma + lane + 32 * j); }
+    if (valid) {
+      const float gsc = __ldg(gscale);                     // the gradient enters the encoder scaled by S
+      for (int s = 0; s < count; ++s) {
+        const int64_t slice = first + s;
+        const int64_t off = slice * T * 256 + lane;
+        const float2 ms = hst[slice];
+        float xh[8], gd[8];
+        float s1 = 0.f, s2 = 0.f;
 #pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        xh[j] = (load1_split(h, h_ps, planes, off + 32 * j) - ms.x) * ms.y;
-        ag[j] += dm[j] * xh[j];
-        ab[j] += dm[j];
-        gd[j] = dm[j] * gam[j];
-        s1 += gd[j];
-        s2 += gd[j] * xh[j];
+        for (int j = 0; j < 8; ++j) {
+          xh[j] = (load1_split(h, h_ps, planes, off + 32 * j) - ms.x) * ms.y;
+          ag[j] += dm[j] * xh[j];
+          ab[j] += dm[j];
+          gd[j] = dm[j] * gam[j];
+          s1 += gd[j];
+          s2 += gd[j] * xh[j];
+        }
+        const float m1 = warp_sum(s1) * (1.f / 256.f);
+        const float m2 = warp_sum(s2) * (1.f / 256.f);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) store1_split(dh, dh_ps, planes, off + 32 * j, ms.y * (gd[j] - m1 - xh[j] * m2) * gsc);
       }
-      const float m1 = warp_sum(s1) * (1.f / 256.f);
-      const float m2 = warp_sum(s2) * (1.f / 256.f);
+    }
+  } else {
+    const float inv_s = 1.f / static_cast<float>(S);       // gradient of every slice's LayerNorm output
+    float gam[8];
 #pragma unroll
-      for (int j = 0; j < 8; ++j) store1_split(dh, dh_ps, planes, off + 32 * j, ms.y * (gd[j] - m1 - xh[j] * m2) * gsc);
+    for (int j = 0; j < 8; ++j) { dm[j] *= inv_s; ag[j] = 0.f; ab[j] = 0.f; gam[j] = __ldg(gamma + lane + 32 * j); }
+    if (valid) {
+      const float gsc = __ldg(gscale);                     // the gradient enters the encoder scaled by S
+      for (int s = 0; s < S; ++s) {
+        const int64_t slice = u * S + s;
+        const int64_t off = slice * T * 256 + lane;
+        const float2 ms = hst[slice];
+        float xh[8], gd[8];
+        float s1 = 0.f, s2 = 0.f;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          xh[j] = (load1_split(h, h_ps, planes, off + 32 * j) - ms.x) * ms.y;
+          ag[j] += dm[j] * xh[j];
+          ab[j] += dm[j];
+          gd[j] = dm[j] * gam[j];
+          s1 += gd[j];
+          s2 += gd[j] * xh[j];
+        }
+        const float m1 = warp_sum(s1) * (1.f / 256.f);
+        const float m2 = warp_sum(s2) * (1.f / 256.f);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) store1_split(dh, dh_ps, planes, off + 32 * j, ms.y * (gd[j] - m1 - xh[j] * m2) * gsc);
+      }
     }
   }
   // ---- dgamma / dbeta: the block's eight utterances meet in shared memory, one atomic per column and block
@@ -767,7 +847,9 @@ static void fill_pack_table(const Plan& pl, const spk_encoder_params& w, PackTab
 
 int encoder_forward(const spk_encoder_config& cfg, const spk_encoder_params& w, const spk_mel_view* mel,
                     const spk_mel_ragged* ragged, int B, int T, int S, int P, int training, uint64_t seed, float* dvec,
-                    void* ws_v, size_t ws_bytes, int keep, cudaStream_t st) {
+                    void* ws_v, size_t ws_bytes, int keep, cudaStream_t st, const int32_t* segments, int utterances) {
+  SPK_CHECK(segments == nullptr || (S == 1 && utterances >= 1 && utterances <= B),
+            "encoder: a segmented call runs at samples 1 with 1 <= utterances <= batch (got %d, %d)", S, utterances);
   Plan pl;
   SPK_TRY(make_plan(cfg, B, T, S, P, keep != 0, pl));
   P = pl.P;     // the upper bits carried the plan options
@@ -874,17 +956,33 @@ int encoder_forward(const spk_encoder_config& cfg, const spk_encoder_params& w, 
   }
   const Split& hl = pl.prune ? pl.last.sub.hout : pl.Lb[pl.L - 1].sub.hout;
   const int head_T = pl.prune ? 1 : T;     // the compact buffer holds one row per slice
+  if (segments != nullptr) {   // variable slice counts per utterance; the plan is the samples = 1 plan (B >= U)
+    ProfScope prof_head("head_fwd_seg", 2.0 * utterances * 256 * 256, 4.0 * B * 256 * 2, st);
+    head_fwd_kernel<true><<<(utterances + HEAD_UPB - 1) / HEAD_UPB, 256, 0, st>>>(
+        c.ptr(hl), hl.ps, P, head_T, 1, w.norm_w, w.norm_b, w.proj_w, w.proj_b, c.f32(pl.hn),
+        reinterpret_cast<float2*>(c.f32(pl.hst)), c.f32(pl.emean), c.f32(pl.epre), dvec,
+        static_cast<int64_t>(utterances), segments, static_cast<int64_t>(B));
+    SPK_CUDA(cudaGetLastError());
+    return 0;
+  }
   ProfScope prof_head("head_fwd", 2.0 * (B / S) * 256 * 256, 4.0 * B * 256 * 2, st);
-  head_fwd_kernel<<<(B / S + HEAD_UPB - 1) / HEAD_UPB, 256, 0, st>>>(
+  head_fwd_kernel<false><<<(B / S + HEAD_UPB - 1) / HEAD_UPB, 256, 0, st>>>(
       c.ptr(hl), hl.ps, P, head_T, S, w.norm_w, w.norm_b, w.proj_w, w.proj_b, c.f32(pl.hn),
-      reinterpret_cast<float2*>(c.f32(pl.hst)), c.f32(pl.emean), c.f32(pl.epre), dvec, static_cast<int64_t>(B / S));
+      reinterpret_cast<float2*>(c.f32(pl.hst)), c.f32(pl.emean), c.f32(pl.epre), dvec, static_cast<int64_t>(B / S),
+      nullptr, 0);
   SPK_CUDA(cudaGetLastError());
   return 0;
 }
 
 int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w, const spk_encoder_params* grads,
                      float* d_mel, const float* d_dvec, int B, int T, int S, int P_fwd, int training, uint64_t seed,
-                     void* ws_v, size_t ws_bytes, cudaStream_t st) {
+                     void* ws_v, size_t ws_bytes, cudaStream_t st, const RaggedGrad* rg) {
+  const int32_t* segments = rg != nullptr ? rg->segments : nullptr;
+  SPK_CHECK(rg == nullptr || (rg->mel != nullptr && rg->utterances >= 1 && rg->utterances <= B &&
+                              (segments != nullptr ? S == 1 : B / rg->utterances == S)),
+            "encoder: ragged backward: bad utterance count %d for batch %d, samples %d", rg ? rg->utterances : 0, B, S);
+  SPK_CHECK(rg == nullptr || d_mel == nullptr, "encoder: d_mel and a ragged input gradient are exclusive");
+  const int64_t U = segments != nullptr ? rg->utterances : B / S;   // d-vectors
   Plan pl;
   SPK_TRY(make_plan(cfg, B, T, S, P_fwd, true, pl));
   P_fwd = pl.P;
@@ -902,7 +1000,7 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
   const DropCfg drop = make_drop(seed, cfg.dropout, training != 0);
   float* gs = c.f32(pl.gscale);   // gradient scale of this pass (device scalars S, 1 / S)
   c.gs = gs;
-  grad_scale_kernel<<<1, 1024, 0, st>>>(d_dvec, static_cast<int64_t>(B / S) * 256, gs, g_grad_scale_log2);
+  grad_scale_kernel<<<1, 1024, 0, st>>>(d_dvec, U * 256, gs, g_grad_scale_log2);
   SPK_CUDA(cudaGetLastError());
 
   // ---- head
@@ -911,15 +1009,26 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
   // dense: the gradient of the last layer's output is zero except the t = 0 rows; pruned: compact [B, 256] in dh_b
   const Split& dhead = pl.prune ? pl.dh_b : pl.dh_a;
   if (!pl.prune) SPK_CUDA(cudaMemsetAsync(c.ptr(pl.dh_a), 0, static_cast<size_t>(pl.dh_a.ps) * P * 2, st));
+  // segmented: a slice that no segment covers (segments[U] < B breaks the ABI's precondition) gets a zero gradient row
+  // instead of whatever the compact buffer held
+  else if (segments != nullptr)
+    SPK_CUDA(cudaMemsetAsync(c.ptr(pl.dh_b), 0, static_cast<size_t>(pl.dh_b.ps) * P * 2, st));
   {
-  ProfScope prof_hb("head_bwd", 4.0 * (B / S) * 256 * 256, 4.0 * B * 256 * 2, st);
-  head_bwd_kernel<<<(B / S + HEAD_UPB - 1) / HEAD_UPB, 256, 0, st>>>(
-      d_dvec, c.f32(pl.epre), w.proj_w, c.ptr(hl), hl.ps, P, reinterpret_cast<const float2*>(c.f32(pl.hst)), w.norm_w,
-      head_T, S, c.f32(pl.de), c.ptr(dhead), dhead.ps, gr.norm_w, gr.norm_b, gs, static_cast<int64_t>(B / S));
+  ProfScope prof_hb(segments != nullptr ? "head_bwd_seg" : "head_bwd", 4.0 * U * 256 * 256, 4.0 * B * 256 * 2, st);
+  if (segments != nullptr)   // variable slice counts per utterance (plan at samples = 1)
+    head_bwd_kernel<true><<<(U + HEAD_UPB - 1) / HEAD_UPB, 256, 0, st>>>(
+        d_dvec, c.f32(pl.epre), w.proj_w, c.ptr(hl), hl.ps, P, reinterpret_cast<const float2*>(c.f32(pl.hst)),
+        w.norm_w, head_T, 1, c.f32(pl.de), c.ptr(dhead), dhead.ps, gr.norm_w, gr.norm_b, gs, U, segments,
+        static_cast<int64_t>(B));
+  else
+    head_bwd_kernel<false><<<(B / S + HEAD_UPB - 1) / HEAD_UPB, 256, 0, st>>>(
+        d_dvec, c.f32(pl.epre), w.proj_w, c.ptr(hl), hl.ps, P, reinterpret_cast<const float2*>(c.f32(pl.hst)),
+        w.norm_w, head_T, S, c.f32(pl.de), c.ptr(dhead), dhead.ps, gr.norm_w, gr.norm_b, gs,
+        static_cast<int64_t>(B / S), nullptr, 0);
   SPK_CUDA(cudaGetLastError());
-  if (c.pgrad) {
-    head_wgrad_kernel<<<dim3(8, (B / S + HEAD_WG_UCH - 1) / HEAD_WG_UCH), 256, 0, st>>>(c.f32(pl.de), c.f32(pl.emean),
-                                                                                        B / S, gr.proj_w, gr.proj_b);
+  if (c.pgrad) {   // de / emean hold one row per d-vector, whatever the slicing
+    head_wgrad_kernel<<<dim3(8, (U + HEAD_WG_UCH - 1) / HEAD_WG_UCH), 256, 0, st>>>(c.f32(pl.de), c.f32(pl.emean), U,
+                                                                                   gr.proj_w, gr.proj_b);
     SPK_CUDA(cudaGetLastError());
   }
   }
@@ -1043,7 +1152,7 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
     }
   }
   SPK_TRY(wgrad(c, "gemm.bwd.prenet_wgrad", Mt, pl.dh_b, D, pl.x0, pl.C, pl.C, gr.prenet_w));
-  if (d_mel != nullptr) {
+  if (d_mel != nullptr || (rg != nullptr && rg->d_data != nullptr)) {
     // ---- input: dX = dU W_pre (fp32, token-major, into dh_a: dead after the prenet backward, Mt * 512 >= Mt * 320
     // bytes), then transposed to the [B, mel, T] layout of the input.  dU carries the gradient scale S: alpha = 1 / S.
     float* dx = reinterpret_cast<float*>(c.ptr(pl.dh_a));
@@ -1052,7 +1161,10 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
     g.epi.alpha_ptr = gs + 1;
     g.epi.out = dx; g.epi.out_ld = pl.C; g.epi.out_planes = 1;
     SPK_TRY(c.run(g));
-    SPK_TRY(mel_grad_unpack(dx, d_mel, B, pl.C, T, st));
+    if (rg != nullptr)   // ragged forward: fold every slice back onto the columns of mel->data it was cut from
+      SPK_TRY(mel_grad_fold(dx, *rg->mel, segments, S, static_cast<int>(U), rg->d_data, B, pl.C, T, st));
+    else
+      SPK_TRY(mel_grad_unpack(dx, d_mel, B, pl.C, T, st));
   }
   return 0;
 }

@@ -171,6 +171,100 @@ int mel_pack_ragged(const spk_mel_ragged& mel, void* out, int64_t plane_stride, 
   return 0;
 }
 
+// Adjoint of mel_pack_ragged_kernel (the input gradient of a ragged forward).  Block (group g, column tiles of g's span
+// strided by gridDim.y): 32 columns x C channels per tile.  Item i of the tile is (column i / C, channel i % C), so a
+// warp reads the C contiguous floats of one token of dX (coalesced) and the tile leaves through shared memory as
+// 32-column runs of every channel (coalesced writes), as in mel_grad_unpack_kernel.
+//   crop row (length > T)  column p = col - start receives frame t = p - offset when 0 <= t < T;
+//   padded row             frames t with (t - pad_left) mod 2 (length - 1) in {p, 2 (length - 1) - p}: two arithmetic
+//                          sequences, walked merged in t order (length 1: every frame).
+// Table and segment entries are clamped: reads stay inside dX and writes inside d_data whatever the device holds.
+template <int C>
+__global__ void __launch_bounds__(256) mel_grad_fold_kernel(const float* __restrict__ dx, const int32_t* __restrict__ table,
+                                                            const int32_t* __restrict__ segments, int rows_per_group,
+                                                            int B, int T, int64_t total, float* __restrict__ d_data) {
+  __shared__ float tile[C][33];
+  __shared__ int64_t span[2];
+  const int g = blockIdx.x;
+  int r0, r1;
+  if (segments != nullptr) {
+    r0 = __ldg(segments + g);
+    r1 = __ldg(segments + g + 1);
+    r0 = r0 < 0 ? 0 : (r0 > B ? B : r0);
+    r1 = r1 < r0 ? r0 : (r1 > B ? B : r1);
+  } else {
+    r0 = g * rows_per_group;
+    r1 = r0 + rows_per_group > B ? B : r0 + rows_per_group;
+  }
+  if (threadIdx.x == 0) {
+    int64_t lo = total, hi = 0;
+    for (int r = r0; r < r1; ++r) {
+      const int64_t start = __ldg(table + 3 * r), len = __ldg(table + 3 * r + 1);
+      if (len < 1) continue;
+      lo = start < lo ? start : lo;
+      hi = start + len > hi ? start + len : hi;
+    }
+    span[0] = lo < 0 ? 0 : lo;
+    span[1] = hi > total ? total : hi;
+  }
+  __syncthreads();
+  const int64_t lo = span[0], hi = span[1];
+  for (int64_t c0 = lo + static_cast<int64_t>(blockIdx.y) * 32; c0 < hi; c0 += static_cast<int64_t>(gridDim.y) * 32) {
+    for (int i = threadIdx.x; i < C * 32; i += blockDim.x) {
+      const int j = i / C, c = i % C;
+      const int64_t col = c0 + j;
+      float acc = 0.f;
+      if (col < hi) {
+        for (int r = r0; r < r1; ++r) {
+          const int start = __ldg(table + 3 * r), len = __ldg(table + 3 * r + 1), off = __ldg(table + 3 * r + 2);
+          const int64_t p64 = col - start;
+          if (len < 1 || p64 < 0 || p64 >= len) continue;
+          const int p = static_cast<int>(p64);
+          const float* s = dx + static_cast<int64_t>(r) * T * C + c;
+          if (len > T) {
+            const int t = p - off;
+            if (t >= 0 && t < T) acc += __ldg(s + static_cast<int64_t>(t) * C);
+          } else if (len == 1) {
+            for (int t = 0; t < T; ++t) acc += __ldg(s + static_cast<int64_t>(t) * C);
+          } else {
+            const int period = 2 * (len - 1), pad_left = (T - len) / 2;
+            int ta = (p + pad_left) % period;                                          // rising pieces
+            int tb = (p == 0 || p == len - 1) ? T : (period - p + pad_left) % period;  // falling pieces (ends: none)
+            while (ta < T || tb < T) {
+              if (ta < tb) { acc += __ldg(s + static_cast<int64_t>(ta) * C); ta += period; }
+              else { acc += __ldg(s + static_cast<int64_t>(tb) * C); tb += period; }
+            }
+          }
+        }
+      }
+      tile[c][j] = acc;
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < C * 32; i += blockDim.x) {
+      const int c = i >> 5, j = i & 31;
+      if (c0 + j < hi) d_data[static_cast<int64_t>(c) * total + c0 + j] = tile[c][j];
+    }
+    __syncthreads();
+  }
+}
+int mel_grad_fold(const float* src, const spk_mel_ragged& mel, const int32_t* segments, int rows_per_group, int groups,
+                  float* d_data, int B, int C, int T, cudaStream_t st) {
+  SPK_CHECK(C == 80, "mel_grad_fold: Mel_Dim %d not supported by this build (80)", C);
+  SPK_CHECK(mel.table != nullptr && mel.total_frames > 0 && d_data != nullptr && groups >= 1 &&
+                (segments != nullptr || rows_per_group >= 1),
+            "mel_grad_fold: bad argument");
+  ProfScope prof("mel_grad_fold", 0, 4.0 * C * (static_cast<double>(B) * T + mel.total_frames), st);
+  // columns outside every group's span are zero; the fold overwrites the spans (disjoint: one writer per column)
+  SPK_CUDA(cudaMemsetAsync(d_data, 0, static_cast<size_t>(C) * mel.total_frames * sizeof(float), st));
+  // enough column tiles per group for an average span; longer spans loop
+  const int64_t tiles = (mel.total_frames / groups + 31) / 32 + 1;
+  dim3 grid(groups, static_cast<unsigned>(tiles < 64 ? tiles : 64));
+  mel_grad_fold_kernel<80><<<grid, 256, 0, st>>>(src, mel.table, segments, rows_per_group, B, T, mel.total_frames,
+                                                 d_data);
+  SPK_CUDA(cudaGetLastError());
+  return 0;
+}
+
 // pe buffer [1, D, max_pos] -> pe_t [T, D]
 __global__ void pe_transpose_kernel(const float* __restrict__ pe, float* __restrict__ pe_t, int D, int max_pos, int T) {
   __shared__ float tile[32][33];

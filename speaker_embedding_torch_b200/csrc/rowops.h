@@ -24,6 +24,14 @@ int mel_pack_ragged(const spk_mel_ragged& mel, void* out, int64_t plane_stride, 
                     cudaStream_t st);
 // token-major fp32 [B*T, C] (the input gradient) -> fp32 [B, C, T], the layout of the mel input
 int mel_grad_unpack(const float* src, float* d_mel, int B, int C, int T, cudaStream_t st);
+// Adjoint of mel_pack_ragged: token-major fp32 [B*T, C] -> d_data fp32 [C, mel.total_frames] (=), every slice folded
+// back onto the columns it was cut from; columns no slice reads receive 0.  Slices form groups: segments[g] ..
+// segments[g+1] - 1 (device int32 [groups + 1]), or runs of rows_per_group slices when segments is null.
+// Precondition: the column spans of different groups (smallest start .. largest start + length of their slices) do not
+// overlap; slices of one group may.  Every column is written by one thread, which adds its group's contributions in
+// slice order and, within a slice, in frame order: no atomics, bit-identical results from identical calls.
+int mel_grad_fold(const float* src, const spk_mel_ragged& mel, const int32_t* segments, int rows_per_group, int groups,
+                  float* d_data, int B, int C, int T, cudaStream_t st);
 int pe_transpose(const float* pe, float* pe_t, int D, int max_pos, int T, cudaStream_t st);
 
 // y[r] = LN(z[r * z_row_step]) over 256 columns; stats[r] = (mean, rstd) (may be null)
