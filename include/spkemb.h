@@ -39,8 +39,9 @@ int spk_abi_version(void);
 const char* spk_last_error(void);
 
 /* Encoder hyper-parameters: the `GE2E:` block + Sound.Mel_Dim of Hyper_Parameters.yaml:3,10-18
- * (read by GE2E.__init__, Modules.py:10-44).  This build supports mel_dim 80, emb 256, heads 4,
- * ffn 1024 (= 4 * emb, hard-wired at Modules.py:29), 1..8 layers, max_pos >= T. */
+ * (read by GE2E.__init__, Modules.py:10-44).  This build supports mel_dim a multiple of 8 in [16, 256], emb 256,
+ * heads 4, ffn 1024 (= 4 * emb, hard-wired at Modules.py:29), 1..8 layers, max_pos >= T.  Any other mel_dim is
+ * refused (workspace size 0, SPK_EINVAL) with a message that states the rule. */
 typedef struct spk_encoder_config {
   int32_t mel_dim, emb, heads, ffn, layers, max_pos;
   float pe_dropout;  /* GE2E.Positional_Encoding.Dropout_Rate */

@@ -127,9 +127,13 @@ int encoder_plan_flags() {
 static int make_plan(const spk_encoder_config& c, int B, int T, int S, int Pflags, bool keep, Plan& pl) {
   const int P = Pflags & 0xFF;
   const int opt = (Pflags & SPK_PLAN_EXPLICIT) ? Pflags : encoder_plan_flags();
-  SPK_CHECK(c.mel_dim == 80 && c.emb == 256 && c.heads == 4 && c.ffn == 1024,
-            "encoder: this build supports Mel_Dim 80, Embedding_Size 256, Head 4 (got %d/%d/%d/%d)", c.mel_dim, c.emb,
-            c.heads, c.ffn);
+  // Mel_Dim is the K of the prenet GEMM and the N of the input dgrad / prenet wgrad: the GEMMs need N % 8 == 0, the
+  // TMA maps of the fp16 x0 [Mt, C] planes 16-byte row strides, and mel_pack stores groups of 8 channels.  With
+  // C % 8 == 0 the packed weights that follow w_pre (256 * C elements) stay 16-byte aligned as well.
+  SPK_CHECK(c.mel_dim % 8 == 0 && c.mel_dim >= 16 && c.mel_dim <= 256,
+            "encoder: Mel_Dim %d must be a multiple of 8 in [16, 256]", c.mel_dim);
+  SPK_CHECK(c.emb == 256 && c.heads == 4 && c.ffn == 1024,
+            "encoder: this build supports Embedding_Size 256, Head 4 (got %d/%d/%d)", c.emb, c.heads, c.ffn);
   SPK_CHECK(c.layers >= 1 && c.layers <= SPK_MAX_LAYERS, "encoder: Num_Layers %d out of range", c.layers);
   SPK_CHECK(B >= 1 && T >= 1 && T <= c.max_pos && T <= 1024, "encoder: frames %d outside [1, %d]", T,
             c.max_pos < 1024 ? c.max_pos : 1024);
@@ -198,6 +202,11 @@ static int make_plan(const spk_encoder_config& c, int B, int T, int S, int Pflag
     pl.dz = take_split(cur, Mt * D, Pb);
     pl.dzd = take_split(cur, Mt * D, Pb);
     pl.df = take_split(cur, Mt * F, Pb);
+    // the input gradient dX (fp32 [Mt, C]) is written into df, dead once the last sublayer backward has run:
+    // 2 * F * Pb >= 2048 bytes per token at every plane count, against 4 * C <= 1024
+    SPK_CHECK(static_cast<size_t>(pl.df.ps) * Pb * 2 >= static_cast<size_t>(Mt) * pl.C * 4,
+              "encoder: the dX region (%lld bytes) is smaller than %lld tokens x %d fp32 channels",
+              (long long)pl.df.ps * Pb * 2, (long long)Mt, pl.C);
     pl.datt = take_split(cur, Mt * D, Pb);
     pl.dqkv = take_split(cur, Mt * 3 * D, Pb);
     pl.ds = take_split(cur, score_elems, Pb);
@@ -1153,9 +1162,10 @@ int encoder_backward(const spk_encoder_config& cfg, const spk_encoder_params& w,
   }
   SPK_TRY(wgrad(c, "gemm.bwd.prenet_wgrad", Mt, pl.dh_b, D, pl.x0, pl.C, pl.C, gr.prenet_w));
   if (d_mel != nullptr || (rg != nullptr && rg->d_data != nullptr)) {
-    // ---- input: dX = dU W_pre (fp32, token-major, into dh_a: dead after the prenet backward, Mt * 512 >= Mt * 320
-    // bytes), then transposed to the [B, mel, T] layout of the input.  dU carries the gradient scale S: alpha = 1 / S.
-    float* dx = reinterpret_cast<float*>(c.ptr(pl.dh_a));
+    // ---- input: dX = dU W_pre (fp32, token-major, into df: dead after the last sublayer backward, and large enough
+    // at every plane count, make_plan), then transposed to the [B, mel, T] layout of the input.  dU carries the
+    // gradient scale S: alpha = 1 / S.
+    float* dx = reinterpret_cast<float*>(c.ptr(pl.df));
     GemmProblem g = dgrad(c, "gemm.bwd.mel_dgrad", pl.dh_b, Mt, D, pl.w_pre, pl.C);
     g.epi.flags = EPI_OUT_F32;
     g.epi.alpha_ptr = gs + 1;

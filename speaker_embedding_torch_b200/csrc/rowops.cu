@@ -39,33 +39,33 @@ int pack_weights(const PackTable& tab, void* dst, int64_t plane_stride, int plan
 // mel view -> token-major split tensor [B*T, C]   (C % 8 == 0).  Slice b = window b / spw, frames
 // [ (b % spw) * hop, + T ) of a [windows, C, L] tensor in fp32 or fp16 (frames contiguous): the overlapping-slice
 // collation and the fp16 -> fp32 upcast of the reference's inference collater happen in this load.
-template <int C, typename TIn>
+// The shared tile is [C][33] floats (dynamic, 33.8 KB at C = 256).
+template <typename TIn>
 __global__ void mel_pack_kernel(const TIn* __restrict__ mel, elem_t* __restrict__ out, int64_t plane_stride,
-                                int planes, int T, int L, int hop, int spw) {
+                                int planes, int C, int T, int L, int hop, int spw) {
   pdl_trigger();   // the next kernel of the stream may start its prologue (ptx.cuh)
-  __shared__ float tile[C][33];
+  extern __shared__ float tile[];
   const int b = blockIdx.y;
   const int t0 = blockIdx.x * 32;
   const TIn* src = mel + static_cast<int64_t>(b / spw) * C * L + static_cast<int64_t>(b % spw) * hop;
   for (int i = threadIdx.x; i < C * 32; i += blockDim.x) {
     const int c = i >> 5, tl = i & 31;
-    tile[c][tl] = (t0 + tl < T) ? static_cast<float>(__ldg(src + static_cast<int64_t>(c) * L + t0 + tl)) : 0.f;
+    tile[c * 33 + tl] = (t0 + tl < T) ? static_cast<float>(__ldg(src + static_cast<int64_t>(c) * L + t0 + tl)) : 0.f;
   }
   __syncthreads();
-  constexpr int G = C / 8;
+  const int G = C / 8;
   for (int i = threadIdx.x; i < G * 32; i += blockDim.x) {
     const int tl = i / G, g = i % G;
     if (t0 + tl >= T) continue;
     float v[8];
 #pragma unroll
-    for (int j = 0; j < 8; ++j) v[j] = tile[g * 8 + j][tl];
+    for (int j = 0; j < 8; ++j) v[j] = tile[(g * 8 + j) * 33 + tl];
     store8_split(out, plane_stride, planes, (static_cast<int64_t>(b) * T + t0 + tl) * C + g * 8, v);
   }
 }
 int mel_pack(const spk_mel_view& mel, void* out, int64_t plane_stride, int planes, int B, int C, int T, cudaStream_t st) {
   const double in_b = mel.dtype == 1 ? 2.0 : 4.0;
   ProfScope prof("mel_pack", 0, 1.0 * B * C * T * (in_b + 2.0 * planes), st);
-  SPK_CHECK(C == 80, "mel_pack: Mel_Dim %d not supported by this build (80)", C);
   SPK_CHECK(mel.data != nullptr && (mel.dtype == 0 || mel.dtype == 1), "mel view: dtype must be 0 (fp32) or 1 (fp16)");
   SPK_CHECK(mel.slices_per_window >= 1 && B % mel.slices_per_window == 0 && mel.hop >= 0,
             "mel view: batch %d is not a multiple of slices_per_window %d", B, mel.slices_per_window);
@@ -73,13 +73,14 @@ int mel_pack(const spk_mel_view& mel, void* out, int64_t plane_stride, int plane
             "mel view: %d slices of %d frames at hop %d do not fit a %d-frame window", mel.slices_per_window, T, mel.hop,
             mel.window_frames);
   dim3 grid((T + 31) / 32, B);
+  const size_t smem = static_cast<size_t>(C) * 33 * sizeof(float);
   auto* o = reinterpret_cast<elem_t*>(out);
   if (mel.dtype == 0)
-    mel_pack_kernel<80, float><<<grid, 256, 0, st>>>(reinterpret_cast<const float*>(mel.data), o, plane_stride, planes, T,
-                                                     mel.window_frames, mel.hop, mel.slices_per_window);
+    mel_pack_kernel<float><<<grid, 256, smem, st>>>(reinterpret_cast<const float*>(mel.data), o, plane_stride, planes, C,
+                                                    T, mel.window_frames, mel.hop, mel.slices_per_window);
   else
-    mel_pack_kernel<80, __half><<<grid, 256, 0, st>>>(reinterpret_cast<const __half*>(mel.data), o, plane_stride, planes,
-                                                      T, mel.window_frames, mel.hop, mel.slices_per_window);
+    mel_pack_kernel<__half><<<grid, 256, smem, st>>>(reinterpret_cast<const __half*>(mel.data), o, plane_stride, planes,
+                                                     C, T, mel.window_frames, mel.hop, mel.slices_per_window);
   SPK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -87,25 +88,24 @@ int mel_pack(const spk_mel_view& mel, void* out, int64_t plane_stride, int plane
 // The mirror of mel_pack_kernel for the input gradient: token-major fp32 [B*T, C] -> d_mel [B, C, T] fp32.  The block's
 // 32 tokens are C * 32 consecutive floats on the read side and 32-frame runs of every channel on the write side; the
 // shared tile turns one into the other so that both are coalesced.
-template <int C>
-__global__ void mel_grad_unpack_kernel(const float* __restrict__ src, float* __restrict__ d_mel, int T) {
-  __shared__ float tile[C][33];
+__global__ void mel_grad_unpack_kernel(const float* __restrict__ src, float* __restrict__ d_mel, int C, int T) {
+  extern __shared__ float tile[];   // [C][33]
   const int b = blockIdx.y;
   const int t0 = blockIdx.x * 32;
   const int nt = T - t0 < 32 ? T - t0 : 32;
   const float* s = src + (static_cast<int64_t>(b) * T + t0) * C;
-  for (int i = threadIdx.x; i < nt * C; i += blockDim.x) tile[i % C][i / C] = __ldg(s + i);
+  for (int i = threadIdx.x; i < nt * C; i += blockDim.x) tile[(i % C) * 33 + i / C] = __ldg(s + i);
   __syncthreads();
   float* dst = d_mel + static_cast<int64_t>(b) * C * T + t0;
   for (int i = threadIdx.x; i < C * 32; i += blockDim.x) {
     const int c = i >> 5, tl = i & 31;
-    if (tl < nt) dst[static_cast<int64_t>(c) * T + tl] = tile[c][tl];
+    if (tl < nt) dst[static_cast<int64_t>(c) * T + tl] = tile[c * 33 + tl];
   }
 }
 int mel_grad_unpack(const float* src, float* d_mel, int B, int C, int T, cudaStream_t st) {
   ProfScope prof("mel_grad_unpack", 0, 8.0 * B * C * T, st);
-  SPK_CHECK(C == 80, "mel_grad_unpack: Mel_Dim %d not supported by this build (80)", C);
-  mel_grad_unpack_kernel<80><<<dim3((T + 31) / 32, B), 256, 0, st>>>(src, d_mel, T);
+  mel_grad_unpack_kernel<<<dim3((T + 31) / 32, B), 256, static_cast<size_t>(C) * 33 * sizeof(float), st>>>(src, d_mel,
+                                                                                                            C, T);
   SPK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -115,10 +115,10 @@ int mel_grad_unpack(const float* src, float* d_mel, int B, int C, int T, cudaStr
 // (start, length, offset) per utterance; every utterance is cut (length > T: frames [offset, offset + T)) or
 // reflect-padded (numpy 'reflect', floor / ceil of the missing frames left / right) to the batch's common T inside the
 // load that packs the token-major operand planes.  Host-side padded / cropped copies never exist.
-template <int C, typename TIn>
+template <typename TIn>
 __global__ void mel_pack_ragged_kernel(const TIn* __restrict__ mel, const int32_t* __restrict__ table, int64_t total,
-                                       elem_t* __restrict__ out, int64_t plane_stride, int planes, int T) {
-  __shared__ float tile[C][33];
+                                       elem_t* __restrict__ out, int64_t plane_stride, int planes, int C, int T) {
+  extern __shared__ float tile[];   // [C][33]
   const int b = blockIdx.y;
   const int t0 = blockIdx.x * 32;
   const int start = __ldg(table + 3 * b), len = __ldg(table + 3 * b + 1), off = __ldg(table + 3 * b + 2);
@@ -140,33 +140,33 @@ __global__ void mel_pack_ragged_kernel(const TIn* __restrict__ mel, const int32_
       }
       v = static_cast<float>(__ldg(mel + static_cast<int64_t>(c) * total + start + idx));
     }
-    tile[c][tl] = v;
+    tile[c * 33 + tl] = v;
   }
   __syncthreads();
-  constexpr int G = C / 8;
+  const int G = C / 8;
   for (int i = threadIdx.x; i < G * 32; i += blockDim.x) {
     const int tl = i / G, g = i % G;
     if (t0 + tl >= T) continue;
     float v[8];
 #pragma unroll
-    for (int j = 0; j < 8; ++j) v[j] = tile[g * 8 + j][tl];
+    for (int j = 0; j < 8; ++j) v[j] = tile[(g * 8 + j) * 33 + tl];
     store8_split(out, plane_stride, planes, (static_cast<int64_t>(b) * T + t0 + tl) * C + g * 8, v);
   }
 }
 int mel_pack_ragged(const spk_mel_ragged& mel, void* out, int64_t plane_stride, int planes, int B, int C, int T,
                     cudaStream_t st) {
   ProfScope prof("mel_pack_ragged", 0, 1.0 * B * C * T * ((mel.dtype == 1 ? 2.0 : 4.0) + 2.0 * planes), st);
-  SPK_CHECK(C == 80, "mel_pack: Mel_Dim %d not supported by this build (80)", C);
   SPK_CHECK(mel.data != nullptr && mel.table != nullptr && (mel.dtype == 0 || mel.dtype == 1) && mel.total_frames > 0,
             "ragged mel: data / table missing or dtype not 0 (fp32) / 1 (fp16)");
   dim3 grid((T + 31) / 32, B);
+  const size_t smem = static_cast<size_t>(C) * 33 * sizeof(float);
   auto* o = reinterpret_cast<elem_t*>(out);
   if (mel.dtype == 0)
-    mel_pack_ragged_kernel<80, float><<<grid, 256, 0, st>>>(reinterpret_cast<const float*>(mel.data), mel.table,
-                                                            mel.total_frames, o, plane_stride, planes, T);
+    mel_pack_ragged_kernel<float><<<grid, 256, smem, st>>>(reinterpret_cast<const float*>(mel.data), mel.table,
+                                                           mel.total_frames, o, plane_stride, planes, C, T);
   else
-    mel_pack_ragged_kernel<80, __half><<<grid, 256, 0, st>>>(reinterpret_cast<const __half*>(mel.data), mel.table,
-                                                             mel.total_frames, o, plane_stride, planes, T);
+    mel_pack_ragged_kernel<__half><<<grid, 256, smem, st>>>(reinterpret_cast<const __half*>(mel.data), mel.table,
+                                                            mel.total_frames, o, plane_stride, planes, C, T);
   SPK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -179,11 +179,10 @@ int mel_pack_ragged(const spk_mel_ragged& mel, void* out, int64_t plane_stride, 
 //   padded row             frames t with (t - pad_left) mod 2 (length - 1) in {p, 2 (length - 1) - p}: two arithmetic
 //                          sequences, walked merged in t order (length 1: every frame).
 // Table and segment entries are clamped: reads stay inside dX and writes inside d_data whatever the device holds.
-template <int C>
 __global__ void __launch_bounds__(256) mel_grad_fold_kernel(const float* __restrict__ dx, const int32_t* __restrict__ table,
                                                             const int32_t* __restrict__ segments, int rows_per_group,
-                                                            int B, int T, int64_t total, float* __restrict__ d_data) {
-  __shared__ float tile[C][33];
+                                                            int B, int C, int T, int64_t total, float* __restrict__ d_data) {
+  extern __shared__ float tile[];   // [C][33]
   __shared__ int64_t span[2];
   const int g = blockIdx.x;
   int r0, r1;
@@ -237,19 +236,18 @@ __global__ void __launch_bounds__(256) mel_grad_fold_kernel(const float* __restr
           }
         }
       }
-      tile[c][j] = acc;
+      tile[c * 33 + j] = acc;
     }
     __syncthreads();
     for (int i = threadIdx.x; i < C * 32; i += blockDim.x) {
       const int c = i >> 5, j = i & 31;
-      if (c0 + j < hi) d_data[static_cast<int64_t>(c) * total + c0 + j] = tile[c][j];
+      if (c0 + j < hi) d_data[static_cast<int64_t>(c) * total + c0 + j] = tile[c * 33 + j];
     }
     __syncthreads();
   }
 }
 int mel_grad_fold(const float* src, const spk_mel_ragged& mel, const int32_t* segments, int rows_per_group, int groups,
                   float* d_data, int B, int C, int T, cudaStream_t st) {
-  SPK_CHECK(C == 80, "mel_grad_fold: Mel_Dim %d not supported by this build (80)", C);
   SPK_CHECK(mel.table != nullptr && mel.total_frames > 0 && d_data != nullptr && groups >= 1 &&
                 (segments != nullptr || rows_per_group >= 1),
             "mel_grad_fold: bad argument");
@@ -259,8 +257,8 @@ int mel_grad_fold(const float* src, const spk_mel_ragged& mel, const int32_t* se
   // enough column tiles per group for an average span; longer spans loop
   const int64_t tiles = (mel.total_frames / groups + 31) / 32 + 1;
   dim3 grid(groups, static_cast<unsigned>(tiles < 64 ? tiles : 64));
-  mel_grad_fold_kernel<80><<<grid, 256, 0, st>>>(src, mel.table, segments, rows_per_group, B, T, mel.total_frames,
-                                                 d_data);
+  mel_grad_fold_kernel<<<grid, 256, static_cast<size_t>(C) * 33 * sizeof(float), st>>>(
+      src, mel.table, segments, rows_per_group, B, C, T, mel.total_frames, d_data);
   SPK_CUDA(cudaGetLastError());
   return 0;
 }

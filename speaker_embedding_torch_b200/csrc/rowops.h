@@ -17,6 +17,7 @@ struct PackTable {
 };
 
 int pack_weights(const PackTable& tab, void* dst, int64_t plane_stride, int planes, cudaStream_t st);
+// The four mel kernels below take C = Mel_Dim at run time: a multiple of 8 in [16, 256], which make_plan checks.
 // mel view (include/spkemb.h spk_mel_view) -> token-major split tensor [B*T, C]
 int mel_pack(const spk_mel_view& mel, void* out, int64_t plane_stride, int planes, int B, int C, int T, cudaStream_t st);
 // ragged batch (include/spkemb.h spk_mel_ragged) -> token-major split tensor, crop / reflect-pad to T in the load
