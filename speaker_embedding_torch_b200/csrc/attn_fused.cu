@@ -19,12 +19,6 @@
 
 namespace spk {
 
-__device__ __forceinline__ float fast_exp2(float x) {   // MUFU.EX2: ~2 ulp, plenty for fp16 probabilities
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-
 constexpr int AF_KV_ROWS = 256;               // max keys (T <= 256)
 constexpr int AF_STAGE = 16384 + 32768 + 32768;   // Q 128 x 128 B | K 256 x 128 B | V 256 x 128 B, double-buffered
 constexpr int AF_SK = 16384;
@@ -211,13 +205,9 @@ int attn_fused_fwd(const void* qkv, void* out, int64_t out_ld, int B, int H, int
   a.mtiles = (T + 127) / 128;
   a.out = reinterpret_cast<elem_t*>(out);
   a.out_ld = out_ld;
-  const elem_t* base = reinterpret_cast<const elem_t*>(qkv);
-  const int64_t ld = 3 * 64 * H;           // qkv row stride
-  const int64_t dims[4] = {64, T, H, B};
-  const int64_t strides[3] = {ld, 64, static_cast<int64_t>(T) * ld};
-  SPK_TRY(encode_map_4d(&a.q_map, base, dims, strides, 128));
-  SPK_TRY(encode_map_4d(&a.k_map, base + 64 * H, dims, strides, a.Tk64));
-  SPK_TRY(encode_map_4d(&a.v_map, base + 2 * 64 * H, dims, strides, a.Tk64));
+  SPK_TRY(encode_qkv_map(&a.q_map, qkv, 0, B, H, T, 128));
+  SPK_TRY(encode_qkv_map(&a.k_map, qkv, 1, B, H, T, a.Tk64));
+  SPK_TRY(encode_qkv_map(&a.v_map, qkv, 2, B, H, T, a.Tk64));
   static PerDeviceOnce once;
   SPK_TRY(once.run([]() -> int {
     SPK_CUDA(cudaFuncSetAttribute(attn_fused_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AF_SMEM));

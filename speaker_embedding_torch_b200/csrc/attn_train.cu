@@ -5,20 +5,22 @@
 // SM.  Reference: torch scaled_dot_product_attention inside nn.TransformerEncoderLayer (Modules.py:25-36,53), scale
 // 1/sqrt(64), dropout on the probabilities.
 //
-// Warp roles (640 threads): 0 = TMA producer, 1 = MMA issuer, 2 = TMEM allocator, 3 idle, 4..19 = sixteen compute
-// warps: warp 4 + 4p + w owns TMEM lane quarter w (tcgen05.ld/st restrict a warp to lanes 32 (warp % 4) ..) and
-// takes every fourth 16-column chunk (p = 0..3).  The per-element work (exp2, Philox, plane splits) is what these
-// kernels are bound by, so it is spread over as many warps as the register file allows.
+// Warp roles: 0 = TMA producer, 1 = MMA issuer, 2 = TMEM allocator, 3 idle, 4.. = compute warps: warp 4 + 4p + w owns
+// TMEM lane quarter w (tcgen05.ld/st restrict a warp to lanes 32 (warp % 4) ..) and takes every (CW / 4)-th 16-column
+// chunk (p = 0 .. CW / 4 - 1).  The per-element work (exp2, Philox, plane splits) is what these kernels are bound by,
+// so it is spread over as many warps as the register file allows: 16 compute warps at one CTA per SM (the backward and
+// the one-CTA forward), 8 in the forwards that run two CTAs per SM.
 //
-// Forward, per (slice, head) and 128-query tile:
+// Forward (attn_fwd_kernel), per (slice, head) and 128-query tile:
 //   TMA       Q tile, K, V (PL planes each) out of the packed qkv buffer [B*T, 768]
-//   tcgen05   S = Q K^T into TMEM (6 plane products for PL = 3, 3 for PL = 2), fp32
-//   8 warps   thread <-> query row (two warps per TMEM lane quarter, alternating 32-key chunks): row max, exp2, row
+//   tcgen05   S = Q K^T into TMEM (6 plane products for PL = 3, 3 for PL = 2, 1 for PL = 1), fp32
+//   CW warps  thread <-> query row (CW / 4 warps per TMEM lane quarter, alternating 16-key chunks): row max, exp2, row
 //             sum, Philox keep mask, split into fp16 planes and written BACK INTO TMEM over the scores they came from
 //             (tcgen05.st): the probabilities are the A operand of the next MMA straight from tensor memory
 //   tcgen05   O = P_drop V  (A from TMEM, V read MN-major from shared memory)
-//   8 warps   O * (1 / ((1 - p) * row sum)) -> PL fp16 planes -> att[(b*T + q) * 256 + h*64 ...]
+//   CW warps  O * (1 / ((1 - p) * row sum)) -> PL fp16 planes -> att[(b*T + q) * 256 + h*64 ...]
 //   kept for the backward: (row max * log2e / 8, row sum) per query and one keep BIT per probability.
+// Inference (PL = 1) has no dropout and keeps nothing.
 //
 // TMEM plane layout of P for key step t (16 keys = one MMA K step = 8 columns of packed fp16 pairs, even key in the low
 // half -- tools/probe/ts_probe.cu): plane 0 at S columns [16t, 16t+8), plane 1 at [16t+8, 16t+16), plane 2 (PL = 3)
@@ -28,11 +30,6 @@
 
 namespace spk {
 
-__device__ __forceinline__ float at_exp2(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
 __device__ __forceinline__ void tmem_st_32x32(uint32_t taddr, const uint32_t (&r)[32]) {
   asm volatile(
       "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
@@ -79,8 +76,9 @@ __device__ __forceinline__ bool elect_one() {
 }
 // descriptor of the same tile `bytes` further on (the start-address field holds address >> 4 in its low 14 bits)
 __device__ __forceinline__ uint64_t desc_add(uint64_t d, uint32_t bytes) { return d + (bytes >> 4); }
-__device__ __forceinline__ void quarter_sync(int quarter) {   // the four warps that share a TMEM lane quarter
-  asm volatile("bar.sync %0, 128;" ::"r"(quarter + 1) : "memory");
+template <int NW = 4>
+__device__ __forceinline__ void quarter_sync(int quarter) {   // the NW warps that share a TMEM lane quarter
+  asm volatile("bar.sync %0, %1;" ::"r"(quarter + 1), "n"(32 * NW) : "memory");
 }
 // keep bits (bit i <-> element idx8 * 8 + i) of one Philox call; same function of (seed, site, element) as dropout_scale8
 __device__ __forceinline__ uint32_t dropout_keep8(uint64_t seed, uint32_t site, uint64_t idx8, uint32_t thresh) {
@@ -96,24 +94,30 @@ __device__ __forceinline__ uint32_t dropout_keep8(uint64_t seed, uint32_t site, 
   return bits;
 }
 
-
-constexpr int ATF_THREADS = 640;
-constexpr int ATF_CW = 16;                                 // compute warps
-constexpr int ATF_TMEM_PLO = 256, ATF_TMEM_O = 384;
+constexpr int ATF_MAX_T = 192;                           // frames of every fused training / two-CTA inference forward
 constexpr float ATF_SC = 0.125f * 1.4426950408889634f;   // 1/sqrt(64) * log2(e)
 
-template <int PL>
-struct AtfCfg {
-  static constexpr int KV_ROWS = PL == 3 ? 192 : 256;            // max frames of the fused path
-  static constexpr int Q_BYTES = 128 * 128, KV_BYTES = KV_ROWS * 128;
-  static constexpr int OFF_K = PL * Q_BYTES, OFF_V = OFF_K + PL * KV_BYTES;
-  static constexpr int OFF_X = OFF_V + PL * KV_BYTES;            // float xmax[4][128], xsum[4][128]
-  static constexpr int OFF_STG = OFF_X + 4096;                   // output staging: one plane, 128 rows x 128 B
+// Footprint of one forward instantiation: PL fp16 planes, CW compute warps (16: one CTA per SM, 512 TMEM columns with
+// plane 2 of P at P_LO; 8: two CTAs per SM, 256 columns) and the load schedule.  KV_SHARED: ONE operand buffer holds K
+// for the score MMAs and is then reloaded with V for the PV MMAs (K and V are needed at different times); otherwise K
+// and V are loaded once per item into buffers of their own.
+template <int PL, int CW, bool KV_SHARED>
+struct AttnFwdLayout {
+  static constexpr int THREADS = 128 + 32 * CW;
+  static constexpr int NP = CW / 4;                           // compute warps per TMEM lane quarter = column parts
+  static constexpr int Q_BYTES = 128 * 128, KV_BYTES = ATF_MAX_T * 128;
+  static constexpr int OFF_K = PL * Q_BYTES, OFF_V = KV_SHARED ? OFF_K : OFF_K + PL * KV_BYTES;
+  static constexpr int OFF_X = OFF_V + PL * KV_BYTES;         // float max parts [NP][128], sum parts [NP][128]
+  static constexpr int OFF_STG = OFF_X + 2 * NP * 128 * 4;    // output staging: one plane, 128 rows x 128 B
   static constexpr int OFF_BAR = OFF_STG + 16384;
   static constexpr int SMEM = OFF_BAR + 128;
+  static constexpr int TMEM_COLS = CW == 16 ? 512 : 256, TMEM_O = CW == 16 ? 384 : 192, TMEM_PLO = 256;
+  // watchdog codes: producer WD + 0 / 1, MMA issuer WD + 0x10 .. 0x13, compute warps WD + 0x20 / 0x21
+  static constexpr uint32_t WD = PL == 1 ? 0x640u : KV_SHARED ? 0x670u : 0x600u;
+  static_assert(CW == 16 || 2 * (SMEM + 1024) <= 228 * 1024, "two CTAs of an 8-warp instantiation must share an SM");
 };
 
-struct AttnTrainFwdArgs {
+struct AttnFwdArgs {
   CUtensorMap q_map[3], k_map[3], v_map[3];
   int B, H, T, Tp, Tk16, Tk64, mtiles, nC;
   elem_t* out;      // [PL][B*T, out_ld], head h at column h*64
@@ -124,16 +128,23 @@ struct AttnTrainFwdArgs {
   uint32_t site;
 };
 
-template <int PL>
-__global__ void __launch_bounds__(ATF_THREADS, 1) attn_train_fwd_kernel(const __grid_constant__ AttnTrainFwdArgs a) {
+// Instantiations: <1, 8, false> inference; <2, 8, true> two-CTA training; <2, 16, false> and <3, 16, false> one-CTA
+// training.  The dropout keep mask, `stats` and `mbits` exist only for PL >= 2.
+template <int PL, int CW, bool KV_SHARED>
+__global__ void __launch_bounds__(128 + 32 * CW, CW == 8 ? 2 : 1) attn_fwd_kernel(const __grid_constant__ AttnFwdArgs a) {
+  using L = AttnFwdLayout<PL, CW, KV_SHARED>;
+  constexpr int NP = L::NP;
+  constexpr uint32_t WD = L::WD;
   pdl_trigger();   // the next kernel of the stream may start its prologue (ptx.cuh)
-  using Cfg = AtfCfg<PL>;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const uint32_t sbase = smem_u32(smem_raw);
-  const uint32_t sQ = sbase, sK = sbase + Cfg::OFF_K, sV = sbase + Cfg::OFF_V;
-  float* xch = reinterpret_cast<float*>(smem_raw + Cfg::OFF_X);   // [0..511] max parts, [512..1023] sum parts
-  const uint32_t bar_kv = sbase + Cfg::OFF_BAR, bar_q = bar_kv + 8, bar_s = bar_kv + 16, bar_p = bar_kv + 24,
-                 bar_o = bar_kv + 32, bar_oe = bar_kv + 40, bar_kvfree = bar_kv + 48, tmem_slot = bar_kv + 56;
+  const uint32_t sQ = sbase, sK = sbase + L::OFF_K, sV = sbase + L::OFF_V;
+  float* xch = reinterpret_cast<float*>(smem_raw + L::OFF_X);   // [0, 128 NP) max parts, [128 NP, 256 NP) sum parts
+  // The first two barriers complete with the operands.  Separate buffers: bar_kv with K and V of an item, bar_q with Q
+  // of a query tile.  Shared buffer: bar_qk with Q and K of a query tile, bar_v with its V.
+  const uint32_t bar_kv = sbase + L::OFF_BAR, bar_q = bar_kv + 8, bar_qk = bar_kv, bar_v = bar_q;
+  const uint32_t bar_s = bar_kv + 16, bar_p = bar_kv + 24, bar_o = bar_kv + 32, bar_oe = bar_kv + 40,
+                 bar_kvfree = bar_kv + 48, tmem_slot = bar_kv + 56;
   // Every waiter of an mbarrier observes EVERY phase of it, in order (a parity wait that skips a phase passes
   // spuriously): per-unit barriers are waited on once per unit, per-item barriers once per item.
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -144,17 +155,18 @@ __global__ void __launch_bounds__(ATF_THREADS, 1) attn_train_fwd_kernel(const __
     for (int p = 0; p < PL; ++p) { tma_prefetch_desc(&a.q_map[p]); tma_prefetch_desc(&a.k_map[p]); tma_prefetch_desc(&a.v_map[p]); }
   }
   if (warp == 1 && lane == 0) {
-    mbar_init(bar_kv, 1); mbar_init(bar_q, 1); mbar_init(bar_s, 1); mbar_init(bar_p, 32 * ATF_CW); mbar_init(bar_o, 1);
-    mbar_init(bar_oe, 32 * ATF_CW); mbar_init(bar_kvfree, 1);
+    mbar_init(bar_kv, 1); mbar_init(bar_q, 1); mbar_init(bar_s, 1); mbar_init(bar_p, 32 * CW); mbar_init(bar_o, 1);
+    mbar_init(bar_oe, 32 * CW);
+    if constexpr (!KV_SHARED) mbar_init(bar_kvfree, 1);
     fence_mbar_init();
   }
-  if (warp == 2) { tmem_alloc(tmem_slot, 512); tmem_relinquish(); }
+  if (warp == 2) { tmem_alloc(tmem_slot, L::TMEM_COLS); tmem_relinquish(); }
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
   uint32_t tmem_base;
   asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
-  const uint32_t tS = tmem_base, tPlo = tmem_base + ATF_TMEM_PLO, tO = tmem_base + ATF_TMEM_O;
+  const uint32_t tS = tmem_base, tPlo = tmem_base + L::TMEM_PLO, tO = tmem_base + L::TMEM_O;
   const int items = a.B * a.H;
   const int kv_plane = a.Tk64 * 128;      // bytes actually loaded per K / V plane
 
@@ -163,18 +175,34 @@ __global__ void __launch_bounds__(ATF_THREADS, 1) attn_train_fwd_kernel(const __
       uint32_t u = 0, it = 0;
       for (int item = blockIdx.x; item < items; item += gridDim.x, ++it) {
         const int h = item % a.H, b = item / a.H;
-        if (it > 0) mbar_wait(bar_kvfree, (it - 1) & 1u, 0x600u);   // last PV of the previous item: K / V are free
-        mbar_arrive_expect_tx(bar_kv, 2u * PL * kv_plane);
+        if constexpr (!KV_SHARED) {
+          if (it > 0) mbar_wait(bar_kvfree, (it - 1) & 1u, WD);   // last PV of the previous item: K / V are free
+          mbar_arrive_expect_tx(bar_kv, 2u * PL * kv_plane);
 #pragma unroll
-        for (int p = 0; p < PL; ++p) {
-          tma_load_4d(sK + p * Cfg::KV_BYTES, &a.k_map[p], bar_kv, 0, 0, h, b);
-          tma_load_4d(sV + p * Cfg::KV_BYTES, &a.v_map[p], bar_kv, 0, 0, h, b);
+          for (int p = 0; p < PL; ++p) {
+            tma_load_4d(sK + p * L::KV_BYTES, &a.k_map[p], bar_kv, 0, 0, h, b);
+            tma_load_4d(sV + p * L::KV_BYTES, &a.v_map[p], bar_kv, 0, 0, h, b);
+          }
         }
         for (int mt = 0; mt < a.mtiles; ++mt, ++u) {
-          if (u > 0) mbar_wait(bar_s, (u - 1) & 1u, 0x601u);     // previous scores issued and retired: Q is free
-          mbar_arrive_expect_tx(bar_q, PL * Cfg::Q_BYTES);
+          if constexpr (KV_SHARED) {
+            if (u > 0) mbar_wait(bar_o, (u - 1) & 1u, WD);        // previous PV retired: the operand buffer (V) and Q are free
+            mbar_arrive_expect_tx(bar_qk, PL * (L::Q_BYTES + kv_plane));
 #pragma unroll
-          for (int p = 0; p < PL; ++p) tma_load_4d(sQ + p * Cfg::Q_BYTES, &a.q_map[p], bar_q, 0, mt * 128, h, b);
+            for (int p = 0; p < PL; ++p) {
+              tma_load_4d(sQ + p * L::Q_BYTES, &a.q_map[p], bar_qk, 0, mt * 128, h, b);
+              tma_load_4d(sK + p * L::KV_BYTES, &a.k_map[p], bar_qk, 0, 0, h, b);
+            }
+            mbar_wait(bar_s, u & 1u, WD + 1);                     // score MMAs retired: K is dead, V takes its place
+            mbar_arrive_expect_tx(bar_v, PL * kv_plane);
+#pragma unroll
+            for (int p = 0; p < PL; ++p) tma_load_4d(sV + p * L::KV_BYTES, &a.v_map[p], bar_v, 0, 0, h, b);
+          } else {
+            if (u > 0) mbar_wait(bar_s, (u - 1) & 1u, WD + 1);    // previous scores issued and retired: Q is free
+            mbar_arrive_expect_tx(bar_q, PL * L::Q_BYTES);
+#pragma unroll
+            for (int p = 0; p < PL; ++p) tma_load_4d(sQ + p * L::Q_BYTES, &a.q_map[p], bar_q, 0, mt * 128, h, b);
+          }
         }
       }
     }
@@ -182,55 +210,60 @@ __global__ void __launch_bounds__(ATF_THREADS, 1) attn_train_fwd_kernel(const __
     // whole warp, converged; one elected lane issues
     const uint32_t idesc_s = umma_idesc_f16(128, a.Tk16, false, false);
     const uint32_t idesc_o = umma_idesc_f16(128, 64, false, true);
-    constexpr int NCOMBO = PL == 3 ? 6 : 3;
-    // plane products, smallest terms first (plane 0 = hi)
-    constexpr int PA3[6] = {1, 0, 2, 0, 1, 0}, PB3[6] = {1, 2, 0, 1, 0, 0};
-    constexpr int PA2[3] = {1, 0, 0}, PB2[3] = {0, 1, 0};
+    // plane products (A plane, B plane), smallest terms first (plane 0 = hi)
+    constexpr int NCOMBO = PL == 3 ? 6 : PL == 2 ? 3 : 1;
+    constexpr int PA[3][6] = {{0}, {1, 0, 0}, {1, 0, 2, 0, 1, 0}}, PB[3][6] = {{0}, {0, 1, 0}, {1, 2, 0, 1, 0, 0}};
     const uint64_t dQ0 = umma_smem_desc(sQ, 16, 1024), dK0 = umma_smem_desc(sK, 16, 1024);
     const uint64_t dV0 = umma_smem_desc(sV, 8192, 1024);
     const int ksteps = a.Tk16 / 16;
     uint32_t u = 0, it = 0;
     for (int item = blockIdx.x; item < items; item += gridDim.x, ++it) {
       for (int mt = 0; mt < a.mtiles; ++mt, ++u) {
-        mbar_wait(bar_q, u & 1u, 0x610u);
-        if (mt == 0) mbar_wait(bar_kv, it & 1u, 0x611u);
+        if constexpr (KV_SHARED) {
+          mbar_wait(bar_qk, u & 1u, WD + 0x10);
+        } else {
+          mbar_wait(bar_q, u & 1u, WD + 0x10);
+          if (mt == 0) mbar_wait(bar_kv, it & 1u, WD + 0x11);
+        }
         tc_fence_after();
         if (elect_one()) {
 #pragma unroll
           for (int cb = 0; cb < NCOMBO; ++cb) {
-            const int pa = PL == 3 ? PA3[cb] : PA2[cb], pb = PL == 3 ? PB3[cb] : PB2[cb];
 #pragma unroll
             for (int k = 0; k < 4; ++k)
-              umma_f16(tS, desc_add(dQ0, pa * Cfg::Q_BYTES + k * 32), desc_add(dK0, pb * Cfg::KV_BYTES + k * 32), idesc_s,
-                        (cb | k) ? 1u : 0u);
+              umma_f16(tS, desc_add(dQ0, PA[PL - 1][cb] * L::Q_BYTES + k * 32), desc_add(dK0, PB[PL - 1][cb] * L::KV_BYTES + k * 32),
+                       idesc_s, (cb | k) ? 1u : 0u);
           }
           umma_commit(bar_s);
         }
         __syncwarp();
-        mbar_wait(bar_p, u & 1u, 0x612u);                       // probabilities are in TMEM
-        if (u > 0) mbar_wait(bar_oe, (u - 1) & 1u, 0x613u);     // previous output tile drained
+        mbar_wait(bar_p, u & 1u, WD + 0x12);                      // probabilities are in TMEM
+        if constexpr (KV_SHARED) mbar_wait(bar_v, u & 1u, WD + 0x11);   // V is in the operand buffer
+        if (u > 0) mbar_wait(bar_oe, (u - 1) & 1u, WD + 0x13);    // previous output tile drained
         tc_fence_after();
         if (elect_one()) {
           for (int t = 0; t < ksteps; ++t) {
             const uint32_t voff = (t >> 2) * 8192 + (t & 3) * 2048;
 #pragma unroll
             for (int cb = 0; cb < NCOMBO; ++cb) {
-              const int pa = PL == 3 ? PA3[cb] : PA2[cb], pb = PL == 3 ? PB3[cb] : PB2[cb];
+              const int pa = PA[PL - 1][cb];
               const uint32_t ta = pa == 0 ? tS + 16 * t : (pa == 1 ? tS + 16 * t + 8 : tPlo + 8 * t);
-              umma_f16_ts(tO, ta, desc_add(dV0, pb * Cfg::KV_BYTES + voff), idesc_o, (t | cb) ? 1u : 0u);
+              umma_f16_ts(tO, ta, desc_add(dV0, PB[PL - 1][cb] * L::KV_BYTES + voff), idesc_o, (t | cb) ? 1u : 0u);
             }
           }
           umma_commit(bar_o);
-          if (mt == a.mtiles - 1) umma_commit(bar_kvfree);
+          if constexpr (!KV_SHARED) {
+            if (mt == a.mtiles - 1) umma_commit(bar_kvfree);
+          }
         }
         __syncwarp();
       }
     }
   } else if (warp >= 4) {
-    const int w = (warp - 4) & 3, part = (warp - 4) >> 2;          // lane quarter, column part (0..3)
+    const int w = (warp - 4) & 3, part = (warp - 4) >> 2;          // lane quarter, column part (0 .. NP - 1)
     const int r = w * 32 + lane;
     const uint32_t t_lane = static_cast<uint32_t>(w * 32) << 16;
-    const bool use_drop = a.drop.thresh != 0;
+    const bool use_drop = PL >= 2 && a.drop.thresh != 0;           // no dropout in inference
     const float inv_keep = use_drop ? a.drop.inv_keep : 1.f;
     const int nchunks = a.Tk16 / 16;                               // 16-key chunks == MMA key steps
     uint32_t u = 0;
@@ -240,12 +273,12 @@ __global__ void __launch_bounds__(ATF_THREADS, 1) attn_train_fwd_kernel(const __
         const uint32_t ph = u & 1u;
         const int q = mt * 128 + r;
         const bool active = mt * 128 + w * 32 < a.T;              // warp-uniform
-        mbar_wait(bar_s, ph, 0x620u);
+        mbar_wait(bar_s, ph, WD + 0x20);
         tc_fence_after();
         uint32_t sreg[16];
         float mx = -INFINITY;
         if (active) {
-          for (int c = part; c * 16 < a.T; c += 4) {
+          for (int c = part; c * 16 < a.T; c += NP) {
             tmem_ld_32x16(tS + t_lane + c * 16, sreg);
             tmem_ld_wait();
 #pragma unroll
@@ -254,75 +287,89 @@ __global__ void __launch_bounds__(ATF_THREADS, 1) attn_train_fwd_kernel(const __
           }
         }
         xch[part * 128 + r] = mx;
-        quarter_sync(w);
-        mx = fmaxf(fmaxf(xch[r], xch[128 + r]), fmaxf(xch[256 + r], xch[384 + r]));
+        quarter_sync<NP>(w);
+        // the parts are combined in a fixed tree, so every row's max and sum are the same whatever the warp count
+        if constexpr (NP == 4) mx = fmaxf(fmaxf(xch[r], xch[128 + r]), fmaxf(xch[256 + r], xch[384 + r]));
+        else mx = fmaxf(xch[r], xch[128 + r]);
         const float mxs = mx * ATF_SC;
         float sum = 0.f;
         if (active) {
           const uint64_t row_idx8 = ((static_cast<uint64_t>(item) * a.T + q) * a.Tp) >> 3;   // Tp % 8 == 0
-          for (int c = part; c < nchunks; c += 4) {
+          for (int c = part; c < nchunks; c += NP) {
             tmem_ld_32x16(tS + t_lane + c * 16, sreg);
             uint32_t keep = 0xFFFFu;
             if (use_drop)
               keep = dropout_keep8(a.drop.seed, a.site, row_idx8 + 2 * c, a.drop.thresh) |
                      (dropout_keep8(a.drop.seed, a.site, row_idx8 + 2 * c + 1, a.drop.thresh) << 8);
             tmem_ld_wait();
-            uint32_t o01[16];
-            uint32_t o2[8];
+            uint32_t o01[PL == 1 ? 8 : 16];                               // planes 0 and 1 of P
+            uint32_t o2[8];                                               // plane 2 (PL = 3)
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
               const int key = c * 16 + 2 * j;
-              float e0 = key < a.T ? at_exp2(__uint_as_float(sreg[2 * j]) * ATF_SC - mxs) : 0.f;
-              float e1 = key + 1 < a.T ? at_exp2(__uint_as_float(sreg[2 * j + 1]) * ATF_SC - mxs) : 0.f;
+              float e0 = key < a.T ? fast_exp2(__uint_as_float(sreg[2 * j]) * ATF_SC - mxs) : 0.f;
+              float e1 = key + 1 < a.T ? fast_exp2(__uint_as_float(sreg[2 * j + 1]) * ATF_SC - mxs) : 0.f;
               sum += e0 + e1;
               e0 = ((keep >> (2 * j)) & 1u) ? e0 : 0.f;
               e1 = ((keep >> (2 * j + 1)) & 1u) ? e1 : 0.f;
               const uint32_t hi = pack2(e0, e1);
               o01[j] = hi;                                                // plane 0 at columns 16c + j
-              e0 -= lo_to_f(hi);
-              e1 -= hi_to_f(hi);
-              const uint32_t mid = pack2(e0, e1);
-              o01[8 + j] = mid;                                           // plane 1 at columns 16c + 8 + j
-              if (PL == 3) {
-                e0 -= lo_to_f(mid);
-                e1 -= hi_to_f(mid);
-                o2[j] = pack2(e0, e1);
+              if constexpr (PL >= 2) {
+                e0 -= lo_to_f(hi);
+                e1 -= hi_to_f(hi);
+                const uint32_t mid = pack2(e0, e1);
+                o01[8 + j] = mid;                                         // plane 1 at columns 16c + 8 + j
+                if constexpr (PL == 3) {
+                  e0 -= lo_to_f(mid);
+                  e1 -= hi_to_f(mid);
+                  o2[j] = pack2(e0, e1);                                  // plane 2 at P_LO + 8c + j
+                }
               }
             }
-            tmem_st_32x16(tS + t_lane + c * 16, o01);
-            if (PL == 3) tmem_st_32x8(tPlo + t_lane + c * 8, o2);
-            if (a.mbits != nullptr && q < a.T)
-              a.mbits[(static_cast<int64_t>(item) * a.nC + c) * a.T + q] = static_cast<uint16_t>(keep);
+            if constexpr (PL == 1) {
+              tmem_st_32x8(tS + t_lane + c * 16, o01);
+            } else {
+              tmem_st_32x16(tS + t_lane + c * 16, o01);
+              if constexpr (PL == 3) tmem_st_32x8(tPlo + t_lane + c * 8, o2);
+              if (a.mbits != nullptr && q < a.T)
+                a.mbits[(static_cast<int64_t>(item) * a.nC + c) * a.T + q] = static_cast<uint16_t>(keep);
+            }
           }
           tmem_st_wait();
         }
-        xch[512 + part * 128 + r] = sum;
+        xch[NP * 128 + part * 128 + r] = sum;
         tc_fence_before();
         mbar_arrive(bar_p);
-        quarter_sync(w);
-        sum = (xch[512 + r] + xch[640 + r]) + (xch[768 + r] + xch[896 + r]);
-        // ---- epilogue: O * inv_keep / sum -> PL planes.  This warp takes 16 of the head's 64 columns out of TMEM; the
+        quarter_sync<NP>(w);
+        if constexpr (NP == 4) sum = (xch[512 + r] + xch[640 + r]) + (xch[768 + r] + xch[896 + r]);
+        else sum = xch[256 + r] + xch[384 + r];
+        // ---- epilogue: O * inv_keep / sum -> PL planes.  This warp takes COLS of the head's 64 columns out of TMEM; the
         //      planes go through a shared-memory tile so that global memory sees full 128-byte rows (8 lanes x 16 B)
-        mbar_wait(bar_o, ph, 0x621u);
+        mbar_wait(bar_o, ph, WD + 0x21);
         tc_fence_after();
-        float v[16];
+        constexpr int COLS = 64 / NP;
+        float v[COLS];
         if (active) {
-          tmem_ld_32x16(tO + t_lane + part * 16, sreg);
-          tmem_ld_wait();
-          const float sc = inv_keep / sum;
 #pragma unroll
-          for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(sreg[i]) * sc;
-          if (part == 0 && q < a.T && a.stats != nullptr) a.stats[static_cast<int64_t>(item) * a.T + q] = make_float2(mxs, sum);
+          for (int hlf = 0; hlf < COLS / 16; ++hlf) {
+            tmem_ld_32x16(tO + t_lane + part * COLS + hlf * 16, sreg);
+            tmem_ld_wait();
+            const float sc = inv_keep / sum;                      // placed after a load, the division overlaps it
+#pragma unroll
+            for (int i = 0; i < 16; ++i) v[hlf * 16 + i] = __uint_as_float(sreg[i]) * sc;
+          }
+          if constexpr (PL >= 2) {
+            if (part == 0 && q < a.T && a.stats != nullptr) a.stats[static_cast<int64_t>(item) * a.T + q] = make_float2(mxs, sum);
+          }
         }
         tc_fence_before();
         mbar_arrive(bar_oe);                                      // the accumulator is free for the next tile's PV
-        if (active) {                                             // uniform over the quarter's four warps
-          const uint32_t stg = sbase + Cfg::OFF_STG;
-          const uint32_t my0 = stg + r * 128 + (((2 * part) ^ (r & 7)) << 4), my1 = stg + r * 128 + (((2 * part + 1) ^ (r & 7)) << 4);
+        if (active) {                                             // uniform over the quarter's NP warps
+          const uint32_t stg = sbase + L::OFF_STG;
 #pragma unroll
           for (int p = 0; p < PL; ++p) {
 #pragma unroll
-            for (int g = 0; g < 2; ++g) {
+            for (int g = 0; g < COLS / 8; ++g) {                  // this warp's 16-byte chunks (COLS / 8) part + g
               uint32_t wv[4];
 #pragma unroll
               for (int i = 0; i < 4; ++i) {
@@ -332,13 +379,13 @@ __global__ void __launch_bounds__(ATF_THREADS, 1) attn_train_fwd_kernel(const __
                   v[g * 8 + 2 * i + 1] -= hi_to_f(wv[i]);
                 }
               }
-              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(g ? my1 : my0), "r"(wv[0]), "r"(wv[1]), "r"(wv[2]),
-                           "r"(wv[3]) : "memory");
+              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stg + r * 128 + ((((COLS / 8) * part + g) ^ (r & 7)) << 4)),
+                           "r"(wv[0]), "r"(wv[1]), "r"(wv[2]), "r"(wv[3]) : "memory");
             }
-            quarter_sync(w);
+            quarter_sync<NP>(w);
 #pragma unroll
-            for (int it = 0; it < 2; ++it) {                      // 8 of the quarter's 32 rows per warp, 4 rows per instruction
-              const int row = w * 32 + part * 8 + it * 4 + (lane >> 3);
+            for (int it = 0; it < 8 / NP; ++it) {                 // 32 / NP of the quarter's 32 rows per warp, 4 rows per instruction
+              const int row = w * 32 + part * (32 / NP) + it * 4 + (lane >> 3);
               uint4 val;
               asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(val.x), "=r"(val.y), "=r"(val.z), "=r"(val.w)
                            : "r"(stg + row * 128 + (((lane & 7) ^ (row & 7)) << 4)) : "memory");
@@ -347,7 +394,7 @@ __global__ void __launch_bounds__(ATF_THREADS, 1) attn_train_fwd_kernel(const __
                 *reinterpret_cast<uint4*>(a.out + p * a.out_ps + (static_cast<int64_t>(b) * a.T + qq) * a.out_ld + h * 64 +
                                           (lane & 7) * 8) = val;
             }
-            quarter_sync(w);
+            quarter_sync<NP>(w);
           }
         }
       }
@@ -358,38 +405,37 @@ __global__ void __launch_bounds__(ATF_THREADS, 1) attn_train_fwd_kernel(const __
   __syncthreads();
   if (warp == 2) {
     tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
+    tmem_dealloc(tmem_base, L::TMEM_COLS);
   }
 }
 
-// two-CTAs-per-SM variant of the two-plane forward (defined below)
-constexpr int ATW_KV_ROWS = 192;
 static int g_attn_fwd_two = 1;     // spk_set_option("training_attention_two_ctas", 0/1)
 void attn_train_set_fwd_two(int on) { g_attn_fwd_two = on; }
-static int attn_train_fwd2_launch(AttnTrainFwdArgs& a, const elem_t* qkv, int64_t qkv_ps, cudaStream_t st);
 
-int attn_train_max_frames(int planes) { return planes == 3 ? AtfCfg<3>::KV_ROWS : AtfCfg<2>::KV_ROWS; }
-
-template <int PL>
-static int attn_train_fwd_launch(AttnTrainFwdArgs& a, const elem_t* qkv, int64_t qkv_ps, cudaStream_t st) {
-  using Cfg = AtfCfg<PL>;
-  const int64_t ld = 3 * 64 * a.H;
-  const int64_t dims[4] = {64, a.T, a.H, a.B};
-  const int64_t strides[3] = {ld, 64, static_cast<int64_t>(a.T) * ld};
+// Fills the map and tile fields of `a` (B, H, T, Tp and the outputs are set) and launches one instantiation.
+template <int PL, int CW, bool KV_SHARED>
+static int attn_fwd_launch(AttnFwdArgs& a, const void* qkv, int64_t qkv_ps, const char* tag, cudaStream_t st) {
+  using L = AttnFwdLayout<PL, CW, KV_SHARED>;
+  a.Tk16 = (a.T + 15) / 16 * 16;
+  a.Tk64 = (a.T + 63) / 64 * 64;
+  a.mtiles = (a.T + 127) / 128;
+  a.nC = (a.Tp + 15) / 16;
   for (int p = 0; p < PL; ++p) {
-    const elem_t* base = qkv + p * qkv_ps;
-    SPK_TRY(encode_map_4d(&a.q_map[p], base, dims, strides, 128));
-    SPK_TRY(encode_map_4d(&a.k_map[p], base + 64 * a.H, dims, strides, a.Tk64));
-    SPK_TRY(encode_map_4d(&a.v_map[p], base + 2 * 64 * a.H, dims, strides, a.Tk64));
+    const elem_t* plane = reinterpret_cast<const elem_t*>(qkv) + p * qkv_ps;
+    SPK_TRY(encode_qkv_map(&a.q_map[p], plane, 0, a.B, a.H, a.T, 128));
+    SPK_TRY(encode_qkv_map(&a.k_map[p], plane, 1, a.B, a.H, a.T, a.Tk64));
+    SPK_TRY(encode_qkv_map(&a.v_map[p], plane, 2, a.B, a.H, a.T, a.Tk64));
   }
   static PerDeviceOnce once;
   SPK_TRY(once.run([]() -> int {
-    SPK_CUDA(cudaFuncSetAttribute(attn_train_fwd_kernel<PL>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM));
+    SPK_CUDA(cudaFuncSetAttribute(attn_fwd_kernel<PL, CW, KV_SHARED>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::SMEM));
     return 0;
   }));
-  const int items = a.B * a.H;
-  const int grid = items < device_sm_count() ? items : device_sm_count();
-  attn_train_fwd_kernel<PL><<<grid, ATF_THREADS, Cfg::SMEM, st>>>(a);
+  const int items = a.B * a.H, ctas = (CW == 8 ? 2 : 1) * device_sm_count();
+  const int grid = items < ctas ? items : ctas;
+  // algorithmic work: QK^T and PV (16-bit dense count); bytes: Q, K, V in, O out
+  ProfScope prof(tag, 4.0 * a.B * a.H * a.T * a.T * 64, 4.0 * a.B * a.T * 64 * a.H * 2.0 * PL, st);
+  attn_fwd_kernel<PL, CW, KV_SHARED><<<grid, L::THREADS, L::SMEM, st>>>(a);
   SPK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -398,493 +444,30 @@ static int attn_train_fwd_launch(AttnTrainFwdArgs& a, const elem_t* qkv, int64_t
 int attn_train_fwd(const void* qkv, int64_t qkv_ps, int planes, void* out, int64_t out_ps, int64_t out_ld, float* stats,
                    uint32_t* mbits, DropCfg drop, uint32_t site, int B, int H, int T, int Tp, cudaStream_t st) {
   SPK_CHECK(planes == 2 || planes == 3, "attn_train_fwd: planes must be 2 or 3");
-  SPK_CHECK(T >= 1 && T <= attn_train_max_frames(planes) && H >= 1, "attn_train_fwd: T=%d outside [1, %d]", T,
-            attn_train_max_frames(planes));
+  SPK_CHECK(T >= 1 && T <= ATF_MAX_T && H >= 1, "attn_train_fwd: T=%d outside [1, %d]", T, ATF_MAX_T);
   SPK_CHECK(drop.thresh == 0 || mbits != nullptr, "attn_train_fwd: dropout needs the keep-bit buffer");
-  AttnTrainFwdArgs a;
+  AttnFwdArgs a;
   memset(&a, 0, sizeof(a));
   a.B = B; a.H = H; a.T = T; a.Tp = Tp;
-  a.Tk16 = (T + 15) / 16 * 16;
-  a.Tk64 = (T + 63) / 64 * 64;
-  a.mtiles = (T + 127) / 128;
-  a.nC = (Tp + 15) / 16;
   a.out = reinterpret_cast<elem_t*>(out);
   a.out_ps = out_ps; a.out_ld = out_ld;
   a.stats = reinterpret_cast<float2*>(stats);
   a.mbits = drop.thresh != 0 ? reinterpret_cast<uint16_t*>(mbits) : nullptr;
   a.drop = drop; a.site = site;
-  // algorithmic work: QK^T and PV (16-bit dense count); bytes: Q, K, V in, O out
-  ProfScope prof("attn_train_fwd", 4.0 * B * H * T * T * 64, 4.0 * B * T * 64 * H * 2.0 * planes, st);
-  if (planes == 3) return attn_train_fwd_launch<3>(a, reinterpret_cast<const elem_t*>(qkv), qkv_ps, st);
-  if (g_attn_fwd_two && T <= ATW_KV_ROWS) return attn_train_fwd2_launch(a, reinterpret_cast<const elem_t*>(qkv), qkv_ps, st);
-  return attn_train_fwd_launch<2>(a, reinterpret_cast<const elem_t*>(qkv), qkv_ps, st);
-}
-
-// =====================================================================================================================
-// Two-CTAs-per-SM variant of the training forward (two planes, T <= 192).  Same arithmetic as attn_train_fwd_kernel<2>;
-// what changes is the footprint: 8 compute warps, 256 TMEM columns (S | P in place at 0, O at 192) and ONE operand buffer
-// that holds K for the score MMAs and is then reloaded with V for the PV MMAs (K and V are needed at different times),
-// so a CTA fits in 99 KB and two of them share an SM: one item's softmax runs under the other item's loads and MMAs.
-// K is fetched again for the second query tile of an item (an L2 hit).
-__device__ __forceinline__ void half_quarter_sync(int quarter) {   // the two warps that share a TMEM lane quarter
-  asm volatile("bar.sync %0, 64;" ::"r"(quarter + 1) : "memory");
-}
-constexpr int ATW_CW = 8, ATW_THREADS = 128 + 32 * ATW_CW;
-constexpr int ATW_Q_BYTES = 16384, ATW_KV_BYTES = ATW_KV_ROWS * 128;
-constexpr int ATW_OFF_KV = 2 * ATW_Q_BYTES, ATW_OFF_X = ATW_OFF_KV + 2 * ATW_KV_BYTES, ATW_OFF_STG = ATW_OFF_X + 2048;
-constexpr int ATW_OFF_BAR = ATW_OFF_STG + 16384, ATW_SMEM = ATW_OFF_BAR + 128;
-constexpr int ATW_TMEM_O = 192;
-
-__global__ void __launch_bounds__(ATW_THREADS, 2) attn_train_fwd2_kernel(const __grid_constant__ AttnTrainFwdArgs a) {
-  pdl_trigger();   // the next kernel of the stream may start its prologue (ptx.cuh)
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  const uint32_t sbase = smem_u32(smem_raw);
-  const uint32_t sQ = sbase, sKV = sbase + ATW_OFF_KV;
-  float* xch = reinterpret_cast<float*>(smem_raw + ATW_OFF_X);   // [0..255] max parts, [256..511] sum parts
-  const uint32_t bar_qk = sbase + ATW_OFF_BAR, bar_v = bar_qk + 8, bar_s = bar_qk + 16, bar_p = bar_qk + 24,
-                 bar_o = bar_qk + 32, bar_oe = bar_qk + 40, tmem_slot = bar_qk + 56;
-  // every barrier completes exactly once per (item, query tile) unit and every waiter waits once per unit
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if ((sbase & 1023u) != 0) __trap();
-  if (warp == 0 && lane == 0) {
-#pragma unroll
-    for (int p = 0; p < 2; ++p) { tma_prefetch_desc(&a.q_map[p]); tma_prefetch_desc(&a.k_map[p]); tma_prefetch_desc(&a.v_map[p]); }
-  }
-  if (warp == 1 && lane == 0) {
-    mbar_init(bar_qk, 1); mbar_init(bar_v, 1); mbar_init(bar_s, 1); mbar_init(bar_p, 32 * ATW_CW); mbar_init(bar_o, 1);
-    mbar_init(bar_oe, 32 * ATW_CW);
-    fence_mbar_init();
-  }
-  if (warp == 2) { tmem_alloc(tmem_slot, 256); tmem_relinquish(); }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
-  const uint32_t tS = tmem_base, tO = tmem_base + ATW_TMEM_O;
-  const int items = a.B * a.H;
-  const int kv_plane = a.Tk64 * 128;      // bytes actually loaded per K / V plane
-
-  if (warp == 0) {
-    if (lane == 0) {
-      uint32_t u = 0;
-      for (int item = blockIdx.x; item < items; item += gridDim.x) {
-        const int h = item % a.H, b = item / a.H;
-        for (int mt = 0; mt < a.mtiles; ++mt, ++u) {
-          if (u > 0) mbar_wait(bar_o, (u - 1) & 1u, 0x670u);      // previous PV retired: the operand buffer (V) and Q are free
-          mbar_arrive_expect_tx(bar_qk, 2u * ATW_Q_BYTES + 2u * kv_plane);
-#pragma unroll
-          for (int p = 0; p < 2; ++p) {
-            tma_load_4d(sQ + p * ATW_Q_BYTES, &a.q_map[p], bar_qk, 0, mt * 128, h, b);
-            tma_load_4d(sKV + p * ATW_KV_BYTES, &a.k_map[p], bar_qk, 0, 0, h, b);
-          }
-          mbar_wait(bar_s, u & 1u, 0x671u);                        // score MMAs retired: K is dead, V takes its place
-          mbar_arrive_expect_tx(bar_v, 2u * kv_plane);
-#pragma unroll
-          for (int p = 0; p < 2; ++p) tma_load_4d(sKV + p * ATW_KV_BYTES, &a.v_map[p], bar_v, 0, 0, h, b);
-        }
-      }
-    }
-  } else if (warp == 1) {
-    const uint32_t idesc_s = umma_idesc_f16(128, a.Tk16, false, false);
-    const uint32_t idesc_o = umma_idesc_f16(128, 64, false, true);
-    constexpr int PA2[3] = {1, 0, 0}, PB2[3] = {0, 1, 0};         // lo*hi, hi*lo, hi*hi
-    const uint64_t dQ0 = umma_smem_desc(sQ, 16, 1024), dK0 = umma_smem_desc(sKV, 16, 1024);
-    const uint64_t dV0 = umma_smem_desc(sKV, 8192, 1024);
-    const int ksteps = a.Tk16 / 16;
-    uint32_t u = 0;
-    for (int item = blockIdx.x; item < items; item += gridDim.x) {
-      for (int mt = 0; mt < a.mtiles; ++mt, ++u) {
-        mbar_wait(bar_qk, u & 1u, 0x680u);
-        tc_fence_after();
-        if (elect_one()) {
-#pragma unroll
-          for (int cb = 0; cb < 3; ++cb) {
-#pragma unroll
-            for (int k = 0; k < 4; ++k)
-              umma_f16(tS, desc_add(dQ0, PA2[cb] * ATW_Q_BYTES + k * 32), desc_add(dK0, PB2[cb] * ATW_KV_BYTES + k * 32), idesc_s,
-                        (cb | k) ? 1u : 0u);
-          }
-          umma_commit(bar_s);
-        }
-        __syncwarp();
-        mbar_wait(bar_p, u & 1u, 0x681u);                          // probabilities are in TMEM
-        mbar_wait(bar_v, u & 1u, 0x682u);                          // V is in the operand buffer
-        if (u > 0) mbar_wait(bar_oe, (u - 1) & 1u, 0x683u);        // previous output tile drained
-        tc_fence_after();
-        if (elect_one()) {
-          for (int t = 0; t < ksteps; ++t) {
-            const uint32_t voff = (t >> 2) * 8192 + (t & 3) * 2048;
-#pragma unroll
-            for (int cb = 0; cb < 3; ++cb)
-              umma_f16_ts(tO, tS + 16 * t + 8 * PA2[cb], desc_add(dV0, PB2[cb] * ATW_KV_BYTES + voff), idesc_o, (t | cb) ? 1u : 0u);
-          }
-          umma_commit(bar_o);
-        }
-        __syncwarp();
-      }
-    }
-  } else if (warp >= 4) {
-    const int w = (warp - 4) & 3, part = (warp - 4) >> 2;          // lane quarter, column part (0..1)
-    const int r = w * 32 + lane;
-    const uint32_t t_lane = static_cast<uint32_t>(w * 32) << 16;
-    const bool use_drop = a.drop.thresh != 0;
-    const float inv_keep = use_drop ? a.drop.inv_keep : 1.f;
-    const int nchunks = a.Tk16 / 16;
-    uint32_t u = 0;
-    for (int item = blockIdx.x; item < items; item += gridDim.x) {
-      const int h = item % a.H, b = item / a.H;
-      for (int mt = 0; mt < a.mtiles; ++mt, ++u) {
-        const uint32_t ph = u & 1u;
-        const int q = mt * 128 + r;
-        const bool active = mt * 128 + w * 32 < a.T;              // warp-uniform
-        mbar_wait(bar_s, ph, 0x690u);
-        tc_fence_after();
-        uint32_t sreg[16];
-        float mx = -INFINITY;
-        if (active) {
-          for (int c = part; c * 16 < a.T; c += 2) {
-            tmem_ld_32x16(tS + t_lane + c * 16, sreg);
-            tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 16; ++i)
-              if (c * 16 + i < a.T) mx = fmaxf(mx, __uint_as_float(sreg[i]));
-          }
-        }
-        xch[part * 128 + r] = mx;
-        half_quarter_sync(w);
-        mx = fmaxf(xch[r], xch[128 + r]);
-        const float mxs = mx * ATF_SC;
-        float sum = 0.f;
-        if (active) {
-          const uint64_t row_idx8 = ((static_cast<uint64_t>(item) * a.T + q) * a.Tp) >> 3;   // Tp % 8 == 0
-          for (int c = part; c < nchunks; c += 2) {
-            tmem_ld_32x16(tS + t_lane + c * 16, sreg);
-            uint32_t keep = 0xFFFFu;
-            if (use_drop)
-              keep = dropout_keep8(a.drop.seed, a.site, row_idx8 + 2 * c, a.drop.thresh) |
-                     (dropout_keep8(a.drop.seed, a.site, row_idx8 + 2 * c + 1, a.drop.thresh) << 8);
-            tmem_ld_wait();
-            uint32_t o01[16];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-              const int key = c * 16 + 2 * j;
-              float e0 = key < a.T ? at_exp2(__uint_as_float(sreg[2 * j]) * ATF_SC - mxs) : 0.f;
-              float e1 = key + 1 < a.T ? at_exp2(__uint_as_float(sreg[2 * j + 1]) * ATF_SC - mxs) : 0.f;
-              sum += e0 + e1;
-              e0 = ((keep >> (2 * j)) & 1u) ? e0 : 0.f;
-              e1 = ((keep >> (2 * j + 1)) & 1u) ? e1 : 0.f;
-              const uint32_t hi = pack2(e0, e1);
-              o01[j] = hi;                                                // plane 0 at columns 16c + j
-              e0 -= lo_to_f(hi);
-              e1 -= hi_to_f(hi);
-              o01[8 + j] = pack2(e0, e1);                                 // plane 1 at columns 16c + 8 + j
-            }
-            tmem_st_32x16(tS + t_lane + c * 16, o01);
-            if (a.mbits != nullptr && q < a.T)
-              a.mbits[(static_cast<int64_t>(item) * a.nC + c) * a.T + q] = static_cast<uint16_t>(keep);
-          }
-          tmem_st_wait();
-        }
-        xch[256 + part * 128 + r] = sum;
-        tc_fence_before();
-        mbar_arrive(bar_p);
-        half_quarter_sync(w);
-        sum = xch[256 + r] + xch[384 + r];
-        mbar_wait(bar_o, ph, 0x691u);
-        tc_fence_after();
-        float v[32];
-        if (active) {
-          uint32_t oreg[16];
-          const float sc = inv_keep / sum;
-#pragma unroll
-          for (int hlf = 0; hlf < 2; ++hlf) {
-            tmem_ld_32x16(tO + t_lane + part * 32 + hlf * 16, oreg);
-            tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 16; ++i) v[hlf * 16 + i] = __uint_as_float(oreg[i]) * sc;
-          }
-          if (part == 0 && q < a.T && a.stats != nullptr) a.stats[static_cast<int64_t>(item) * a.T + q] = make_float2(mxs, sum);
-        }
-        tc_fence_before();
-        mbar_arrive(bar_oe);                                      // the accumulator is free for the next tile's PV
-        if (active) {                                             // uniform over the quarter's two warps
-          const uint32_t stg = sbase + ATW_OFF_STG;
-#pragma unroll
-          for (int p = 0; p < 2; ++p) {
-#pragma unroll
-            for (int g = 0; g < 4; ++g) {                         // this warp's 32 columns = 16-byte chunks 4 part .. 4 part + 3
-              uint32_t wv[4];
-#pragma unroll
-              for (int i = 0; i < 4; ++i) {
-                wv[i] = pack2(v[g * 8 + 2 * i], v[g * 8 + 2 * i + 1]);
-                if (p == 0) {
-                  v[g * 8 + 2 * i] -= lo_to_f(wv[i]);
-                  v[g * 8 + 2 * i + 1] -= hi_to_f(wv[i]);
-                }
-              }
-              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stg + r * 128 + (((4 * part + g) ^ (r & 7)) << 4)),
-                           "r"(wv[0]), "r"(wv[1]), "r"(wv[2]), "r"(wv[3]) : "memory");
-            }
-            half_quarter_sync(w);
-#pragma unroll
-            for (int it = 0; it < 4; ++it) {                      // 16 of the quarter's 32 rows per warp, 4 rows per instruction
-              const int row = w * 32 + part * 16 + it * 4 + (lane >> 3);
-              uint4 val;
-              asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(val.x), "=r"(val.y), "=r"(val.z), "=r"(val.w)
-                           : "r"(stg + row * 128 + (((lane & 7) ^ (row & 7)) << 4)) : "memory");
-              const int qq = mt * 128 + row;
-              if (qq < a.T)
-                *reinterpret_cast<uint4*>(a.out + p * a.out_ps + (static_cast<int64_t>(b) * a.T + qq) * a.out_ld + h * 64 +
-                                          (lane & 7) * 8) = val;
-            }
-            half_quarter_sync(w);
-          }
-        }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 256);
-  }
-}
-
-static int attn_train_fwd2_launch(AttnTrainFwdArgs& a, const elem_t* qkv, int64_t qkv_ps, cudaStream_t st) {
-  const int64_t ld = 3 * 64 * a.H;
-  const int64_t dims[4] = {64, a.T, a.H, a.B};
-  const int64_t strides[3] = {ld, 64, static_cast<int64_t>(a.T) * ld};
-  for (int p = 0; p < 2; ++p) {
-    const elem_t* base = qkv + p * qkv_ps;
-    SPK_TRY(encode_map_4d(&a.q_map[p], base, dims, strides, 128));
-    SPK_TRY(encode_map_4d(&a.k_map[p], base + 64 * a.H, dims, strides, a.Tk64));
-    SPK_TRY(encode_map_4d(&a.v_map[p], base + 2 * 64 * a.H, dims, strides, a.Tk64));
-  }
-  static PerDeviceOnce once;
-  SPK_TRY(once.run([]() -> int {
-    SPK_CUDA(cudaFuncSetAttribute(attn_train_fwd2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ATW_SMEM));
-    return 0;
-  }));
-  const int items = a.B * a.H;
-  const int grid = items < 2 * device_sm_count() ? items : 2 * device_sm_count();
-  attn_train_fwd2_kernel<<<grid, ATW_THREADS, ATW_SMEM, st>>>(a);
-  SPK_CUDA(cudaGetLastError());
-  return 0;
-}
-
-// =====================================================================================================================
-// Inference variant (one fp16 plane, no dropout, nothing kept), T <= 192: the same structure with 8 compute warps,
-// 85 KB of shared memory and 256 TMEM columns, so that TWO CTAs share an SM and one item's softmax runs under the other
-// item's loads and MMAs (each item on its own is a serial chain TMA -> QK^T -> softmax -> PV -> store of ~8 us).
-constexpr int ATI_CW = 8, ATI_THREADS = 128 + 32 * ATI_CW, ATI_KV_ROWS = 192;
-constexpr int ATI_OFF_K = 16384, ATI_OFF_V = ATI_OFF_K + ATI_KV_ROWS * 128, ATI_OFF_X = ATI_OFF_V + ATI_KV_ROWS * 128;
-constexpr int ATI_OFF_STG = ATI_OFF_X + 2048, ATI_OFF_BAR = ATI_OFF_STG + 16384, ATI_SMEM = ATI_OFF_BAR + 128;
-constexpr int ATI_TMEM_O = 192;
-
-__global__ void __launch_bounds__(ATI_THREADS, 2) attn_infer_fwd_kernel(const __grid_constant__ AttnTrainFwdArgs a) {
-  pdl_trigger();   // the next kernel of the stream may start its prologue (ptx.cuh)
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  const uint32_t sbase = smem_u32(smem_raw);
-  const uint32_t sQ = sbase, sK = sbase + ATI_OFF_K, sV = sbase + ATI_OFF_V;
-  float* xch = reinterpret_cast<float*>(smem_raw + ATI_OFF_X);   // [0..255] max parts, [256..511] sum parts
-  const uint32_t bar_kv = sbase + ATI_OFF_BAR, bar_q = bar_kv + 8, bar_s = bar_kv + 16, bar_p = bar_kv + 24,
-                 bar_o = bar_kv + 32, bar_oe = bar_kv + 40, bar_kvfree = bar_kv + 48, tmem_slot = bar_kv + 56;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if ((sbase & 1023u) != 0) __trap();
-  if (warp == 0 && lane == 0) { tma_prefetch_desc(&a.q_map[0]); tma_prefetch_desc(&a.k_map[0]); tma_prefetch_desc(&a.v_map[0]); }
-  if (warp == 1 && lane == 0) {
-    mbar_init(bar_kv, 1); mbar_init(bar_q, 1); mbar_init(bar_s, 1); mbar_init(bar_p, 32 * ATI_CW); mbar_init(bar_o, 1);
-    mbar_init(bar_oe, 32 * ATI_CW); mbar_init(bar_kvfree, 1);
-    fence_mbar_init();
-  }
-  if (warp == 2) { tmem_alloc(tmem_slot, 256); tmem_relinquish(); }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
-  const uint32_t tS = tmem_base, tO = tmem_base + ATI_TMEM_O;
-  const int items = a.B * a.H;
-  const int kv_plane = a.Tk64 * 128;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      uint32_t u = 0, it = 0;
-      for (int item = blockIdx.x; item < items; item += gridDim.x, ++it) {
-        const int h = item % a.H, b = item / a.H;
-        if (it > 0) mbar_wait(bar_kvfree, (it - 1) & 1u, 0x640u);
-        mbar_arrive_expect_tx(bar_kv, 2u * kv_plane);
-        tma_load_4d(sK, &a.k_map[0], bar_kv, 0, 0, h, b);
-        tma_load_4d(sV, &a.v_map[0], bar_kv, 0, 0, h, b);
-        for (int mt = 0; mt < a.mtiles; ++mt, ++u) {
-          if (u > 0) mbar_wait(bar_s, (u - 1) & 1u, 0x641u);
-          mbar_arrive_expect_tx(bar_q, 16384);
-          tma_load_4d(sQ, &a.q_map[0], bar_q, 0, mt * 128, h, b);
-        }
-      }
-    }
-  } else if (warp == 1) {
-    const uint32_t idesc_s = umma_idesc_f16(128, a.Tk16, false, false);
-    const uint32_t idesc_o = umma_idesc_f16(128, 64, false, true);
-    const uint64_t dQ0 = umma_smem_desc(sQ, 16, 1024), dK0 = umma_smem_desc(sK, 16, 1024);
-    const uint64_t dV0 = umma_smem_desc(sV, 8192, 1024);
-    const int ksteps = a.Tk16 / 16;
-    uint32_t u = 0, it = 0;
-    for (int item = blockIdx.x; item < items; item += gridDim.x, ++it) {
-      for (int mt = 0; mt < a.mtiles; ++mt, ++u) {
-        mbar_wait(bar_q, u & 1u, 0x650u);
-        if (mt == 0) mbar_wait(bar_kv, it & 1u, 0x651u);
-        tc_fence_after();
-        if (elect_one()) {
-#pragma unroll
-          for (int k = 0; k < 4; ++k) umma_f16(tS, desc_add(dQ0, k * 32), desc_add(dK0, k * 32), idesc_s, k ? 1u : 0u);
-          umma_commit(bar_s);
-        }
-        __syncwarp();
-        mbar_wait(bar_p, u & 1u, 0x652u);
-        if (u > 0) mbar_wait(bar_oe, (u - 1) & 1u, 0x653u);
-        tc_fence_after();
-        if (elect_one()) {
-          for (int t = 0; t < ksteps; ++t)
-            umma_f16_ts(tO, tS + 16 * t, desc_add(dV0, (t >> 2) * 8192 + (t & 3) * 2048), idesc_o, t ? 1u : 0u);
-          umma_commit(bar_o);
-          if (mt == a.mtiles - 1) umma_commit(bar_kvfree);
-        }
-        __syncwarp();
-      }
-    }
-  } else if (warp >= 4) {
-    const int w = (warp - 4) & 3, part = (warp - 4) >> 2;          // lane quarter, column part (0..1)
-    const int r = w * 32 + lane;
-    const uint32_t t_lane = static_cast<uint32_t>(w * 32) << 16;
-    const int nchunks = a.Tk16 / 16;
-    uint32_t u = 0;
-    for (int item = blockIdx.x; item < items; item += gridDim.x) {
-      const int h = item % a.H, b = item / a.H;
-      for (int mt = 0; mt < a.mtiles; ++mt, ++u) {
-        const uint32_t ph = u & 1u;
-        const bool active = mt * 128 + w * 32 < a.T;              // warp-uniform
-        mbar_wait(bar_s, ph, 0x660u);
-        tc_fence_after();
-        uint32_t sreg[16];
-        float mx = -INFINITY;
-        if (active) {
-          for (int c = part; c * 16 < a.T; c += 2) {
-            tmem_ld_32x16(tS + t_lane + c * 16, sreg);
-            tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 16; ++i)
-              if (c * 16 + i < a.T) mx = fmaxf(mx, __uint_as_float(sreg[i]));
-          }
-        }
-        xch[part * 128 + r] = mx;
-        half_quarter_sync(w);
-        mx = fmaxf(xch[r], xch[128 + r]);
-        const float mxs = mx * ATF_SC;
-        float sum = 0.f;
-        if (active) {
-          for (int c = part; c < nchunks; c += 2) {
-            tmem_ld_32x16(tS + t_lane + c * 16, sreg);
-            tmem_ld_wait();
-            uint32_t o8[8];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-              const int key = c * 16 + 2 * j;
-              const float e0 = key < a.T ? at_exp2(__uint_as_float(sreg[2 * j]) * ATF_SC - mxs) : 0.f;
-              const float e1 = key + 1 < a.T ? at_exp2(__uint_as_float(sreg[2 * j + 1]) * ATF_SC - mxs) : 0.f;
-              sum += e0 + e1;
-              o8[j] = pack2(e0, e1);                                      // columns 16c + j: the A operand of key step c
-            }
-            tmem_st_32x8(tS + t_lane + c * 16, o8);
-          }
-          tmem_st_wait();
-        }
-        xch[256 + part * 128 + r] = sum;
-        tc_fence_before();
-        mbar_arrive(bar_p);
-        half_quarter_sync(w);
-        sum = xch[256 + r] + xch[384 + r];
-        mbar_wait(bar_o, ph, 0x661u);
-        tc_fence_after();
-        float v[32];
-        if (active) {
-          uint32_t oreg[16];
-          const float sc = 1.f / sum;
-#pragma unroll
-          for (int hlf = 0; hlf < 2; ++hlf) {
-            tmem_ld_32x16(tO + t_lane + part * 32 + hlf * 16, oreg);
-            tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 16; ++i) v[hlf * 16 + i] = __uint_as_float(oreg[i]) * sc;
-          }
-        }
-        tc_fence_before();
-        mbar_arrive(bar_oe);
-        if (active) {                                             // uniform over the quarter's two warps
-          const uint32_t stg = sbase + ATI_OFF_STG;
-#pragma unroll
-          for (int g = 0; g < 4; ++g) {                           // this warp's 32 columns = 16-byte chunks 4 part .. 4 part + 3
-            uint32_t wv[4];
-#pragma unroll
-            for (int i = 0; i < 4; ++i) wv[i] = pack2(v[g * 8 + 2 * i], v[g * 8 + 2 * i + 1]);
-            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stg + r * 128 + (((4 * part + g) ^ (r & 7)) << 4)),
-                         "r"(wv[0]), "r"(wv[1]), "r"(wv[2]), "r"(wv[3]) : "memory");
-          }
-          half_quarter_sync(w);
-#pragma unroll
-          for (int it = 0; it < 4; ++it) {                        // 16 of the quarter's 32 rows per warp, 4 rows per instruction
-            const int row = w * 32 + part * 16 + it * 4 + (lane >> 3);
-            uint4 val;
-            asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(val.x), "=r"(val.y), "=r"(val.z), "=r"(val.w)
-                         : "r"(stg + row * 128 + (((lane & 7) ^ (row & 7)) << 4)) : "memory");
-            const int qq = mt * 128 + row;
-            if (qq < a.T)
-              *reinterpret_cast<uint4*>(a.out + (static_cast<int64_t>(b) * a.T + qq) * a.out_ld + h * 64 + (lane & 7) * 8) = val;
-          }
-          half_quarter_sync(w);
-        }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 256);
-  }
+  if (planes == 3) return attn_fwd_launch<3, 16, false>(a, qkv, qkv_ps, "attn_train_fwd", st);
+  if (g_attn_fwd_two) return attn_fwd_launch<2, 8, true>(a, qkv, qkv_ps, "attn_train_fwd", st);
+  return attn_fwd_launch<2, 16, false>(a, qkv, qkv_ps, "attn_train_fwd", st);
 }
 
 // qkv: [B*T, 768] one plane; out: [B*T, out_ld] one plane (head h at column h*64).  T <= 192.
 int attn_infer_fwd(const void* qkv, void* out, int64_t out_ld, int B, int H, int T, cudaStream_t st) {
-  SPK_CHECK(T >= 1 && T <= ATI_KV_ROWS && H >= 1, "attn_infer_fwd: T=%d outside [1, %d]", T, ATI_KV_ROWS);
-  AttnTrainFwdArgs a;
+  SPK_CHECK(T >= 1 && T <= ATF_MAX_T && H >= 1, "attn_infer_fwd: T=%d outside [1, %d]", T, ATF_MAX_T);
+  AttnFwdArgs a;
   memset(&a, 0, sizeof(a));
-  a.B = B; a.H = H; a.T = T; a.Tp = (T + 7) / 8 * 8;
-  a.Tk16 = (T + 15) / 16 * 16;
-  a.Tk64 = (T + 63) / 64 * 64;
-  a.mtiles = (T + 127) / 128;
+  a.B = B; a.H = H; a.T = T;
   a.out = reinterpret_cast<elem_t*>(out);
   a.out_ld = out_ld;
-  const int64_t ld = 3 * 64 * H;
-  const int64_t dims[4] = {64, T, H, B};
-  const int64_t strides[3] = {ld, 64, static_cast<int64_t>(T) * ld};
-  const elem_t* base = reinterpret_cast<const elem_t*>(qkv);
-  SPK_TRY(encode_map_4d(&a.q_map[0], base, dims, strides, 128));
-  SPK_TRY(encode_map_4d(&a.k_map[0], base + 64 * H, dims, strides, a.Tk64));
-  SPK_TRY(encode_map_4d(&a.v_map[0], base + 2 * 64 * H, dims, strides, a.Tk64));
-  static PerDeviceOnce once;
-  SPK_TRY(once.run([]() -> int {
-    SPK_CUDA(cudaFuncSetAttribute(attn_infer_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ATI_SMEM));
-    return 0;
-  }));
-  const int items = B * H;
-  const int grid = items < 2 * device_sm_count() ? items : 2 * device_sm_count();
-  ProfScope prof("attn_fused_fwd", 4.0 * B * H * T * T * 64, 4.0 * B * T * 64 * H * 2.0, st);
-  attn_infer_fwd_kernel<<<grid, ATI_THREADS, ATI_SMEM, st>>>(a);
-  SPK_CUDA(cudaGetLastError());
-  return 0;
+  return attn_fwd_launch<1, 8, false>(a, qkv, 0, "attn_fused_fwd", st);
 }
 
 // =====================================================================================================================
@@ -1236,7 +819,7 @@ __global__ void __launch_bounds__(ATB_THREADS, 1) attn_train_bwd_kernel(const __
                   const int x = 2 * jj + e;
                   const float2 st = strow[x];                      // (m + log2 l, delta); +inf past the slice -> p = 0
                   const float kf = (word & (1u << x)) ? a.inv_keep : 0.f;
-                  const float p = at_exp2(fmaf(__uint_as_float(s_[x]), ATF_SC, -st.x));
+                  const float p = fast_exp2(fmaf(__uint_as_float(s_[x]), ATF_SC, -st.x));
                   pd[e] = p * kf;
                   ds[e] = (p * 0.125f) * fmaf(__uint_as_float(d_[x]), kf, -st.y);
                 }
@@ -1429,15 +1012,13 @@ int attn_train_bwd(const void* qkv, int64_t qkv_ps, const void* out, int64_t out
   a.inv_keep = drop.thresh != 0 ? drop.inv_keep : 1.f;
   a.timeline = g_attn_timeline;
   a.timeline_slots = g_attn_timeline_slots;
-  const int64_t ld = 3 * 64 * H;
   const int64_t dims[4] = {64, T, H, B};
-  const int64_t strides[3] = {ld, 64, static_cast<int64_t>(T) * ld};
   const int64_t ostrides[3] = {64 * H, 64, static_cast<int64_t>(T) * 64 * H};
   for (int p = 0; p < 2; ++p) {
-    const elem_t* base = reinterpret_cast<const elem_t*>(qkv) + p * qkv_ps;
-    SPK_TRY(encode_map_4d(&a.q_map[p], base, dims, strides, a.Tk64));
-    SPK_TRY(encode_map_4d(&a.k_map[p], base + 64 * H, dims, strides, 128));
-    SPK_TRY(encode_map_4d(&a.v_map[p], base + 2 * 64 * H, dims, strides, 128));
+    const elem_t* plane = reinterpret_cast<const elem_t*>(qkv) + p * qkv_ps;
+    SPK_TRY(encode_qkv_map(&a.q_map[p], plane, 0, B, H, T, a.Tk64));
+    SPK_TRY(encode_qkv_map(&a.k_map[p], plane, 1, B, H, T, 128));
+    SPK_TRY(encode_qkv_map(&a.v_map[p], plane, 2, B, H, T, 128));
     SPK_TRY(encode_map_4d(&a.do_map[p], reinterpret_cast<const elem_t*>(dout) + p * dout_ps, dims, ostrides, a.Tk64));
   }
   static PerDeviceOnce once;

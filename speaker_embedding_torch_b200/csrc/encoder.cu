@@ -19,7 +19,6 @@ int attn_row0_bwd(const void* datt0, int64_t da_ps, int g_planes, const void* q0
                   int64_t dkv_ps, float* dbias, const float* gscale, int B, int H, int T, int Tp, cudaStream_t st);
 int attn_fused_fwd(const void* qkv, void* out, int64_t out_ld, int B, int H, int T, cudaStream_t st);
 int attn_infer_fwd(const void* qkv, void* out, int64_t out_ld, int B, int H, int T, cudaStream_t st);
-int attn_train_max_frames(int planes);
 int attn_train_fwd(const void* qkv, int64_t qkv_ps, int planes, void* out, int64_t out_ps, int64_t out_ld, float* stats,
                    uint32_t* mbits, DropCfg drop, uint32_t site, int B, int H, int T, int Tp, cudaStream_t st);
 int attn_train_bwd(const void* qkv, int64_t qkv_ps, const void* out, int64_t out_ps, const void* dout, int64_t dout_ps,
@@ -164,7 +163,7 @@ static int make_plan(const spk_encoder_config& c, int B, int T, int S, int Pflag
   pl.h0bits = keep ? take_f32(cur, Mt * (D / 32)) : 0;     // 1-bit ReLU mask of the prenet (backward)
   pl.pe_t = take_f32(cur, static_cast<int64_t>(T) * D);
   // fused training attention (scores never leave the SM): multi-plane training plans up to 192 frames
-  pl.attn_tr = keep && pl.fused_train && P >= 2 && T <= 192 && T <= attn_train_max_frames(P) && pl.H == 4;
+  pl.attn_tr = keep && pl.fused_train && P >= 2 && T <= 192 && pl.H == 4;
   const int64_t score_elems = pl.attn_tr ? 128 : pl.BH * T * pl.Tp;     // the materialised path's score tensors
   pl.scr = take_split(cur, score_elems, P < 2 ? 2 : P);   // also holds fp32 scores / dP (4 B per element)
   const bool drop = keep;   // P_drop is only distinct in training; allocate with the stash

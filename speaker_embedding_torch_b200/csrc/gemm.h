@@ -105,4 +105,13 @@ void gemm_set_cta_pairs(int on);   // route eligible multi-plane GEMMs through t
 // box {64, box_rows, 1, 1}, 128-byte swizzle, out-of-bounds elements read as zero.
 int encode_map_4d(CUtensorMap* map, const void* base, const int64_t dims[4], const int64_t strides[3], int box_rows);
 
+// Map of Q (which = 0), K (1) or V (2) of one plane of the packed attention input qkv [B*T, 3*64*H], in which head h of
+// Q / K / V sits at column which*64*H + h*64: dims {64, T, H, B}, so rows >= T of a (slice, head) read as zeros.
+inline int encode_qkv_map(CUtensorMap* map, const void* qkv_plane, int which, int B, int H, int T, int box_rows) {
+  const int64_t ld = 3 * 64 * H;
+  const int64_t dims[4] = {64, T, H, B};
+  const int64_t strides[3] = {ld, 64, static_cast<int64_t>(T) * ld};
+  return encode_map_4d(map, static_cast<const elem_t*>(qkv_plane) + which * 64 * H, dims, strides, box_rows);
+}
+
 }  // namespace spk

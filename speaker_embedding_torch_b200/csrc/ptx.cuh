@@ -17,6 +17,12 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) {
 
 __device__ __forceinline__ uint32_t lane_id() { return threadIdx.x & 31; }
 
+__device__ __forceinline__ float fast_exp2(float x) {   // MUFU.EX2: ~2 ulp, plenty for fp16 probabilities
+  float y;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
+}
+
 // ----------------------------------------------------------------------------- mbarrier
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");

@@ -439,7 +439,7 @@ def test_fused_layernorm_training_forward_matches_the_separate_pass(frames, trai
 
 @pytest.mark.parametrize("frames", [1, 15, 16, 17, 100, 128, 129, 160, 191, 192])
 def test_two_cta_inference_attention_matches_the_one_cta_kernel(frames):
-    """attn_infer_fwd_kernel (two CTAs per SM, T <= 192) against attn_fused_fwd_kernel on the same input, and both
+    """attn_fwd_kernel<1, 8, false> (two CTAs per SM, T <= 192) against attn_fused_fwd_kernel on the same input, and both
     against the fp64 oracle (one fp16 plane: cosine >= 0.9999)."""
     from speaker_embedding_torch_b200 import _native
     m, state = _model(9)
@@ -464,8 +464,9 @@ def test_two_cta_inference_attention_matches_the_one_cta_kernel(frames):
 @pytest.mark.parametrize("frames", [1, 16, 100, 129, 160, 192])
 @pytest.mark.parametrize("train", [False, True])
 def test_two_cta_training_attention_forward_matches_the_one_cta_kernel(frames, train):
-    """attn_train_fwd2_kernel (two CTAs per SM, one operand buffer for K then V) against attn_train_fwd_kernel<2>: same
-    d-vectors, same saved statistics / keep bits (checked through the gradients of the shared backward)."""
+    """attn_fwd_kernel<2, 8, true> (two CTAs per SM, one operand buffer for K then V) against
+    attn_fwd_kernel<2, 16, false>: same d-vectors, same saved statistics / keep bits (checked through the gradients of
+    the shared backward)."""
     from speaker_embedding_torch_b200 import GE2E_Loss, _native
     nspk, utt = 3, 2
     mel = torch.as_tensor(synth.make_mel(500 + frames, nspk * utt, frames)).cuda()
