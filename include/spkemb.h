@@ -220,6 +220,23 @@ int spk_ge2e_loss(const float* emb, int speakers, int per_speaker, int dim, cons
                   const float* bias, float* loss, float* d_emb, float* d_weight, float* d_bias,
                   void* workspace, size_t workspace_bytes, void* stream);
 
+/* The GE2E paper's loss variants (Wan et al., 2018).  `mode` ORs one loss with one centroid rule:
+ *   SPK_GE2E_SOFTMAX    mean over rows of logsumexp_k z_ik - z_i,own (eq. 6; spk_ge2e_loss)
+ *   SPK_GE2E_CONTRAST   mean over rows of 1 - sigmoid(z_i,own) + sigmoid(max_{k != own} z_ik) (eq. 7); ties in the
+ *                       maximum go to the lowest speaker index.  Needs speakers >= 2.
+ *   SPK_GE2E_EXCLUSIVE  the own-speaker column of row i uses the centroid of the speaker's other rows (eq. 8); every
+ *                       other column keeps the inclusive centroid (eq. 9).  Needs per_speaker >= 2.
+ * Mode 0 runs the kernels of spk_ge2e_loss, and spk_ge2e_workspace_bytes_ex(n, m, 0) equals
+ * spk_ge2e_workspace_bytes(n, m).  Unknown mode bits and the shape limits above return SPK_EINVAL (workspace query: 0)
+ * before any CUDA call.  With SPK_GE2E_CONTRAST, d_bias is no longer zero. */
+#define SPK_GE2E_SOFTMAX 0
+#define SPK_GE2E_CONTRAST 1
+#define SPK_GE2E_EXCLUSIVE (1 << 8)
+size_t spk_ge2e_workspace_bytes_ex(int speakers, int per_speaker, int mode);
+int spk_ge2e_loss_ex(const float* emb, int speakers, int per_speaker, int dim, int mode, const float* weight,
+                     const float* bias, float* loss, float* d_emb, float* d_weight, float* d_bias,
+                     void* workspace, size_t workspace_bytes, void* stream);
+
 /* Fused optimiser over a list of tensors (replaces Radam.py:25-90 / torch AdamW + the
  * clip_grad_norm_ site Train.py:154-159).  One launch computes the global grad norm, one applies
  * clip + update.  kind: 0 = RAdam (Radam.py), 1 = AdamW.  step is 1-based.

@@ -4,8 +4,8 @@ Same public surface as /root/reference/Modules.py:
   * ``GE2E(hyper_parameters)``; ``forward(features[B*S, Mel_Dim, T], samples=1) -> [B, Embedding_Size]``
     (Modules.py:5-59), same sub-module / parameter names, ``state_dict`` keys and shapes
     (SURVEY.md Appendix A), so reference checkpoints load with ``strict=True`` and vice versa;
-  * ``GE2E_Loss(init_weight=10.0, init_bias=-5.0)``; ``forward(embeddings[N*M, D], pattern_per_speaker)``
-    -> 0-dim loss (Modules.py:112-156), ``weight`` / ``bias`` 0-dim parameters;
+  * ``GE2E_Loss(init_weight=10.0, init_bias=-5.0, loss_method="softmax", centroids="inclusive")``;
+    ``forward(embeddings[N*M, D], pattern_per_speaker)`` -> 0-dim loss (Modules.py:112-156), ``weight`` / ``bias`` 0-dim parameters;
   * ``Conv1d`` and ``Positional_Encoding`` helper modules (Modules.py:61-109).
 
 The modules only OWN parameters; the arithmetic runs in libspkemb.so (hand-written sm_100a
@@ -540,10 +540,10 @@ def Overlapped_Slices(windows: torch.Tensor, frame_length: int, overlap_length: 
 
 
 class _GE2ELossFunction(torch.autograd.Function):
-    """Loss and gradients from ONE fused kernel launch (spk_ge2e_loss); backward only rescales."""
+    """Loss and gradients from ONE fused kernel launch (spk_ge2e_loss_ex); backward only rescales."""
 
     @staticmethod
-    def forward(ctx, embeddings, weight, bias, per_speaker):
+    def forward(ctx, embeddings, weight, bias, per_speaker, mode=0):
         N.require_cuda(embeddings, "embeddings")
         emb = embeddings.detach().contiguous().float()
         if emb.dim() != 2 or emb.size(0) % per_speaker != 0:
@@ -553,17 +553,20 @@ class _GE2ELossFunction(torch.autograd.Function):
         device = emb.device
         need_grad = any(ctx.needs_input_grad[:3])
         with torch.cuda.device(device):
-            wsb = N.lib().spk_ge2e_workspace_bytes(speakers, per_speaker)
+            wsb = N.lib().spk_ge2e_workspace_bytes_ex(speakers, per_speaker, mode)
+            if wsb == 0:                                                   # refused mode / shape
+                raise RuntimeError("spk_ge2e_workspace_bytes_ex failed: %s"
+                                   % N.lib().spk_last_error().decode("utf-8", "replace"))
             ws = torch.empty(wsb, dtype=torch.uint8, device=device)
             scal = torch.empty(3, dtype=torch.float32, device=device)      # loss, dw, db
             d_emb = torch.empty_like(emb) if need_grad else None
-            N.check(N.lib().spk_ge2e_loss(N.ptr(emb), speakers, per_speaker, emb.size(1),
-                                          N.ptr(weight.detach().float().contiguous()),
-                                          N.ptr(bias.detach().float().contiguous()),
-                                          ctypes.c_void_p(scal.data_ptr()), N.ptr(d_emb),
-                                          ctypes.c_void_p(scal.data_ptr() + 4) if need_grad else None,
-                                          ctypes.c_void_p(scal.data_ptr() + 8) if need_grad else None,
-                                          N.ptr(ws), wsb, N.stream_ptr(device)), "spk_ge2e_loss")
+            N.check(N.lib().spk_ge2e_loss_ex(N.ptr(emb), speakers, per_speaker, emb.size(1), mode,
+                                             N.ptr(weight.detach().float().contiguous()),
+                                             N.ptr(bias.detach().float().contiguous()),
+                                             ctypes.c_void_p(scal.data_ptr()), N.ptr(d_emb),
+                                             ctypes.c_void_p(scal.data_ptr() + 4) if need_grad else None,
+                                             ctypes.c_void_p(scal.data_ptr() + 8) if need_grad else None,
+                                             N.ptr(ws), wsb, N.stream_ptr(device)), "spk_ge2e_loss_ex")
         ctx.d_emb, ctx.scal = d_emb, scal
         return scal[0].clone()
 
@@ -573,27 +576,45 @@ class _GE2ELossFunction(torch.autograd.Function):
         g_e = d_emb * grad_loss if ctx.needs_input_grad[0] else None
         g_w = scal[1] * grad_loss if ctx.needs_input_grad[1] else None
         g_b = scal[2] * grad_loss if ctx.needs_input_grad[2] else None
-        return g_e, g_w, g_b, None
+        return g_e, g_w, g_b, None, None
+
+
+_GE2E_METHODS = {"softmax": 0, "contrast": N.GE2E_CONTRAST}
+_GE2E_CENTROIDS = {"inclusive": 0, "exclusive": N.GE2E_EXCLUSIVE}
 
 
 class GE2E_Loss(torch.nn.Module):
-    """GE2E softmax loss, logits = weight * cos(e, centroid) - bias (Modules.py:112-156).
+    """GE2E loss, logits = weight * cos(e, centroid) - bias (Modules.py:112-156).
 
-    The reference's "within" similarity uses the inclusive sum-centroid, which after cosine
-    normalisation is the diagonal block of the "between" matrix, so the loss is plain
-    cross-entropy of the [N*M, N] scaled cosine matrix against the row's speaker (SURVEY.md D2)."""
+    The defaults are the reference's: the softmax loss with inclusive centroids.  Its "within" similarity uses the
+    inclusive sum-centroid, which after cosine normalisation is the diagonal block of the "between" matrix, so the loss
+    is plain cross-entropy of the [N*M, N] scaled cosine matrix against the row's speaker (SURVEY.md D2).
 
-    def __init__(self, init_weight=10.0, init_bias=-5.0):
+    The GE2E paper's variants (DESIGN.md §3.3): ``loss_method="contrast"`` is
+    ``1 - sigmoid(z_own) + max_{k != own} sigmoid(z_k)`` (eq. 7; needs two speakers), and ``centroids="exclusive"``
+    computes each row's own-speaker similarity against the mean of the speaker's other utterances (eq. 8; needs two
+    utterances per speaker)."""
+
+    def __init__(self, init_weight=10.0, init_bias=-5.0, loss_method="softmax", centroids="inclusive"):
         super().__init__()
+        if loss_method not in _GE2E_METHODS:
+            raise ValueError("loss_method must be one of %s, got %r" % (sorted(_GE2E_METHODS), loss_method))
+        if centroids not in _GE2E_CENTROIDS:
+            raise ValueError("centroids must be one of %s, got %r" % (sorted(_GE2E_CENTROIDS), centroids))
         self.weight = torch.nn.Parameter(torch.tensor(init_weight))
         self.bias = torch.nn.Parameter(torch.tensor(init_bias))
+        self.loss_method, self.centroids = loss_method, centroids
+        self._mode = _GE2E_METHODS[loss_method] | _GE2E_CENTROIDS[centroids]
+
+    def extra_repr(self):
+        return "loss_method=%r, centroids=%r" % (self.loss_method, self.centroids)
 
     def forward(self, embeddings, pattern_per_speaker):
-        """embeddings: [Batch, Emb_dim], speaker-major rows; returns the mean cross-entropy (0-dim)."""
+        """embeddings: [Batch, Emb_dim], speaker-major rows; returns the mean loss over the rows (0-dim)."""
         if not torch.is_grad_enabled():
             return _GE2ELossFunction.apply(embeddings.detach(), self.weight.detach(), self.bias.detach(),
-                                           int(pattern_per_speaker))
-        loss = _GE2ELossFunction.apply(embeddings, self.weight, self.bias, int(pattern_per_speaker))
+                                           int(pattern_per_speaker), self._mode)
+        loss = _GE2ELossFunction.apply(embeddings, self.weight, self.bias, int(pattern_per_speaker), self._mode)
         LAST_TRAINING_LOSS[loss.device] = loss.detach()      # picked up by distributed.allreduce_gradients
         return loss
 

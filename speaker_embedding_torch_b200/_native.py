@@ -18,6 +18,8 @@ CSRC = os.path.join(_HERE, "csrc")
 SPK_MAX_LAYERS = 8
 OPTIM_MAX_CHUNKS = 16      # SPK_OPTIM_MAX_CHUNKS
 ABI_VERSION = 2
+GE2E_CONTRAST = 1          # SPK_GE2E_CONTRAST
+GE2E_EXCLUSIVE = 1 << 8    # SPK_GE2E_EXCLUSIVE
 
 EXPORTS = (
     "spk_abi_version", "spk_last_error", "spk_encoder_workspace_bytes", "spk_encoder_forward",
@@ -28,6 +30,7 @@ EXPORTS = (
     "spk_mel_frames", "spk_mel_spectrogram", "spk_set_debug_buffer", "spk_encoder_backward_input",
     "spk_mel_backward_workspace_bytes", "spk_mel_spectrogram_backward",
     "spk_encoder_forward_segments", "spk_encoder_backward_segments",
+    "spk_ge2e_workspace_bytes_ex", "spk_ge2e_loss_ex",
 )
 
 c_f32p = ctypes.c_void_p  # device pointers travel as integers
@@ -155,6 +158,10 @@ def lib():
         L.spk_ge2e_workspace_bytes.argtypes = [i32, i32]
         L.spk_ge2e_loss.restype = i32
         L.spk_ge2e_loss.argtypes = [vp, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, sz, vp]
+        L.spk_ge2e_workspace_bytes_ex.restype = sz
+        L.spk_ge2e_workspace_bytes_ex.argtypes = [i32, i32, i32]
+        L.spk_ge2e_loss_ex.restype = i32
+        L.spk_ge2e_loss_ex.argtypes = [vp, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, sz, vp]
         L.spk_optim_step.restype = i32
         L.spk_optim_step.argtypes = [ctypes.POINTER(OptimTensors), i32, i64, f32, f32, f32, f32, f32, f32, f32,
                                      vp, i32, i32, i32, vp]

@@ -156,6 +156,34 @@ int spk_ge2e_loss(const float* emb, int speakers, int per_speaker, int dim, cons
                     workspace_bytes, as_stream(stream));
 }
 
+static_assert(SPK_GE2E_CONTRAST == GE2E_CONTRAST && SPK_GE2E_EXCLUSIVE == GE2E_EXCLUSIVE, "GE2E mode bits");
+
+// Mode checks shared by the two variant entry points; host-only.
+static int check_ge2e_mode(const char* fn, int speakers, int per_speaker, int mode) {
+  SPK_CHECK((mode & ~GE2E_MODE_BITS) == 0, "%s: unknown mode bits 0x%x (SPK_GE2E_CONTRAST | SPK_GE2E_EXCLUSIVE)", fn,
+            mode & ~GE2E_MODE_BITS);
+  SPK_CHECK(!(mode & GE2E_EXCLUSIVE) || per_speaker >= 2,
+            "%s: exclusive centroids need at least 2 utterances per speaker (got %d)", fn, per_speaker);
+  SPK_CHECK(!(mode & GE2E_CONTRAST) || speakers >= 2, "%s: the contrast loss needs at least 2 speakers (got %d)", fn,
+            speakers);
+  return 0;
+}
+
+size_t spk_ge2e_workspace_bytes_ex(int speakers, int per_speaker, int mode) {
+  if (check_ge2e_mode("spk_ge2e_workspace_bytes_ex", speakers, per_speaker, mode) != 0) return 0;
+  return ge2e_workspace_bytes(speakers, per_speaker, mode);
+}
+
+int spk_ge2e_loss_ex(const float* emb, int speakers, int per_speaker, int dim, int mode, const float* weight,
+                     const float* bias, float* loss, float* d_emb, float* d_weight, float* d_bias, void* workspace,
+                     size_t workspace_bytes, void* stream) {
+  SPK_CHECK(emb && weight && bias && loss && workspace, "spk_ge2e_loss_ex: null argument");
+  SPK_CHECK(d_emb == nullptr || (d_weight && d_bias), "spk_ge2e_loss_ex: d_weight/d_bias required with d_emb");
+  SPK_TRY(check_ge2e_mode("spk_ge2e_loss_ex", speakers, per_speaker, mode));
+  return ge2e_fused(emb, speakers, per_speaker, dim, weight, bias, loss, d_emb, d_weight, d_bias, workspace,
+                    workspace_bytes, as_stream(stream), mode);
+}
+
 int spk_optim_step(const spk_optim_tensors* tensors, int kind, int64_t step, float lr, float beta1, float beta2,
                    float eps, float weight_decay, float max_grad_norm, float grad_scale, float* norm_scratch,
                    int phase, int chunk, int nchunks, void* stream) {

@@ -15,6 +15,7 @@
 // D is fixed at 256 (= Embedding_Size of the reference hyper-parameters): thread <-> column.
 #include "common.cuh"
 #include "ge2e.h"
+#include "ge2e_excl.cuh"
 #include "ptx.cuh"
 
 namespace spk {
@@ -46,12 +47,16 @@ __device__ __forceinline__ float block_sum_256(float v, float* red8) {
   return s;
 }
 
+// EXCL: exclusive own-speaker centroids (ge2e_excl.cuh): phase 1 also writes each row's diagonal cosine `cos_own` and
+// `urinv` = 1 / max(|u_i| / (M-1), eps); phase 3 adds the diagonal's gradient `gdiag` (written by the row stage).
+template <bool EXCL>
 __global__ void __launch_bounds__(256, 2)
 ge2e_fused_kernel(const float* __restrict__ E, int N, int M, const float* __restrict__ w_ptr,
                   const float* __restrict__ b_ptr, float* __restrict__ loss, float* __restrict__ dE,
                   float* __restrict__ dw, float* __restrict__ db, float* __restrict__ chat,
                   float* __restrict__ cinv, float* __restrict__ einv, float* __restrict__ dchat, int need_grad,
-                  float eps, int phase) {
+                  float eps, int phase, float* __restrict__ cos_own, float* __restrict__ urinv,
+                  const float* __restrict__ gdiag) {
   // `phase` selects one of the three stages; the launcher enqueues them back to back on one stream (stream order is the
   // grid-wide barrier: a cooperative launch with two grid.sync() cost 32 us at the training size, mostly in the syncs)
   extern __shared__ __align__(16) uint8_t smem_raw[];
@@ -89,18 +94,46 @@ ge2e_fused_kernel(const float* __restrict__ E, int N, int M, const float* __rest
     float cv = 0.f;
 #pragma unroll
     for (int wv = 0; wv < 8; ++wv) cv += sm.e[wv][tid];
+    if constexpr (EXCL) sm.e[8][tid] = cv;       // the speaker's column sum (visible after block_sum_256's barriers)
     cv *= 1.f / static_cast<float>(M);
     const float nrm = fmaxf(sqrtf(block_sum_256(cv * cv, red8)), eps);
     chat[static_cast<int64_t>(k) * GD + tid] = cv / nrm;
     if (need_grad) dchat[static_cast<int64_t>(k) * GD + tid] = 0.f;
     if (tid == 0) cinv[k] = 1.f / nrm;
+    if constexpr (EXCL) {
+      // warp per row, as above (lane 0 wrote einv of these rows): u_i = sum - e_i, formed directly
+      const float inv_m1 = 1.f / static_cast<float>(M - 1);
+      for (int m = warp; m < M; m += 8) {
+        const int64_t r = static_cast<int64_t>(k) * M + m;
+        const float4 a0 = __ldg(reinterpret_cast<const float4*>(E + r * GD + lane * 8));
+        const float4 a1 = __ldg(reinterpret_cast<const float4*>(E + r * GD + lane * 8 + 4));
+        const float4 s0 = *reinterpret_cast<const float4*>(&sm.e[8][lane * 8]);
+        const float4 s1 = *reinterpret_cast<const float4*>(&sm.e[8][lane * 8 + 4]);
+        const float v[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
+        const float sv[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w};
+        float qu = 0.f, qeu = 0.f;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          const float u = sv[i] - v[i];
+          qu += u * u;
+          qeu += v[i] * u;
+        }
+        qu = warp_sum(qu);
+        qeu = warp_sum(qeu);
+        if (lane == 0) {
+          const float ur = 1.f / fmaxf(sqrtf(qu) * inv_m1, eps);
+          urinv[r] = ur;
+          cos_own[r] = qeu * einv[r] * (ur * inv_m1);
+        }
+      }
+    }
     __syncthreads();
   }
   return;
   }
 
-  // ------------------------------------------------------------------ phase 2
-  if (phase == 2) {
+  // ------------------------------------------------------------------ phase 2 (mode 0 only: the first row stage)
+  if (!EXCL && phase == 2) {
   const int r_loc = tid >> 4;      // 0..15 : row within tile (S-tile compute mapping)
   const int cgp = tid & 15;        // columns cgp, cgp+16, cgp+32, cgp+48 of the centroid tile
   const int64_t row_tiles = (NM + TR - 1) / TR;
@@ -287,7 +320,11 @@ ge2e_fused_kernel(const float* __restrict__ E, int N, int M, const float* __rest
     const float ch = chat[static_cast<int64_t>(k) * GD + tid];
     const float dot = block_sum_256(dc * ch, red8);
     const float u = (dc - dot * ch) * cinv[k] * (1.f / static_cast<float>(M));
-    for (int m = 0; m < M; ++m) dE[(static_cast<int64_t>(k) * M + m) * GD + tid] += u;
+    if constexpr (EXCL) {
+      ge2e_excl_diag_grad(E, k, M, einv, cos_own, urinv, gdiag, dE, u);
+    } else {
+      for (int m = 0; m < M; ++m) dE[(static_cast<int64_t>(k) * M + m) * GD + tid] += u;
+    }
   }
 }
 
@@ -327,11 +364,17 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
                : "memory");
 }
 
+// MODE (GE2E_CONTRAST | GE2E_EXCLUSIVE bits): with GE2E_EXCLUSIVE the own-speaker cosine of each row is replaced by
+// `cos_own` (stage 1) after pass A, and its G goes to `gdiag` instead of G^T, so that the inclusive centroid does not
+// receive it; with GE2E_CONTRAST the log-sum-exp gives way to the own / strongest-impostor rule.
+template <int MODE>
 __global__ void __launch_bounds__(TILE_THREADS, 2)
 ge2e_rows_tile_kernel(const float* __restrict__ E, int N, int M, const float* __restrict__ w_ptr,
                       const float* __restrict__ b_ptr, float* __restrict__ loss, float* __restrict__ dE,
                       float* __restrict__ dw, float* __restrict__ db, const float* __restrict__ chat,
-                      const float* __restrict__ einv, float* __restrict__ dchat, int need_grad) {
+                      const float* __restrict__ einv, float* __restrict__ dchat, int need_grad,
+                      const float* __restrict__ cos_own, float* __restrict__ gdiag) {
+  constexpr bool EXCL = (MODE & GE2E_EXCLUSIVE) != 0, CONTRAST = (MODE & GE2E_CONTRAST) != 0;
   extern __shared__ __align__(16) uint8_t smem_raw[];
   Ge2eTileSmem& sm = *reinterpret_cast<Ge2eTileSmem*>(smem_raw);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -425,30 +468,72 @@ ge2e_rows_tile_kernel(const float* __restrict__ E, int N, int M, const float* __
     const int64_t gi = row0 + warp;
     const bool live = gi < NM;
     const int label = live ? static_cast<int>(gi / M) : -1;
-    float mx = -INFINITY;
-    for (int j = lane; j < N; j += 32) mx = fmaxf(mx, w * sm.s[warp][j] - b);
-    mx = warp_max(mx);
-    float sum = 0.f;
-    for (int j = lane; j < N; j += 32) sum += expf(w * sm.s[warp][j] - b - mx);
-    sum = warp_sum(sum);
-    const float lse = mx + logf(sum);
+    if constexpr (EXCL) {
+      if (live && lane == 0) sm.s[warp][label] = __ldg(cos_own + gi);
+      __syncwarp();
+    }
     float lrow = 0.f, dw_part = 0.f, db_part = 0.f;
-    if (live && lane == 0) lrow = lse - (w * sm.s[warp][label] - b);
-    if (need_grad) {
+    if constexpr (CONTRAST) {
+      // L = 1 - sigmoid(z_own) + sigmoid(z_k*), k* = the largest off-diagonal logit, ties to the lowest column
+      float bz = -INFINITY;
+      int bj = N;
       for (int j = lane; j < N; j += 32) {
-        float gval = 0.f;
-        if (live) {
-          const float sv = sm.s[warp][j];
-          const float p = expf(w * sv - b - lse);
-          const float pm = (p - (j == label ? 1.f : 0.f)) * inv_nm;
-          dw_part += pm * sv;
-          db_part -= pm;
-          gval = w * pm;
-        }
-        sm.gt[j][warp] = gval;
+        const float z = w * sm.s[warp][j] - b;
+        if (j != label && z > bz) { bz = z; bj = j; }
       }
-      dw_part = warp_sum(dw_part);
-      db_part = warp_sum(db_part);
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        const float oz = __shfl_xor_sync(0xffffffffu, bz, o);
+        const int oj = __shfl_xor_sync(0xffffffffu, bj, o);
+        if (oz > bz || (oz == bz && oj < bj)) { bz = oz; bj = oj; }
+      }
+      // sigmoid(z) and sigmoid(-z) = 1 - sigmoid(z) each from its own exp: no cancellation when |z| is large
+      const float zo = live ? w * sm.s[warp][label] - b : 0.f;
+      const float so = 1.f / (1.f + expf(-zo)), son = 1.f / (1.f + expf(zo));
+      const float sk = 1.f / (1.f + expf(-bz)), skn = 1.f / (1.f + expf(bz));
+      if (live && lane == 0) lrow = son + sk;
+      if (need_grad) {
+        const float go = -so * son * inv_nm, gk = sk * skn * inv_nm;
+        for (int j = lane; j < N; j += 32) {
+          float gval = 0.f;
+          if (live && (j == label || j == bj)) {
+            const float pm = j == label ? go : gk;
+            dw_part += pm * sm.s[warp][j];
+            db_part -= pm;
+            gval = w * pm;
+            if (EXCL && j == label) { gdiag[gi] = gval; gval = 0.f; }
+          }
+          sm.gt[j][warp] = gval;
+        }
+        dw_part = warp_sum(dw_part);
+        db_part = warp_sum(db_part);
+      }
+    } else {
+      float mx = -INFINITY;
+      for (int j = lane; j < N; j += 32) mx = fmaxf(mx, w * sm.s[warp][j] - b);
+      mx = warp_max(mx);
+      float sum = 0.f;
+      for (int j = lane; j < N; j += 32) sum += expf(w * sm.s[warp][j] - b - mx);
+      sum = warp_sum(sum);
+      const float lse = mx + logf(sum);
+      if (live && lane == 0) lrow = lse - (w * sm.s[warp][label] - b);
+      if (need_grad) {
+        for (int j = lane; j < N; j += 32) {
+          float gval = 0.f;
+          if (live) {
+            const float sv = sm.s[warp][j];
+            const float p = expf(w * sv - b - lse);
+            const float pm = (p - (j == label ? 1.f : 0.f)) * inv_nm;
+            dw_part += pm * sv;
+            db_part -= pm;
+            gval = w * pm;
+            if (EXCL && j == label) { gdiag[gi] = gval; gval = 0.f; }
+          }
+          sm.gt[j][warp] = gval;
+        }
+        dw_part = warp_sum(dw_part);
+        db_part = warp_sum(db_part);
+      }
     }
     if (lane == 0) { sm.scal[0][warp] = lrow; sm.scal[1][warp] = dw_part; sm.scal[2][warp] = db_part; }
   }
@@ -534,46 +619,66 @@ void ge2e_set_tile_v2(int on) { g_ge2e_tile_v2 = on != 0; }
 static int g_ge2e_pdl = 1;         // spk_set_option("ge2e_dependent_launch", 0/1): programmatic dependent launch of stages 2, 3
 void ge2e_set_pdl(int on) { g_ge2e_pdl = on != 0; }
 
-static size_t ge2e_simt_workspace_bytes(int N, int M) {
+static size_t ge2e_simt_workspace_bytes(int N, int M, int mode) {
   const size_t NM = static_cast<size_t>(N) * M;
-  return (2 * static_cast<size_t>(N) * GD + N + NM) * sizeof(float) + 256;
+  const size_t excl = (mode & GE2E_EXCLUSIVE) ? 3 * NM : 0;      // cos_own, urinv, gdiag
+  return (2 * static_cast<size_t>(N) * GD + N + NM + excl) * sizeof(float) + 256;
 }
-size_t ge2e_workspace_bytes(int N, int M) {
-  return N >= GE2E_TC_MIN_SPEAKERS ? ge2e_tc_workspace_bytes(N, M) : ge2e_simt_workspace_bytes(N, M);
+size_t ge2e_workspace_bytes(int N, int M, int mode) {
+  return N >= GE2E_TC_MIN_SPEAKERS ? ge2e_tc_workspace_bytes(N, M, mode) : ge2e_simt_workspace_bytes(N, M, mode);
 }
 
 int ge2e_fused(const float* E, int N, int M, int D, const float* w, const float* b, float* loss, float* dE, float* dw,
-               float* db, void* ws, size_t ws_bytes, cudaStream_t st) {
+               float* db, void* ws, size_t ws_bytes, cudaStream_t st, int mode) {
   SPK_CHECK(D == GD, "ge2e: embedding size %d not supported by this build (256)", D);
   SPK_CHECK(N >= 1 && M >= 1, "ge2e: need at least one speaker and one utterance");
   SPK_CHECK((reinterpret_cast<uintptr_t>(E) & 15) == 0, "ge2e: embeddings must be 16-byte aligned");
   if (N >= GE2E_TC_MIN_SPEAKERS)   // intensity 0.75 N FLOP/B: tensor-core composition (ge2e_tc.cu)
-    return ge2e_tc(E, N, M, w, b, loss, dE, dw, db, ws, ws_bytes, st);
-  if (ws_bytes < ge2e_simt_workspace_bytes(N, M)) {
-    set_error("ge2e: workspace too small (%zu < %zu)", ws_bytes, ge2e_simt_workspace_bytes(N, M));
+    return ge2e_tc(E, N, M, w, b, loss, dE, dw, db, ws, ws_bytes, st, mode);
+  if (ws_bytes < ge2e_simt_workspace_bytes(N, M, mode)) {
+    set_error("ge2e: workspace too small (%zu < %zu)", ws_bytes, ge2e_simt_workspace_bytes(N, M, mode));
     return SPK_ENOMEM;
   }
   const int need_grad = (dE != nullptr);
+  const bool excl = (mode & GE2E_EXCLUSIVE) != 0;
   float* chat = reinterpret_cast<float*>(ws);
   float* dchat = chat + static_cast<size_t>(N) * GD;
   float* cinv = dchat + static_cast<size_t>(N) * GD;
   float* einv = cinv + N;
+  float* cos_own = excl ? einv + static_cast<size_t>(N) * M : nullptr;
+  float* urinv = excl ? cos_own + static_cast<size_t>(N) * M : nullptr;
+  float* gdiag = excl ? urinv + static_cast<size_t>(N) * M : nullptr;
 
   static PerDeviceOnce once;
   const int smem = static_cast<int>(sizeof(Ge2eSmem));
   const int smem2 = static_cast<int>(sizeof(Ge2eTileSmem));
   SPK_TRY(once.run([&]() -> int {
-    SPK_CUDA(cudaFuncSetAttribute(ge2e_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    SPK_CUDA(cudaFuncSetAttribute(ge2e_rows_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
+    SPK_CUDA(cudaFuncSetAttribute(ge2e_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    SPK_CUDA(cudaFuncSetAttribute(ge2e_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    SPK_CUDA(cudaFuncSetAttribute(ge2e_rows_tile_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
+    SPK_CUDA(cudaFuncSetAttribute(ge2e_rows_tile_kernel<GE2E_CONTRAST>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  smem2));
+    SPK_CUDA(cudaFuncSetAttribute(ge2e_rows_tile_kernel<GE2E_EXCLUSIVE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  smem2));
+    SPK_CUDA(cudaFuncSetAttribute(ge2e_rows_tile_kernel<GE2E_EXCLUSIVE | GE2E_CONTRAST>,
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
     return 0;
   }));
+  auto* centroid_stage = excl ? ge2e_fused_kernel<true> : ge2e_fused_kernel<false>;
+  auto* row_stage = ge2e_rows_tile_kernel<0>;
+  if (mode == GE2E_CONTRAST) row_stage = ge2e_rows_tile_kernel<GE2E_CONTRAST>;
+  if (mode == GE2E_EXCLUSIVE) row_stage = ge2e_rows_tile_kernel<GE2E_EXCLUSIVE>;
+  if (mode == (GE2E_EXCLUSIVE | GE2E_CONTRAST)) row_stage = ge2e_rows_tile_kernel<GE2E_EXCLUSIVE | GE2E_CONTRAST>;
+  // the variants exist only in the re-tiled row stage; "ge2e_row_tile_v2" = 0 selects the first one for mode 0 alone
+  const bool tile_v2 = g_ge2e_tile_v2 || mode != 0;
   const long long NM = 1LL * N * M;
   const int row_tiles = static_cast<int>((NM + TR - 1) / TR);
   const float eps = 1e-8f;
   ProfScope prof(need_grad ? "ge2e_fused_fwd_bwd" : "ge2e_fused_fwd", (need_grad ? 6.0 : 2.0) * NM * N * GD,
                  (need_grad ? 2.0 : 1.0) * NM * GD * 4.0, st);
   // three launches in stream order: centroids | row tiles (loss, dE row part, dC) | centroid part of dE
-  ge2e_fused_kernel<<<N, 256, smem, st>>>(E, N, M, w, b, loss, dE, dw, db, chat, cinv, einv, dchat, need_grad, eps, 1);
+  centroid_stage<<<N, 256, smem, st>>>(E, N, M, w, b, loss, dE, dw, db, chat, cinv, einv, dchat, need_grad, eps, 1,
+                                       cos_own, urinv, gdiag);
   SPK_CUDA(cudaGetLastError());
   cudaLaunchAttribute pdl_attr[1];
   pdl_attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -582,26 +687,29 @@ int ge2e_fused(const float* E, int N, int M, int D, const float* w, const float*
   cfg.blockDim = dim3(256);
   cfg.stream = st;
   cfg.attrs = pdl_attr;
-  const bool pdl = g_ge2e_tile_v2 && g_ge2e_pdl;
+  const bool pdl = tile_v2 && g_ge2e_pdl;
   cfg.numAttrs = pdl ? 1 : 0;
   const float* chat_c = chat;
   const float* einv_c = einv;
-  if (g_ge2e_tile_v2) {
+  const float* cos_own_c = cos_own;
+  const float* gdiag_c = gdiag;
+  if (tile_v2) {
     cfg.gridDim = dim3(static_cast<unsigned>((NM + RT - 1) / RT));
     cfg.blockDim = dim3(TILE_THREADS);
     cfg.dynamicSmemBytes = smem2;
-    SPK_CUDA(cudaLaunchKernelEx(&cfg, ge2e_rows_tile_kernel, E, N, M, w, b, loss, dE, dw, db, chat_c, einv_c, dchat,
-                                need_grad));
+    SPK_CUDA(cudaLaunchKernelEx(&cfg, row_stage, E, N, M, w, b, loss, dE, dw, db, chat_c, einv_c, dchat, need_grad,
+                                cos_own_c, gdiag));
   } else {
-    ge2e_fused_kernel<<<row_tiles, 256, smem, st>>>(E, N, M, w, b, loss, dE, dw, db, chat, cinv, einv, dchat, need_grad, eps, 2);
+    ge2e_fused_kernel<false><<<row_tiles, 256, smem, st>>>(E, N, M, w, b, loss, dE, dw, db, chat, cinv, einv, dchat,
+                                                           need_grad, eps, 2, nullptr, nullptr, nullptr);
     SPK_CUDA(cudaGetLastError());
   }
   if (need_grad) {
     cfg.gridDim = dim3(N);
     cfg.blockDim = dim3(256);
     cfg.dynamicSmemBytes = smem;
-    SPK_CUDA(cudaLaunchKernelEx(&cfg, ge2e_fused_kernel, E, N, M, w, b, loss, dE, dw, db, chat, cinv, einv, dchat, need_grad,
-                                eps, 3));
+    SPK_CUDA(cudaLaunchKernelEx(&cfg, centroid_stage, E, N, M, w, b, loss, dE, dw, db, chat, cinv, einv, dchat, need_grad,
+                                eps, 3, cos_own, urinv, gdiag_c));
   }
   return 0;
 }

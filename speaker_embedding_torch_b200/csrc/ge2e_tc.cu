@@ -9,10 +9,12 @@
 //   GEMM    dEhat = G Chat     (Chat read MN-major), fp32 output
 //   GEMM    dChat = G^T Ehat   (both MN-major, split-K, fp32 atomics)
 //   finish  (warp / row)       normalisation Jacobians, centroid scatter: dE
+//   excl    (block / speaker)  exclusive centroids only: the diagonal's two gradient terms (ge2e_excl.cuh)
 //
 // The [NM, N] logits are materialised here (1 GB at N = 4096) -- what the small-N kernel avoids -- but the
 // reference's two [NM, N, D] operands (2 x 257 GB at N = 4096) still never exist.
 #include "ge2e.h"
+#include "ge2e_excl.cuh"
 #include "gemm.h"
 #include "rowops.h"
 
@@ -27,9 +29,10 @@ struct TcPlan {
   size_t ehat, chat, g;          // split tensors (byte offsets); plane strides below
   int64_t ehat_ps, chat_ps, g_ps;
   size_t chat32, einv, cinv, s, dehat, dchat, scal, total;
+  size_t cos_own = 0, urinv = 0, gdiag = 0;     // exclusive centroids only
 };
 
-static TcPlan tc_plan(int N, int M) {
+static TcPlan tc_plan(int N, int M, int mode) {
   TcPlan p;
   p.NM = static_cast<int64_t>(N) * M;
   p.Np = (N + 7) / 8 * 8;
@@ -55,20 +58,28 @@ static TcPlan tc_plan(int N, int M) {
   p.dehat = f32(p.NM * TD);
   p.dchat = f32(static_cast<int64_t>(N) * TD);
   p.scal = f32(4);
+  if (mode & GE2E_EXCLUSIVE) {
+    p.cos_own = f32(p.NM);
+    p.urinv = f32(p.NM);
+    p.gdiag = f32(p.NM);
+  }
   p.total = cur + 256;
   return p;
 }
 
-size_t ge2e_tc_workspace_bytes(int N, int M) { return tc_plan(N, M).total; }
+size_t ge2e_tc_workspace_bytes(int N, int M, int mode) { return tc_plan(N, M, mode).total; }
 
 // ---- prep: one block (256 threads = 8 warps) per speaker
+// EXCL: also each row's exclusive diagonal cosine `cos_own` and `urinv` = 1 / max(|u_i| / (M-1), eps), u_i = sum - e_i
+template <bool EXCL>
 __global__ void __launch_bounds__(256) ge2e_prep_kernel(const float* __restrict__ E, int N, int M,
                                                         elem_t* __restrict__ ehat, int64_t e_ps,
                                                         elem_t* __restrict__ chat, int64_t c_ps,
                                                         float* __restrict__ chat32, float* __restrict__ einv,
                                                         float* __restrict__ cinv, float* __restrict__ loss,
                                                         float* __restrict__ dw, float* __restrict__ db,
-                                                        float* __restrict__ dchat, float eps) {
+                                                        float* __restrict__ dchat, float eps,
+                                                        float* __restrict__ cos_own, float* __restrict__ urinv) {
   __shared__ float part[8][TD];
   __shared__ float red[8];
   const int k = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -98,6 +109,7 @@ __global__ void __launch_bounds__(256) ge2e_prep_kernel(const float* __restrict_
   float cv = 0.f;
 #pragma unroll
   for (int w = 0; w < 8; ++w) cv += part[w][tid];
+  const float csum = cv;
   cv *= 1.f / static_cast<float>(M);
   float q = warp_sum(cv * cv);
   if (lane == 0) red[warp] = q;
@@ -110,14 +122,45 @@ __global__ void __launch_bounds__(256) ge2e_prep_kernel(const float* __restrict_
   chat32[static_cast<int64_t>(k) * TD + tid] = ch;
   store1_split(chat, c_ps, 2, static_cast<int64_t>(k) * TD + tid, ch);
   if (tid == 0) cinv[k] = 1.f / nrm;
+  if constexpr (EXCL) {
+    part[0][tid] = csum;                       // every read of `part` is behind the barrier above
+    __syncthreads();
+    const float inv_m1 = 1.f / static_cast<float>(M - 1);
+    for (int m = warp; m < M; m += 8) {        // warp per row, as above (lane 0 wrote einv of these rows)
+      const int64_t row = static_cast<int64_t>(k) * M + m;
+      const float4 a0 = __ldg(reinterpret_cast<const float4*>(E + row * TD + lane * 8));
+      const float4 a1 = __ldg(reinterpret_cast<const float4*>(E + row * TD + lane * 8 + 4));
+      const float v[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
+      float qu = 0.f, qeu = 0.f;
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        const float u = part[0][lane * 8 + i] - v[i];
+        qu += u * u;
+        qeu += v[i] * u;
+      }
+      qu = warp_sum(qu);
+      qeu = warp_sum(qeu);
+      if (lane == 0) {
+        const float ur = 1.f / fmaxf(sqrtf(qu) * inv_m1, eps);
+        urinv[row] = ur;
+        cos_own[row] = qeu * einv[row] * (ur * inv_m1);
+      }
+    }
+  }
 }
 
 // ---- rows: one warp per embedding row; lane handles columns lane*8 + 256*c
+// MODE (GE2E_CONTRAST | GE2E_EXCLUSIVE bits): GE2E_EXCLUSIVE replaces each row's own-speaker cosine by `cos_own` (prep)
+// and writes that column's G to `gdiag` (dL/dcos_own) and a zero to the G planes, so that neither GEMM carries it;
+// GE2E_CONTRAST replaces the log-sum-exp by the own / strongest-impostor rule.
+template <int MODE>
 __global__ void __launch_bounds__(256) ge2e_rows_kernel(const float* __restrict__ S, int64_t NM, int N, int Np, int M,
                                                         const float* __restrict__ w_ptr, const float* __restrict__ b_ptr,
                                                         elem_t* __restrict__ G, int64_t g_ps,
                                                         float* __restrict__ loss, float* __restrict__ dw,
-                                                        float* __restrict__ db, int need_grad) {
+                                                        float* __restrict__ db, int need_grad,
+                                                        const float* __restrict__ cos_own, float* __restrict__ gdiag) {
+  constexpr bool EXCL = (MODE & GE2E_EXCLUSIVE) != 0, CONTRAST = (MODE & GE2E_CONTRAST) != 0;
   __shared__ float red[3][8];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
   const int64_t warp = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
@@ -128,13 +171,61 @@ __global__ void __launch_bounds__(256) ge2e_rows_kernel(const float* __restrict_
   for (int64_t r = warp; r < NM; r += nwarps) {
     const float* srow = S + r * Np;
     const int label = static_cast<int>(r / M);
+    const float own = EXCL ? __ldg(cos_own + r) : 0.f;
+    if constexpr (CONTRAST) {
+      // L = 1 - sigmoid(z_own) + sigmoid(z_k*), k* = the largest off-diagonal logit, ties to the lowest column
+      float bz = -INFINITY;
+      int bj = N;
+      for (int c0 = lane * 8; c0 < Np; c0 += 256) {
+        const float4 a0 = *reinterpret_cast<const float4*>(srow + c0);
+        const float4 a1 = *reinterpret_cast<const float4*>(srow + c0 + 4);
+        const float v[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          const float z = w * v[i] - b;
+          if (c0 + i < N && c0 + i != label && z > bz) { bz = z; bj = c0 + i; }
+        }
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        const float oz = __shfl_xor_sync(0xffffffffu, bz, o);
+        const int oj = __shfl_xor_sync(0xffffffffu, bj, o);
+        if (oz > bz || (oz == bz && oj < bj)) { bz = oz; bj = oj; }
+      }
+      const float s_own = EXCL ? own : srow[label];
+      // sigmoid(z) and sigmoid(-z) = 1 - sigmoid(z) each from its own exp: no cancellation when |z| is large
+      const float zo = w * s_own - b;
+      const float so = 1.f / (1.f + expf(-zo)), son = 1.f / (1.f + expf(zo));
+      const float sk = 1.f / (1.f + expf(-bz)), skn = 1.f / (1.f + expf(bz));
+      if (lane == 0) loss_acc += son + sk;
+      if (need_grad) {
+        const float go = -so * son, gk = sk * skn;      // dL/dz (x NM)
+        if (lane == 0) {
+          dw_acc += (go * s_own + gk * srow[bj]) * inv_nm;
+          db_acc -= (go + gk) * inv_nm;
+          if (EXCL) gdiag[r] = w * go * inv_nm;
+        }
+        for (int c0 = lane * 8; c0 < Np; c0 += 256) {
+          float g[8];
+#pragma unroll
+          for (int i = 0; i < 8; ++i)
+            g[i] = (c0 + i == label && !EXCL) ? w * go : (c0 + i == bj ? w * gk : 0.f);
+          store8_split(G, g_ps, 2, r * Np + c0, g);
+        }
+      }
+      continue;
+    }
     // one sweep for the maximum and the sum (per-lane running pair, rescaled when the maximum moves): the logits are
     // read twice per call (here and for G) instead of three times
     float mx = -INFINITY, sum = 0.f;
     for (int c0 = lane * 8; c0 < Np; c0 += 256) {
       const float4 a0 = *reinterpret_cast<const float4*>(srow + c0);
       const float4 a1 = *reinterpret_cast<const float4*>(srow + c0 + 4);
-      const float v[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
+      float v[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
+      if constexpr (EXCL) {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) v[i] = (c0 + i == label) ? own : v[i];
+      }
       float z[8], cm = -INFINITY;
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
@@ -156,14 +247,18 @@ __global__ void __launch_bounds__(256) ge2e_rows_kernel(const float* __restrict_
       mx = all;
     }
     const float lse = mx + logf(sum);
-    if (lane == 0) loss_acc += lse - (w * srow[label] - b);
+    if (lane == 0) loss_acc += lse - (w * (EXCL ? own : srow[label]) - b);
     if (need_grad) {
       // (keeping the row in shared memory for this sweep was measured: 8 warps x 16 KB leaves one block per SM at
       // N = 4096 and the kernel ran 1.8x slower than re-reading the row, most of which L2 still holds)
       for (int c0 = lane * 8; c0 < Np; c0 += 256) {
         const float4 a0 = *reinterpret_cast<const float4*>(srow + c0);
         const float4 a1 = *reinterpret_cast<const float4*>(srow + c0 + 4);
-        const float v[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
+        float v[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
+        if constexpr (EXCL) {
+#pragma unroll
+          for (int i = 0; i < 8; ++i) v[i] = (c0 + i == label) ? own : v[i];
+        }
         float g[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
@@ -175,6 +270,10 @@ __global__ void __launch_bounds__(256) ge2e_rows_kernel(const float* __restrict_
             dw_acc += pm * v[i];
             db_acc -= pm;
             g[i] = w * pm1;      // G * NM: O(w), well inside the fp16 planes' range; 1 / NM is the GEMMs' alpha
+            if (EXCL && c0 + i == label) {
+              gdiag[r] = w * pm;
+              g[i] = 0.f;
+            }
           }
         }
         store8_split(G, g_ps, 2, r * Np + c0, g);
@@ -233,9 +332,17 @@ __global__ void __launch_bounds__(256) ge2e_finish_kernel(const float* __restric
   }
 }
 
+// ---- exclusive centroids: the diagonal's gradient terms, one block per speaker (after finish)
+__global__ void __launch_bounds__(256) ge2e_excl_kernel(const float* __restrict__ E, int M, const float* __restrict__ einv,
+                                                        const float* __restrict__ cos_own, const float* __restrict__ urinv,
+                                                        const float* __restrict__ gdiag, float* __restrict__ dE) {
+  ge2e_excl_diag_grad(E, blockIdx.x, M, einv, cos_own, urinv, gdiag, dE, 0.f);
+}
+
 int ge2e_tc(const float* E, int N, int M, const float* w, const float* b, float* loss, float* dE, float* dw, float* db,
-            void* ws_v, size_t ws_bytes, cudaStream_t st) {
-  const TcPlan pl = tc_plan(N, M);
+            void* ws_v, size_t ws_bytes, cudaStream_t st, int mode) {
+  const TcPlan pl = tc_plan(N, M, mode);
+  const bool excl = (mode & GE2E_EXCLUSIVE) != 0;
   if (ws_bytes < pl.total) {
     set_error("ge2e: workspace too small (%zu < %zu)", ws_bytes, pl.total);
     return SPK_ENOMEM;
@@ -247,9 +354,11 @@ int ge2e_tc(const float* E, int N, int M, const float* w, const float* b, float*
   const int64_t NM = pl.NM;
   {
     ProfScope prof("ge2e_tc.prep", 0, 4.0 * NM * TD + 6.0 * NM * TD, st);
-    ge2e_prep_kernel<<<N, 256, 0, st>>>(E, N, M, bf(pl.ehat), pl.ehat_ps, bf(pl.chat), pl.chat_ps, fp(pl.chat32),
-                                        fp(pl.einv), fp(pl.cinv), loss, need_grad ? dw : nullptr, need_grad ? db : nullptr,
-                                        need_grad ? fp(pl.dchat) : nullptr, 1e-8f);
+    auto* prep = excl ? ge2e_prep_kernel<true> : ge2e_prep_kernel<false>;
+    prep<<<N, 256, 0, st>>>(E, N, M, bf(pl.ehat), pl.ehat_ps, bf(pl.chat), pl.chat_ps, fp(pl.chat32), fp(pl.einv),
+                            fp(pl.cinv), loss, need_grad ? dw : nullptr, need_grad ? db : nullptr,
+                            need_grad ? fp(pl.dchat) : nullptr, 1e-8f, excl ? fp(pl.cos_own) : nullptr,
+                            excl ? fp(pl.urinv) : nullptr);
     SPK_CUDA(cudaGetLastError());
   }
   {  // S = Ehat Chat^T
@@ -265,8 +374,12 @@ int ge2e_tc(const float* E, int N, int M, const float* w, const float* b, float*
   {
     ProfScope prof("ge2e_tc.rows", 0, (need_grad ? 2.0 : 1.0) * NM * pl.Np * 4.0 + (need_grad ? 4.0 * NM * pl.Np : 0.0), st);
     const int blocks = static_cast<int>(std::min<int64_t>((NM + 7) / 8, static_cast<int64_t>(device_sm_count()) * 8));
-    ge2e_rows_kernel<<<blocks, 256, 0, st>>>(fp(pl.s), NM, N, static_cast<int>(pl.Np), M, w, b, bf(pl.g), pl.g_ps, loss, dw, db,
-                                             need_grad);
+    auto* rows = ge2e_rows_kernel<0>;
+    if (mode == GE2E_CONTRAST) rows = ge2e_rows_kernel<GE2E_CONTRAST>;
+    if (mode == GE2E_EXCLUSIVE) rows = ge2e_rows_kernel<GE2E_EXCLUSIVE>;
+    if (mode == (GE2E_EXCLUSIVE | GE2E_CONTRAST)) rows = ge2e_rows_kernel<GE2E_EXCLUSIVE | GE2E_CONTRAST>;
+    rows<<<blocks, 256, 0, st>>>(fp(pl.s), NM, N, static_cast<int>(pl.Np), M, w, b, bf(pl.g), pl.g_ps, loss, dw, db,
+                                 need_grad, excl ? fp(pl.cos_own) : nullptr, excl ? fp(pl.gdiag) : nullptr);
     SPK_CUDA(cudaGetLastError());
   }
   if (need_grad) {
@@ -303,6 +416,11 @@ int ge2e_tc(const float* E, int N, int M, const float* w, const float* b, float*
       const int blocks = static_cast<int>(std::min<int64_t>((NM + 7) / 8, 148 * 8));
       ge2e_finish_kernel<<<blocks, 256, 0, st>>>(E, fp(pl.einv), fp(pl.chat32), fp(pl.cinv), fp(pl.dehat), fp(pl.dchat),
                                                  dE, NM, M);
+      SPK_CUDA(cudaGetLastError());
+    }
+    if (excl) {
+      ProfScope prof("ge2e_tc.excl", 0, 12.0 * NM * TD, st);
+      ge2e_excl_kernel<<<N, 256, 0, st>>>(E, M, fp(pl.einv), fp(pl.cos_own), fp(pl.urinv), fp(pl.gdiag), dE);
       SPK_CUDA(cudaGetLastError());
     }
   }
