@@ -226,7 +226,6 @@ int spk_set_option(const char* name, int value) {
   if (strcmp(name, "fused_training_attention") == 0) { encoder_set_fused_train_attn(value != 0); return 0; }
   if (strcmp(name, "grad_scale_log2") == 0) { encoder_set_grad_scale_log2(value); return 0; }
   if (strcmp(name, "ge2e_dependent_launch") == 0) { ge2e_set_pdl(value); return 0; }
-  if (strcmp(name, "ge2e_row_tile_v2") == 0) { ge2e_set_tile_v2(value); return 0; }
   if (strcmp(name, "gemm_dependent_launch") == 0) { gemm_set_dependent_launch(value); return 0; }
   if (strcmp(name, "gemm_cta_pairs") == 0) { gemm_set_cta_pairs(value != 0); return 0; }
   set_error("spk_set_option: unknown option '%s'", name);

@@ -1,40 +1,30 @@
-// Fused GE2E loss: one kernel, three stream-ordered launches (stages), computes centroids, row/centroid normalisation, the
-// N*M x N cosine-similarity matrix, w*S - b, log-softmax cross-entropy, and its gradient
+// Fused GE2E loss for N < 256 speakers: three stream-ordered launches (stages) compute centroids, row/centroid
+// normalisation, the N*M x N cosine-similarity matrix, w*S - b, log-softmax cross-entropy, and its gradient
 // (dE, dw, db) without ever materialising the [N*M, N] logits or the reference's two
 // [N*M, N, D] expanded operands (/root/reference/Modules.py:121-156; math: SURVEY.md App. B).
 //
-//   phase 1  (block per speaker)   c_k = mean_m E ; ehat scale 1/max(|E_i|,eps) ; chat_k ; zero dchat
-//   phase 2  (block per 16 rows)   pass A: S tile -> online (max, sum) -> lse, loss
-//                                  pass B: recompute S tile -> G = (w/NM)(softmax - onehot)
-//                                          dehat += G * Chat   (registers)
-//                                          dchat += G^T * Ehat (coalesced fp32 RED)
-//                                  dE_i  = (dehat - (dehat.ehat) ehat) / |E_i|
-//   phase 3  (block per speaker)   dE_i += (1/M) (dchat_j - (dchat_j.chat_j) chat_j) / |c_j|
+//   stage 1  ge2e_centroid_kernel       (block per speaker)  c_k = mean_m E ; ehat scale 1/max(|E_i|,eps) ; chat_k ;
+//                                                            zero dchat (also the tensor-core path's first kernel)
+//   stage 2  ge2e_rows_tile_kernel      (block per 8 rows)   S rows -> log-sum-exp, loss ; G = (w/NM)(softmax - onehot)
+//                                                            dehat += G * Chat   (registers)
+//                                                            dchat += G^T * Ehat (fp32 RED)
+//                                                            dE_i  = (dehat - (dehat.ehat) ehat) / |E_i|
+//   stage 3  ge2e_centroid_grad_kernel  (block per speaker)  dE_i += (1/M) (dchat_j - (dchat_j.chat_j) chat_j) / |c_j|
 //
 // fp32 SIMT math throughout (bit-for-bit deterministic except the fp32 atomics of dchat/loss).
 // D is fixed at 256 (= Embedding_Size of the reference hyper-parameters): thread <-> column.
 #include "common.cuh"
 #include "ge2e.h"
-#include "ge2e_excl.cuh"
+#include "ge2e_common.cuh"
 #include "ptx.cuh"
 
 namespace spk {
 
 constexpr int GD = 256;        // embedding size
-constexpr int TR = 16;         // rows per block tile
 constexpr int TC = 64;         // centroids per tile
 constexpr int CPAD = GD + 4;   // padded centroid row (floats), keeps 16-B alignment, breaks bank aliasing
 
-struct Ge2eSmem {
-  float e[TR][GD];         // normalised rows
-  float c[TC][CPAD];       // normalised centroids tile
-  float g[TR][TC];         // G tile, row-major (for dchat)
-  float gt[TC][TR];        // G tile, transposed (for dehat)
-  float red[8][TR];
-  float rowv[TR];
-};
-
-// Programmatic dependent launch (pdl_trigger / pdl_wait, ptx.cuh): the three stages are launched back to back with the
+// Programmatic dependent launch (pdl_trigger / pdl_wait, ptx.cuh): the stages are launched back to back with the
 // stream-serialisation attribute; a stage touches its predecessor's results only after pdl_wait().
 __device__ __forceinline__ float block_sum_256(float v, float* red8) {
   v = warp_sum(v);
@@ -47,290 +37,128 @@ __device__ __forceinline__ float block_sum_256(float v, float* red8) {
   return s;
 }
 
-// EXCL: exclusive own-speaker centroids (ge2e_excl.cuh): phase 1 also writes each row's diagonal cosine `cos_own` and
-// `urinv` = 1 / max(|u_i| / (M-1), eps); phase 3 adds the diagonal's gradient `gdiag` (written by the row stage).
-template <bool EXCL>
-__global__ void __launch_bounds__(256, 2)
-ge2e_fused_kernel(const float* __restrict__ E, int N, int M, const float* __restrict__ w_ptr,
-                  const float* __restrict__ b_ptr, float* __restrict__ loss, float* __restrict__ dE,
-                  float* __restrict__ dw, float* __restrict__ db, float* __restrict__ chat,
-                  float* __restrict__ cinv, float* __restrict__ einv, float* __restrict__ dchat, int need_grad,
-                  float eps, int phase, float* __restrict__ cos_own, float* __restrict__ urinv,
-                  const float* __restrict__ gdiag) {
-  // `phase` selects one of the three stages; the launcher enqueues them back to back on one stream (stream order is the
-  // grid-wide barrier: a cooperative launch with two grid.sync() cost 32 us at the training size, mostly in the syncs)
-  extern __shared__ __align__(16) uint8_t smem_raw[];
-  Ge2eSmem& sm = *reinterpret_cast<Ge2eSmem*>(smem_raw);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int64_t NM = static_cast<int64_t>(N) * M;
-  const float w = __ldg(w_ptr), b = __ldg(b_ptr);
-  float* red8 = &sm.red[0][0];
-
-  // ------------------------------------------------------------------ phase 1
-  if (phase == 1) {
-  pdl_trigger();
-  if (blockIdx.x == 0 && tid == 0) {
-    loss[0] = 0.f;
-    if (need_grad) { dw[0] = 0.f; db[0] = 0.f; }
+// Stage 1 of both paths (ge2e_centroids), one block per speaker: warp per row for the row norms and the column partial
+// sums (lane owns columns lane*8 .. +7), thread <-> column for the centroid.  EXCL: exclusive own-speaker centroids,
+// each row's diagonal cosine `cos_own` and `urinv` = 1 / max(|u_i| / (M-1), eps), u_i = sum - e_i.  SPLIT: Ehat and
+// Chat also as two fp16 planes for the tensor-core GEMMs.
+template <bool EXCL, bool SPLIT>
+__global__ void __launch_bounds__(256) ge2e_centroid_kernel(const Ge2eCentroids c) {
+  __shared__ float part[8][GD];
+  __shared__ float colsum[GD];
+  __shared__ float red8[8];
+  const int k = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const float eps = 1e-8f;
+  pdl_trigger();      // the next launch reads nothing of this one before its pdl_wait()
+  if (k == 0 && tid == 0) {
+    c.loss[0] = 0.f;
+    if (c.dw != nullptr) { c.dw[0] = 0.f; c.db[0] = 0.f; }
   }
-  for (int k = blockIdx.x; k < N; k += gridDim.x) {
-    // warp per row: row norm + partial centroid (lane owns columns lane*8 .. +7)
-    float cpart[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-    for (int m = warp; m < M; m += 8) {
-      const float* row = E + (static_cast<int64_t>(k) * M + m) * GD + lane * 8;
-      const float4 a0 = __ldg(reinterpret_cast<const float4*>(row));
-      const float4 a1 = __ldg(reinterpret_cast<const float4*>(row + 4));
+  if (c.dchat != nullptr) c.dchat[static_cast<int64_t>(k) * GD + tid] = 0.f;
+  float cp[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  for (int m = warp; m < c.M; m += 8) {
+    const int64_t row = static_cast<int64_t>(k) * c.M + m;
+    const float4 a0 = __ldg(reinterpret_cast<const float4*>(c.E + row * GD + lane * 8));
+    const float4 a1 = __ldg(reinterpret_cast<const float4*>(c.E + row * GD + lane * 8 + 4));
+    float v[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
+    float q = 0.f;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) { q += v[i] * v[i]; cp[i] += v[i]; }
+    const float inv = 1.f / fmaxf(sqrtf(warp_sum(q)), eps);
+    if (lane == 0) c.einv[row] = inv;
+    if constexpr (SPLIT) {
+#pragma unroll
+      for (int i = 0; i < 8; ++i) v[i] *= inv;
+      store8_split(c.ehat_planes, c.ehat_ps, 2, row * GD + lane * 8, v);   // two fp16 planes carry an fp32 mantissa
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < 8; ++i) part[warp][lane * 8 + i] = cp[i];
+  __syncthreads();
+  float cv = 0.f;
+#pragma unroll
+  for (int w = 0; w < 8; ++w) cv += part[w][tid];
+  if constexpr (EXCL) colsum[tid] = cv;        // the speaker's column sum (visible after block_sum_256's barriers)
+  cv *= 1.f / static_cast<float>(c.M);
+  const float nrm = fmaxf(sqrtf(block_sum_256(cv * cv, red8)), eps);
+  const float ch = cv / nrm;
+  c.chat[static_cast<int64_t>(k) * GD + tid] = ch;
+  if constexpr (SPLIT) store1_split(c.chat_planes, c.chat_ps, 2, static_cast<int64_t>(k) * GD + tid, ch);
+  if (tid == 0) c.cinv[k] = 1.f / nrm;
+  if constexpr (EXCL) {
+    // warp per row, as above (lane 0 wrote einv of these rows): u_i = sum - e_i, formed directly
+    const float inv_m1 = 1.f / static_cast<float>(c.M - 1);
+    for (int m = warp; m < c.M; m += 8) {
+      const int64_t r = static_cast<int64_t>(k) * c.M + m;
+      const float4 a0 = __ldg(reinterpret_cast<const float4*>(c.E + r * GD + lane * 8));
+      const float4 a1 = __ldg(reinterpret_cast<const float4*>(c.E + r * GD + lane * 8 + 4));
+      const float4 s0 = *reinterpret_cast<const float4*>(&colsum[lane * 8]);
+      const float4 s1 = *reinterpret_cast<const float4*>(&colsum[lane * 8 + 4]);
       const float v[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-      float q = 0.f;
+      const float sv[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w};
+      float qu = 0.f, qeu = 0.f;
 #pragma unroll
-      for (int i = 0; i < 8; ++i) { q += v[i] * v[i]; cpart[i] += v[i]; }
-      q = warp_sum(q);
-      if (lane == 0) einv[static_cast<int64_t>(k) * M + m] = 1.f / fmaxf(sqrtf(q), eps);
-    }
-    __syncthreads();
-#pragma unroll
-    for (int i = 0; i < 8; ++i) sm.e[warp][lane * 8 + i] = cpart[i];
-    __syncthreads();
-    float cv = 0.f;
-#pragma unroll
-    for (int wv = 0; wv < 8; ++wv) cv += sm.e[wv][tid];
-    if constexpr (EXCL) sm.e[8][tid] = cv;       // the speaker's column sum (visible after block_sum_256's barriers)
-    cv *= 1.f / static_cast<float>(M);
-    const float nrm = fmaxf(sqrtf(block_sum_256(cv * cv, red8)), eps);
-    chat[static_cast<int64_t>(k) * GD + tid] = cv / nrm;
-    if (need_grad) dchat[static_cast<int64_t>(k) * GD + tid] = 0.f;
-    if (tid == 0) cinv[k] = 1.f / nrm;
-    if constexpr (EXCL) {
-      // warp per row, as above (lane 0 wrote einv of these rows): u_i = sum - e_i, formed directly
-      const float inv_m1 = 1.f / static_cast<float>(M - 1);
-      for (int m = warp; m < M; m += 8) {
-        const int64_t r = static_cast<int64_t>(k) * M + m;
-        const float4 a0 = __ldg(reinterpret_cast<const float4*>(E + r * GD + lane * 8));
-        const float4 a1 = __ldg(reinterpret_cast<const float4*>(E + r * GD + lane * 8 + 4));
-        const float4 s0 = *reinterpret_cast<const float4*>(&sm.e[8][lane * 8]);
-        const float4 s1 = *reinterpret_cast<const float4*>(&sm.e[8][lane * 8 + 4]);
-        const float v[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-        const float sv[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w};
-        float qu = 0.f, qeu = 0.f;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const float u = sv[i] - v[i];
-          qu += u * u;
-          qeu += v[i] * u;
-        }
-        qu = warp_sum(qu);
-        qeu = warp_sum(qeu);
-        if (lane == 0) {
-          const float ur = 1.f / fmaxf(sqrtf(qu) * inv_m1, eps);
-          urinv[r] = ur;
-          cos_own[r] = qeu * einv[r] * (ur * inv_m1);
-        }
+      for (int i = 0; i < 8; ++i) {
+        const float u = sv[i] - v[i];
+        qu += u * u;
+        qeu += v[i] * u;
       }
-    }
-    __syncthreads();
-  }
-  return;
-  }
-
-  // ------------------------------------------------------------------ phase 2 (mode 0 only: the first row stage)
-  if (!EXCL && phase == 2) {
-  const int r_loc = tid >> 4;      // 0..15 : row within tile (S-tile compute mapping)
-  const int cgp = tid & 15;        // columns cgp, cgp+16, cgp+32, cgp+48 of the centroid tile
-  const int64_t row_tiles = (NM + TR - 1) / TR;
-  const int col_tiles = (N + TC - 1) / TC;
-  const float inv_nm = 1.f / static_cast<float>(NM);
-
-  for (int64_t rt = blockIdx.x; rt < row_tiles; rt += gridDim.x) {
-    const int64_t row0 = rt * TR;
-    __syncthreads();
-    // load + normalise 16 rows: warp handles rows warp, warp+8
-    for (int r = warp; r < TR; r += 8) {
-      const int64_t gi = row0 + r;
-      float v[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-      if (gi < NM) {
-        const float sc = einv[gi];
-        const float4 a0 = __ldg(reinterpret_cast<const float4*>(E + gi * GD + lane * 8));
-        const float4 a1 = __ldg(reinterpret_cast<const float4*>(E + gi * GD + lane * 8 + 4));
-        v[0] = a0.x * sc; v[1] = a0.y * sc; v[2] = a0.z * sc; v[3] = a0.w * sc;
-        v[4] = a1.x * sc; v[5] = a1.y * sc; v[6] = a1.z * sc; v[7] = a1.w * sc;
+      qu = warp_sum(qu);
+      qeu = warp_sum(qeu);
+      if (lane == 0) {
+        const float ur = 1.f / fmaxf(sqrtf(qu) * inv_m1, eps);
+        c.urinv[r] = ur;
+        c.cos_own[r] = qeu * c.einv[r] * (ur * inv_m1);
       }
-#pragma unroll
-      for (int i = 0; i < 8; ++i) sm.e[r][lane * 8 + i] = v[i];
-    }
-    const int64_t my_row = row0 + r_loc;
-    const int my_label = (my_row < NM) ? static_cast<int>(my_row / M) : -1;
-    float run_max = -INFINITY, run_sum = 0.f, z_true = 0.f;
-    float lse = 0.f;
-    float dacc[TR];
-#pragma unroll
-    for (int r = 0; r < TR; ++r) dacc[r] = 0.f;
-    float dw_part = 0.f, db_part = 0.f;
-
-    float s[4] = {0.f, 0.f, 0.f, 0.f};
-    for (int pass = 0; pass < (need_grad ? 2 : 1); ++pass) {
-      for (int ct = 0; ct < col_tiles; ++ct) {
-        const int c0 = ct * TC;
-        // N <= 64 (the training configuration): one centroid tile -- the second sweep reuses the tile in shared
-        // memory and the S values still held in registers instead of recomputing them.
-        const bool reuse = (pass == 1 && col_tiles == 1);
-        if (!reuse) {
-          __syncthreads();
-          // centroid tile -> smem (coalesced float4)
-          for (int i = tid; i < TC * (GD / 4); i += 256) {
-            const int cr = i / (GD / 4), c4 = i % (GD / 4);
-            float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (c0 + cr < N) v = __ldg(reinterpret_cast<const float4*>(chat + static_cast<int64_t>(c0 + cr) * GD) + c4);
-            *reinterpret_cast<float4*>(&sm.c[cr][c4 * 4]) = v;
-          }
-          __syncthreads();
-          // S tile: 4 dot products of length 256 per thread
-          s[0] = s[1] = s[2] = s[3] = 0.f;
-#pragma unroll 4
-          for (int d = 0; d < GD; d += 4) {
-            const float4 ev = *reinterpret_cast<const float4*>(&sm.e[r_loc][d]);
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const float4 cvv = *reinterpret_cast<const float4*>(&sm.c[cgp + 16 * j][d]);
-              s[j] = fmaf(ev.x, cvv.x, s[j]);
-              s[j] = fmaf(ev.y, cvv.y, s[j]);
-              s[j] = fmaf(ev.z, cvv.z, s[j]);
-              s[j] = fmaf(ev.w, cvv.w, s[j]);
-            }
-          }
-        }
-        if (pass == 0) {
-          float tmax = -INFINITY;
-          float z[4];
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const int col = c0 + cgp + 16 * j;
-            z[j] = (col < N) ? w * s[j] - b : -INFINITY;
-            if (col == my_label) z_true = z[j];
-            tmax = fmaxf(tmax, z[j]);
-          }
-#pragma unroll
-          for (int o = 8; o > 0; o >>= 1) tmax = fmaxf(tmax, __shfl_xor_sync(0xffffffffu, tmax, o));
-          const float new_max = fmaxf(run_max, tmax);
-          float part = 0.f;
-#pragma unroll
-          for (int j = 0; j < 4; ++j) part += (z[j] == -INFINITY) ? 0.f : expf(z[j] - new_max);
-#pragma unroll
-          for (int o = 8; o > 0; o >>= 1) part += __shfl_xor_sync(0xffffffffu, part, o);
-          run_sum = run_sum * ((run_max == -INFINITY) ? 0.f : expf(run_max - new_max)) + part;
-          run_max = new_max;
-        } else {
-          // G tile
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const int cl = cgp + 16 * j, col = c0 + cl;
-            float gval = 0.f;
-            if (col < N && my_row < NM) {
-              const float p = expf(w * s[j] - b - lse);
-              const float pm = (p - (col == my_label ? 1.f : 0.f)) * inv_nm;
-              dw_part += pm * s[j];
-              db_part -= pm;
-              gval = w * pm;
-            }
-            sm.g[r_loc][cl] = gval;
-            sm.gt[cl][r_loc] = gval;
-          }
-          __syncthreads();
-          // dehat[r][tid] += sum_c G[r][c] * chat[c][tid]
-#pragma unroll 4
-          for (int c = 0; c < TC; ++c) {
-            const float cvl = sm.c[c][tid];
-#pragma unroll
-            for (int r4 = 0; r4 < TR; r4 += 4) {
-              const float4 gv = *reinterpret_cast<const float4*>(&sm.gt[c][r4]);
-              dacc[r4 + 0] = fmaf(gv.x, cvl, dacc[r4 + 0]);
-              dacc[r4 + 1] = fmaf(gv.y, cvl, dacc[r4 + 1]);
-              dacc[r4 + 2] = fmaf(gv.z, cvl, dacc[r4 + 2]);
-              dacc[r4 + 3] = fmaf(gv.w, cvl, dacc[r4 + 3]);
-            }
-          }
-          // dchat[c][tid] += sum_r G[r][c] * ehat[r][tid]   (16 centroids at a time to bound registers)
-#pragma unroll 1
-          for (int cb = 0; cb < TC; cb += 16) {
-            if (c0 + cb >= N) break;
-            float a2[16];
-#pragma unroll
-            for (int i = 0; i < 16; ++i) a2[i] = 0.f;
-#pragma unroll
-            for (int r = 0; r < TR; ++r) {
-              const float evl = sm.e[r][tid];
-#pragma unroll
-              for (int c4 = 0; c4 < 16; c4 += 4) {
-                const float4 gv = *reinterpret_cast<const float4*>(&sm.g[r][cb + c4]);
-                a2[c4 + 0] = fmaf(gv.x, evl, a2[c4 + 0]);
-                a2[c4 + 1] = fmaf(gv.y, evl, a2[c4 + 1]);
-                a2[c4 + 2] = fmaf(gv.z, evl, a2[c4 + 2]);
-                a2[c4 + 3] = fmaf(gv.w, evl, a2[c4 + 3]);
-              }
-            }
-#pragma unroll
-            for (int i = 0; i < 16; ++i)
-              if (c0 + cb + i < N) atomicAdd(dchat + static_cast<int64_t>(c0 + cb + i) * GD + tid, a2[i]);
-          }
-        }
-      }
-      if (pass == 0) {
-        lse = run_max + logf(run_sum);
-        // loss contribution: one thread per row (cgp == 0 holds the reduced values; z_true lives in one lane)
-#pragma unroll
-        for (int o = 8; o > 0; o >>= 1) z_true += __shfl_xor_sync(0xffffffffu, z_true, o);
-        float lrow = (cgp == 0 && my_row < NM) ? (lse - z_true) : 0.f;
-        const float lsum = block_sum_256(lrow, red8);
-        if (tid == 0) atomicAdd(loss, lsum * inv_nm);
-      }
-    }
-
-    if (need_grad) {
-      const float dws = block_sum_256(dw_part, red8);
-      const float dbs = block_sum_256(db_part, red8);
-      if (tid == 0) { atomicAdd(dw, dws); atomicAdd(db, dbs); }
-      // project out the radial component and write the row part of dE
-      __syncthreads();
-#pragma unroll
-      for (int r = 0; r < TR; ++r) {
-        float dot = warp_sum(dacc[r] * sm.e[r][tid]);
-        if (lane == 0) sm.red[warp][r] = dot;
-      }
-      __syncthreads();
-      if (tid < TR) {
-        float s = 0.f;
-#pragma unroll
-        for (int wv = 0; wv < 8; ++wv) s += sm.red[wv][tid];
-        sm.rowv[tid] = s;
-      }
-      __syncthreads();
-#pragma unroll
-      for (int r = 0; r < TR; ++r) {
-        const int64_t gi = row0 + r;
-        if (gi < NM) dE[gi * GD + tid] = (dacc[r] - sm.rowv[r] * sm.e[r][tid]) * einv[gi];
-      }
-    }
-  }
-  return;
-  }
-
-  // ------------------------------------------------------------------ phase 3
-  pdl_wait();
-  for (int k = blockIdx.x; k < N; k += gridDim.x) {
-    const float dc = dchat[static_cast<int64_t>(k) * GD + tid];
-    const float ch = chat[static_cast<int64_t>(k) * GD + tid];
-    const float dot = block_sum_256(dc * ch, red8);
-    const float u = (dc - dot * ch) * cinv[k] * (1.f / static_cast<float>(M));
-    if constexpr (EXCL) {
-      ge2e_excl_diag_grad(E, k, M, einv, cos_own, urinv, gdiag, dE, u);
-    } else {
-      for (int m = 0; m < M; ++m) dE[(static_cast<int64_t>(k) * M + m) * GD + tid] += u;
     }
   }
 }
 
-// ------------------------------------------------------------------------------------------------ row-tile stage, v2
-// Same mathematics as phase 2 above, re-tiled for the shared-memory pipe (ncu of the first version: L1/shared 64 % busy on
-// the 60 SMs it used, 20 us of the 32 us call at N = 64):
+// The per-speaker stages of the small-N path (1 and 3) are launched with 80 KB of dynamic shared memory that they do not
+// use, so that at most two of their blocks share an SM.  Measured on a B200 at 1000 W (CUDA-graph replay): without it on
+// stage 1 the call at N = 64 took 21.3 us instead of 17.5 us in every mode; without it on stage 3 the exclusive modes
+// took 1.4 us more at N = 64; a larger reservation (90 KB) cost the exclusive modes 0.6 - 0.9 us at N = 64 and 128.
+// The tensor-core path launches stage 1 without one.
+constexpr int CENTROID_SPREAD_SMEM = 80 * 1024;
+
+int ge2e_centroids(const Ge2eCentroids& c, cudaStream_t st) {
+  static PerDeviceOnce once;
+  SPK_TRY(once.run([]() -> int {
+    for (auto* k : {ge2e_centroid_kernel<false, false>, ge2e_centroid_kernel<true, false>})
+      SPK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, CENTROID_SPREAD_SMEM));
+    return 0;
+  }));
+  auto* kernel = c.cos_own ? (c.ehat_planes ? ge2e_centroid_kernel<true, true> : ge2e_centroid_kernel<true, false>)
+                           : (c.ehat_planes ? ge2e_centroid_kernel<false, true> : ge2e_centroid_kernel<false, false>);
+  kernel<<<c.N, 256, c.ehat_planes ? 0 : CENTROID_SPREAD_SMEM, st>>>(c);
+  SPK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+// Stage 3, one block per speaker: the centroid part of dE; EXCL adds the diagonal's terms from `gdiag` (written by the
+// row stage, ge2e_common.cuh)
+template <bool EXCL>
+__global__ void __launch_bounds__(256)
+ge2e_centroid_grad_kernel(const float* __restrict__ E, int M, const float* __restrict__ chat,
+                          const float* __restrict__ cinv, const float* __restrict__ dchat,
+                          const float* __restrict__ einv, const float* __restrict__ cos_own,
+                          const float* __restrict__ urinv, const float* __restrict__ gdiag, float* __restrict__ dE) {
+  __shared__ float red8[8];
+  const int k = blockIdx.x, tid = threadIdx.x;
+  pdl_wait();
+  const float dc = dchat[static_cast<int64_t>(k) * GD + tid];
+  const float ch = chat[static_cast<int64_t>(k) * GD + tid];
+  const float dot = block_sum_256(dc * ch, red8);
+  const float u = (dc - dot * ch) * cinv[k] * (1.f / static_cast<float>(M));
+  if constexpr (EXCL) {
+    ge2e_excl_diag_grad(E, k, M, einv, cos_own, urinv, gdiag, dE, u);
+  } else {
+    for (int m = 0; m < M; ++m) dE[(static_cast<int64_t>(k) * M + m) * GD + tid] += u;
+  }
+}
+
+// ------------------------------------------------------------------------------------------------ stage 2: row tiles
+// Tiled for the shared-memory pipe (ncu of a first 16-row version, since retired: L1/shared 64 % busy on the 60 SMs it
+// used, 20 us of the 32 us call at N = 64):
 //   * 8 rows per block instead of 16 -> 120 blocks at the training size (148 SMs), two blocks per SM;
 //   * the centroid tile arrives by bulk copy (cp.async.bulk -> mbarrier), one 1 KB row per copy, while the block
 //     normalises its rows;
@@ -485,12 +313,11 @@ ge2e_rows_tile_kernel(const float* __restrict__ E, int N, int M, const float* __
       for (int o = 16; o > 0; o >>= 1) {
         const float oz = __shfl_xor_sync(0xffffffffu, bz, o);
         const int oj = __shfl_xor_sync(0xffffffffu, bj, o);
-        if (oz > bz || (oz == bz && oj < bj)) { bz = oz; bj = oj; }
+        if (ge2e_argmax_takes(bz, bj, oz, oj)) { bz = oz; bj = oj; }
       }
-      // sigmoid(z) and sigmoid(-z) = 1 - sigmoid(z) each from its own exp: no cancellation when |z| is large
-      const float zo = live ? w * sm.s[warp][label] - b : 0.f;
-      const float so = 1.f / (1.f + expf(-zo)), son = 1.f / (1.f + expf(zo));
-      const float sk = 1.f / (1.f + expf(-bz)), skn = 1.f / (1.f + expf(bz));
+      float so, son, sk, skn;
+      ge2e_sigmoid_pair(live ? w * sm.s[warp][label] - b : 0.f, so, son);
+      ge2e_sigmoid_pair(bz, sk, skn);
       if (live && lane == 0) lrow = son + sk;
       if (need_grad) {
         const float go = -so * son * inv_nm, gk = sk * skn * inv_nm;
@@ -614,8 +441,6 @@ ge2e_rows_tile_kernel(const float* __restrict__ E, int N, int M, const float* __
   }
 }
 
-static int g_ge2e_tile_v2 = 1;     // spk_set_option("ge2e_row_tile_v2", 0/1): 0 = the first 16-row stage (A/B, tests)
-void ge2e_set_tile_v2(int on) { g_ge2e_tile_v2 = on != 0; }
 static int g_ge2e_pdl = 1;         // spk_set_option("ge2e_dependent_launch", 0/1): programmatic dependent launch of stages 2, 3
 void ge2e_set_pdl(int on) { g_ge2e_pdl = on != 0; }
 
@@ -626,6 +451,10 @@ static size_t ge2e_simt_workspace_bytes(int N, int M, int mode) {
 }
 size_t ge2e_workspace_bytes(int N, int M, int mode) {
   return N >= GE2E_TC_MIN_SPEAKERS ? ge2e_tc_workspace_bytes(N, M, mode) : ge2e_simt_workspace_bytes(N, M, mode);
+}
+
+static auto rows_tile_kernel_for(int mode) {
+  return ge2e_for_mode(mode, [](auto m) { return ge2e_rows_tile_kernel<decltype(m)::value>; });
 }
 
 int ge2e_fused(const float* E, int N, int M, int D, const float* w, const float* b, float* loss, float* dE, float* dw,
@@ -650,66 +479,44 @@ int ge2e_fused(const float* E, int N, int M, int D, const float* w, const float*
   float* gdiag = excl ? urinv + static_cast<size_t>(N) * M : nullptr;
 
   static PerDeviceOnce once;
-  const int smem = static_cast<int>(sizeof(Ge2eSmem));
-  const int smem2 = static_cast<int>(sizeof(Ge2eTileSmem));
+  const int smem = static_cast<int>(sizeof(Ge2eTileSmem));
   SPK_TRY(once.run([&]() -> int {
-    SPK_CUDA(cudaFuncSetAttribute(ge2e_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    SPK_CUDA(cudaFuncSetAttribute(ge2e_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    SPK_CUDA(cudaFuncSetAttribute(ge2e_rows_tile_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
-    SPK_CUDA(cudaFuncSetAttribute(ge2e_rows_tile_kernel<GE2E_CONTRAST>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  smem2));
-    SPK_CUDA(cudaFuncSetAttribute(ge2e_rows_tile_kernel<GE2E_EXCLUSIVE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  smem2));
-    SPK_CUDA(cudaFuncSetAttribute(ge2e_rows_tile_kernel<GE2E_EXCLUSIVE | GE2E_CONTRAST>,
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
+    for (int m : {0, GE2E_CONTRAST, GE2E_EXCLUSIVE, GE2E_CONTRAST | GE2E_EXCLUSIVE})
+      SPK_CUDA(cudaFuncSetAttribute(rows_tile_kernel_for(m), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    for (auto* k : {ge2e_centroid_grad_kernel<false>, ge2e_centroid_grad_kernel<true>})
+      SPK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, CENTROID_SPREAD_SMEM));
     return 0;
   }));
-  auto* centroid_stage = excl ? ge2e_fused_kernel<true> : ge2e_fused_kernel<false>;
-  auto* row_stage = ge2e_rows_tile_kernel<0>;
-  if (mode == GE2E_CONTRAST) row_stage = ge2e_rows_tile_kernel<GE2E_CONTRAST>;
-  if (mode == GE2E_EXCLUSIVE) row_stage = ge2e_rows_tile_kernel<GE2E_EXCLUSIVE>;
-  if (mode == (GE2E_EXCLUSIVE | GE2E_CONTRAST)) row_stage = ge2e_rows_tile_kernel<GE2E_EXCLUSIVE | GE2E_CONTRAST>;
-  // the variants exist only in the re-tiled row stage; "ge2e_row_tile_v2" = 0 selects the first one for mode 0 alone
-  const bool tile_v2 = g_ge2e_tile_v2 || mode != 0;
   const long long NM = 1LL * N * M;
-  const int row_tiles = static_cast<int>((NM + TR - 1) / TR);
-  const float eps = 1e-8f;
   ProfScope prof(need_grad ? "ge2e_fused_fwd_bwd" : "ge2e_fused_fwd", (need_grad ? 6.0 : 2.0) * NM * N * GD,
                  (need_grad ? 2.0 : 1.0) * NM * GD * 4.0, st);
-  // three launches in stream order: centroids | row tiles (loss, dE row part, dC) | centroid part of dE
-  centroid_stage<<<N, 256, smem, st>>>(E, N, M, w, b, loss, dE, dw, db, chat, cinv, einv, dchat, need_grad, eps, 1,
-                                       cos_own, urinv, gdiag);
-  SPK_CUDA(cudaGetLastError());
+  // three launches in stream order: centroids | row tiles (loss, dE row part, dC) | centroid part of dE (stream order is
+  // the grid-wide barrier: a cooperative launch with two grid.sync() cost 32 us at the training size, mostly in the syncs)
+  Ge2eCentroids c = {};
+  c.E = E; c.N = N; c.M = M;
+  c.loss = loss;
+  if (need_grad) { c.dw = dw; c.db = db; c.dchat = dchat; }
+  c.einv = einv; c.chat = chat; c.cinv = cinv;
+  c.cos_own = cos_own; c.urinv = urinv;
+  SPK_TRY(ge2e_centroids(c, st));
   cudaLaunchAttribute pdl_attr[1];
   pdl_attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   pdl_attr[0].val.programmaticStreamSerializationAllowed = 1;
   cudaLaunchConfig_t cfg = {};
-  cfg.blockDim = dim3(256);
   cfg.stream = st;
   cfg.attrs = pdl_attr;
-  const bool pdl = tile_v2 && g_ge2e_pdl;
-  cfg.numAttrs = pdl ? 1 : 0;
-  const float* chat_c = chat;
-  const float* einv_c = einv;
-  const float* cos_own_c = cos_own;
-  const float* gdiag_c = gdiag;
-  if (tile_v2) {
-    cfg.gridDim = dim3(static_cast<unsigned>((NM + RT - 1) / RT));
-    cfg.blockDim = dim3(TILE_THREADS);
-    cfg.dynamicSmemBytes = smem2;
-    SPK_CUDA(cudaLaunchKernelEx(&cfg, row_stage, E, N, M, w, b, loss, dE, dw, db, chat_c, einv_c, dchat, need_grad,
-                                cos_own_c, gdiag));
-  } else {
-    ge2e_fused_kernel<false><<<row_tiles, 256, smem, st>>>(E, N, M, w, b, loss, dE, dw, db, chat, cinv, einv, dchat,
-                                                           need_grad, eps, 2, nullptr, nullptr, nullptr);
-    SPK_CUDA(cudaGetLastError());
-  }
+  cfg.numAttrs = g_ge2e_pdl ? 1 : 0;
+  cfg.gridDim = dim3(static_cast<unsigned>((NM + RT - 1) / RT));
+  cfg.blockDim = dim3(TILE_THREADS);
+  cfg.dynamicSmemBytes = smem;
+  SPK_CUDA(cudaLaunchKernelEx(&cfg, rows_tile_kernel_for(mode), E, N, M, w, b, loss, dE, dw, db, chat, einv, dchat,
+                              need_grad, cos_own, gdiag));
   if (need_grad) {
     cfg.gridDim = dim3(N);
     cfg.blockDim = dim3(256);
-    cfg.dynamicSmemBytes = smem;
-    SPK_CUDA(cudaLaunchKernelEx(&cfg, centroid_stage, E, N, M, w, b, loss, dE, dw, db, chat, cinv, einv, dchat, need_grad,
-                                eps, 3, cos_own, urinv, gdiag_c));
+    cfg.dynamicSmemBytes = CENTROID_SPREAD_SMEM;
+    SPK_CUDA(cudaLaunchKernelEx(&cfg, excl ? ge2e_centroid_grad_kernel<true> : ge2e_centroid_grad_kernel<false>, E, M,
+                                chat, cinv, dchat, einv, cos_own, urinv, gdiag, dE));
   }
   return 0;
 }

@@ -3,18 +3,18 @@
 // the threshold the loss is composed from the tcgen05 GEMM of gemm_tc.cu and three row kernels instead of
 // the single fp32 SIMT kernel of ge2e.cu:
 //
-//   prep    (block / speaker)  row norms, centroids; Ehat, Chat as split-fp16 planes (+ fp32 Chat)
+//   prep    (block / speaker)  row norms, centroids; Ehat, Chat as split-fp16 planes (+ fp32 Chat): ge2e_centroids
 //   GEMM    S = Ehat Chat^T    3 planes (fp32-equivalent), fp32 output [NM, Np]
 //   rows    (warp / row)       z = w S - b, log-sum-exp, loss, dw, db, G = (w/NM)(softmax - onehot) -> 2 planes
 //   GEMM    dEhat = G Chat     (Chat read MN-major), fp32 output
 //   GEMM    dChat = G^T Ehat   (both MN-major, split-K, fp32 atomics)
 //   finish  (warp / row)       normalisation Jacobians, centroid scatter: dE
-//   excl    (block / speaker)  exclusive centroids only: the diagonal's two gradient terms (ge2e_excl.cuh)
+//   excl    (block / speaker)  exclusive centroids only: the diagonal's two gradient terms (ge2e_common.cuh)
 //
 // The [NM, N] logits are materialised here (1 GB at N = 4096) -- what the small-N kernel avoids -- but the
 // reference's two [NM, N, D] operands (2 x 257 GB at N = 4096) still never exist.
 #include "ge2e.h"
-#include "ge2e_excl.cuh"
+#include "ge2e_common.cuh"
 #include "gemm.h"
 #include "rowops.h"
 
@@ -69,86 +69,6 @@ static TcPlan tc_plan(int N, int M, int mode) {
 
 size_t ge2e_tc_workspace_bytes(int N, int M, int mode) { return tc_plan(N, M, mode).total; }
 
-// ---- prep: one block (256 threads = 8 warps) per speaker
-// EXCL: also each row's exclusive diagonal cosine `cos_own` and `urinv` = 1 / max(|u_i| / (M-1), eps), u_i = sum - e_i
-template <bool EXCL>
-__global__ void __launch_bounds__(256) ge2e_prep_kernel(const float* __restrict__ E, int N, int M,
-                                                        elem_t* __restrict__ ehat, int64_t e_ps,
-                                                        elem_t* __restrict__ chat, int64_t c_ps,
-                                                        float* __restrict__ chat32, float* __restrict__ einv,
-                                                        float* __restrict__ cinv, float* __restrict__ loss,
-                                                        float* __restrict__ dw, float* __restrict__ db,
-                                                        float* __restrict__ dchat, float eps,
-                                                        float* __restrict__ cos_own, float* __restrict__ urinv) {
-  __shared__ float part[8][TD];
-  __shared__ float red[8];
-  const int k = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (k == 0 && tid == 0) {                  // the accumulators of the row kernel: the caller's own scalars
-    loss[0] = 0.f;
-    if (dw != nullptr) { dw[0] = 0.f; db[0] = 0.f; }
-  }
-  if (dchat != nullptr) dchat[static_cast<int64_t>(k) * TD + tid] = 0.f;   // split-K target of the dChat GEMM
-  float cp[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-  for (int m = warp; m < M; m += 8) {
-    const int64_t row = static_cast<int64_t>(k) * M + m;
-    const float4 a0 = __ldg(reinterpret_cast<const float4*>(E + row * TD + lane * 8));
-    const float4 a1 = __ldg(reinterpret_cast<const float4*>(E + row * TD + lane * 8 + 4));
-    float v[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-    float q = 0.f;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) { q += v[i] * v[i]; cp[i] += v[i]; }
-    const float inv = 1.f / fmaxf(sqrtf(warp_sum(q)), eps);
-    if (lane == 0) einv[row] = inv;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) v[i] *= inv;
-    store8_split(ehat, e_ps, 2, row * TD + lane * 8, v);      // two fp16 planes carry an fp32 mantissa
-  }
-#pragma unroll
-  for (int i = 0; i < 8; ++i) part[warp][lane * 8 + i] = cp[i];
-  __syncthreads();
-  float cv = 0.f;
-#pragma unroll
-  for (int w = 0; w < 8; ++w) cv += part[w][tid];
-  const float csum = cv;
-  cv *= 1.f / static_cast<float>(M);
-  float q = warp_sum(cv * cv);
-  if (lane == 0) red[warp] = q;
-  __syncthreads();
-  float tot = 0.f;
-#pragma unroll
-  for (int w = 0; w < 8; ++w) tot += red[w];
-  const float nrm = fmaxf(sqrtf(tot), eps);
-  const float ch = cv / nrm;
-  chat32[static_cast<int64_t>(k) * TD + tid] = ch;
-  store1_split(chat, c_ps, 2, static_cast<int64_t>(k) * TD + tid, ch);
-  if (tid == 0) cinv[k] = 1.f / nrm;
-  if constexpr (EXCL) {
-    part[0][tid] = csum;                       // every read of `part` is behind the barrier above
-    __syncthreads();
-    const float inv_m1 = 1.f / static_cast<float>(M - 1);
-    for (int m = warp; m < M; m += 8) {        // warp per row, as above (lane 0 wrote einv of these rows)
-      const int64_t row = static_cast<int64_t>(k) * M + m;
-      const float4 a0 = __ldg(reinterpret_cast<const float4*>(E + row * TD + lane * 8));
-      const float4 a1 = __ldg(reinterpret_cast<const float4*>(E + row * TD + lane * 8 + 4));
-      const float v[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-      float qu = 0.f, qeu = 0.f;
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        const float u = part[0][lane * 8 + i] - v[i];
-        qu += u * u;
-        qeu += v[i] * u;
-      }
-      qu = warp_sum(qu);
-      qeu = warp_sum(qeu);
-      if (lane == 0) {
-        const float ur = 1.f / fmaxf(sqrtf(qu) * inv_m1, eps);
-        urinv[row] = ur;
-        cos_own[row] = qeu * einv[row] * (ur * inv_m1);
-      }
-    }
-  }
-}
-
 // ---- rows: one warp per embedding row; lane handles columns lane*8 + 256*c
 // MODE (GE2E_CONTRAST | GE2E_EXCLUSIVE bits): GE2E_EXCLUSIVE replaces each row's own-speaker cosine by `cos_own` (prep)
 // and writes that column's G to `gdiag` (dL/dcos_own) and a zero to the G planes, so that neither GEMM carries it;
@@ -190,13 +110,12 @@ __global__ void __launch_bounds__(256) ge2e_rows_kernel(const float* __restrict_
       for (int o = 16; o > 0; o >>= 1) {
         const float oz = __shfl_xor_sync(0xffffffffu, bz, o);
         const int oj = __shfl_xor_sync(0xffffffffu, bj, o);
-        if (oz > bz || (oz == bz && oj < bj)) { bz = oz; bj = oj; }
+        if (ge2e_argmax_takes(bz, bj, oz, oj)) { bz = oz; bj = oj; }
       }
       const float s_own = EXCL ? own : srow[label];
-      // sigmoid(z) and sigmoid(-z) = 1 - sigmoid(z) each from its own exp: no cancellation when |z| is large
-      const float zo = w * s_own - b;
-      const float so = 1.f / (1.f + expf(-zo)), son = 1.f / (1.f + expf(zo));
-      const float sk = 1.f / (1.f + expf(-bz)), skn = 1.f / (1.f + expf(bz));
+      float so, son, sk, skn;
+      ge2e_sigmoid_pair(w * s_own - b, so, son);
+      ge2e_sigmoid_pair(bz, sk, skn);
       if (lane == 0) loss_acc += son + sk;
       if (need_grad) {
         const float go = -so * son, gk = sk * skn;      // dL/dz (x NM)
@@ -354,12 +273,15 @@ int ge2e_tc(const float* E, int N, int M, const float* w, const float* b, float*
   const int64_t NM = pl.NM;
   {
     ProfScope prof("ge2e_tc.prep", 0, 4.0 * NM * TD + 6.0 * NM * TD, st);
-    auto* prep = excl ? ge2e_prep_kernel<true> : ge2e_prep_kernel<false>;
-    prep<<<N, 256, 0, st>>>(E, N, M, bf(pl.ehat), pl.ehat_ps, bf(pl.chat), pl.chat_ps, fp(pl.chat32), fp(pl.einv),
-                            fp(pl.cinv), loss, need_grad ? dw : nullptr, need_grad ? db : nullptr,
-                            need_grad ? fp(pl.dchat) : nullptr, 1e-8f, excl ? fp(pl.cos_own) : nullptr,
-                            excl ? fp(pl.urinv) : nullptr);
-    SPK_CUDA(cudaGetLastError());
+    Ge2eCentroids c = {};
+    c.E = E; c.N = N; c.M = M;
+    c.loss = loss;
+    if (need_grad) { c.dw = dw; c.db = db; c.dchat = fp(pl.dchat); }   // dchat: split-K target of the dChat GEMM
+    c.einv = fp(pl.einv); c.chat = fp(pl.chat32); c.cinv = fp(pl.cinv);
+    if (excl) { c.cos_own = fp(pl.cos_own); c.urinv = fp(pl.urinv); }
+    c.ehat_planes = bf(pl.ehat); c.ehat_ps = pl.ehat_ps;
+    c.chat_planes = bf(pl.chat); c.chat_ps = pl.chat_ps;
+    SPK_TRY(ge2e_centroids(c, st));
   }
   {  // S = Ehat Chat^T
     GemmProblem g;
@@ -374,10 +296,7 @@ int ge2e_tc(const float* E, int N, int M, const float* w, const float* b, float*
   {
     ProfScope prof("ge2e_tc.rows", 0, (need_grad ? 2.0 : 1.0) * NM * pl.Np * 4.0 + (need_grad ? 4.0 * NM * pl.Np : 0.0), st);
     const int blocks = static_cast<int>(std::min<int64_t>((NM + 7) / 8, static_cast<int64_t>(device_sm_count()) * 8));
-    auto* rows = ge2e_rows_kernel<0>;
-    if (mode == GE2E_CONTRAST) rows = ge2e_rows_kernel<GE2E_CONTRAST>;
-    if (mode == GE2E_EXCLUSIVE) rows = ge2e_rows_kernel<GE2E_EXCLUSIVE>;
-    if (mode == (GE2E_EXCLUSIVE | GE2E_CONTRAST)) rows = ge2e_rows_kernel<GE2E_EXCLUSIVE | GE2E_CONTRAST>;
+    auto* rows = ge2e_for_mode(mode, [](auto m) { return ge2e_rows_kernel<decltype(m)::value>; });
     rows<<<blocks, 256, 0, st>>>(fp(pl.s), NM, N, static_cast<int>(pl.Np), M, w, b, bf(pl.g), pl.g_ps, loss, dw, db,
                                  need_grad, excl ? fp(pl.cos_own) : nullptr, excl ? fp(pl.gdiag) : nullptr);
     SPK_CUDA(cudaGetLastError());

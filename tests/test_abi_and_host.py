@@ -47,14 +47,13 @@ def test_workspace_query_is_host_only(native):
     assert L.spk_ge2e_workspace_bytes(64, 15) > 64 * 256 * 8
 
 
-def test_option_switches_are_host_only_and_documented(native):
+def test_option_switches_are_host_only_documented_and_retired_ones_unknown(native):
     """spk_set_option touches no device: every switch INTEGRATION.md lists is accepted here (and put back to its
-    default), an unknown name is rejected with a message."""
+    default), an unknown name is rejected with a message, and so is the switch of the retired first GE2E row stage."""
     text = open(os.path.join(ROOT, "INTEGRATION.md")).read()
     defaults = {"prune_last_layer": 1, "fused_training_attention": 1, "fused_inference_attention": 1,
                 "inference_attention_two_ctas": 1, "training_attention_two_ctas": 1, "fused_layernorm": 2,
-                "gemm_cta_pairs": 1, "gemm_dependent_launch": 2, "ge2e_row_tile_v2": 1, "ge2e_dependent_launch": 1,
-                "grad_scale_log2": 12}
+                "gemm_cta_pairs": 1, "gemm_dependent_launch": 2, "ge2e_dependent_launch": 1, "grad_scale_log2": 12}
     flags = native.plan_flags()
     for name, default in defaults.items():
         assert "`%s`" % name in text, name
@@ -63,6 +62,8 @@ def test_option_switches_are_host_only_and_documented(native):
     assert native.plan_flags() == flags
     with pytest.raises(RuntimeError, match="unknown option"):
         native.set_option("no_such_option", 1)
+    with pytest.raises(RuntimeError, match="unknown option"):
+        native.set_option("ge2e_row_tile_v2", 0)
 
 
 def _model():

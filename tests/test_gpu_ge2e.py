@@ -92,31 +92,19 @@ def test_grad_scaling_and_errors():
 
 @pytest.mark.parametrize("n,m", [(1, 1), (1, 4), (2, 1), (3, 7), (5, 13), (64, 15), (65, 3), (100, 9), (128, 15), (129, 2),
                                  (192, 5), (255, 3)])
-def test_row_tile_stage_v2_matches_v1_and_the_closed_form(n, m):
-    """ge2e_rows_tile_kernel (8-row tiles, bulk-copied centroid tiles, K split over warp halves) against the first
-    16-row stage on the same input, and both against the fp64 closed form; every tile shape of the N < 256 path: rows
-    not a multiple of 8, 1 .. 4 centroid tiles, a ragged last tile."""
-    from speaker_embedding_torch_b200 import _native
+def test_row_tile_stage_matches_the_closed_form(n, m):
+    """ge2e_rows_tile_kernel (8-row tiles, bulk-copied centroid tiles, K split over warp halves) against the fp64 closed
+    form; every tile shape of the N < 256 path: rows not a multiple of 8, 1 .. 4 centroid tiles, a ragged last tile."""
     E = synth.make_embeddings(1700 + n, n, m, unit_norm=(n % 2 == 1))
     l_ref, dE_ref, dw_ref, db_ref = O.ge2e_loss_and_grads_closed_form(E, m)
-    out = {}
-    try:
-        for v2 in (1, 0):
-            _native.set_option("ge2e_row_tile_v2", v2)
-            out[v2] = _run(E, m)
-            l_ng, _, _, _ = _run(E, m, grad=False)
-            assert abs(l_ng - out[v2][0]) <= 1e-6 * max(1.0, abs(out[v2][0]))
-    finally:
-        _native.set_option("ge2e_row_tile_v2", 1)
+    loss, dE, dw, db = _run(E, m)
+    l_ng, _, _, _ = _run(E, m, grad=False)
+    assert abs(l_ng - loss) <= 1e-6 * max(1.0, abs(loss))
+    assert abs(loss - l_ref) <= 2e-5 * max(1.0, abs(l_ref))
     den = np.linalg.norm(dE_ref)
-    for loss, dE, dw, db in out.values():
-        assert abs(loss - l_ref) <= 2e-5 * max(1.0, abs(l_ref))
-        if den > 1e-12:
-            assert np.linalg.norm(dE - dE_ref) / den <= 3e-4
-        else:
-            assert np.abs(dE).max() <= 1e-6
-        assert abs(dw - dw_ref) <= 2e-4 * abs(dw_ref) + 1e-6
-        assert abs(db) <= 1e-5
-    assert abs(out[1][0] - out[0][0]) <= 2e-6 * max(1.0, abs(out[0][0]))
     if den > 1e-12:
-        assert np.linalg.norm(out[1][1] - out[0][1]) / den <= 2e-5
+        assert np.linalg.norm(dE - dE_ref) / den <= 3e-4
+    else:
+        assert np.abs(dE).max() <= 1e-6
+    assert abs(dw - dw_ref) <= 2e-4 * abs(dw_ref) + 1e-6
+    assert abs(db) <= 1e-5
